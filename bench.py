@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """bench.py — `himut call` hot-path throughput on synthetic 30x CCS data (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--contig-mb M] [--genome-mb G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--contig-mb M] [--genome-mb G] [--dump-outputs DIR]
+
+--dump-outputs DIR (N = 1, --impl ours only): the records and counters of the headline call's last timed step as .npy.
 
 A step is one pass of the whole `himut call` device path (k_call_pairs -> k_site_sort -> k_call_scan -> k_site_reduce,
 one host synchronisation, host som_seen replay) over the workload's packed read batches.
@@ -37,6 +39,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np  # noqa: E402
 
 METRIC = "aligned CCS bases/sec (himut call, 30x synthetic)"
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this much in all
 # chr1 .. chr22, X, Y in Mb (GRCh38, rounded): the length ratios of BASELINE configs[2]'s 3.1 Gb genome
 HUMAN_MB = [248, 242, 198, 190, 181, 171, 159, 145, 138, 133, 135, 133, 114, 107, 102, 90, 83, 80, 58, 64, 46, 50, 156, 57]
 
@@ -295,6 +298,29 @@ class Timer:
         return e0.elapsed_time(e1)
 
 
+def dump_outputs(path, rec, log):
+    """the site records and the 15 log counters a call returns, as DIR/records_<field>.npy and DIR/log.npy in float64
+    (every field is an integer that float64 holds exactly).  The device returns records in no particular order: they
+    are sorted on all their fields first, so that two builds can be compared array for array.  Past DUMP_BYTES, the
+    records whose (chunk, tpos, ref, alt) hash lowest are written: the choice depends on each record's key alone, so
+    two builds whose record sets differ in a few sites still write the same sample apart from those sites."""
+    os.makedirs(path, exist_ok=True)
+    rec = np.sort(rec, order=["chunk", "tpos", "ref", "alt"])  # the fields not named break the ties
+    fields = [n for n in rec.dtype.names if n != "pad0"]
+    row_bytes = 8 * sum(int(np.prod(rec.dtype[n].shape)) for n in fields)
+    cap = (DUMP_BYTES - (1 << 20)) // row_bytes  # 1 MB for the counters and the .npy headers
+    if rec.size > cap:
+        u = np.uint64
+        h = (rec["chunk"].astype(u) << u(40)) ^ (rec["tpos"].astype(u) << u(8)) ^ (rec["ref"].astype(u) << u(4)) ^ rec["alt"].astype(u)
+        for shift, mul in ((30, 0xBF58476D1CE4E5B9), (27, 0x94D049BB133111EB)):  # splitmix64 finaliser
+            h = (h ^ (h >> u(shift))) * u(mul)
+        h ^= h >> u(31)
+        rec = rec[np.sort(np.lexsort((np.arange(rec.size), h))[:cap])]
+    for n in fields:
+        np.save(os.path.join(path, "records_%s.npy" % n), rec[n].astype(np.float64))
+    np.save(os.path.join(path, "log.npy"), np.asarray(log, np.float64))
+
+
 def kernel_breakdown(ctx, fn, reps=3):
     """per-kernel CUDA-event times and the launch count of a call, measured outside the timed loops"""
     ctx.kernel_timing(True)
@@ -355,6 +381,8 @@ def leg_contig(args, T, ctx, d, params, chunks, tmpdir):
     ms_total = T.run(step, args.steps, after=drain, streams=streams)
     rec, log = state["rec"].copy(), state["log"]
     assert ctx.last_call_path() == 2, "the fused device path did not run"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rec, log)
     # the same call, one context, each call collected before the next is enqueued (what hm_call_chunks alone gives)
     sync_state = {}
 
@@ -427,8 +455,7 @@ def leg_contig(args, T, ctx, d, params, chunks, tmpdir):
         ctx.call_batch(batch, chunks, view=True)
 
     step_plain()
-    n_plain = max(2, args.steps // 3)
-    ms_plain = T.run(step_plain, n_plain) / n_plain
+    ms_plain = T.run(step_plain, args.steps) / args.steps
     ctx.unpin(batch)
     ctx.unpin_arrays(pinned)
     nb.close()
@@ -502,7 +529,7 @@ def leg_phase(args, T, ctx, d):
 
     for _ in range(2):
         step()
-    n = max(3, args.steps // 2)
+    n = args.steps
     ms = T.run(step, n, after=ctx.records_wait) / n
     k_ms, launches = kernel_breakdown(ctx, step)
     ctx.records_wait()
@@ -523,7 +550,7 @@ def leg_normcounts(args, T, ctx, d, chunks):
     with one quality byte per base"""
     from himut_b200 import bamdec
     batch = d.batch
-    n_norm = max(2, args.steps // 3)
+    n_norm = args.steps
     state = {}
 
     def step():
@@ -773,12 +800,18 @@ def main():
     ap.add_argument("--no-bam-leg", action="store_true")
     ap.add_argument("--no-genome", action="store_true")
     ap.add_argument("--no-phase", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the records and log counters of the headline call's last step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the one-GPU headline call's outputs: N = 1 and --impl ours only")
 
     import __graft_entry__ as g
     if args.impl == "reference":

@@ -2,7 +2,7 @@
 integer test of the kernel (restated here from make_norm_cert in himut_b200.cu and the consumer epilogue in
 normfast.cuh) certifies a pure position — n reads of the reference allele with qualities b_i — the unmodified
 `himut.gtlib.get_germ_gt` must call it hom-ref with GQ >= min_gq.  Random depths, quality mixes, priors and GQ
-thresholds; build container only (needs /root/reference)."""
+thresholds.  The comparisons with the reference run where its unmodified sources are present (tests/refshim.py)."""
 import math
 import random
 
@@ -11,7 +11,7 @@ import pytest
 import refshim
 from himut_b200 import gtmodel
 
-pytestmark = pytest.mark.skipif(not refshim.have_reference(), reason="reference sources are not present")
+needs_reference = pytest.mark.skipif(not refshim.have_reference(), reason="reference sources are not present")
 
 
 def make_cert(prior, min_gq, min_bq=93):
@@ -63,6 +63,7 @@ def quality_mix(rnd, n):
     return [rnd.randrange(1, 256) for _ in range(n)]               # beyond what PacBio writes
 
 
+@needs_reference
 @pytest.mark.parametrize("prior", [1e-3, 1e-2, 5e-4, 0.3])
 @pytest.mark.parametrize("min_gq", [0, 5, 20, 60, 99])
 def test_certified_positions_are_homref_with_enough_gq(prior, min_gq):
@@ -98,6 +99,7 @@ def test_thirty_reads_at_q93_are_certified_by_default():
     assert make_cert(1e-3, 20, min_bq=200) is None           # outside the certified domain: exact pass only
 
 
+@needs_reference
 def test_every_table_entry_is_the_references_value():
     """the per-BQ terms and priors the kernels add are the reference's own functions' values, bit for bit, over the whole
     table (tests/test_kat.py pins four entries without the reference)"""
