@@ -67,6 +67,14 @@ class BqCompact:
         return self.mask.nbytes + self.n_exc + self.exc_off.nbytes
 
 
+class hm_bgzf_plan(C.Structure):
+    """a BAM region planned for the device decoder (include/himut_b200.h)"""
+    _fields_ = [("comp", C.c_void_p), ("comp_bytes", C.c_uint64), ("n_blocks", C.c_uint64),
+                ("blk_coff", C.c_void_p), ("blk_csize", C.c_void_p), ("blk_isize", C.c_void_p), ("blk_uoff", C.c_void_p),
+                ("blk_crc", C.c_void_p), ("entry", C.c_void_p), ("n_entry", C.c_uint64), ("walk_end", C.c_uint64),
+                ("path", C.c_char_p)]
+
+
 class hm_chunk(C.Structure):
     _fields_ = [("start", C.c_int32), ("end", C.c_int32), ("read_lo", C.c_uint32),
                 ("read_hi", C.c_uint32), ("phase_set", C.c_int32), ("reserved", C.c_int32)]

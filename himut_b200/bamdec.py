@@ -17,7 +17,7 @@ from . import abi, pack
 _LIB = None
 EXPORTS = ["hm_bam_open", "hm_bam_close", "hm_bam_error", "hm_bam_header_text", "hm_bam_n_refs", "hm_bam_ref_name",
            "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bq_compact_build",
-           "hm_bq_compact_free"]
+           "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames"]
 
 
 def lib_path():
@@ -56,6 +56,8 @@ def load():
         lib.hm_bam_n_qnames.restype = C.c_uint32
         lib.hm_bam_qname.argtypes = [vp, C.c_uint32]
         lib.hm_bam_qname.restype = C.c_char_p
+        lib.hm_bam_region_plan.argtypes = [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(abi.hm_bgzf_plan)]
+        lib.hm_bam_intern_qnames.argtypes = [vp, vp, vp, C.c_size_t, vp]
         _LIB = lib
     return _LIB
 
@@ -117,6 +119,7 @@ class NativeBam:
         self.references = [self.lib.hm_bam_ref_name(self.h, i).decode() for i in range(self.lib.hm_bam_n_refs(self.h))]
         self.lengths = [self.lib.hm_bam_ref_len(self.h, i) for i in range(len(self.references))]
         self.header_text = self.lib.hm_bam_header_text(self.h).decode()
+        self.has_index = os.path.exists(os.fsencode(path) + b".bai")
 
     def read_batch(self, chrom, start, end, copy=True, seq=True, compact=False, buffer_set=0):
         """seq=False: the batch comes without its 2-bit base stream (HM_BAM_OPT_NO_SEQ), as `call` and the phase
@@ -153,6 +156,25 @@ class NativeBam:
         exc = cp(_view(q.exc, (n_exc + 31) & ~15, np.uint8))  # the decoder keeps 32 readable bytes past the last exception
         exc_off = cp(_view(q.exc_off, n + 1, np.uint64))
         return batch, abi.BqCompact(mask, exc, exc_off, int(q.modal), n_exc)
+
+    def plan(self, chrom, start, end):
+        """abi.hm_bgzf_plan of the records read_batch(chrom, start, end) visits, for Context.decode_region: the
+        compressed blocks and the record starts the BAI knows, nothing inflated.  Valid until the next plan()."""
+        if chrom not in self.references:
+            raise KeyError(chrom)
+        p = abi.hm_bgzf_plan()
+        if self.lib.hm_bam_region_plan(self.h, self.references.index(chrom), int(max(start, 0)), int(end), C.byref(p)) != 0:
+            raise pack.BatchFormatError(self.lib.hm_bam_error(self.h).decode())
+        return p
+
+    def intern_qnames(self, blob, off, n):
+        """query-name ids (the ones read_batch gives) of n NUL-terminated names, name i at blob + off[i]"""
+        ids = np.zeros(n, np.uint32)
+        off = np.ascontiguousarray(off, np.uint64)
+        blob_p = blob if isinstance(blob, int) else blob.ctypes.data
+        if n and self.lib.hm_bam_intern_qnames(self.h, C.c_void_p(blob_p), off.ctypes.data_as(C.c_void_p), n, ids.ctypes.data_as(C.c_void_p)) != 0:
+            raise RuntimeError(self.lib.hm_bam_error(self.h).decode())
+        return ids
 
     def window_qlens(self, chrom, start, end):
         """len(query_sequence) of the records overlapping [start, end) with MAPQ > 0 and tp:A:P, fetch order

@@ -10,6 +10,10 @@ from . import abi, gtmodel, records, vcfio, worker
 
 _RESTATES = (abi.ST_GERM_HET, abi.ST_GERM_HETALT, abi.ST_GERM_HOMALT, abi.ST_GERM_HOMREF)
 
+# compressed BAM bytes per decode group from which call_region(decode="auto") decodes on the device: below it the host
+# decoder's threads finish a group first (tools/decode_trace.py, profiles/decode_trace_r03.json)
+DEVICE_DECODE_MIN_BYTES = 48 << 20
+
 
 def _log_from_records(rec, num_ccs):
     """chrom2tsbs_log vector (caller.py:625-641) from record statuses"""
@@ -69,18 +73,32 @@ def carry_som_seen(parts, later_starts):
     return out
 
 
-def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_names=False, ctx2=None):
+def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_names=False, ctx2=None, decode="auto"):
     """the device path over a contig's chunk list (or a run of it), pipelined: group k + 1 is decoded on a thread of its
     own while group k is uploaded; with a second context (configured like the first) the two alternate from group to
     group, so upload(k + 1) also overlaps kernels(k) and the record copy of k - 1:
         decode(k + 1) || H2D(k + 1) || kernels(k) || D2H(k - 1).
+    decode: "device" inflates and parses each group on the GPU from the compressed file (Context.decode_region): the
+    context that calls a group decodes it, and with two contexts the decode of group k + 1 runs while the kernels of
+    group k do.  It needs a context with the device decoder and a BAM with a BAI; without either the host decoder runs.
+    "host" is the pipeline above (the native host decoder).  "auto" takes the device decoder when it can run and the
+    groups average at least DEVICE_DECODE_MIN_BYTES of compressed BAM (below that the host decoder is faster).
     -> (records incl. germline restatements, number of distinct query names that passed the read gates,
         names blob (want_names) or None)"""
+    if decode not in ("auto", "host", "device"):
+        raise ValueError("decode must be 'auto', 'host' or 'device'")
     src = worker.RegionSource(bam_file)
     tally = worker.QnameTally()
     kept, laters = [], []
     starts = [s for _, s, _e in chunkloci_lst]
     groups = worker.group_chunks(chunkloci_lst)
+    if decode != "host" and not (hasattr(ctx, "decode_region") and src.reader.has_index):
+        decode = "host"
+    if decode == "auto" and not starts:
+        decode = "host"
+    if decode == "auto":
+        lo, hi = min(starts), max(e for _, _s, e in chunkloci_lst) + (1 if phase else 0)
+        decode = "device" if src.reader.plan(chrom, lo, hi).comp_bytes >= DEVICE_DECODE_MIN_BYTES * len(groups) else "host"
     ctxs = [ctx] if (ctx2 is None or len(groups) == 1 or not hasattr(ctx, "call_chunks_submit")) else [ctx, ctx2]
     pins = worker.PinCache(ctx, enabled=len(groups) > 1)
     # `call` never needs the read bases as a stream: substituted bases are in the ops, and under a cs match the read
@@ -101,6 +119,36 @@ def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_nam
         laters.append(min(starts[idx[-1] + 1:], default=None))
 
     lap = worker.Laps("call_region %s" % chrom)  # HIMUT_B200_WORKER_TIMING=1: where the host time of a contig goes
+    if decode == "device":
+        try:
+            k = 0
+            for idx in groups:
+                loci = [chunkloci_lst[i] for i in idx]
+                c = ctxs[k % len(ctxs)]  # never the context whose call is pending
+                region = c.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci) + (1 if phase else 0))
+                lap("device decode")
+                if region.n_reads == 0:
+                    continue
+                k += 1
+                table = region.chunk_table([(s, e) for _, s, e in loci], None if chunk_sets is None else [chunk_sets[i] for i in idx])
+                if len(ctxs) > 1:
+                    c.call_chunks_submit(table)
+                    if pending is not None:
+                        finish(pending)
+                    pending = (c, idx)
+                else:
+                    finish((c, idx, c.call_chunks(table)))
+                lap("submit + collect")
+            if pending is not None:
+                finish(pending)
+            names = src.reader.qnames_blob(tally.seen) if want_names else None
+        finally:
+            src.close()
+        kept = carry_som_seen(kept, laters)
+        rec = np.concatenate(kept) if kept else np.zeros(0, abi.SITE_DTYPE)
+        lap("merge")
+        lap.report()
+        return rec, tally.count(), names
     try:
         k = 0
         for idx, batch, cq, table, release in worker.pipelined_groups(src, chrom, chunkloci_lst, groups, chunk_sets, seq=False,

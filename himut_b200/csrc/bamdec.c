@@ -30,6 +30,7 @@
 #include "../../include/himut_io.h"
 #include "inflate_fast.h"
 #include "crc32_clmul.h"
+#include "bamerr.h"
 
 /* crc32(0, p, n) of zlib: carry-less-multiply folding over the multiple-of-16 body when the CPU has it
  * (crc32_clmul.h), zlib for the tail and everywhere else */
@@ -52,6 +53,10 @@ typedef struct {
   uint64_t* lin; /* linear index */
   int32_t n_lin;
   int has_index;
+  uint32_t* bin;     /* BAI bins (the pseudo-bin 37450 left out) ... */
+  uint64_t* bin_end; /* ... the largest chunk end of each ... */
+  uint64_t* bin_beg; /* ... and the smallest chunk begin */
+  int32_t n_bin;
 } bam_ref_t;
 
 typedef struct {
@@ -105,6 +110,12 @@ typedef struct hm_bam {
     uint64_t n_qexc;
   } other; /* the set that is not active */
   int cur_set;
+  /* the last hm_bam_region_plan: block table, entry points, and the compressed range when the file is not mapped */
+  uint64_t *p_coff, *p_uoff, *p_entry;
+  uint32_t *p_csize, *p_isize, *p_crc;
+  size_t cap_plan_blocks, cap_plan_entry;
+  uint8_t* p_comp;
+  size_t cap_p_comp;
 } hm_bam;
 
 /* swap the active output buffers with the parked set */
@@ -413,7 +424,23 @@ static int load_bai(hm_bam* b) {
   int32_t nref = (int32_t)rd32(d + 4);
   for (int32_t r = 0; r < nref && r < b->n_ref; r++) {
     int32_t nbin = (int32_t)rd32(d + q); q += 4;
-    for (int32_t k = 0; k < nbin; k++) { int32_t nchunk = (int32_t)rd32(d + q + 4); q += 8 + 16 * (size_t)nchunk; }
+    b->refs[r].bin = (uint32_t*)malloc(((size_t)nbin + 1) * 4);
+    b->refs[r].bin_end = (uint64_t*)malloc(((size_t)nbin + 1) * 8);
+    b->refs[r].bin_beg = (uint64_t*)malloc(((size_t)nbin + 1) * 8);
+    if (!b->refs[r].bin || !b->refs[r].bin_end || !b->refs[r].bin_beg) { free(d); return -1; }
+    for (int32_t k = 0; k < nbin; k++) {
+      const uint32_t bin = rd32(d + q);
+      int32_t nchunk = (int32_t)rd32(d + q + 4);
+      uint64_t e = 0, bg = UINT64_MAX;
+      for (int32_t c = 0; c < nchunk; c++) {
+        uint64_t cb, ce;
+        memcpy(&cb, d + q + 8 + 16 * (size_t)c, 8); memcpy(&ce, d + q + 8 + 16 * (size_t)c + 8, 8);
+        if (ce > e) e = ce;
+        if (cb < bg) bg = cb;
+      }
+      if (bin != 37450) { b->refs[r].bin[b->refs[r].n_bin] = bin; b->refs[r].bin_beg[b->refs[r].n_bin] = bg; b->refs[r].bin_end[b->refs[r].n_bin++] = e; }
+      q += 8 + 16 * (size_t)nchunk;
+    }
     int32_t nintv = (int32_t)rd32(d + q); q += 4;
     b->refs[r].lin = (uint64_t*)malloc(((size_t)nintv + 1) * 8);
     b->refs[r].n_lin = nintv;
@@ -429,8 +456,9 @@ void hm_bam_close(hm_bam* b) {
   if (!b) return;
   if (b->map) munmap((void*)b->map, b->map_len);
   if (b->f) fclose(b->f);
-  for (int32_t i = 0; i < b->n_ref; i++) { free(b->refs[i].name); free(b->refs[i].lin); }
+  for (int32_t i = 0; i < b->n_ref; i++) { free(b->refs[i].name); free(b->refs[i].lin); free(b->refs[i].bin); free(b->refs[i].bin_end); free(b->refs[i].bin_beg); }
   free(b->refs); free(b->header); free(b->path);
+  free(b->p_coff); free(b->p_uoff); free(b->p_entry); free(b->p_csize); free(b->p_isize); free(b->p_crc); free(b->p_comp);
   for (uint32_t i = 0; i < b->qt.n; i++) free(b->qt.names[i]);
   free(b->qt.names); free(b->qt.keys_hash); free(b->qt.ids);
   for (int k = 0; k < 2; k++) { /* both buffer sets */
@@ -559,13 +587,6 @@ typedef struct {
   long err_arg;
 } rec_t;
 
-enum { E_CS_TOKEN = 1, E_CS_PAST, E_N_MATCH, E_CS_LONG, E_SUB_N, E_SPAN_REF, E_SPAN_QRY };
-static const char* const REC_ERR[] = {
-    "", "%s: unsupported cs token (%ld)", "%s: cs runs past the read (%ld)",
-    "%s: read base outside A/C/G/T under a cs match (reference: KeyError) (%ld)",
-    "%s: cs long-form bases disagree with SEQ at query %ld",
-    "%s: substitution to a base outside A/C/G/T (the reference pileup raises KeyError) (%ld)",
-    "%s: cs reference span != CIGAR span (%ld)", "%s: cs query span != aligned query span (%ld)"};
 
 typedef struct {
   hm_bam* b;
@@ -789,7 +810,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
       if (st < 0) { rc = fail(b, "truncated BAM %s (%ld)", b->path, 0); break; }
       {
         uint32_t bs0 = rd32(s.buf + s.pos);
-        if (stream_need(&s, 4 + (size_t)bs0)) { rc = fail(b, "truncated BAM record in %s (%ld)", b->path, 0); break; }
+        if (stream_need(&s, 4 + (size_t)bs0)) { rc = fail(b, REC_ERR[E_TRUNC_REC], b->path, 0); break; }
       }
       double tA = now_s();
       size_t nsel = 0, seg_ops = 0, seg_exc = 0;
@@ -802,13 +823,13 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         int32_t ref_id = (int32_t)rd32(r), pos = (int32_t)rd32(r + 4);
         if (ref_id != rid) { if (ref_id > rid || ref_id < 0) { done = 1; break; } continue; }
         if (pos >= end) { done = 1; break; }
-        if (bs < 32) { rc = fail(b, "malformed BAM record in %s: block_size %ld", b->path, (long)bs); break; }
+        if (bs < 32) { rc = fail(b, REC_ERR[E_BLOCK_SIZE], b->path, (long)bs); break; }
         uint32_t l_name = r[8], mapq = r[9], n_cig = r[12] | (r[13] << 8), flag = r[14] | (r[15] << 8);
         int32_t l_seq = (int32_t)rd32(r + 16);
         /* the fixed part, name, CIGAR, SEQ and QUAL must lie inside the record before any of them is touched */
         if (l_seq < 0 || l_name == 0 || 32 + (uint64_t)l_name + 4 * (uint64_t)n_cig + ((uint64_t)l_seq + 1) / 2 + (uint64_t)l_seq > (uint64_t)bs ||
             r[32 + l_name - 1] != 0) {
-          rc = fail(b, "malformed BAM record in %s: fields run past block_size %ld", b->path, (long)bs);
+          rc = fail(b, REC_ERR[E_FIELDS], b->path, (long)bs);
           break;
         }
         const char* qname = (const char*)(r + 32);
@@ -835,7 +856,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
           size_t adv;
           if (ty == 'Z' || ty == 'H') {
             const void* z = memchr(v, 0, left); /* the string must end inside the record */
-            if (!z) { rc = fail(b, "malformed BAM record %s: unterminated %ld tag", qname, (long)ty); break; }
+            if (!z) { rc = fail(b, REC_ERR[E_TAG_UNTERM], qname, (long)ty); break; }
             adv = (size_t)((const uint8_t*)z - v) + 1;
             if (tag[0] == 'c' && tag[1] == 's' && ty == 'Z') cs = (const char*)v;
           }
@@ -843,20 +864,20 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
           else if (ty == 's' || ty == 'S') adv = 2;
           else if (ty == 'i' || ty == 'I' || ty == 'f') adv = 4;
           else if (ty == 'B') {
-            if (left < 5) { rc = fail(b, "malformed BAM record %s: truncated B tag (%ld)", qname, (long)left); break; }
+            if (left < 5) { rc = fail(b, REC_ERR[E_TAG_B], qname, (long)left); break; }
             char sub = (char)v[0]; uint32_t cnt = rd32(v + 1);
             adv = 5 + (size_t)cnt * ((sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4);
           }
-          else { rc = fail(b, "unknown tag type in record %s (%ld)", qname, ty); break; }
-          if (adv > left) { rc = fail(b, "malformed BAM record %s: a tag runs past the record (%ld)", qname, (long)adv); break; }
+          else { rc = fail(b, REC_ERR[E_TAG_TYPE], qname, ty); break; }
+          if (adv > left) { rc = fail(b, REC_ERR[E_TAG_PAST], qname, (long)adv); break; }
           tag = v + adv;
         }
         if (rc) break;
-        if (!cs) { rc = fail(b, "%s has no cs:Z tag (the reference raises KeyError in BAM.__init__) (%ld)", qname, 0); break; }
+        if (!cs) { rc = fail(b, REC_ERR[E_NO_CS], qname, 0); break; }
         /* hard clips: pysam's query_sequence and query_alignment_start leave them out (SEQ holds no hard-clipped base),
          * so cs2tuple indexes consistently and the reference processes such records (minimap2 writes them for
          * supplementary alignments without -Y); lead / trail above count soft clips only */
-        if (l_seq <= 0 || qual[0] == 0xff) { rc = fail(b, "%s has no base qualities (%ld)", qname, 0); break; }
+        if (l_seq <= 0 || qual[0] == 0xff) { rc = fail(b, REC_ERR[E_NO_QUAL], qname, 0); break; }
         if (nsel == recs_cap) {
           size_t nc = recs_cap ? recs_cap * 2 : 8192;
           rec_t* nr = (rec_t*)realloc(recs, nc * sizeof(rec_t));
@@ -978,6 +999,196 @@ int hm_bam_last_compact(hm_bam* b, hm_bq_compact* out) {
   return HM_OK;
 }
 
+/* ------------------------------------------------------------------ region plan for the device decoder */
+/* the bins of the UCSC binning scheme that overlap [beg, end) (SAM spec 5.3) */
+static int reg2bins(int64_t beg, int64_t end, uint32_t* list) {
+  int n = 0;
+  --end;
+  list[n++] = 0;
+  for (int64_t k = 1 + (beg >> 26); k <= 1 + (end >> 26); ++k) list[n++] = (uint32_t)k;
+  for (int64_t k = 9 + (beg >> 23); k <= 9 + (end >> 23); ++k) list[n++] = (uint32_t)k;
+  for (int64_t k = 73 + (beg >> 20); k <= 73 + (end >> 20); ++k) list[n++] = (uint32_t)k;
+  for (int64_t k = 585 + (beg >> 17); k <= 585 + (end >> 17); ++k) list[n++] = (uint32_t)k;
+  for (int64_t k = 4681 + (beg >> 14); k <= 4681 + (end >> 14); ++k) list[n++] = (uint32_t)k;
+  return n;
+}
+
+/* first reference position of a bin of the binning scheme */
+static int64_t bin_start(uint32_t bin) {
+  if (bin >= 4681) return (int64_t)(bin - 4681) << 14;
+  if (bin >= 585) return (int64_t)(bin - 585) << 17;
+  if (bin >= 73) return (int64_t)(bin - 73) << 20;
+  if (bin >= 9) return (int64_t)(bin - 9) << 23;
+  if (bin >= 1) return (int64_t)(bin - 1) << 26;
+  return 0;
+}
+
+/* the BGZF header at coff: 0 and *blk filled, 1 end of file, -1 not a BGZF block */
+static int block_at(hm_bam* b, uint64_t coff, blk_t* blk, uint32_t* crc) {
+  if (!b->map) {
+    const int st = read_block_header(b->f, coff, blk);
+    if (st) return st;
+    uint8_t t[4];
+    if (fseeko(b->f, (off_t)(coff + blk->csize - 8), SEEK_SET) || fread(t, 1, 4, b->f) != 4) return -1;
+    *crc = rd32(t);
+    return 0;
+  }
+  if (coff >= b->map_len) return 1;
+  const uint8_t* h = b->map + coff;
+  if (b->map_len - coff < 18 || h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return -1;
+  const uint16_t xlen = (uint16_t)(h[10] | (h[11] << 8));
+  if (coff + 12 + xlen > b->map_len) return -1;
+  int bsize = -1;
+  for (int q = 0; q + 4 <= xlen;) {
+    const int slen = h[12 + q + 2] | (h[12 + q + 3] << 8);
+    if (h[12 + q] == 66 && h[12 + q + 1] == 67 && slen == 2) bsize = h[12 + q + 4] | (h[12 + q + 5] << 8);
+    q += 4 + slen;
+  }
+  if (bsize < 0 || (size_t)bsize + 1 < 12u + xlen + 8u || coff + (uint64_t)bsize + 1 > b->map_len) return -1;
+  blk->coff = coff; blk->csize = (uint32_t)bsize + 1;
+  blk->usize = rd32(h + blk->csize - 4);
+  *crc = rd32(h + blk->csize - 8);
+  return 0;
+}
+
+static int plan_range(hm_bam* b, uint64_t v_lo, uint64_t v_hi, const uint64_t* ventry, size_t n_ventry, hm_bgzf_plan* out);
+
+int hm_bam_region_plan(hm_bam* b, int rid, int32_t start, int32_t end, hm_bgzf_plan* out) {
+  if (!b || !out) return HM_ERR_ARG;
+  if (rid < 0 || rid >= b->n_ref) return fail(b, "invalid contig index%s %ld", NULL, rid);
+  memset(out, 0, sizeof(*out));
+  out->path = b->path;
+  if (start < 0) start = 0;
+  if (end > b->refs[rid].len) end = b->refs[rid].len;
+  uint64_t v_lo = b->first_record, v_hi = UINT64_MAX; /* UINT64_MAX: to the end of the file */
+  uint64_t* ventry = NULL; /* virtual offsets of the later entry points */
+  size_t n_ventry = 0;
+  if (b->have_bai) {
+    const bam_ref_t* R = &b->refs[rid];
+    if (!R->has_index) return HM_OK; /* no reads on this contig: an empty plan */
+    /* the window hm_bam_read_batch seeks to, then the linear-index entries of the windows the region covers */
+    int32_t w0 = start >> 14;
+    if (w0 >= R->n_lin) w0 = R->n_lin - 1;
+    int32_t w = w0;
+    uint64_t v = 0;
+    for (; w >= 0 && !v; w--) v = R->lin[w];
+    if (v) v_lo = v;
+    /* every record that overlaps the region (hm_bam_read_batch's rule: pos < end, reference end > start) lies in a
+     * chunk of a bin that overlaps [min(start, end), max(start, end) + 1): the range ends at their largest end.  The
+     * large bins (64 and 512 Mb) overlap every region and their chunks reach to the far end of the contig, so the range
+     * also ends at the first chunk of any bin that starts at or past `end`: every record there has pos >= end, where
+     * hm_bam_read_batch stops, and it is a record start. */
+    const int64_t rb = start < end ? start : end, re = (start > end ? start : end) + 1;
+    uint8_t* in_region = (uint8_t*)calloc(37450, 1);
+    uint32_t* bins = (uint32_t*)malloc(37450 * sizeof(uint32_t));
+    if (!in_region || !bins) { free(in_region); free(bins); return fail(b, "out of memory%s (%ld)", NULL, 0); }
+    const int nbins = reg2bins(rb, re, bins);
+    for (int j = 0; j < nbins; j++) if (bins[j] < 37450) in_region[bins[j]] = 1;
+    free(bins);
+    v_hi = 0;
+    for (int32_t k = 0; k < R->n_bin; k++)
+      if (R->bin[k] < 37450 && in_region[R->bin[k]] && R->bin_end[k] > v_hi) v_hi = R->bin_end[k];
+    free(in_region);
+    for (int32_t k = 0; k < R->n_bin; k++)
+      if (R->bin[k] < 37450 && bin_start(R->bin[k]) >= (int64_t)end && R->bin_beg[k] < v_hi) v_hi = R->bin_beg[k];
+    if (v_hi <= v_lo) return HM_OK; /* no record overlaps the region */
+    const int32_t w_last = (int32_t)((re - 1) >> 14) < R->n_lin - 1 ? (int32_t)((re - 1) >> 14) : R->n_lin - 1;
+    if (w_last > w0) {
+      ventry = (uint64_t*)malloc((size_t)(w_last - w0) * sizeof(uint64_t));
+      if (!ventry) return fail(b, "out of memory%s (%ld)", NULL, 0);
+    }
+    for (int32_t k = w0 + 1; k <= w_last; k++)
+      if (R->lin[k] > v_lo && R->lin[k] < v_hi && (!n_ventry || R->lin[k] > ventry[n_ventry - 1])) ventry[n_ventry++] = R->lin[k];
+  }
+  const int rc = plan_range(b, v_lo, v_hi, ventry, n_ventry, out);
+  free(ventry);
+  return rc;
+}
+
+/* hm_bam_region_plan from virtual offsets: the first entry point, the end of the range (UINT64_MAX: the end of the
+ * file) and the later entry points, ascending */
+static int plan_range(hm_bam* b, uint64_t v_lo, uint64_t v_hi, const uint64_t* ventry, size_t n_ventry, hm_bgzf_plan* out) {
+  /* the block table of the compressed range, by the header walk stream_fill does */
+  const uint64_t c_lo = v_lo >> 16;
+  size_t nb = 0;
+  uint64_t usum = 0, coff = c_lo;
+  for (;;) {
+    if (v_hi != UINT64_MAX && (coff > (v_hi >> 16) || (coff == (v_hi >> 16) && (v_hi & 0xffff) == 0))) break;
+    blk_t blk;
+    uint32_t crc = 0;
+    const int st = block_at(b, coff, &blk, &crc);
+    if (st == 1 && v_hi == UINT64_MAX) break;
+    if (st) return fail(b, "cannot read BGZF blocks of %s (%ld)", b->path, (long)coff);
+    if (nb + 2 > b->cap_plan_blocks) {
+      const size_t nc = b->cap_plan_blocks ? 2 * b->cap_plan_blocks : 4096;
+#define RP(ptr, type) do { type* np_ = (type*)realloc(ptr, nc * sizeof(type)); if (!np_) return fail(b, "out of memory%s (%ld)", NULL, (long)nc); ptr = np_; } while (0)
+      RP(b->p_coff, uint64_t); RP(b->p_uoff, uint64_t); RP(b->p_csize, uint32_t); RP(b->p_isize, uint32_t); RP(b->p_crc, uint32_t);
+#undef RP
+      b->cap_plan_blocks = nc;
+    }
+    b->p_coff[nb] = coff - c_lo; b->p_csize[nb] = blk.csize; b->p_isize[nb] = blk.usize; b->p_crc[nb] = crc; b->p_uoff[nb] = usum;
+    if (blk.usize > 65536) return fail(b, "cannot read BGZF blocks of %s (%ld)", b->path, (long)coff);
+    usum += blk.usize; coff += blk.csize; nb++;
+  }
+  if (nb == 0) return HM_OK;
+  b->p_coff[nb] = coff - c_lo;
+  b->p_uoff[nb] = usum;
+  /* virtual offset -> offset in the inflated range; an in-block offset equal to ISIZE is the next block's start */
+#define V2U(v, dst)                                                                                              \
+  do {                                                                                                           \
+    const uint64_t c_ = ((v) >> 16) - c_lo;                                                                      \
+    size_t lo_ = 0, hi_ = nb;                                                                                    \
+    while (lo_ < hi_) { const size_t m_ = (lo_ + hi_) / 2; if (b->p_coff[m_] < c_) lo_ = m_ + 1; else hi_ = m_; } \
+    if (b->p_coff[lo_] != c_ || (lo_ < nb && ((v) & 0xffff) > b->p_isize[lo_]) || (lo_ == nb && ((v) & 0xffff)))  \
+      return fail(b, "BAI virtual offset outside the BGZF blocks of %s (%ld)", b->path, (long)((v) >> 16));      \
+    (dst) = b->p_uoff[lo_] + ((v) & 0xffff);                                                                     \
+  } while (0)
+  uint64_t u_end = usum;
+  if (v_hi != UINT64_MAX) V2U(v_hi, u_end);
+  if (n_ventry + 1 > b->cap_plan_entry) {
+    uint64_t* np_ = (uint64_t*)realloc(b->p_entry, (n_ventry + 1) * sizeof(uint64_t));
+    if (!np_) return fail(b, "out of memory%s (%ld)", NULL, 0);
+    b->p_entry = np_; b->cap_plan_entry = n_ventry + 1;
+  }
+  size_t ne = 0;
+  V2U(v_lo, b->p_entry[ne]);
+  ne++;
+  for (size_t k = 0; k < n_ventry; k++) {
+    uint64_t u;
+    V2U(ventry[k], u);
+    if (u > b->p_entry[ne - 1] && u < u_end) b->p_entry[ne++] = u;
+  }
+#undef V2U
+  if (b->map) out->comp = b->map + c_lo;
+  else {
+    if (coff - c_lo > b->cap_p_comp) {
+      uint8_t* np_ = (uint8_t*)realloc(b->p_comp, coff - c_lo);
+      if (!np_) return fail(b, "out of memory%s (%ld)", NULL, 0);
+      b->p_comp = np_; b->cap_p_comp = coff - c_lo;
+    }
+    if (fseeko(b->f, (off_t)c_lo, SEEK_SET) || fread(b->p_comp, 1, coff - c_lo, b->f) != coff - c_lo)
+      return fail(b, "cannot read BGZF blocks of %s (%ld)", b->path, (long)c_lo);
+    out->comp = b->p_comp;
+  }
+  out->comp_bytes = coff - c_lo;
+  out->n_blocks = nb;
+  out->blk_coff = b->p_coff; out->blk_csize = b->p_csize; out->blk_isize = b->p_isize; out->blk_uoff = b->p_uoff; out->blk_crc = b->p_crc;
+  out->entry = b->p_entry; out->n_entry = ne;
+  out->walk_end = u_end;
+  return HM_OK;
+}
+
+int hm_bam_intern_qnames(hm_bam* b, const char* blob, const uint64_t* off, size_t n, uint32_t* ids) {
+  if (!b || (n && (!blob || !off || !ids))) return HM_ERR_ARG;
+  for (size_t i = 0; i < n; i++) {
+    const char* s = blob + off[i];
+    const int64_t id = qt_get(&b->qt, s, strlen(s));
+    if (id < 0) return fail(b, "out of memory%s (%ld)", NULL, 0);
+    ids[i] = (uint32_t)id;
+  }
+  return HM_OK;
+}
+
 /* ------------------------------------------------------------------ pre-pass: read lengths of a window */
 /* bamlib.get_thresholds (src/himut/bamlib.py:137-178) fetches 100 random 100 kb windows per contig and keeps
  * len(query_sequence) of every record with mapping_quality > 0 and tp:A:P (secondary / supplementary records
@@ -1012,18 +1223,18 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
     if (st == 1) break;
     if (st < 0) { rc = fail(b, "truncated BAM %s (%ld)", b->path, 0); break; }
     uint32_t bs = rd32(s.buf + s.pos);
-    if (stream_need(&s, 4 + (size_t)bs)) { rc = fail(b, "truncated BAM record in %s (%ld)", b->path, 0); break; }
+    if (stream_need(&s, 4 + (size_t)bs)) { rc = fail(b, REC_ERR[E_TRUNC_REC], b->path, 0); break; }
     const uint8_t* r = s.buf + s.pos + 4;
     s.pos += 4 + (size_t)bs;
     int32_t ref_id = (int32_t)rd32(r), pos = (int32_t)rd32(r + 4);
     if (ref_id != rid) { if (ref_id > rid || ref_id < 0) break; continue; }
     if (pos >= end) break;
-    if (bs < 32) { rc = fail(b, "malformed BAM record in %s: block_size %ld", b->path, (long)bs); break; }
+    if (bs < 32) { rc = fail(b, REC_ERR[E_BLOCK_SIZE], b->path, (long)bs); break; }
     uint32_t l_name = r[8], mapq = r[9], n_cig = r[12] | (r[13] << 8);
     int32_t l_seq = (int32_t)rd32(r + 16);
     if (l_seq < 0 || l_name == 0 || 32 + (uint64_t)l_name + 4 * (uint64_t)n_cig + ((uint64_t)l_seq + 1) / 2 + (uint64_t)l_seq > (uint64_t)bs ||
         r[32 + l_name - 1] != 0) {
-      rc = fail(b, "malformed BAM record in %s: fields run past block_size %ld", b->path, (long)bs);
+      rc = fail(b, REC_ERR[E_FIELDS], b->path, (long)bs);
       break;
     }
     const uint8_t* cig = r + 32 + l_name;
@@ -1044,19 +1255,19 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
       size_t adv;
       if (ty == 'Z' || ty == 'H') {
         const void* z = memchr(v, 0, left);
-        if (!z) { rc = fail(b, "malformed BAM record %s: unterminated %ld tag", (const char*)(r + 32), (long)ty); break; }
+        if (!z) { rc = fail(b, REC_ERR[E_TAG_UNTERM], (const char*)(r + 32), (long)ty); break; }
         adv = (size_t)((const uint8_t*)z - v) + 1;
       }
       else if (ty == 'A' || ty == 'c' || ty == 'C') { adv = 1; if (left >= 1 && tag[0] == 't' && tag[1] == 'p' && ty == 'A') tp_primary = (v[0] == 'P'); }
       else if (ty == 's' || ty == 'S') adv = 2;
       else if (ty == 'i' || ty == 'I' || ty == 'f') adv = 4;
       else if (ty == 'B') {
-        if (left < 5) { rc = fail(b, "malformed BAM record %s: truncated B tag (%ld)", (const char*)(r + 32), (long)left); break; }
+        if (left < 5) { rc = fail(b, REC_ERR[E_TAG_B], (const char*)(r + 32), (long)left); break; }
         char sub = (char)v[0]; uint32_t cnt = rd32(v + 1);
         adv = 5 + (size_t)cnt * ((sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4);
       }
-      else { rc = fail(b, "unknown tag type in record %s (%ld)", (const char*)(r + 32), ty); break; }
-      if (adv > left) { rc = fail(b, "malformed BAM record %s: a tag runs past the record (%ld)", (const char*)(r + 32), (long)adv); break; }
+      else { rc = fail(b, REC_ERR[E_TAG_TYPE], (const char*)(r + 32), ty); break; }
+      if (adv > left) { rc = fail(b, REC_ERR[E_TAG_PAST], (const char*)(r + 32), (long)adv); break; }
       tag = v + adv;
     }
     if (rc) break;

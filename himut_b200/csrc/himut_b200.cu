@@ -27,6 +27,7 @@
 #include "normfast.cuh"
 #include "callfused.cuh"
 #include "normbits.cuh"
+#include "bamgpu.cuh"
 
 #define HM_BOUNDARY_CAP_DEFAULT 65536   // boundary records the device list holds (HIMUT_B200_BOUNDARY_CAP overrides: tests)
 #define HM_BOUNDARY_FIRST 2048  // ... of which this many travel with the counters
@@ -154,6 +155,17 @@ struct hm_ctx {
   DevBuf b_cw_off, b_calw, b_impure, b_ref2, b_tri8, b_thr, b_span_off, b_exc_minmax, b_exp_total, b_sdiff, b_cal_ok;
   bool compact_resident = false;            // the resident batch came as bitmap + exceptions: both are still on the device
   uint32_t modal = 0;
+  // device BAM decoder (hm_decode_bam_*, bamgpu.cuh)
+  DevBuf b_comp, b_pcoff, b_pcsize, b_pisize, b_puoff, b_pcrc, b_pentry, b_inflated, b_blk_code, b_derr, b_seg_cnt,
+      b_seg_off, b_recoff, b_recinfo, b_cnt4, b_scan4, b_ecode, b_earg, b_names, b_name_off;
+  PinVec<int32_t> hd_tstart, hd_tend, hd_qstart, hd_qlen;   // per-read arrays of the last hm_decode_bam_begin
+  PinVec<uint32_t> hd_n_ops;
+  PinVec<uint64_t> hd_bq_off, hd_op_off, hd_name_off, hd_scal; // hd_scal: walk / scan totals read back
+  PinVec<char> hd_names;
+  PinVec<bamgpu::Err> hd_err;
+  std::vector<uint8_t> hd_flags;
+  uint64_t dec_n = 0, dec_ops = 0, dec_bq = 0;
+  bool dec_ready = false;                   // hm_decode_bam_begin succeeded, hm_decode_bam_end has not run
 };
 
 namespace {
@@ -336,6 +348,7 @@ size_t hm_abi_sizeof(int which) {
     case 2: return sizeof(hm_params);
     case 3: return sizeof(hm_site_record);
     case 4: return sizeof(hm_bq_compact);
+    case 5: return sizeof(hm_bgzf_plan);
     default: return 0;
   }
 }
@@ -383,12 +396,18 @@ void hm_destroy(hm_ctx* ctx) {
                     &ctx->b_pair_off, &ctx->b_pair_hap, &ctx->b_qseen, &ctx->b_keys, &ctx->b_keys_sorted, &ctx->b_cub,
                     &ctx->b_records, &ctx->b_counters, &ctx->b_ref, &ctx->b_norm_out, &ctx->b_lut, &ctx->b_tile_off, &ctx->b_agg, &ctx->b_geom, &ctx->b_bidx, &ctx->b_brecs, &ctx->b_sites, &ctx->b_push, &ctx->b_span_cnt, &ctx->b_koff, &ctx->b_tile_info, &ctx->b_edge_counts, &ctx->b_edge_hpos, &ctx->b_edge_href, &ctx->b_bqmask, &ctx->b_bqexc, &ctx->b_bqexc_off,
                     &ctx->b_cgeom, &ctx->b_seg_keys, &ctx->b_seg_read, &ctx->b_keys_tmp, &ctx->b_gscratch, &ctx->b_czero, &ctx->b_first_pair, &ctx->b_tiles, &ctx->b_site_valid, &ctx->b_pair_c,
-                    &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_exp_total, &ctx->b_sdiff, &ctx->b_cal_ok};
+                    &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_exp_total, &ctx->b_sdiff, &ctx->b_cal_ok,
+                    &ctx->b_comp, &ctx->b_pcoff, &ctx->b_pcsize, &ctx->b_pisize, &ctx->b_puoff, &ctx->b_pcrc, &ctx->b_pentry, &ctx->b_inflated,
+                    &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt4,
+                    &ctx->b_scan4, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off};
   for (DevBuf* b : bufs) b->release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_cnt_pin) cudaFreeHost(ctx->h_cnt_pin);
   if (ctx->h_geom_pin) cudaFreeHost(ctx->h_geom_pin);
   ctx->h_pmax.release(); ctx->h_tix_off.release(); ctx->h_cw_off.release();
+  ctx->hd_tstart.release(); ctx->hd_tend.release(); ctx->hd_qstart.release(); ctx->hd_qlen.release(); ctx->hd_n_ops.release();
+  ctx->hd_bq_off.release(); ctx->hd_op_off.release(); ctx->hd_name_off.release(); ctx->hd_scal.release(); ctx->hd_names.release();
+  ctx->hd_err.release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -505,39 +524,12 @@ int hm_upload_wait(hm_ctx* ctx) {
   return HM_OK;
 }
 
-static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact* cq, bool wait) {
-  if (!ctx || !b) return HM_ERR_ARG;
-  if (!cq && !b->bq) return fail(ctx, HM_ERR_ARG, "batch has no quality stream");
-  // seq == NULL: no base stream.  The bases of match runs are then the reference allele of the site that asks
-  // (what a cs match means, cslib.py:22-29); substituted bases travel in the ops.  `call` and the phase edges
-  // need nothing else; normcounts does (for now) and refuses such a batch.
-  const bool has_seq = b->seq != nullptr;
-  if (!has_seq && b->seq_bytes) return fail(ctx, HM_ERR_ARG, "seq is NULL but seq_bytes is not 0");
-  if (has_seq && !b->seq_off) return fail(ctx, HM_ERR_ARG, "seq without seq_off");
-  if (cq) {
-    if (!cq->mask || !cq->exc_off || (cq->exc_bytes && !cq->exc)) return fail(ctx, HM_ERR_ARG, "incomplete hm_bq_compact");
-    if (cq->mask_bytes * 8 != b->bq_bytes) return fail(ctx, HM_ERR_ARG, "hm_bq_compact.mask_bytes must be bq_bytes / 8");
-  }
-  CU(cudaSetDevice(ctx->device));
-  if (ctx->upload_pending) { // an upload that was not waited for: its copies still read the page-locked tables rewritten below
-    CU(cudaEventSynchronize(ctx->ev_up));
-    ctx->upload_pending = false;
-  }
-  ctx->have_batch = false;
+// The O(reads) checks of a batch on the host and the tables derived from it (running maximum of tend, tile and
+// cal-word offsets, op prefix, shared query names, entry slots per site), for both ways a batch becomes resident
+// (hm_upload_batch*, hm_decode_bam_end).  A batch that fails is never used; the stream is waited for before the error
+// returns, so the caller may free its buffers.
+static int batch_tables(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact* cq, bool has_seq) {
   const uint64_t n = b->n_reads;
-  if (n >= (1ull << 32)) return fail(ctx, HM_ERR_ARG, "too many reads in one batch");
-  if ((b->seq_bytes & 15) || (b->bq_bytes & 15)) return fail(ctx, HM_ERR_ARG, "seq / bq buffers must be padded to 16 bytes");
-  // The large streams leave first (copy engine, in stream order); the O(reads) validation below runs on the host while
-  // they move.  A batch that fails it is never used (have_batch stays false); the copies are waited for before the
-  // error is returned, so the caller may free its buffers.
-  int rc;
-#define UP(buf, field, count) if ((rc = upload(ctx, ctx->buf, b->field, (size_t)(count)))) return rc
-  if (cq) {
-    if ((rc = upload(ctx, ctx->b_bqmask, cq->mask, (size_t)cq->mask_bytes))) return rc;
-    if ((rc = upload(ctx, ctx->b_bqexc, cq->exc, (size_t)cq->exc_bytes, 16))) return rc;
-  } else { UP(b_bq, bq, b->bq_bytes); }
-  if (has_seq) { UP(b_seq, seq, b->seq_bytes); }
-  UP(b_ops, ops, b->n_ops_total);
 #define BAD(...) do { cudaStreamSynchronize(ctx->stream); return fail(ctx, HM_ERR_ARG, __VA_ARGS__); } while (0)
   // structural validation (cheap, O(reads)); the kernels binary-search on these invariants
   if (!ctx->h_pmax.resize(n) || !ctx->h_tix_off.resize(n + 1) || !ctx->h_cw_off.resize(n + 1)) BAD("out of page-locked host memory for %llu reads", (unsigned long long)n);
@@ -588,24 +580,22 @@ static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_co
       named[b->qname_id[r]] = 1;
     }
   }
-  UP(b_tstart, tstart, n); UP(b_tend, tend, n); UP(b_qstart, qstart, n); UP(b_qlen, qlen, n);
-  UP(b_mapq, mapq, n); UP(b_flags, flags, n); UP(b_qname, qname_id, n);
-  UP(b_bq_off, bq_off, n); UP(b_op_off, op_off, n); UP(b_n_ops, n_ops, n);
-  if (has_seq) { UP(b_seq_off, seq_off, n); }
-  if (cq) {
-    CU(ctx->b_bq.ensure(b->bq_bytes + 16));
-    if ((rc = upload(ctx, ctx->b_bqexc_off, cq->exc_off, (size_t)n + 1))) return rc;
-  }
-#undef UP
   if (b->n_reads && (b->tstart[0] < 0 || n_tix >= (1ull << 32))) BAD("negative reference_start, or too many (read, tile) pairs in one batch");
 #undef BAD
   ctx->h_tix_off[n] = (uint32_t)n_tix;
   ctx->n_tix = n_tix;
-  if ((rc = upload(ctx, ctx->b_pmax, ctx->h_pmax.data(), n))) return rc;
-  if ((rc = upload(ctx, ctx->b_tix_off, ctx->h_tix_off.data(), n + 1))) return rc;
   ctx->h_cw_off[n] = (uint32_t)n_cw;
   ctx->n_cw = n_cw;
-  if (n_cw < (1ull << 32) && (rc = upload(ctx, ctx->b_cw_off, ctx->h_cw_off.data(), n + 1))) return rc;
+  return HM_OK;
+}
+
+// the derived tables to the device and the resident batch's device view (the per-read arrays are in place)
+static int bind_batch(hm_ctx* ctx, const hm_read_batch* b, bool has_seq) {
+  const uint64_t n = b->n_reads;
+  int rc;
+  if ((rc = upload(ctx, ctx->b_pmax, ctx->h_pmax.data(), n))) return rc;
+  if ((rc = upload(ctx, ctx->b_tix_off, ctx->h_tix_off.data(), n + 1))) return rc;
+  if (ctx->n_cw < (1ull << 32) && (rc = upload(ctx, ctx->b_cw_off, ctx->h_cw_off.data(), n + 1))) return rc;
   const size_t no = (size_t)b->n_ops_total;
   CU(ctx->b_op_t.ensure(no * 4 + 16)); CU(ctx->b_op_q.ensure(no * 4 + 16)); CU(ctx->b_mm.ensure(no * 4 + 16));
   CU(ctx->b_bq_total.ensure(n * 8 + 16)); CU(ctx->b_n_match.ensure(n * 4 + 16)); CU(ctx->b_n_sub.ensure(n * 4 + 16));
@@ -623,6 +613,53 @@ static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_co
   d.n_sub = ctx->b_n_sub.as<int32_t>(); d.ins_len = ctx->b_ins_len.as<int32_t>(); d.del_len = ctx->b_del_len.as<int32_t>();
   d.n_mm = ctx->b_n_mm.as<int32_t>(); d.gate = ctx->b_gate.as<uint8_t>(); d.pmax_tend = ctx->b_pmax.as<int32_t>();
   ctx->n_reads = n; ctx->n_ops_total = b->n_ops_total; ctx->seq_bytes = b->seq_bytes; ctx->bq_bytes = b->bq_bytes;
+  return HM_OK;
+}
+
+static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact* cq, bool wait) {
+  if (!ctx || !b) return HM_ERR_ARG;
+  if (!cq && !b->bq) return fail(ctx, HM_ERR_ARG, "batch has no quality stream");
+  // seq == NULL: no base stream.  The bases of match runs are then the reference allele of the site that asks
+  // (what a cs match means, cslib.py:22-29); substituted bases travel in the ops.  `call` and the phase edges
+  // need nothing else; normcounts does (for now) and refuses such a batch.
+  const bool has_seq = b->seq != nullptr;
+  if (!has_seq && b->seq_bytes) return fail(ctx, HM_ERR_ARG, "seq is NULL but seq_bytes is not 0");
+  if (has_seq && !b->seq_off) return fail(ctx, HM_ERR_ARG, "seq without seq_off");
+  if (cq) {
+    if (!cq->mask || !cq->exc_off || (cq->exc_bytes && !cq->exc)) return fail(ctx, HM_ERR_ARG, "incomplete hm_bq_compact");
+    if (cq->mask_bytes * 8 != b->bq_bytes) return fail(ctx, HM_ERR_ARG, "hm_bq_compact.mask_bytes must be bq_bytes / 8");
+  }
+  CU(cudaSetDevice(ctx->device));
+  if (ctx->upload_pending) { // an upload that was not waited for: its copies still read the page-locked tables rewritten below
+    CU(cudaEventSynchronize(ctx->ev_up));
+    ctx->upload_pending = false;
+  }
+  ctx->have_batch = false;
+  const uint64_t n = b->n_reads;
+  if (n >= (1ull << 32)) return fail(ctx, HM_ERR_ARG, "too many reads in one batch");
+  if ((b->seq_bytes & 15) || (b->bq_bytes & 15)) return fail(ctx, HM_ERR_ARG, "seq / bq buffers must be padded to 16 bytes");
+  // The large streams leave first (copy engine, in stream order); the O(reads) validation below runs on the host while
+  // they move.  A batch that fails it is never used (have_batch stays false); the copies are waited for before the
+  // error is returned, so the caller may free its buffers.
+  int rc;
+#define UP(buf, field, count) if ((rc = upload(ctx, ctx->buf, b->field, (size_t)(count)))) return rc
+  if (cq) {
+    if ((rc = upload(ctx, ctx->b_bqmask, cq->mask, (size_t)cq->mask_bytes))) return rc;
+    if ((rc = upload(ctx, ctx->b_bqexc, cq->exc, (size_t)cq->exc_bytes, 16))) return rc;
+  } else { UP(b_bq, bq, b->bq_bytes); }
+  if (has_seq) { UP(b_seq, seq, b->seq_bytes); }
+  UP(b_ops, ops, b->n_ops_total);
+  if ((rc = batch_tables(ctx, b, cq, has_seq))) return rc;
+  UP(b_tstart, tstart, n); UP(b_tend, tend, n); UP(b_qstart, qstart, n); UP(b_qlen, qlen, n);
+  UP(b_mapq, mapq, n); UP(b_flags, flags, n); UP(b_qname, qname_id, n);
+  UP(b_bq_off, bq_off, n); UP(b_op_off, op_off, n); UP(b_n_ops, n_ops, n);
+  if (has_seq) { UP(b_seq_off, seq_off, n); }
+  if (cq) {
+    CU(ctx->b_bq.ensure(b->bq_bytes + 16));
+    if ((rc = upload(ctx, ctx->b_bqexc_off, cq->exc_off, (size_t)n + 1))) return rc;
+  }
+#undef UP
+  if ((rc = bind_batch(ctx, b, has_seq))) return rc;
   ctx->compact_resident = false;
   CU(cudaEventRecord(ctx->ev_up, ctx->stream)); // every host buffer has been read once this fires
   if (cq && n) {
@@ -641,6 +678,167 @@ static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_co
   if (wait) CU(cudaEventSynchronize(ctx->ev_up)); // the caller may reuse its buffers after return; k_bq_expand may still be running
   ctx->upload_pending = !wait;
   ctx->have_batch = true;
+  return HM_OK;
+}
+
+// ------------------------------------------------------------------ device BAM decoder (bamgpu.cuh)
+// the message of the first failing record (index r of the walk) of the last decode, as the host decoder words it
+static int decode_record_error(hm_ctx* ctx, const hm_bgzf_plan* pl, unsigned long long r) {
+  uint8_t code = 0;
+  long long arg = 0;
+  bamgpu::RecInfo info;
+  CU(cudaMemcpyAsync(&code, ctx->b_ecode.as<uint8_t>() + r, 1, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(&arg, ctx->b_earg.as<long long>() + r, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(&info, ctx->b_recinfo.as<bamgpu::RecInfo>() + r, sizeof(info), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (code == 0 || code >= E_N_CODES) return fail(ctx, HM_ERR_ARG, "device BAM decoder: record %llu failed without a code", r);
+  if (REC_ERR_ON_PATH(code)) return fail(ctx, HM_ERR_ARG, REC_ERR[code], pl->path ? pl->path : "", (long)arg);
+  char name[257];  // the record passed the field checks: its name ends inside it, within 256 bytes
+  CU(cudaMemcpyAsync(name, ctx->b_inflated.as<uint8_t>() + info.p + 4 + 32, 256, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  name[256] = 0;
+  return fail(ctx, HM_ERR_ARG, REC_ERR[code], name, (long)arg);
+}
+
+static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32_t start, int32_t end, uint64_t* n_reads) {
+  using namespace bamgpu;
+  const uint64_t nb = pl->n_blocks, ne = pl->n_entry;
+  ctx->dec_n = ctx->dec_ops = 0;
+  ctx->dec_bq = 16;
+  if (nb == 0 || ne == 0) return HM_OK;
+  // the plan comes from outside: every offset the kernels follow is checked here
+  if (!pl->comp || !pl->blk_coff || !pl->blk_csize || !pl->blk_isize || !pl->blk_uoff || !pl->blk_crc || !pl->entry)
+    return fail(ctx, HM_ERR_ARG, "incomplete hm_bgzf_plan");
+  for (uint64_t i = 0; i < nb; i++)
+    if (pl->blk_coff[i] + pl->blk_csize[i] != pl->blk_coff[i + 1] || pl->blk_csize[i] < 20 || pl->blk_isize[i] > 65536 ||
+        pl->blk_uoff[i] + pl->blk_isize[i] != pl->blk_uoff[i + 1])
+      return fail(ctx, HM_ERR_ARG, "hm_bgzf_plan: block %llu is inconsistent", (unsigned long long)i);
+  const uint64_t total = pl->blk_uoff[nb];
+  if (pl->blk_coff[0] != 0 || pl->blk_coff[nb] != pl->comp_bytes || pl->blk_uoff[0] != 0 || pl->walk_end > total)
+    return fail(ctx, HM_ERR_ARG, "hm_bgzf_plan: the block table does not cover the range");
+  for (uint64_t e = 0; e < ne; e++)
+    if (pl->entry[e] >= pl->walk_end || (e && pl->entry[e] <= pl->entry[e - 1]))
+      return fail(ctx, HM_ERR_ARG, "hm_bgzf_plan: entry point %llu is out of order", (unsigned long long)e);
+  int rc;
+  t_begin(ctx, "h2d_compressed");
+  if ((rc = upload(ctx, ctx->b_comp, pl->comp, pl->comp_bytes))) return rc;
+  t_end(ctx);
+  if ((rc = upload(ctx, ctx->b_pcoff, pl->blk_coff, nb + 1))) return rc;
+  if ((rc = upload(ctx, ctx->b_pcsize, pl->blk_csize, nb))) return rc;
+  if ((rc = upload(ctx, ctx->b_pisize, pl->blk_isize, nb))) return rc;
+  if ((rc = upload(ctx, ctx->b_puoff, pl->blk_uoff, nb + 1))) return rc;
+  if ((rc = upload(ctx, ctx->b_pcrc, pl->blk_crc, nb))) return rc;
+  if ((rc = upload(ctx, ctx->b_pentry, pl->entry, ne))) return rc;
+  CU(ctx->b_inflated.ensure(total + 64));  // 64 zero bytes past the end: the fixed part of a short last record reads there
+  CU(cudaMemsetAsync(ctx->b_inflated.as<uint8_t>() + total, 0, 64, ctx->stream));
+  CU(ctx->b_blk_code.ensure(nb));
+  CU(ctx->b_derr.ensure(sizeof(Err)));
+  CU(cudaMemsetAsync(ctx->b_derr.p, 0xff, sizeof(Err), ctx->stream));
+  if (!ctx->hd_err.resize(1) || !ctx->hd_scal.resize(4)) return fail(ctx, HM_ERR_ARG, "out of page-locked host memory");
+  Err* derr = ctx->b_derr.as<Err>();
+  Err& herr = ctx->hd_err[0];
+  // inflate: one block per warp (bamgpu.cuh says why)
+  const uint64_t per_cta = 1;
+  const Plan dpl{ctx->b_comp.as<uint8_t>(), ctx->b_pcoff.as<uint64_t>(), ctx->b_pcsize.as<uint32_t>(), ctx->b_pisize.as<uint32_t>(),
+                 ctx->b_puoff.as<uint64_t>(), ctx->b_pcrc.as<uint32_t>(), nb};
+  t_begin(ctx, "k_bgzf_inflate");
+  k_bgzf_inflate<<<(unsigned)((nb + per_cta - 1) / per_cta), 32, 0, ctx->stream>>>(dpl, ctx->b_inflated.as<uint8_t>(), (uint32_t)per_cta,
+                                                                                ctx->b_blk_code.as<uint8_t>(), derr);
+  t_end(ctx);
+  CU(cudaGetLastError());
+  // walk: records per segment, their scan, then the offsets
+  CU(ctx->b_seg_cnt.ensure((ne + 1) * 8));
+  CU(ctx->b_seg_off.ensure((ne + 1) * 8));
+  CU(cudaMemsetAsync(ctx->b_seg_cnt.as<unsigned long long>() + ne, 0, 8, ctx->stream));
+  const uint8_t* buf = ctx->b_inflated.as<uint8_t>();
+  t_begin(ctx, "k_bam_walk");
+  k_bam_walk<<<(unsigned)((ne + 127) / 128), 128, 0, ctx->stream>>>(buf, ctx->b_pentry.as<uint64_t>(), ne, pl->walk_end,
+                                                                     ctx->b_seg_cnt.as<unsigned long long>(), nullptr, nullptr, derr);
+  t_end(ctx);
+  CU(cudaGetLastError());
+  size_t tmp = 0;
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, ctx->b_seg_cnt.as<unsigned long long>(), ctx->b_seg_off.as<unsigned long long>(), (int)(ne + 1), ctx->stream));
+  CU(ctx->b_cub.ensure(tmp));
+  CU(cub::DeviceScan::ExclusiveSum(ctx->b_cub.p, tmp, ctx->b_seg_cnt.as<unsigned long long>(), ctx->b_seg_off.as<unsigned long long>(), (int)(ne + 1), ctx->stream));
+  CU(cudaMemcpyAsync(&ctx->hd_scal[0], ctx->b_seg_off.as<unsigned long long>() + ne, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(&herr, derr, sizeof(Err), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (herr.block != ~0ull) {
+    uint8_t code = 0;
+    CU(cudaMemcpy(&code, ctx->b_blk_code.as<uint8_t>() + herr.block, 1, cudaMemcpyDeviceToHost));
+    return fail(ctx, HM_ERR_ARG, REC_ERR[code == E_CRC ? E_CRC : E_INFLATE], pl->path ? pl->path : "", (long)herr.block);
+  }
+  if (herr.entry != ~0ull) return fail(ctx, HM_ERR_ARG, REC_ERR[E_BAI_ENTRY], pl->path ? pl->path : "", (long)herr.entry);
+  const uint64_t n_rec = ctx->hd_scal[0];
+  if (n_rec == 0) return HM_OK;
+  if (n_rec >= (1ull << 31)) return fail(ctx, HM_ERR_ARG, "too many records in one region (%llu)", (unsigned long long)n_rec);
+  CU(ctx->b_recoff.ensure(n_rec * 8));
+  k_bam_walk<<<(unsigned)((ne + 127) / 128), 128, 0, ctx->stream>>>(buf, ctx->b_pentry.as<uint64_t>(), ne, pl->walk_end, nullptr,
+                                                                     ctx->b_seg_off.as<unsigned long long>(), ctx->b_recoff.as<uint64_t>(), derr);
+  CU(cudaGetLastError());
+  // select and count
+  const uint64_t stride = n_rec + 1;
+  CU(ctx->b_recinfo.ensure(n_rec * sizeof(RecInfo)));
+  CU(ctx->b_cnt4.ensure(4 * stride * 8));
+  CU(ctx->b_scan4.ensure(4 * stride * 8));
+  CU(ctx->b_ecode.ensure(n_rec));
+  CU(ctx->b_earg.ensure(n_rec * 8));
+  t_begin(ctx, "k_bam_select");
+  k_bam_select<<<(unsigned)((n_rec + 127) / 128), 128, 0, ctx->stream>>>(buf, ctx->b_recoff.as<uint64_t>(), n_rec, pl->walk_end, rid, start, end,
+                                                                          ctx->b_recinfo.as<RecInfo>(), ctx->b_cnt4.as<unsigned long long>(),
+                                                                          ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
+  t_end(ctx);
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(&herr, derr, sizeof(Err), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  const uint64_t stop = std::min<uint64_t>(herr.stop, n_rec);  // records from here on are never looked at by the host
+  if (herr.rec < stop) return decode_record_error(ctx, pl, herr.rec);
+  if (stop == 0) return HM_OK;
+  // output offsets: exclusive scans of the four counts (read index, first op, first quality byte, first name byte)
+  unsigned long long* cnt4 = ctx->b_cnt4.as<unsigned long long>();
+  unsigned long long* scan4 = ctx->b_scan4.as<unsigned long long>();
+  tmp = 0;
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt4, scan4, (int)stride, ctx->stream));
+  CU(ctx->b_cub.ensure(tmp));
+  t_begin(ctx, "cub_scan_records");
+  for (int k = 0; k < 4; k++) CU(cub::DeviceScan::ExclusiveSum(ctx->b_cub.p, tmp, cnt4 + k * stride, scan4 + k * stride, (int)stride, ctx->stream));
+  t_end(ctx);
+  for (int k = 0; k < 4; k++) CU(cudaMemcpyAsync(&ctx->hd_scal[k], scan4 + k * stride + stop, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  const uint64_t n = ctx->hd_scal[0], n_ops = ctx->hd_scal[1], n_bq = ctx->hd_scal[2], n_nm = ctx->hd_scal[3];
+  // the resident batch's buffers, written in place
+  CU(ctx->b_tstart.ensure(n * 4 + 16)); CU(ctx->b_tend.ensure(n * 4 + 16)); CU(ctx->b_qstart.ensure(n * 4 + 16));
+  CU(ctx->b_qlen.ensure(n * 4 + 16)); CU(ctx->b_mapq.ensure(n + 16)); CU(ctx->b_flags.ensure(n + 16)); CU(ctx->b_qname.ensure(n * 4 + 16));
+  CU(ctx->b_n_ops.ensure(n * 4 + 16)); CU(ctx->b_bq_off.ensure(n * 8 + 16)); CU(ctx->b_op_off.ensure(n * 8 + 16));
+  CU(ctx->b_bq.ensure(n_bq + 32)); CU(ctx->b_ops.ensure(n_ops * 4 + 16)); CU(ctx->b_names.ensure(n_nm + 16));
+  CU(ctx->b_name_off.ensure(n * 8 + 16));
+  ParseOut o{ctx->b_tstart.as<int32_t>(), ctx->b_tend.as<int32_t>(), ctx->b_qstart.as<int32_t>(), ctx->b_qlen.as<int32_t>(),
+             ctx->b_mapq.as<uint8_t>(), ctx->b_flags.as<uint8_t>(), ctx->b_n_ops.as<uint32_t>(), ctx->b_bq_off.as<uint64_t>(),
+             ctx->b_op_off.as<uint64_t>(), ctx->b_name_off.as<uint64_t>(), ctx->b_bq.as<uint8_t>(), ctx->b_ops.as<uint32_t>(),
+             ctx->b_names.as<char>()};
+  t_begin(ctx, "k_bam_parse");
+  k_bam_parse<<<(unsigned)((stop * 32 + 255) / 256), 256, 0, ctx->stream>>>(buf, ctx->b_recinfo.as<RecInfo>(), stop, scan4, stride, o,
+                                                                             ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
+  t_end(ctx);
+  CU(cudaGetLastError());
+  if (!ctx->hd_tstart.resize(n) || !ctx->hd_tend.resize(n) || !ctx->hd_qstart.resize(n) || !ctx->hd_qlen.resize(n) ||
+      !ctx->hd_n_ops.resize(n) || !ctx->hd_bq_off.resize(n) || !ctx->hd_op_off.resize(n) || !ctx->hd_name_off.resize(n) ||
+      !ctx->hd_names.resize(n_nm + 1))
+    return fail(ctx, HM_ERR_ARG, "out of page-locked host memory for %llu reads", (unsigned long long)n);
+  t_begin(ctx, "d2h_reads_names");
+#define DOWN(h, d, bytes) CU(cudaMemcpyAsync(ctx->h.data(), ctx->d.p, (bytes), cudaMemcpyDeviceToHost, ctx->stream))
+  DOWN(hd_tstart, b_tstart, n * 4); DOWN(hd_tend, b_tend, n * 4); DOWN(hd_qstart, b_qstart, n * 4); DOWN(hd_qlen, b_qlen, n * 4);
+  DOWN(hd_n_ops, b_n_ops, n * 4); DOWN(hd_bq_off, b_bq_off, n * 8); DOWN(hd_op_off, b_op_off, n * 8);
+  DOWN(hd_name_off, b_name_off, n * 8); DOWN(hd_names, b_names, n_nm);
+#undef DOWN
+  t_end(ctx);
+  CU(cudaMemcpyAsync(&herr, derr, sizeof(Err), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (herr.parse != ~0ull) return decode_record_error(ctx, pl, herr.parse);
+  ctx->dec_n = n;
+  ctx->dec_ops = n_ops;
+  ctx->dec_bq = n_bq ? n_bq : 16;
+  *n_reads = n;
   return HM_OK;
 }
 
@@ -1487,6 +1685,108 @@ int hm_last_kernel_times(hm_ctx* ctx, const char** names, float* ms, size_t cap,
   }
   *n = k;
   return HM_OK;
+}
+
+int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint64_t* n_reads) {
+  if (!ctx || !plan || !n_reads) return HM_ERR_ARG;
+  *n_reads = 0;
+  CU(cudaSetDevice(ctx->device));
+  if (ctx->upload_pending) { // the copies of an upload that was not waited for still read their host buffers
+    CU(cudaEventSynchronize(ctx->ev_up));
+    ctx->upload_pending = false;
+  }
+  ctx->have_batch = false;
+  ctx->dec_ready = false;
+  t_reset(ctx);
+  if (start < 0) start = 0;
+  const int rc = decode_begin_impl(ctx, plan, rid, start, end, n_reads);
+  if (rc) { cudaStreamSynchronize(ctx->stream); return rc; }
+  t_collect(ctx);
+  ctx->dec_ready = true;
+  return HM_OK;
+}
+
+int hm_decode_bam_names(hm_ctx* ctx, const char** names, const uint64_t** name_off, const int32_t** tstart, const int32_t** tend,
+                        uint64_t* n_reads) {
+  if (!ctx || !names || !name_off || !tstart || !tend || !n_reads) return HM_ERR_ARG;
+  if (!ctx->dec_ready) return fail(ctx, HM_ERR_STATE, "no decoded region: call hm_decode_bam_begin first");
+  *names = ctx->hd_names.data(); *name_off = ctx->hd_name_off.data();
+  *tstart = ctx->hd_tstart.data(); *tend = ctx->hd_tend.data();
+  *n_reads = ctx->dec_n;
+  return HM_OK;
+}
+
+int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id) {
+  if (!ctx) return HM_ERR_ARG;
+  if (!ctx->dec_ready) return fail(ctx, HM_ERR_STATE, "no decoded region: call hm_decode_bam_begin first");
+  const uint64_t n = ctx->dec_n;
+  if (n && !qname_id) return fail(ctx, HM_ERR_ARG, "qname_id is NULL");
+  CU(cudaSetDevice(ctx->device));
+  ctx->dec_ready = false;
+  ctx->hd_flags.assign(n, 0);
+  hm_read_batch b;
+  memset(&b, 0, sizeof(b));
+  b.n_reads = n;
+  b.tstart = ctx->hd_tstart.data(); b.tend = ctx->hd_tend.data(); b.qstart = ctx->hd_qstart.data(); b.qlen = ctx->hd_qlen.data();
+  b.flags = ctx->hd_flags.data(); b.qname_id = qname_id; b.bq_off = ctx->hd_bq_off.data(); b.op_off = ctx->hd_op_off.data();
+  b.n_ops = ctx->hd_n_ops.data(); b.bq_bytes = ctx->dec_bq; b.n_ops_total = ctx->dec_ops;
+  int rc;
+  if ((rc = batch_tables(ctx, &b, nullptr, false))) return rc;
+  if (n == 0) { // the host decoder's empty batch: 16 zero quality bytes
+    CU(ctx->b_bq.ensure(32));
+    CU(cudaMemsetAsync(ctx->b_bq.p, 0, 16, ctx->stream));
+    CU(ctx->b_ops.ensure(16));
+    for (DevBuf* d : {&ctx->b_tstart, &ctx->b_tend, &ctx->b_qstart, &ctx->b_qlen, &ctx->b_mapq, &ctx->b_flags, &ctx->b_qname,
+                      &ctx->b_n_ops, &ctx->b_bq_off, &ctx->b_op_off})
+      CU(d->ensure(16));
+  }
+  if ((rc = upload(ctx, ctx->b_qname, qname_id, n))) return rc;
+  if ((rc = bind_batch(ctx, &b, false))) return rc;
+  ctx->compact_resident = false;
+  CU(cudaStreamSynchronize(ctx->stream));
+  ctx->have_batch = true;
+  return HM_OK;
+}
+
+/* diagnostics (tests): the resident batch back to caller buffers (NULL: skip); sizes as hm_decode_bam_begin / the upload
+ * left them: n_reads entries per read, bq_bytes quality bytes, n_ops_total ops */
+int hm_batch_read_back(hm_ctx* ctx, hm_read_batch* out, int32_t* tstart, int32_t* tend, int32_t* qstart, int32_t* qlen,
+                       uint8_t* mapq, uint32_t* qname_id, uint64_t* bq_off, uint64_t* op_off, uint32_t* n_ops, uint8_t* bq, uint32_t* ops) {
+  if (!ctx || !out) return HM_ERR_ARG;
+  if (!ctx->have_batch) return fail(ctx, HM_ERR_STATE, "no resident batch");
+  CU(cudaSetDevice(ctx->device));
+  memset(out, 0, sizeof(*out));
+  const uint64_t n = ctx->n_reads;
+  out->n_reads = n; out->bq_bytes = ctx->bq_bytes; out->n_ops_total = ctx->n_ops_total;
+  const struct { void* dst; const DevBuf* src; size_t bytes; } cp[] = {
+      {tstart, &ctx->b_tstart, n * 4}, {tend, &ctx->b_tend, n * 4}, {qstart, &ctx->b_qstart, n * 4}, {qlen, &ctx->b_qlen, n * 4},
+      {mapq, &ctx->b_mapq, n}, {qname_id, &ctx->b_qname, n * 4}, {bq_off, &ctx->b_bq_off, n * 8}, {op_off, &ctx->b_op_off, n * 8},
+      {n_ops, &ctx->b_n_ops, n * 4}, {bq, &ctx->b_bq, ctx->bq_bytes}, {ops, &ctx->b_ops, ctx->n_ops_total * 4}};
+  for (const auto& c : cp)
+    if (c.dst && c.bytes) CU(cudaMemcpyAsync(c.dst, c.src->p, c.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  return HM_OK;
+}
+
+/* tests: k_bgzf_inflate's decoder on one raw DEFLATE stream that must inflate to exactly out_len bytes with CRC32 `crc`;
+ * 0 ok, else the error code of bamerr.h (E_INFLATE, E_CRC) */
+int hm_inflate_device_test(hm_ctx* ctx, const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len, uint32_t crc) {
+  if (!ctx || (in_len && !in) || (out_len && !out) || out_len > 65536 || in_len >= (1ull << 31)) return HM_ERR_ARG;
+  CU(cudaSetDevice(ctx->device));
+  DevBuf din, dout, drc;
+  CU(din.ensure(in_len + 16));
+  CU(dout.ensure(out_len + 16));
+  CU(drc.ensure(16));
+  if (in_len) CU(cudaMemcpyAsync(din.p, in, in_len, cudaMemcpyHostToDevice, ctx->stream));
+  bamgpu::k_inflate_one<<<1, 32, 0, ctx->stream>>>(din.as<uint8_t>(), (uint32_t)in_len, dout.as<uint8_t>(), (uint32_t)out_len, crc, drc.as<int>());
+  int rc = 0;
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(&rc, drc.p, 4, cudaMemcpyDeviceToHost, ctx->stream);
+  if (e == cudaSuccess && out_len) e = cudaMemcpyAsync(out, dout.p, out_len, cudaMemcpyDeviceToHost, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  din.release(); dout.release(); drc.release();
+  if (e != cudaSuccess) return fail(ctx, HM_ERR_CUDA, "hm_inflate_device_test: %s", cudaGetErrorString(e));
+  return rc;
 }
 
 }  // extern "C"

@@ -8,7 +8,7 @@ import os
 
 import numpy as np
 
-from . import abi
+from . import abi, pack
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HIMUT_B200_LIB") or os.path.join(_HERE, "libhimut_b200.so")  # override: instrumented builds
@@ -21,6 +21,7 @@ EXPORTS = [
     "hm_read_stats", "hm_last_timing", "hm_last_kernel_times", "hm_set_stream", "hm_host_register",
     "hm_host_unregister", "hm_abi_sizeof", "hm_last_records", "hm_qname_seen", "hm_set_reference", "hm_ref_tricounts", "hm_last_norm_exact_sites",
     "hm_phase_edges_begin", "hm_phase_edges_add", "hm_phase_edges_end", "hm_upload_batch_compact", "hm_call_batch_compact", "hm_call_chunks_async", "hm_records_wait", "hm_set_option", "hm_last_call_path", "hm_call_chunks_submit", "hm_call_chunks_collect", "hm_device_count", "hm_upload_batch_compact_begin", "hm_upload_wait",
+    "hm_decode_bam_begin", "hm_decode_bam_names", "hm_decode_bam_end", "hm_batch_read_back", "hm_inflate_device_test",
 ]
 
 
@@ -80,6 +81,11 @@ def load():
         lib.hm_last_call_path.restype = C.c_int
         lib.hm_host_register.argtypes = [vp, vp, sz]
         lib.hm_host_unregister.argtypes = [vp, vp]
+        lib.hm_decode_bam_begin.argtypes = [vp, C.POINTER(abi.hm_bgzf_plan), C.c_int, C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]
+        lib.hm_decode_bam_names.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_uint64)]
+        lib.hm_decode_bam_end.argtypes = [vp, vp]
+        lib.hm_batch_read_back.argtypes = [vp, C.POINTER(abi.hm_read_batch)] + [vp] * 11
+        lib.hm_inflate_device_test.argtypes = [vp, C.c_char_p, sz, vp, sz, C.c_uint32]
         _LIB = lib
     return _LIB
 
@@ -91,6 +97,15 @@ def _p(a):
 def device_count():
     """cudaGetDeviceCount through the library (0 when no driver / device)"""
     return int(load().hm_device_count())
+
+
+class DecodedRegion:
+    """what Context.decode_region leaves on the host: the per-read coordinates the chunk table needs"""
+
+    chunk_table = abi.ReadBatch.chunk_table
+
+    def __init__(self, tstart, tend):
+        self.n_reads, self.tstart, self.tend = int(tstart.size), tstart, tend
 
 
 class Context:
@@ -181,6 +196,49 @@ class Context:
         else:
             self._uploading = (batch, cq)  # alive until the copies are done
             self._chk(self.lib.hm_upload_batch_compact_begin(self.h, C.byref(batch.as_struct()), C.byref(cq.struct)))
+
+    def decode_region(self, reader, chrom, start, end):
+        """the records reader.read_batch(chrom, start, end, seq=False) returns, decoded on the device from the
+        compressed file (reader: bamdec.NativeBam) and left resident as upload() would leave that batch.  Query-name
+        ids come from the reader's table.  Rejected input raises pack.BatchFormatError with the host decoder's text.
+        -> DecodedRegion (n_reads, tstart, tend, chunk_table)"""
+        rid = reader.references.index(chrom)
+        start, end = int(max(start, 0)), int(min(end, reader.lengths[rid]))
+        plan = reader.plan(chrom, start, end)
+        n = C.c_uint64(0)
+        rc = self.lib.hm_decode_bam_begin(self.h, C.byref(plan), rid, start, end, C.byref(n))
+        if rc == abi.HM_ERR_ARG:
+            raise pack.BatchFormatError(self.lib.hm_last_error(self.h).decode())
+        self._chk(rc)
+        self.last_decode_times = self.last_kernel_times()
+        names, off, ts, te = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        self._chk(self.lib.hm_decode_bam_names(self.h, C.byref(names), C.byref(off), C.byref(ts), C.byref(te), C.byref(n)))
+        nr = int(n.value)
+        view = lambda p, dt: np.ctypeslib.as_array(C.cast(p, C.POINTER(dt)), (nr,)) if nr else np.zeros(0, dt)
+        ids = reader.intern_qnames(names.value or 0, view(off, C.c_uint64), nr)
+        self._chk(self.lib.hm_decode_bam_end(self.h, _p(ids)))
+        return DecodedRegion(view(ts, C.c_int32).copy(), view(te, C.c_int32).copy())
+
+    def read_back(self):
+        """diagnostics (tests): the resident batch as an abi.ReadBatch without seq (mapq, qname_id, qualities, ops
+        included; flags as uploaded by a decoder: 0)"""
+        s = abi.hm_read_batch()
+        self._chk(self.lib.hm_batch_read_back(self.h, C.byref(s), *([None] * 11)))
+        n, nbq, nops = int(s.n_reads), int(s.bq_bytes), int(s.n_ops_total)
+        a = dict(tstart=np.zeros(n, np.int32), tend=np.zeros(n, np.int32), qstart=np.zeros(n, np.int32), qlen=np.zeros(n, np.int32),
+                 mapq=np.zeros(n, np.uint8), qname_id=np.zeros(n, np.uint32), bq_off=np.zeros(n, np.uint64), op_off=np.zeros(n, np.uint64),
+                 n_ops=np.zeros(n, np.uint32), bq=np.zeros(nbq, np.uint8), ops=np.zeros(nops, np.uint32))
+        order = ("tstart", "tend", "qstart", "qlen", "mapq", "qname_id", "bq_off", "op_off", "n_ops", "bq", "ops")
+        self._chk(self.lib.hm_batch_read_back(self.h, C.byref(s), *[_p(a[k]) for k in order]))
+        return abi.ReadBatch(flags=np.zeros(n, np.uint8), seq_off=np.zeros(0, np.uint64), seq=np.zeros(0, np.uint8), **a)
+
+    def inflate_test(self, comp, n, crc):
+        """tests: the device decoder of k_bgzf_inflate on one raw DEFLATE stream -> (rc, bytes)"""
+        out = np.zeros(max(n, 1), np.uint8)
+        rc = self.lib.hm_inflate_device_test(self.h, bytes(comp), len(comp), _p(out), n, crc & 0xffffffff)
+        if rc == abi.HM_ERR_CUDA:
+            self._chk(rc)
+        return rc, out[:n].tobytes()
 
     def upload_wait(self):
         """the copies of the last upload_compact(..., wait=False) are done: its arrays may be reused"""

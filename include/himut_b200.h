@@ -121,6 +121,24 @@ typedef struct hm_bq_compact {
  * smallest file-order index range that contains every record pysam's
  * fetch(chrom, start, end) would return; the library re-applies the overlap rule
  * tstart < end && tend > start inside the range.                                           */
+/* A BAM region planned for the device decoder (hm_bam_region_plan of himut_io.h fills it, hm_decode_bam_begin reads
+ * it): whole BGZF blocks of the file and the points of their inflated stream where a record is known to start.
+ * Offsets into the inflated stream count from the first block of the range.  Valid until the next plan of the handle. */
+typedef struct hm_bgzf_plan {
+  const uint8_t* comp;        /* the compressed range (n_blocks whole BGZF blocks)                         */
+  uint64_t comp_bytes;
+  uint64_t n_blocks;
+  const uint64_t* blk_coff;   /* n_blocks + 1: offset of each block in comp (last: comp_bytes)             */
+  const uint32_t* blk_csize;  /* whole block size (BSIZE + 1)                                              */
+  const uint32_t* blk_isize;  /* ISIZE of the footer                                                       */
+  const uint64_t* blk_uoff;   /* n_blocks + 1: offset of the block's payload in the inflated stream        */
+  const uint32_t* blk_crc;    /* CRC32 of the footer                                                       */
+  const uint64_t* entry;      /* ascending inflated offsets of record starts (BAI linear index entries)    */
+  uint64_t n_entry;           /* 0: nothing to decode                                                      */
+  uint64_t walk_end;          /* records are walked up to this inflated offset                             */
+  const char* path;           /* the BAM file, for messages                                                */
+} hm_bgzf_plan;
+
 typedef struct hm_chunk {
   int32_t start;
   int32_t end;
@@ -376,6 +394,30 @@ int hm_read_stats(hm_ctx* ctx, int64_t* bq_total, int32_t* n_match, int32_t* n_s
  * events): total device milliseconds and the number of own kernels the call launched (fused `call` path: counted
  * launch by launch; elsewhere: the number of timed kernel groups).  names/ms give per-kernel
  * figures for up to `cap` kernels; returns how many were written in *n.                    */
+/* Device BAM decoder: a region planned on the host (hm_bgzf_plan, hm_bam_region_plan of himut_io.h) becomes the
+ * resident batch of `call` (no base stream) without being inflated on the host.  In two halves, so that a worker
+ * can decode the next group on one context while the kernels of the current one run on another:
+ *   hm_decode_bam_begin copies the compressed range up (cudaMemcpyAsync), inflates every BGZF block (CRC32 and
+ *   ISIZE checked), walks the records from the entry points, selects and parses them with hm_bam_read_batch's rules
+ *   (file order, same messages for rejected input: HM_ERR_ARG) and brings back the query names and the per-read
+ *   coordinates; *n_reads = the batch's reads.  `end` is clamped to the contig by the caller.
+ *   hm_decode_bam_names: views of those host arrays (valid until the next begin): NUL-terminated names at
+ *   names + name_off[i], tstart / tend per read.
+ *   hm_decode_bam_end takes the query-name ids (interned by the BAM handle: hm_bam_intern_qnames) and makes the batch
+ *   resident; afterwards every call behaves as after hm_upload_batch of hm_bam_read_batch's batch without seq. */
+int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint64_t* n_reads);
+int hm_decode_bam_names(hm_ctx* ctx, const char** names, const uint64_t** name_off, const int32_t** tstart,
+                        const int32_t** tend, uint64_t* n_reads);
+int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id);
+
+/* diagnostics (tests): the resident batch back into caller buffers (any may be NULL); *out gets n_reads, bq_bytes and
+ * n_ops_total, which size them */
+int hm_batch_read_back(hm_ctx* ctx, hm_read_batch* out, int32_t* tstart, int32_t* tend, int32_t* qstart, int32_t* qlen,
+                       uint8_t* mapq, uint32_t* qname_id, uint64_t* bq_off, uint64_t* op_off, uint32_t* n_ops, uint8_t* bq,
+                       uint32_t* ops);
+/* tests: the device inflate of one raw DEFLATE stream (exactly out_len bytes, CRC32 crc); 0 ok, else an error code */
+int hm_inflate_device_test(hm_ctx* ctx, const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len, uint32_t crc);
+
 int hm_last_timing(hm_ctx* ctx, float* total_ms, int* n_launches);
 /* which device path the last hm_call_chunks took: 2 the fused one (one pass over the quality stream, no library
  * sort, one synchronisation), 1 the first version (chunk spans of 2^28 positions and more, or HIMUT_B200_CALL_V1 set),

@@ -83,6 +83,17 @@ int hm_bq_compact_build(const hm_read_batch* b, int threads, uint8_t* mask, uint
                         uint64_t* exc_bytes, uint8_t* modal_out);
 void hm_bq_compact_free(uint8_t* exc);
 
+/* plan of the records hm_bam_read_batch would visit for [start, end) of contig `rid`, for the device decoder
+ * (hm_decode_bam_begin of himut_b200.h): nothing is inflated.  The range starts at the BAI linear-index entry
+ * hm_bam_read_batch seeks to and ends at the largest chunk end of the BAI bins that overlap the region; the entry
+ * points are the linear-index entries of the windows the region covers.  Without a BAI: one entry point at the first
+ * record and the range runs to the end of the file.  An empty contig gives n_entry = 0.  The arrays (and the
+ * compressed range, when the file is not mapped) belong to the handle until its next plan. */
+int hm_bam_region_plan(hm_bam* b, int rid, int32_t start, int32_t end, hm_bgzf_plan* out);
+/* the ids of `n` NUL-terminated names (name i at blob + off[i]) in the handle's query-name table: the ids
+ * hm_bam_read_batch gives the same names */
+int hm_bam_intern_qnames(hm_bam* b, const char* blob, const uint64_t* off, size_t n, uint32_t* ids);
+
 /* query names are interned per handle: qname_id of a batch indexes this table, ids are stable
  * across hm_bam_read_batch calls (m.num_ccs counts distinct names per contig, caller.py:318-320) */
 uint32_t hm_bam_n_qnames(const hm_bam* b);
