@@ -92,13 +92,8 @@ def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_nam
     kept, laters = [], []
     starts = [s for _, s, _e in chunkloci_lst]
     groups = worker.group_chunks(chunkloci_lst)
-    if decode != "host" and not (hasattr(ctx, "decode_region") and src.reader.has_index):
-        decode = "host"
-    if decode == "auto" and not starts:
-        decode = "host"
-    if decode == "auto":
-        lo, hi = min(starts), max(e for _, _s, e in chunkloci_lst) + (1 if phase else 0)
-        decode = "device" if src.reader.plan(chrom, lo, hi).comp_bytes >= DEVICE_DECODE_MIN_BYTES * len(groups) else "host"
+    lo, hi = (min(starts), max(e for _, _s, e in chunkloci_lst) + (1 if phase else 0)) if starts else (None, None)
+    decode = worker.choose_decode(decode, ctx, src.reader, chrom, lo, hi, len(groups), DEVICE_DECODE_MIN_BYTES)
     ctxs = [ctx] if (ctx2 is None or len(groups) == 1 or not hasattr(ctx, "call_chunks_submit")) else [ctx, ctx2]
     pins = worker.PinCache(ctx, enabled=len(groups) > 1)
     # `call` never needs the read bases as a stream: substituted bases are in the ops, and under a cs match the read

@@ -1,11 +1,12 @@
-// bamgpu.cuh — a BAM region decoded on the device, from the compressed BGZF blocks to the resident batch of `call`
-// (no base stream, one quality byte per base).  The rules are hm_bam_read_batch's (csrc/bamdec.c), which stays the
-// reference the tests compare against; the messages come from the same table (bamerr.h).
+// bamgpu.cuh — a BAM region decoded on the device, from the compressed BGZF blocks to a resident batch with one
+// quality byte per base: without a base stream for `call` and the phase edges, with the 2-bit base stream for
+// normcounts.  The rules are hm_bam_read_batch's (csrc/bamdec.c), which stays the reference the tests compare against;
+// the messages come from the same table (bamerr.h).
 //
 //   k_bgzf_inflate   one thread per BGZF block: raw DEFLATE (stored, fixed, dynamic), ISIZE and CRC32 checked
 //   k_bam_walk       one thread per entry point (BAI linear-index entry): follows block_size to the next one
 //   k_bam_select     one thread per record: hm_bam_read_batch's selection and checks, counts for the output scans
-//   k_bam_parse      one warp per selected record: qualities, cs -> ops, coordinates, the query name
+//   k_bam_parse      one warp per selected record: qualities, 2-bit bases (if asked), cs -> ops, coordinates, the name
 //
 // Shape of k_bgzf_inflate: a BGZF block is an independent stream of at most 64 KB whose decode is one serial chain
 // (each symbol's length is known only once it is decoded), so one thread decodes one block, and it is the only
@@ -267,7 +268,8 @@ __global__ void k_bam_walk(const uint8_t* buf, const uint64_t* entry, uint64_t n
 }
 
 // ------------------------------------------------------------------------------------------ k_bam_select
-// counts per record for the exclusive scans: [0] selected, [1] ops, [2] quality bytes (16-byte padded), [3] name bytes
+// counts per record for the exclusive scans: [0] selected, [1] ops, [2] quality bytes (16-byte padded), [3] name bytes,
+// and with the base stream (n_cnt 5) [4] its bytes, ceil(l_seq / 4) padded to 16 as the host decoder lays them out
 __device__ __forceinline__ void sel_fail(Err* err, uint8_t* code, long long* arg, uint64_t r, int c, long long a) {
   code[r] = (uint8_t)c;
   arg[r] = a;
@@ -300,14 +302,14 @@ __device__ uint32_t cs_count(const char* c) {
 }
 
 __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n_rec, uint64_t walk_end, int32_t rid,
-                             int32_t start, int32_t end, RecInfo* info, unsigned long long* cnt4, uint8_t* code,
+                             int32_t start, int32_t end, RecInfo* info, unsigned long long* cnt, int n_cnt, uint8_t* code,
                              long long* arg, Err* err) {
   const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const uint64_t stride = n_rec + 1;  // cnt4: four arrays of n_rec + 1 (the last entry 0: the scan's total)
-  if (r == 0) cnt4[n_rec] = cnt4[stride + n_rec] = cnt4[2 * stride + n_rec] = cnt4[3 * stride + n_rec] = 0;
+  const uint64_t stride = n_rec + 1;  // cnt: n_cnt (4 or 5) arrays of n_rec + 1 (the last entry 0: the scan's total)
+  if (r == 0)
+    for (int k = 0; k < n_cnt; k++) cnt[k * stride + n_rec] = 0;
   if (r >= n_rec) return;
-  unsigned long long* c4[4] = {cnt4 + r, cnt4 + stride + r, cnt4 + 2 * stride + r, cnt4 + 3 * stride + r};
-  *c4[0] = *c4[1] = *c4[2] = *c4[3] = 0;
+  for (int k = 0; k < n_cnt; k++) cnt[k * stride + r] = 0;
   RecInfo I;
   I.keep = 0;
   I.p = rec[r];
@@ -375,10 +377,11 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
   I.pos = pos; I.l_seq = l_seq; I.lead = lead; I.trail = trail; I.ref_span = ref_span;
   I.n_ops = cs_count((const char*)cs);
   info[r] = I;
-  *c4[0] = 1;
-  *c4[1] = I.n_ops;
-  *c4[2] = ((uint64_t)l_seq + 15) & ~(uint64_t)15;
-  *c4[3] = l_name;
+  cnt[r] = 1;
+  cnt[stride + r] = I.n_ops;
+  cnt[2 * stride + r] = ((uint64_t)l_seq + 15) & ~(uint64_t)15;
+  cnt[3 * stride + r] = l_name;
+  if (n_cnt == 5) cnt[4 * stride + r] = (((uint64_t)l_seq + 3) / 4 + 15) & ~(uint64_t)15;
 }
 
 // ------------------------------------------------------------------------------------------ k_bam_parse
@@ -390,6 +393,8 @@ struct ParseOut {
   uint8_t* bq;
   uint32_t* ops;
   char* names;
+  uint64_t* seq_off;  // both nullptr: no base stream (the batch of `call` and the phase edges)
+  uint8_t* seq;
 };
 
 // the code of read base q (A0 T1 G2 C3, 0xff anything else)
@@ -402,18 +407,22 @@ __device__ __forceinline__ int base_code(char c) {
   switch (c) { case 'A': case 'a': return 0; case 'T': case 't': return 1; case 'G': case 'g': return 2; case 'C': case 'c': return 3; default: return -1; }
 }
 
+// 2-bit code of each BAM nibble at bits 2 * nibble: A (1) 0, C (2) 3, G (4) 2, T (8) 1; N, IUPAC codes and '=' 0, as
+// the host decoder's pack_codes_* store them
+constexpr uint32_t kNibBits = (3u << 2 * 2) | (2u << 2 * 4) | (1u << 2 * 8);
+
 // Every lane of the warp walks the cs string (the same bytes: broadcast loads, no divergence); checks over a run of
-// read bases are split over the lanes, and lane 0 writes the ops.  scan4: exclusive prefix sums of k_bam_select's
-// four counts (stride apart) = the record's read index and its first op, quality byte and name byte.  n_rec: the
-// records before the one that ends the region.
-__global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_rec, const unsigned long long* scan4,
+// read bases are split over the lanes, and lane 0 writes the ops.  scan: exclusive prefix sums of k_bam_select's
+// counts (stride apart) = the record's read index and its first op, quality byte, name byte and (o.seq) base byte.
+// n_rec: the records before the one that ends the region.
+__global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_rec, const unsigned long long* scan,
                             uint64_t stride, ParseOut o, uint8_t* code, long long* arg, Err* err) {
   const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (r >= n_rec) return;
   const RecInfo I = info[r];
   if (!I.keep) return;
-  const uint64_t rd = scan4[r], op0 = scan4[stride + r], bq0 = scan4[2 * stride + r], nm0 = scan4[3 * stride + r];
+  const uint64_t rd = scan[r], op0 = scan[stride + r], bq0 = scan[2 * stride + r], nm0 = scan[3 * stride + r];
   const uint8_t* R = buf + I.p + 4;
   const uint32_t l_name = R[8], n_cig = R[12] | (R[13] << 8);
   const int32_t l_seq = I.l_seq;
@@ -422,6 +431,21 @@ __global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_
   const uint64_t qb16 = ((uint64_t)l_seq + 15) & ~(uint64_t)15;
   for (uint64_t k = lane; k < qb16; k += 32) o.bq[bq0 + k] = k < (uint64_t)l_seq ? qual[k] : 0;
   for (uint32_t k = lane; k < l_name; k += 32) o.names[nm0 + k] = (char)R[32 + k];
+  const uint64_t sq0 = o.seq ? scan[4 * stride + r] : 0;
+  if (o.seq) {  // a lane packs 16 bases (8 nibble bytes) into one aligned word: base 16 w + j at bits 2 j of word w
+    const uint64_t n_words = ((((uint64_t)l_seq + 3) / 4 + 15) & ~(uint64_t)15) / 4;  // the padding words are zero
+    uint32_t* dst = (uint32_t*)(o.seq + sq0);
+    for (uint64_t w = lane; w < n_words; w += 32) {
+      const int64_t b0 = 16 * (int64_t)w, nb = min((int64_t)16, (int64_t)l_seq - b0);
+      uint32_t v = 0;
+      for (int64_t j = 0; j < nb; j += 2) {  // the high nibble is the even base
+        const uint32_t by = seq4[(b0 + j) >> 1];
+        v |= ((kNibBits >> 2 * (by >> 4)) & 3u) << 2 * j;
+        if (j + 1 < nb) v |= ((kNibBits >> 2 * (by & 15)) & 3u) << 2 * (j + 1);
+      }
+      dst[w] = v;
+    }
+  }
   const char* cs = (const char*)(R + I.cs);
   const char* c = cs;
   uint32_t* ops = o.ops + op0;
@@ -499,6 +523,7 @@ __global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_
   o.bq_off[rd] = bq0;
   o.op_off[rd] = op0;
   o.name_off[rd] = nm0;
+  if (o.seq) o.seq_off[rd] = sq0;
 }
 
 }  // namespace bamgpu

@@ -157,14 +157,14 @@ struct hm_ctx {
   uint32_t modal = 0;
   // device BAM decoder (hm_decode_bam_*, bamgpu.cuh)
   DevBuf b_comp, b_pcoff, b_pcsize, b_pisize, b_puoff, b_pcrc, b_pentry, b_inflated, b_blk_code, b_derr, b_seg_cnt,
-      b_seg_off, b_recoff, b_recinfo, b_cnt4, b_scan4, b_ecode, b_earg, b_names, b_name_off;
+      b_seg_off, b_recoff, b_recinfo, b_cnt, b_scan, b_ecode, b_earg, b_names, b_name_off;
   PinVec<int32_t> hd_tstart, hd_tend, hd_qstart, hd_qlen;   // per-read arrays of the last hm_decode_bam_begin
   PinVec<uint32_t> hd_n_ops;
-  PinVec<uint64_t> hd_bq_off, hd_op_off, hd_name_off, hd_scal; // hd_scal: walk / scan totals read back
+  PinVec<uint64_t> hd_bq_off, hd_op_off, hd_name_off, hd_seq_off, hd_scal; // hd_scal: walk / scan totals read back
   PinVec<char> hd_names;
   PinVec<bamgpu::Err> hd_err;
   std::vector<uint8_t> hd_flags;
-  uint64_t dec_n = 0, dec_ops = 0, dec_bq = 0;
+  uint64_t dec_n = 0, dec_ops = 0, dec_bq = 0, dec_seq = 0;  // dec_seq: base-stream bytes (0: decoded without it)
   bool dec_ready = false;                   // hm_decode_bam_begin succeeded, hm_decode_bam_end has not run
 };
 
@@ -398,15 +398,15 @@ void hm_destroy(hm_ctx* ctx) {
                     &ctx->b_cgeom, &ctx->b_seg_keys, &ctx->b_seg_read, &ctx->b_keys_tmp, &ctx->b_gscratch, &ctx->b_czero, &ctx->b_first_pair, &ctx->b_tiles, &ctx->b_site_valid, &ctx->b_pair_c,
                     &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_exp_total, &ctx->b_sdiff, &ctx->b_cal_ok,
                     &ctx->b_comp, &ctx->b_pcoff, &ctx->b_pcsize, &ctx->b_pisize, &ctx->b_puoff, &ctx->b_pcrc, &ctx->b_pentry, &ctx->b_inflated,
-                    &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt4,
-                    &ctx->b_scan4, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off};
+                    &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt,
+                    &ctx->b_scan, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off};
   for (DevBuf* b : bufs) b->release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_cnt_pin) cudaFreeHost(ctx->h_cnt_pin);
   if (ctx->h_geom_pin) cudaFreeHost(ctx->h_geom_pin);
   ctx->h_pmax.release(); ctx->h_tix_off.release(); ctx->h_cw_off.release();
   ctx->hd_tstart.release(); ctx->hd_tend.release(); ctx->hd_qstart.release(); ctx->hd_qlen.release(); ctx->hd_n_ops.release();
-  ctx->hd_bq_off.release(); ctx->hd_op_off.release(); ctx->hd_name_off.release(); ctx->hd_scal.release(); ctx->hd_names.release();
+  ctx->hd_bq_off.release(); ctx->hd_op_off.release(); ctx->hd_name_off.release(); ctx->hd_seq_off.release(); ctx->hd_scal.release(); ctx->hd_names.release();
   ctx->hd_err.release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -700,11 +700,13 @@ static int decode_record_error(hm_ctx* ctx, const hm_bgzf_plan* pl, unsigned lon
   return fail(ctx, HM_ERR_ARG, REC_ERR[code], name, (long)arg);
 }
 
-static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32_t start, int32_t end, uint64_t* n_reads) {
+static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32_t start, int32_t end, bool want_seq,
+                             uint64_t* n_reads) {
   using namespace bamgpu;
   const uint64_t nb = pl->n_blocks, ne = pl->n_entry;
   ctx->dec_n = ctx->dec_ops = 0;
   ctx->dec_bq = 16;
+  ctx->dec_seq = want_seq ? 16 : 0;  // the host decoder's empty batch: 16 zero bytes of each stream it has
   if (nb == 0 || ne == 0) return HM_OK;
   // the plan comes from outside: every offset the kernels follow is checked here
   if (!pl->comp || !pl->blk_coff || !pl->blk_csize || !pl->blk_isize || !pl->blk_uoff || !pl->blk_crc || !pl->entry)
@@ -734,7 +736,7 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   CU(ctx->b_blk_code.ensure(nb));
   CU(ctx->b_derr.ensure(sizeof(Err)));
   CU(cudaMemsetAsync(ctx->b_derr.p, 0xff, sizeof(Err), ctx->stream));
-  if (!ctx->hd_err.resize(1) || !ctx->hd_scal.resize(4)) return fail(ctx, HM_ERR_ARG, "out of page-locked host memory");
+  if (!ctx->hd_err.resize(1) || !ctx->hd_scal.resize(5)) return fail(ctx, HM_ERR_ARG, "out of page-locked host memory");
   Err* derr = ctx->b_derr.as<Err>();
   Err& herr = ctx->hd_err[0];
   // inflate: one block per warp (bamgpu.cuh says why)
@@ -778,14 +780,15 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   CU(cudaGetLastError());
   // select and count
   const uint64_t stride = n_rec + 1;
+  const int n_cnt = want_seq ? 5 : 4;
   CU(ctx->b_recinfo.ensure(n_rec * sizeof(RecInfo)));
-  CU(ctx->b_cnt4.ensure(4 * stride * 8));
-  CU(ctx->b_scan4.ensure(4 * stride * 8));
+  CU(ctx->b_cnt.ensure(n_cnt * stride * 8));
+  CU(ctx->b_scan.ensure(n_cnt * stride * 8));
   CU(ctx->b_ecode.ensure(n_rec));
   CU(ctx->b_earg.ensure(n_rec * 8));
   t_begin(ctx, "k_bam_select");
   k_bam_select<<<(unsigned)((n_rec + 127) / 128), 128, 0, ctx->stream>>>(buf, ctx->b_recoff.as<uint64_t>(), n_rec, pl->walk_end, rid, start, end,
-                                                                          ctx->b_recinfo.as<RecInfo>(), ctx->b_cnt4.as<unsigned long long>(),
+                                                                          ctx->b_recinfo.as<RecInfo>(), ctx->b_cnt.as<unsigned long long>(), n_cnt,
                                                                           ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
   t_end(ctx);
   CU(cudaGetLastError());
@@ -794,42 +797,46 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   const uint64_t stop = std::min<uint64_t>(herr.stop, n_rec);  // records from here on are never looked at by the host
   if (herr.rec < stop) return decode_record_error(ctx, pl, herr.rec);
   if (stop == 0) return HM_OK;
-  // output offsets: exclusive scans of the four counts (read index, first op, first quality byte, first name byte)
-  unsigned long long* cnt4 = ctx->b_cnt4.as<unsigned long long>();
-  unsigned long long* scan4 = ctx->b_scan4.as<unsigned long long>();
+  // output offsets: exclusive scans of the counts (read index, first op, first quality byte, first name byte, and with
+  // the base stream its first byte)
+  unsigned long long* cnt = ctx->b_cnt.as<unsigned long long>();
+  unsigned long long* scan = ctx->b_scan.as<unsigned long long>();
   tmp = 0;
-  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt4, scan4, (int)stride, ctx->stream));
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, scan, (int)stride, ctx->stream));
   CU(ctx->b_cub.ensure(tmp));
   t_begin(ctx, "cub_scan_records");
-  for (int k = 0; k < 4; k++) CU(cub::DeviceScan::ExclusiveSum(ctx->b_cub.p, tmp, cnt4 + k * stride, scan4 + k * stride, (int)stride, ctx->stream));
+  for (int k = 0; k < n_cnt; k++) CU(cub::DeviceScan::ExclusiveSum(ctx->b_cub.p, tmp, cnt + k * stride, scan + k * stride, (int)stride, ctx->stream));
   t_end(ctx);
-  for (int k = 0; k < 4; k++) CU(cudaMemcpyAsync(&ctx->hd_scal[k], scan4 + k * stride + stop, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  for (int k = 0; k < n_cnt; k++) CU(cudaMemcpyAsync(&ctx->hd_scal[k], scan + k * stride + stop, 8, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   const uint64_t n = ctx->hd_scal[0], n_ops = ctx->hd_scal[1], n_bq = ctx->hd_scal[2], n_nm = ctx->hd_scal[3];
+  const uint64_t n_seq = want_seq ? ctx->hd_scal[4] : 0;
   // the resident batch's buffers, written in place
   CU(ctx->b_tstart.ensure(n * 4 + 16)); CU(ctx->b_tend.ensure(n * 4 + 16)); CU(ctx->b_qstart.ensure(n * 4 + 16));
   CU(ctx->b_qlen.ensure(n * 4 + 16)); CU(ctx->b_mapq.ensure(n + 16)); CU(ctx->b_flags.ensure(n + 16)); CU(ctx->b_qname.ensure(n * 4 + 16));
   CU(ctx->b_n_ops.ensure(n * 4 + 16)); CU(ctx->b_bq_off.ensure(n * 8 + 16)); CU(ctx->b_op_off.ensure(n * 8 + 16));
   CU(ctx->b_bq.ensure(n_bq + 32)); CU(ctx->b_ops.ensure(n_ops * 4 + 16)); CU(ctx->b_names.ensure(n_nm + 16));
   CU(ctx->b_name_off.ensure(n * 8 + 16));
+  if (want_seq) { CU(ctx->b_seq.ensure(n_seq + 32)); CU(ctx->b_seq_off.ensure(n * 8 + 16)); }
   ParseOut o{ctx->b_tstart.as<int32_t>(), ctx->b_tend.as<int32_t>(), ctx->b_qstart.as<int32_t>(), ctx->b_qlen.as<int32_t>(),
              ctx->b_mapq.as<uint8_t>(), ctx->b_flags.as<uint8_t>(), ctx->b_n_ops.as<uint32_t>(), ctx->b_bq_off.as<uint64_t>(),
              ctx->b_op_off.as<uint64_t>(), ctx->b_name_off.as<uint64_t>(), ctx->b_bq.as<uint8_t>(), ctx->b_ops.as<uint32_t>(),
-             ctx->b_names.as<char>()};
+             ctx->b_names.as<char>(), want_seq ? ctx->b_seq_off.as<uint64_t>() : nullptr, want_seq ? ctx->b_seq.as<uint8_t>() : nullptr};
   t_begin(ctx, "k_bam_parse");
-  k_bam_parse<<<(unsigned)((stop * 32 + 255) / 256), 256, 0, ctx->stream>>>(buf, ctx->b_recinfo.as<RecInfo>(), stop, scan4, stride, o,
+  k_bam_parse<<<(unsigned)((stop * 32 + 255) / 256), 256, 0, ctx->stream>>>(buf, ctx->b_recinfo.as<RecInfo>(), stop, scan, stride, o,
                                                                              ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
   t_end(ctx);
   CU(cudaGetLastError());
   if (!ctx->hd_tstart.resize(n) || !ctx->hd_tend.resize(n) || !ctx->hd_qstart.resize(n) || !ctx->hd_qlen.resize(n) ||
       !ctx->hd_n_ops.resize(n) || !ctx->hd_bq_off.resize(n) || !ctx->hd_op_off.resize(n) || !ctx->hd_name_off.resize(n) ||
-      !ctx->hd_names.resize(n_nm + 1))
+      !ctx->hd_names.resize(n_nm + 1) || (want_seq && !ctx->hd_seq_off.resize(n)))
     return fail(ctx, HM_ERR_ARG, "out of page-locked host memory for %llu reads", (unsigned long long)n);
   t_begin(ctx, "d2h_reads_names");
 #define DOWN(h, d, bytes) CU(cudaMemcpyAsync(ctx->h.data(), ctx->d.p, (bytes), cudaMemcpyDeviceToHost, ctx->stream))
   DOWN(hd_tstart, b_tstart, n * 4); DOWN(hd_tend, b_tend, n * 4); DOWN(hd_qstart, b_qstart, n * 4); DOWN(hd_qlen, b_qlen, n * 4);
   DOWN(hd_n_ops, b_n_ops, n * 4); DOWN(hd_bq_off, b_bq_off, n * 8); DOWN(hd_op_off, b_op_off, n * 8);
   DOWN(hd_name_off, b_name_off, n * 8); DOWN(hd_names, b_names, n_nm);
+  if (want_seq) DOWN(hd_seq_off, b_seq_off, n * 8);
 #undef DOWN
   t_end(ctx);
   CU(cudaMemcpyAsync(&herr, derr, sizeof(Err), cudaMemcpyDeviceToHost, ctx->stream));
@@ -838,6 +845,7 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   ctx->dec_n = n;
   ctx->dec_ops = n_ops;
   ctx->dec_bq = n_bq ? n_bq : 16;
+  if (want_seq) ctx->dec_seq = n_seq ? n_seq : 16;
   *n_reads = n;
   return HM_OK;
 }
@@ -1688,8 +1696,14 @@ int hm_last_kernel_times(hm_ctx* ctx, const char** names, float* ms, size_t cap,
 }
 
 int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint64_t* n_reads) {
+  return hm_decode_bam_begin_opts(ctx, plan, rid, start, end, 0, n_reads);
+}
+
+int hm_decode_bam_begin_opts(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint32_t opts,
+                             uint64_t* n_reads) {
   if (!ctx || !plan || !n_reads) return HM_ERR_ARG;
   *n_reads = 0;
+  if (opts & ~HM_DECODE_SEQ) return fail(ctx, HM_ERR_ARG, "unknown decode option bits 0x%x", opts & ~HM_DECODE_SEQ);
   CU(cudaSetDevice(ctx->device));
   if (ctx->upload_pending) { // the copies of an upload that was not waited for still read their host buffers
     CU(cudaEventSynchronize(ctx->ev_up));
@@ -1699,7 +1713,7 @@ int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t 
   ctx->dec_ready = false;
   t_reset(ctx);
   if (start < 0) start = 0;
-  const int rc = decode_begin_impl(ctx, plan, rid, start, end, n_reads);
+  const int rc = decode_begin_impl(ctx, plan, rid, start, end, (opts & HM_DECODE_SEQ) != 0, n_reads);
   if (rc) { cudaStreamSynchronize(ctx->stream); return rc; }
   t_collect(ctx);
   ctx->dec_ready = true;
@@ -1724,24 +1738,31 @@ int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id) {
   CU(cudaSetDevice(ctx->device));
   ctx->dec_ready = false;
   ctx->hd_flags.assign(n, 0);
+  const bool has_seq = ctx->dec_seq != 0;
   hm_read_batch b;
   memset(&b, 0, sizeof(b));
   b.n_reads = n;
   b.tstart = ctx->hd_tstart.data(); b.tend = ctx->hd_tend.data(); b.qstart = ctx->hd_qstart.data(); b.qlen = ctx->hd_qlen.data();
   b.flags = ctx->hd_flags.data(); b.qname_id = qname_id; b.bq_off = ctx->hd_bq_off.data(); b.op_off = ctx->hd_op_off.data();
   b.n_ops = ctx->hd_n_ops.data(); b.bq_bytes = ctx->dec_bq; b.n_ops_total = ctx->dec_ops;
+  if (has_seq) { b.seq_off = ctx->hd_seq_off.data(); b.seq_bytes = ctx->dec_seq; }  // b.seq stays NULL: the stream is on the device
   int rc;
-  if ((rc = batch_tables(ctx, &b, nullptr, false))) return rc;
-  if (n == 0) { // the host decoder's empty batch: 16 zero quality bytes
+  if ((rc = batch_tables(ctx, &b, nullptr, has_seq))) return rc;
+  if (n == 0) { // the host decoder's empty batch: 16 zero quality bytes (and 16 zero base bytes with the base stream)
     CU(ctx->b_bq.ensure(32));
     CU(cudaMemsetAsync(ctx->b_bq.p, 0, 16, ctx->stream));
     CU(ctx->b_ops.ensure(16));
     for (DevBuf* d : {&ctx->b_tstart, &ctx->b_tend, &ctx->b_qstart, &ctx->b_qlen, &ctx->b_mapq, &ctx->b_flags, &ctx->b_qname,
                       &ctx->b_n_ops, &ctx->b_bq_off, &ctx->b_op_off})
       CU(d->ensure(16));
+    if (has_seq) {
+      CU(ctx->b_seq.ensure(32));
+      CU(cudaMemsetAsync(ctx->b_seq.p, 0, 16, ctx->stream));
+      CU(ctx->b_seq_off.ensure(16));
+    }
   }
   if ((rc = upload(ctx, ctx->b_qname, qname_id, n))) return rc;
-  if ((rc = bind_batch(ctx, &b, false))) return rc;
+  if ((rc = bind_batch(ctx, &b, has_seq))) return rc;
   ctx->compact_resident = false;
   CU(cudaStreamSynchronize(ctx->stream));
   ctx->have_batch = true;
@@ -1764,6 +1785,20 @@ int hm_batch_read_back(hm_ctx* ctx, hm_read_batch* out, int32_t* tstart, int32_t
       {n_ops, &ctx->b_n_ops, n * 4}, {bq, &ctx->b_bq, ctx->bq_bytes}, {ops, &ctx->b_ops, ctx->n_ops_total * 4}};
   for (const auto& c : cp)
     if (c.dst && c.bytes) CU(cudaMemcpyAsync(c.dst, c.src->p, c.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  return HM_OK;
+}
+
+/* diagnostics (tests): the resident base stream back to caller buffers (NULL: skip): n_reads offsets, *seq_bytes bytes;
+ * *seq_bytes = 0 when the resident batch has no base stream */
+int hm_batch_read_back_seq(hm_ctx* ctx, uint64_t* seq_off, uint8_t* seq, uint64_t* seq_bytes) {
+  if (!ctx || !seq_bytes) return HM_ERR_ARG;
+  if (!ctx->have_batch) return fail(ctx, HM_ERR_STATE, "no resident batch");
+  *seq_bytes = ctx->db.seq ? ctx->seq_bytes : 0;
+  if (!ctx->db.seq) return HM_OK;
+  CU(cudaSetDevice(ctx->device));
+  if (seq_off && ctx->n_reads) CU(cudaMemcpyAsync(seq_off, ctx->b_seq_off.p, ctx->n_reads * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (seq) CU(cudaMemcpyAsync(seq, ctx->b_seq.p, ctx->seq_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return HM_OK;
 }

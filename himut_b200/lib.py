@@ -22,6 +22,7 @@ EXPORTS = [
     "hm_host_unregister", "hm_abi_sizeof", "hm_last_records", "hm_qname_seen", "hm_set_reference", "hm_ref_tricounts", "hm_last_norm_exact_sites",
     "hm_phase_edges_begin", "hm_phase_edges_add", "hm_phase_edges_end", "hm_upload_batch_compact", "hm_call_batch_compact", "hm_call_chunks_async", "hm_records_wait", "hm_set_option", "hm_last_call_path", "hm_call_chunks_submit", "hm_call_chunks_collect", "hm_device_count", "hm_upload_batch_compact_begin", "hm_upload_wait",
     "hm_decode_bam_begin", "hm_decode_bam_names", "hm_decode_bam_end", "hm_batch_read_back", "hm_inflate_device_test",
+    "hm_decode_bam_begin_opts", "hm_batch_read_back_seq",
 ]
 
 
@@ -82,9 +83,12 @@ def load():
         lib.hm_host_register.argtypes = [vp, vp, sz]
         lib.hm_host_unregister.argtypes = [vp, vp]
         lib.hm_decode_bam_begin.argtypes = [vp, C.POINTER(abi.hm_bgzf_plan), C.c_int, C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]
+        lib.hm_decode_bam_begin_opts.argtypes = [vp, C.POINTER(abi.hm_bgzf_plan), C.c_int, C.c_int32, C.c_int32, C.c_uint32,
+                                                 C.POINTER(C.c_uint64)]
         lib.hm_decode_bam_names.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_uint64)]
         lib.hm_decode_bam_end.argtypes = [vp, vp]
         lib.hm_batch_read_back.argtypes = [vp, C.POINTER(abi.hm_read_batch)] + [vp] * 11
+        lib.hm_batch_read_back_seq.argtypes = [vp, vp, vp, C.POINTER(C.c_uint64)]
         lib.hm_inflate_device_test.argtypes = [vp, C.c_char_p, sz, vp, sz, C.c_uint32]
         _LIB = lib
     return _LIB
@@ -197,16 +201,20 @@ class Context:
             self._uploading = (batch, cq)  # alive until the copies are done
             self._chk(self.lib.hm_upload_batch_compact_begin(self.h, C.byref(batch.as_struct()), C.byref(cq.struct)))
 
-    def decode_region(self, reader, chrom, start, end):
-        """the records reader.read_batch(chrom, start, end, seq=False) returns, decoded on the device from the
-        compressed file (reader: bamdec.NativeBam) and left resident as upload() would leave that batch.  Query-name
-        ids come from the reader's table.  Rejected input raises pack.BatchFormatError with the host decoder's text.
+    def decode_region(self, reader, chrom, start, end, seq=False):
+        """the records reader.read_batch(chrom, start, end, seq=seq) returns, decoded on the device from the
+        compressed file (reader: bamdec.NativeBam) and left resident as upload() would leave that batch: seq=True
+        with the 2-bit base stream normcounts reads, seq=False without it (`call`, phase edges).  Query-name ids come
+        from the reader's table.  Rejected input raises pack.BatchFormatError with the host decoder's text.
         -> DecodedRegion (n_reads, tstart, tend, chunk_table)"""
         rid = reader.references.index(chrom)
         start, end = int(max(start, 0)), int(min(end, reader.lengths[rid]))
         plan = reader.plan(chrom, start, end)
         n = C.c_uint64(0)
-        rc = self.lib.hm_decode_bam_begin(self.h, C.byref(plan), rid, start, end, C.byref(n))
+        if seq:
+            rc = self.lib.hm_decode_bam_begin_opts(self.h, C.byref(plan), rid, start, end, abi.HM_DECODE_SEQ, C.byref(n))
+        else:
+            rc = self.lib.hm_decode_bam_begin(self.h, C.byref(plan), rid, start, end, C.byref(n))
         if rc == abi.HM_ERR_ARG:
             raise pack.BatchFormatError(self.lib.hm_last_error(self.h).decode())
         self._chk(rc)
@@ -219,9 +227,10 @@ class Context:
         self._chk(self.lib.hm_decode_bam_end(self.h, _p(ids)))
         return DecodedRegion(view(ts, C.c_int32).copy(), view(te, C.c_int32).copy())
 
-    def read_back(self):
-        """diagnostics (tests): the resident batch as an abi.ReadBatch without seq (mapq, qname_id, qualities, ops
-        included; flags as uploaded by a decoder: 0)"""
+    def read_back(self, seq=False):
+        """diagnostics (tests): the resident batch as an abi.ReadBatch (mapq, qname_id, qualities, ops included; flags
+        as uploaded by a decoder: 0); seq=True also brings back seq_off / seq (empty when the batch has no base
+        stream), seq=False leaves them empty"""
         s = abi.hm_read_batch()
         self._chk(self.lib.hm_batch_read_back(self.h, C.byref(s), *([None] * 11)))
         n, nbq, nops = int(s.n_reads), int(s.bq_bytes), int(s.n_ops_total)
@@ -230,7 +239,14 @@ class Context:
                  n_ops=np.zeros(n, np.uint32), bq=np.zeros(nbq, np.uint8), ops=np.zeros(nops, np.uint32))
         order = ("tstart", "tend", "qstart", "qlen", "mapq", "qname_id", "bq_off", "op_off", "n_ops", "bq", "ops")
         self._chk(self.lib.hm_batch_read_back(self.h, C.byref(s), *[_p(a[k]) for k in order]))
-        return abi.ReadBatch(flags=np.zeros(n, np.uint8), seq_off=np.zeros(0, np.uint64), seq=np.zeros(0, np.uint8), **a)
+        seq_off, seq_b = np.zeros(0, np.uint64), np.zeros(0, np.uint8)
+        if seq:
+            nseq = C.c_uint64(0)
+            self._chk(self.lib.hm_batch_read_back_seq(self.h, None, None, C.byref(nseq)))
+            if nseq.value:
+                seq_off, seq_b = np.zeros(n, np.uint64), np.zeros(int(nseq.value), np.uint8)
+                self._chk(self.lib.hm_batch_read_back_seq(self.h, _p(seq_off), _p(seq_b), C.byref(nseq)))
+        return abi.ReadBatch(flags=np.zeros(n, np.uint8), seq_off=seq_off, seq=seq_b, **a)
 
     def inflate_test(self, comp, n, crc):
         """tests: the device decoder of k_bgzf_inflate on one raw DEFLATE stream -> (rc, bytes)"""

@@ -12,6 +12,66 @@ from . import abi, gtmodel, vcfio, worker
 # mutlib.tri_lst (src/himut/mutlib.py:17-50)
 TRI_LST = [a + c + b for a in "ACGT" for c in "CT" for b in "ACGT"]
 
+# compressed BAM bytes per decode group from which normcounts_region(decode="auto") decodes on the device.  The worker
+# is faster on the device decoder at every size measured (profiles/decode_trace_norm_r04.json): 22 ms vs 29 ms on the
+# 1 Mb BAM (15.6 MB, one group), although the decode alone is slower there (15.7 ms vs 8.8 ms), because the host path
+# still uploads the bases and the compact qualities and expands them; smaller groups are not measured and stay on the
+# host decoder.
+DEVICE_DECODE_MIN_BYTES = 14 << 20
+
+
+def normcounts_region(ctx, bam_file, chrom, refseq, chunkloci_lst, chunk_sets, decode="auto"):
+    """the device path of normcounts over a contig's chunk list, decode group by decode group.
+    decode: "device" inflates and parses each group on the GPU from the compressed file with the 2-bit base stream
+    (Context.decode_region(..., seq=True)); "host" decodes with the native host decoder one group ahead of the device;
+    "auto" takes the device decoder when the groups average at least DEVICE_DECODE_MIN_BYTES of compressed BAM.  Either
+    needs a context with the device decoder and a BAM with a BAI; without them the host decoder runs.
+    -> (ccs_tri[33], ref_tri[33], log[14], n_alt_tie, distinct query names that passed the read gates); log[0] is
+    that count"""
+    src = worker.RegionSource(bam_file)
+    tally = worker.QnameTally()
+    ccs = np.zeros(abi.TRI_BINS, np.int64)
+    ref = np.zeros(abi.TRI_BINS, np.int64)
+    log = np.zeros(abi.NORM_LOG_LEN, np.int64)
+    ties = 0
+    groups = worker.group_chunks(chunkloci_lst)
+    lo, hi = (min(s for _, s, _e in chunkloci_lst), max(e for _, _s, e in chunkloci_lst)) if chunkloci_lst else (None, None)
+
+    def add(table):
+        nonlocal ties
+        c, r, l, t = ctx.normcounts_chunks(refseq, table)
+        tally.add(ctx.qname_seen())
+        ccs[:] += c; ref[:] += r; log[:] += l
+        ties += t
+
+    try:
+        decode = worker.choose_decode(decode, ctx, src.reader, chrom, lo, hi, len(groups), DEVICE_DECODE_MIN_BYTES)
+        if decode == "device":
+            for idx in groups:
+                loci = [chunkloci_lst[i] for i in idx]
+                region = ctx.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci), seq=True)
+                if region.n_reads == 0:
+                    continue
+                add(region.chunk_table([(s, e) for _, s, e in loci], None if chunk_sets is None else [chunk_sets[i] for i in idx]))
+        else:
+            pins = worker.PinCache(ctx, enabled=len(groups) > 1)
+            try:
+                # qualities in the decoder's compact form, bases as a stream (the tile kernel reads them), decode one group ahead
+                for _idx, batch, cq, table, release in worker.pipelined_groups(src, chrom, chunkloci_lst, groups, chunk_sets, seq=True):
+                    if batch.n_reads == 0:
+                        release()
+                        continue
+                    pins.pin([cq.mask, cq.exc, batch.ops, batch.seq])
+                    ctx.upload_compact(batch, cq)
+                    release()
+                    add(table)
+            finally:
+                pins.close()
+    finally:
+        src.close()
+    log[0] = tally.count()
+    return ccs, ref, log, ties, int(log[0])
+
 
 def get_callable_tricounts(
     chrom, seq, bam_file, common_snps, panel_of_normals, chunkloci_lst, phase_set2hbit_lst, phase_set2hpos_lst,
@@ -35,31 +95,7 @@ def get_callable_tricounts(
         table, chunk_sets = vcfio.phase_tables(chunkloci_lst, phase_set2hbit_lst, phase_set2hpos_lst, phase_set2hetsnp_lst)
         ctx.set_phase_sets(table)
     refseq = seq.encode() if isinstance(seq, str) else bytes(seq)
-
-    src = worker.RegionSource(bam_file)
-    tally = worker.QnameTally()
-    ccs = np.zeros(abi.TRI_BINS, np.int64)
-    ref = np.zeros(abi.TRI_BINS, np.int64)
-    log = np.zeros(abi.NORM_LOG_LEN, np.int64)
-    ties = 0
-    groups = worker.group_chunks(chunkloci_lst)
-    pins = worker.PinCache(ctx, enabled=len(groups) > 1)
-    try:
-        # qualities in the decoder's compact form, bases as a stream (the tile kernel reads them), decode one group ahead
-        for _idx, batch, cq, table, release in worker.pipelined_groups(src, chrom, chunkloci_lst, groups, chunk_sets, seq=True):
-            if batch.n_reads == 0:
-                release()
-                continue
-            pins.pin([cq.mask, cq.exc, batch.ops, batch.seq])
-            ctx.upload_compact(batch, cq)
-            release()
-            c, r, l, t = ctx.normcounts_chunks(refseq, table)
-            tally.add(ctx.qname_seen())
-            ccs += c; ref += r; log += l; ties += t
-    finally:
-        pins.close()
-    src.close()
-    log[0] = tally.count()
+    ccs, ref, log, ties, _ = normcounts_region(ctx, bam_file, chrom, refseq, chunkloci_lst, chunk_sets)
     ccs_d = {tri: int(ccs[i]) for i, tri in enumerate(TRI_LST)}
     ref_d = {tri: int(ref[i]) for i, tri in enumerate(TRI_LST)}
     if ccs[32] or ref[32]:

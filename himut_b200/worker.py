@@ -69,6 +69,22 @@ def group_chunks(chunkloci_lst, span=None):
     return groups
 
 
+def choose_decode(decode, ctx, reader, chrom, lo, hi, n_groups, min_bytes):
+    """which decoder reads [lo, hi) of chrom in n_groups groups: "device" (Context.decode_region) or "host" (the
+    native host decoder).  "device" needs a context with the device decoder and a BAM with a BAI, else the host
+    decoder runs; "auto" also needs the groups to average at least min_bytes of compressed BAM (below that the host
+    decoder's threads finish first).  lo None: nothing to decode."""
+    if decode not in ("auto", "host", "device"):
+        raise ValueError("decode must be 'auto', 'host' or 'device'")
+    if decode != "host" and not (hasattr(ctx, "decode_region") and reader.has_index):
+        return "host"
+    if decode == "auto":
+        if lo is None:
+            return "host"
+        return "device" if reader.plan(chrom, lo, hi).comp_bytes >= min_bytes * n_groups else "host"
+    return decode
+
+
 class RegionSource:
     """decodes the records a group of chunks fetches into one packed batch"""
 

@@ -394,18 +394,24 @@ int hm_read_stats(hm_ctx* ctx, int64_t* bq_total, int32_t* n_match, int32_t* n_s
  * events): total device milliseconds and the number of own kernels the call launched (fused `call` path: counted
  * launch by launch; elsewhere: the number of timed kernel groups).  names/ms give per-kernel
  * figures for up to `cap` kernels; returns how many were written in *n.                    */
-/* Device BAM decoder: a region planned on the host (hm_bgzf_plan, hm_bam_region_plan of himut_io.h) becomes the
- * resident batch of `call` (no base stream) without being inflated on the host.  In two halves, so that a worker
- * can decode the next group on one context while the kernels of the current one run on another:
+/* Device BAM decoder: a region planned on the host (hm_bgzf_plan, hm_bam_region_plan of himut_io.h) becomes a
+ * resident batch without being inflated on the host: the batch of `call` and the phase edges (no base stream), or with
+ * HM_DECODE_SEQ the batch of normcounts (with the 2-bit base stream).  In two halves, so that a worker can decode the
+ * next group on one context while the kernels of the current one run on another:
  *   hm_decode_bam_begin copies the compressed range up (cudaMemcpyAsync), inflates every BGZF block (CRC32 and
  *   ISIZE checked), walks the records from the entry points, selects and parses them with hm_bam_read_batch's rules
  *   (file order, same messages for rejected input: HM_ERR_ARG) and brings back the query names and the per-read
- *   coordinates; *n_reads = the batch's reads.  `end` is clamped to the contig by the caller.
+ *   coordinates; *n_reads = the batch's reads.  `end` is clamped to the contig by the caller.  It decodes without the
+ *   base stream; hm_decode_bam_begin_opts takes option bits (HM_DECODE_SEQ; others: HM_ERR_ARG).
  *   hm_decode_bam_names: views of those host arrays (valid until the next begin): NUL-terminated names at
  *   names + name_off[i], tstart / tend per read.
  *   hm_decode_bam_end takes the query-name ids (interned by the BAM handle: hm_bam_intern_qnames) and makes the batch
- *   resident; afterwards every call behaves as after hm_upload_batch of hm_bam_read_batch's batch without seq. */
+ *   resident; afterwards every call behaves as after hm_upload_batch of hm_bam_read_batch's batch without seq, or
+ *   with HM_DECODE_SEQ of its batch with seq (one quality byte per base either way). */
+#define HM_DECODE_SEQ 1u /* hm_decode_bam_begin_opts: pack the 2-bit base stream too (seq / seq_off of hm_read_batch) */
 int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint64_t* n_reads);
+int hm_decode_bam_begin_opts(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint32_t opts,
+                             uint64_t* n_reads);
 int hm_decode_bam_names(hm_ctx* ctx, const char** names, const uint64_t** name_off, const int32_t** tstart,
                         const int32_t** tend, uint64_t* n_reads);
 int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id);
@@ -415,6 +421,9 @@ int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id);
 int hm_batch_read_back(hm_ctx* ctx, hm_read_batch* out, int32_t* tstart, int32_t* tend, int32_t* qstart, int32_t* qlen,
                        uint8_t* mapq, uint32_t* qname_id, uint64_t* bq_off, uint64_t* op_off, uint32_t* n_ops, uint8_t* bq,
                        uint32_t* ops);
+/* diagnostics (tests): the resident base stream back into caller buffers (either may be NULL): n_reads offsets and
+ * *seq_bytes bytes; *seq_bytes = 0 when the resident batch has none */
+int hm_batch_read_back_seq(hm_ctx* ctx, uint64_t* seq_off, uint8_t* seq, uint64_t* seq_bytes);
 /* tests: the device inflate of one raw DEFLATE stream (exactly out_len bytes, CRC32 crc); 0 ok, else an error code */
 int hm_inflate_device_test(hm_ctx* ctx, const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len, uint32_t crc);
 
