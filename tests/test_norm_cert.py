@@ -37,15 +37,30 @@ def make_cert(prior, min_gq, min_bq=93):
     a_bq = 10.0 / 30.0 * (1.0 - 1e-12)
     a_x = 10.0 * f1 / 254.0 * (1.0 + 1e-12)
     c_oth = 10.0 * (lp[0] - max(lp[2], lp[3])) - margin
-    return dict(n_min=int(n_min), ia_bq=math.floor(a_bq * 1048576.0), ia_x=math.ceil(a_x * 1048576.0),
+    cert = dict(n_min=int(n_min), ia_bq=math.floor(a_bq * 1048576.0), ia_x=math.ceil(a_x * 1048576.0),
                 i_need=math.ceil((need - c_oth) * 1048576.0))
+    # thr[n]: the smallest callable count that certifies depth n from the lower bound s1 >= min_bq cal + (n - cal)
+    # (k_norm_bits), made non-decreasing in n; 0xffff: none
+    thr, run = [], 0
+    for n in range(256):
+        t = 0xffff
+        if n >= cert["n_min"]:
+            t = next((cal for cal in range(n + 1) if certified_sum(cert, n, min_bq * cal + (n - cal))), 0xffff)
+            t = run = max(t, run)
+        thr.append(t)
+    cert["thr"] = thr
+    return cert
+
+
+def certified_sum(cert, n, s1):
+    """the integer test on depth n and quality sum s1 (without the depth bound n >= n_min)"""
+    x = min(254 * n, 255 * n - s1)
+    return s1 * cert["ia_bq"] - x * cert["ia_x"] >= cert["i_need"]
 
 
 def certified(cert, bqs):
     """the consumer epilogue's test (normfast.cuh: `n >= cert.n_min && s1 * ia_bq - x * ia_x >= i_need`)"""
-    n, s1 = len(bqs), sum(bqs)
-    x = min(254 * n, 255 * n - s1)
-    return n >= cert["n_min"] and s1 * cert["ia_bq"] - x * cert["ia_x"] >= cert["i_need"]
+    return len(bqs) >= cert["n_min"] and certified_sum(cert, len(bqs), sum(bqs))
 
 
 def quality_mix(rnd, n):
