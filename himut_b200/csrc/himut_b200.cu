@@ -75,6 +75,31 @@ struct PinVec {
 
 struct KTime { const char* name; cudaEvent_t a, b; float ms; };
 
+// Certified verdict of the genotype model at a pure position (computed from hm_params by
+// make_norm_cert; k_norm_bits receives n_min and the table thr derived from it).  With n reads
+// of the reference allele r and qualities b_i:
+//   PL_rr     = -10 (M0 + lp_homref)        M0 = sum lut_hom[b_i]
+//   PL_het    = -10 (M1 + lp_het)           M1 = sum lut_het[b_i]   (= M0 - n log10 2 up to 1e-13)
+//   PL_hetalt = -10 (M2 + lp_hetalt)        M2 = sum lut_err[b_i]   (= -sum b_i / 30 up to 1e-13)
+//   PL_homalt = -10 (M2 + lp_homalt)
+// every other genotype equals one of these four (adding exact zeros is exact).  Homref is the
+// argmin and GQ = int(second - best) >= min_gq iff both differences are >= max(min_gq, 0) and > 0:
+//   PL_het - PL_rr      = 10 n log10 2 + 10 (lp_homref - lp_het)                    -> n >= n_min
+//   PL_other - PL_rr   >= 10 (sum b_i / 30 - f1 * x / 254) + 10 (lp_homref - max(lp_hetalt, lp_homalt))
+//     with x = min(254 n, 255 n - sum b_i), f1 = -lut_hom[1]: -lut_hom is convex and decreasing,
+//     so -M0 <= f1 * (255 n - sum b_i) / 254 and trivially <= f1 * n  (all b_i >= 1).
+// `margin` keeps the comparison away from the fp64 rounding of the reference's own sums (1e-9 at
+// most for depth <= 255); a position that fails the test is simply evaluated exactly.
+struct NormCert {
+  int32_t enabled;
+  int32_t n_min;       // smallest depth whose het - homref difference is certified
+  double a_bq;         // 10 / 30
+  double a_x;          // 10 * f1 / 254
+  double c_oth;        // 10 (lp_homref - max(lp_hetalt, lp_homalt))
+  double need;         // max(min_gq, 0) + margin
+  long long ia_bq, ia_x, i_need; // floor(a_bq 2^20), ceil(a_x 2^20), ceil((need - c_oth) 2^20)
+};
+
 }  // namespace
 
 struct hm_ctx {
@@ -89,12 +114,10 @@ struct hm_ctx {
   uint64_t n_reads = 0, n_ops_total = 0, seq_bytes = 0, bq_bytes = 0;
   uint32_t max_qname_id = 0;
   PinVec<int32_t> h_pmax;
-  PinVec<uint32_t> h_tix_off; // per read: first entry of its tile index (k_tile_index)
   bool upload_pending = false;  // hm_upload_batch_compact_begin: the copies of the last upload have not been waited for
-  uint64_t n_tix = 0;
   DevBuf b_tstart, b_tend, b_qstart, b_qlen, b_mapq, b_flags, b_qname, b_seq_off, b_bq_off, b_op_off, b_n_ops,
       b_seq, b_bq, b_ops, b_op_t, b_op_q, b_mm, b_bq_total, b_n_match, b_n_sub, b_ins_len, b_del_len, b_n_mm, b_gate,
-      b_pmax, b_tix_off, b_tix;
+      b_pmax;
   DevBatch db;
   // sets / phase
   DevBuf b_common, b_pon, b_hpos, b_href, b_halt, b_hbit, b_set_off;
@@ -128,7 +151,7 @@ struct hm_ctx {
   float last_total_ms = 0.f;
   int last_launches = 0;
   size_t ref_len = 0; // length of the contig left resident by hm_set_reference (0: none)
-  NormCert cert;      // certified-verdict constants of the normcounts fast pass
+  NormCert cert;      // certified-verdict constants of the normcounts bit-vector pass
   unsigned long long last_norm_sites = 0; // positions the last normcounts call evaluated exactly
   DevBuf b_push, b_span_cnt; // k_norm_bits: 32 site words and a site count per span
   DevBuf b_sites, b_koff, b_tile_info, b_edge_counts, b_edge_hpos, b_edge_href, b_bqmask, b_bqexc, b_bqexc_off;
@@ -226,9 +249,9 @@ void make_dev_params(hm_ctx* ctx) {
   d.min_sequence_identity = p.min_sequence_identity; d.min_trim = p.min_trim; d.md_threshold = p.md_threshold;
 }
 
-// Constants of the certified homref verdict at pure positions (normfast.cuh).  The derivation
+// Constants of the certified homref verdict at pure positions (NormCert above).  The derivation
 // assumes the three per-BQ tables are the reference's own (gtlib.py:47-69); that is verified here
-// numerically, and the fast pass is switched off for anything else.
+// numerically, and the bit-vector pass is switched off for anything else.
 void make_norm_cert(hm_ctx* ctx) {
   const hm_params& p = ctx->params;
   NormCert& c = ctx->cert;
@@ -391,7 +414,7 @@ void hm_destroy(hm_ctx* ctx) {
   DevBuf* bufs[] = {&ctx->b_tstart, &ctx->b_tend, &ctx->b_qstart, &ctx->b_qlen, &ctx->b_mapq, &ctx->b_flags, &ctx->b_qname,
                     &ctx->b_seq_off, &ctx->b_bq_off, &ctx->b_op_off, &ctx->b_n_ops, &ctx->b_seq, &ctx->b_bq, &ctx->b_ops,
                     &ctx->b_op_t, &ctx->b_op_q, &ctx->b_mm, &ctx->b_bq_total, &ctx->b_n_match, &ctx->b_n_sub,
-                    &ctx->b_ins_len, &ctx->b_del_len, &ctx->b_n_mm, &ctx->b_gate, &ctx->b_pmax, &ctx->b_tix_off, &ctx->b_tix, &ctx->b_common, &ctx->b_pon,
+                    &ctx->b_ins_len, &ctx->b_del_len, &ctx->b_n_mm, &ctx->b_gate, &ctx->b_pmax, &ctx->b_common, &ctx->b_pon,
                     &ctx->b_hpos, &ctx->b_href, &ctx->b_halt, &ctx->b_hbit, &ctx->b_set_off, &ctx->b_chunks,
                     &ctx->b_pair_off, &ctx->b_pair_hap, &ctx->b_qseen, &ctx->b_keys, &ctx->b_keys_sorted, &ctx->b_cub,
                     &ctx->b_records, &ctx->b_counters, &ctx->b_ref, &ctx->b_norm_out, &ctx->b_lut, &ctx->b_tile_off, &ctx->b_agg, &ctx->b_geom, &ctx->b_bidx, &ctx->b_brecs, &ctx->b_sites, &ctx->b_push, &ctx->b_span_cnt, &ctx->b_koff, &ctx->b_tile_info, &ctx->b_edge_counts, &ctx->b_edge_hpos, &ctx->b_edge_href, &ctx->b_bqmask, &ctx->b_bqexc, &ctx->b_bqexc_off,
@@ -404,7 +427,7 @@ void hm_destroy(hm_ctx* ctx) {
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_cnt_pin) cudaFreeHost(ctx->h_cnt_pin);
   if (ctx->h_geom_pin) cudaFreeHost(ctx->h_geom_pin);
-  ctx->h_pmax.release(); ctx->h_tix_off.release(); ctx->h_cw_off.release();
+  ctx->h_pmax.release(); ctx->h_cw_off.release();
   ctx->hd_tstart.release(); ctx->hd_tend.release(); ctx->hd_qstart.release(); ctx->hd_qlen.release(); ctx->hd_n_ops.release();
   ctx->hd_bq_off.release(); ctx->hd_op_off.release(); ctx->hd_name_off.release(); ctx->hd_seq_off.release(); ctx->hd_scal.release(); ctx->hd_names.release();
   ctx->hd_err.release();
@@ -524,7 +547,7 @@ int hm_upload_wait(hm_ctx* ctx) {
   return HM_OK;
 }
 
-// The O(reads) checks of a batch on the host and the tables derived from it (running maximum of tend, tile and
+// The O(reads) checks of a batch on the host and the tables derived from it (running maximum of tend,
 // cal-word offsets, op prefix, shared query names, entry slots per site), for both ways a batch becomes resident
 // (hm_upload_batch*, hm_decode_bam_end).  A batch that fails is never used; the stream is waited for before the error
 // returns, so the caller may free its buffers.
@@ -532,8 +555,8 @@ static int batch_tables(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact
   const uint64_t n = b->n_reads;
 #define BAD(...) do { cudaStreamSynchronize(ctx->stream); return fail(ctx, HM_ERR_ARG, __VA_ARGS__); } while (0)
   // structural validation (cheap, O(reads)); the kernels binary-search on these invariants
-  if (!ctx->h_pmax.resize(n) || !ctx->h_tix_off.resize(n + 1) || !ctx->h_cw_off.resize(n + 1)) BAD("out of page-locked host memory for %llu reads", (unsigned long long)n);
-  uint64_t n_tix = 0, n_cw = 0, span_sum = 0;
+  if (!ctx->h_pmax.resize(n) || !ctx->h_cw_off.resize(n + 1)) BAD("out of page-locked host memory for %llu reads", (unsigned long long)n);
+  uint64_t n_cw = 0, span_sum = 0;
   int32_t run = INT32_MIN;
   uint32_t max_q = 0;
   for (uint64_t r = 0; r < n; r++) {
@@ -549,8 +572,6 @@ static int batch_tables(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact
     if (b->tend[r] > run) run = b->tend[r];
     span_sum += (uint64_t)(b->tend[r] - b->tstart[r]);
     ctx->h_pmax[r] = run;
-    ctx->h_tix_off[r] = (uint32_t)n_tix;
-    n_tix += (uint64_t)((b->tend[r] >> 11) - (b->tstart[r] >> 11) + 1);
     ctx->h_cw_off[r] = (uint32_t)n_cw;
     if (b->tend[r] > b->tstart[r] && b->tstart[r] >= 0) n_cw += (uint64_t)(((b->tend[r] - 1) >> 5) - (b->tstart[r] >> 5) + 1);
     if (b->qname_id[r] > max_q) max_q = b->qname_id[r];
@@ -580,10 +601,8 @@ static int batch_tables(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_compact
       named[b->qname_id[r]] = 1;
     }
   }
-  if (b->n_reads && (b->tstart[0] < 0 || n_tix >= (1ull << 32))) BAD("negative reference_start, or too many (read, tile) pairs in one batch");
+  if (b->n_reads && b->tstart[0] < 0) BAD("negative reference_start");
 #undef BAD
-  ctx->h_tix_off[n] = (uint32_t)n_tix;
-  ctx->n_tix = n_tix;
   ctx->h_cw_off[n] = (uint32_t)n_cw;
   ctx->n_cw = n_cw;
   return HM_OK;
@@ -594,7 +613,6 @@ static int bind_batch(hm_ctx* ctx, const hm_read_batch* b, bool has_seq) {
   const uint64_t n = b->n_reads;
   int rc;
   if ((rc = upload(ctx, ctx->b_pmax, ctx->h_pmax.data(), n))) return rc;
-  if ((rc = upload(ctx, ctx->b_tix_off, ctx->h_tix_off.data(), n + 1))) return rc;
   if (ctx->n_cw < (1ull << 32) && (rc = upload(ctx, ctx->b_cw_off, ctx->h_cw_off.data(), n + 1))) return rc;
   const size_t no = (size_t)b->n_ops_total;
   CU(ctx->b_op_t.ensure(no * 4 + 16)); CU(ctx->b_op_q.ensure(no * 4 + 16)); CU(ctx->b_mm.ensure(no * 4 + 16));
@@ -1279,24 +1297,15 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
                                                                               site_lo, site_n);
       t_end(ctx);
       CU(cudaGetLastError());
-      const bool by_site = getenv("HIMUT_B200_ENTRIES_BY_SITE") != nullptr; // the earlier thread-per-(site, read) gather (A/B)
-      if (by_site) {
-        t_begin(ctx, "k_site_entries");
-        k_site_entries<<<(unsigned)((n_unique + 15) / 16), 1024, 0, ctx->stream>>>(
-            ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), ctx->b_pair_off.as<uint64_t>(), ctx->b_pair_hap.as<uint8_t>(), k_in,
-            d_cnt + 1, site_lo, site_n, entries, stride);
-        t_end(ctx);
-      } else {
-        CU(ctx->b_koff.ensure((n_chunks + 2) * 4));
-        t_begin(ctx, "k_site_entries_by_read");
-        CU(cudaMemsetAsync(entries, 0xff, stride * HM_SITE_SLOTS * 4, ctx->stream));
-        k_chunk_key_ranges<<<(unsigned)((n_chunks + 1 + 127) / 128), 128, 0, ctx->stream>>>(k_in, d_cnt + 1, (uint32_t)n_chunks, ctx->b_koff.as<uint32_t>());
-        auto gather = ctx->db.seq ? k_site_entries_by_read<true> : k_site_entries_by_read<false>;
-        gather<<<(unsigned)((n_pairs * 32 + 255) / 256), 256, 0, ctx->stream>>>(
-            ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(), n_pairs,
-            ctx->b_pair_hap.as<uint8_t>(), k_in, ctx->b_koff.as<uint32_t>(), site_lo, site_n, entries, stride);
-        t_end(ctx);
-      }
+      CU(ctx->b_koff.ensure((n_chunks + 2) * 4));
+      t_begin(ctx, "k_site_entries_by_read");
+      CU(cudaMemsetAsync(entries, 0xff, stride * HM_SITE_SLOTS * 4, ctx->stream));
+      k_chunk_key_ranges<<<(unsigned)((n_chunks + 1 + 127) / 128), 128, 0, ctx->stream>>>(k_in, d_cnt + 1, (uint32_t)n_chunks, ctx->b_koff.as<uint32_t>());
+      auto gather = ctx->db.seq ? k_site_entries_by_read<true> : k_site_entries_by_read<false>;
+      gather<<<(unsigned)((n_pairs * 32 + 255) / 256), 256, 0, ctx->stream>>>(
+          ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(), n_pairs,
+          ctx->b_pair_hap.as<uint8_t>(), k_in, ctx->b_koff.as<uint32_t>(), site_lo, site_n, entries, stride);
+      t_end(ctx);
       CU(cudaGetLastError());
       t_begin(ctx, "k_site_reduce");
       k_site_reduce<<<(unsigned)((n_unique + 127) / 128), 128, 0, ctx->stream>>>(
@@ -1843,19 +1852,13 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
   int rc = upload_chunks(ctx, chunks, n_chunks, pair_off);
   if (rc) return rc;
   const uint64_t n_pairs = pair_off.back();
-  // tile prefix sums for the 256-wide (v1) and 512-wide (TMA) kernels, back to back
-  std::vector<uint64_t> tile_off(3 * (n_chunks + 1), 0);
-  uint64_t* tile_off2 = tile_off.data() + n_chunks + 1;
-  uint64_t* tile_off3 = tile_off.data() + 2 * (n_chunks + 1);
-  uint64_t total_span = 0;
+  // tile prefix sums of k_norm_tiles_tma (512-position tiles from each chunk's start)
+  std::vector<uint64_t> tile_off(n_chunks + 1, 0);
   for (size_t i = 0; i < n_chunks; i++) {
     const int64_t span = (int64_t)chunks[i].end - (int64_t)chunks[i].start;
-    tile_off[i + 1] = tile_off[i] + (span > 0 ? (uint64_t)((span + HM_TILE_W - 1) / HM_TILE_W) : 0);
-    tile_off2[i + 1] = tile_off2[i] + (span > 0 ? (uint64_t)((span + HM_TW - 1) / HM_TW) : 0);
-    tile_off3[i + 1] = tile_off3[i] + (span > 0 ? (uint64_t)(((chunks[i].end - 1) >> 11) - (chunks[i].start >> 11) + 1) : 0); // absolute 2048 grid
-    if (span > 0) total_span += (uint64_t)span;
+    tile_off[i + 1] = tile_off[i] + (span > 0 ? (uint64_t)((span + HM_TW - 1) / HM_TW) : 0);
   }
-  const uint64_t n_tiles = tile_off[n_chunks], n_tiles_tma = tile_off2[n_chunks], n_tiles_fast = tile_off3[n_chunks];
+  const uint64_t n_tiles = tile_off[n_chunks];
   if (n_tiles >= (1ull << 31)) return fail(ctx, HM_ERR_ARG, "too many tiles in one call");
   if ((rc = upload(ctx, ctx->b_tile_off, tile_off.data(), tile_off.size()))) return rc;
   if (refseq) { // per-call reference: replaces whatever hm_set_reference left
@@ -1863,12 +1866,10 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     ctx->ref_len = 0;
     ctx->packed_pos = 0;
   }
-  // which pass runs in front of the exact pass: bit vectors (normbits.cuh) unless the parameters are outside the
-  // certified domain or an earlier kernel is asked for (A/B: HIMUT_B200_NORM_V1 / _V2 single pass, _V3 byte tiles)
-  const bool use_v1 = getenv("HIMUT_B200_NORM_V1") != nullptr;
-  const bool use_v2 = getenv("HIMUT_B200_NORM_V2") != nullptr;
-  const bool use_v3 = getenv("HIMUT_B200_NORM_V3") != nullptr;
-  bool use_bits = !use_v1 && !use_v2 && !use_v3 && ctx->cert.enabled && ctx->n_reads > 0 && ctx->n_cw < (1ull << 32) && n_pairs > 0;
+  // bit vectors (normbits.cuh) in front of the exact pass; the single pass k_norm_tiles_tma where they do not apply:
+  // parameters outside the certified domain, a chunk that starts below 0 (the spans lie on the absolute 1024 grid),
+  // cal words that a 32-bit offset cannot address
+  bool use_bits = ctx->cert.enabled && ctx->n_reads > 0 && ctx->n_cw < (1ull << 32) && n_pairs > 0;
   std::vector<uint64_t> span_off(n_chunks + 1, 0);
   int64_t max_end = 0;
   for (size_t i = 0; i < n_chunks; i++) {
@@ -1904,7 +1905,7 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     t_begin(ctx, "k_norm_prep");
     k_norm_prep<<<(unsigned)((ctx->n_reads + NB_PREP_WARPS - 1) / NB_PREP_WARPS), 32 * NB_PREP_WARPS, sizeof(PrepWarp) * NB_PREP_WARPS, ctx->stream>>>(
         ctx->db, ctx->dp, ctx->b_ref2.as<uint32_t>(), ctx->b_cw_off.as<uint32_t>(), ctx->b_calw.as<uint32_t>(), ctx->b_impure.as<uint32_t>(), imp_words,
-        ctx->compact_resident && !getenv("HIMUT_B200_NORM_BYTES") ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->b_exc_minmax.as<uint8_t>(),
+        ctx->compact_resident ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->b_exc_minmax.as<uint8_t>(),
         ctx->b_exp_total.as<unsigned long long>(), ctx->modal, ctx->b_sdiff.as<uint32_t>(), ctx->b_cal_ok.as<uint8_t>());
     t_end(ctx);
     CU(cudaGetLastError());
@@ -1929,141 +1930,72 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     CU(cudaGetLastError());
     int n_sm = 148;
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, ctx->device);
-    if (use_v1) {
-      t_begin(ctx, "k_norm_tiles");
-      k_norm_tiles<<<(unsigned)n_tiles, HM_TILE_W, 0, ctx->stream>>>(ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(),
-                                                                     (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(),
-                                                                     ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_off.as<uint64_t>(),
-                                                                     ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len,
-                                                                     ctx->b_norm_out.as<NormOut>());
-      t_end(ctx);
-    } else if (use_v2 || !ctx->cert.enabled) {
+    if (!use_bits) {
       const size_t smem = sizeof(TileStage) * HM_NSTAGE;
       static bool attr_set = false;
       if (!attr_set) {
         CU(cudaFuncSetAttribute(k_norm_tiles_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_set = true;
       }
-      unsigned grid = (unsigned)std::min<uint64_t>(n_tiles_tma, (uint64_t)n_sm);
-      if (const char* g = getenv("HIMUT_B200_NORM_GRID")) grid = (unsigned)std::max(1, std::min<int>(atoi(g), (int)n_tiles_tma));
+      const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles, (uint64_t)n_sm);
       t_begin(ctx, "k_norm_tiles_tma");
       k_norm_tiles_tma<<<grid, HM_TW + 32 * HM_NPROD, smem, ctx->stream>>>(ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(),
                                                                 (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(),
-                                                                ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_off.as<uint64_t>() + n_chunks + 1,
-                                                                (uint32_t)n_tiles_tma, ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len,
+                                                                ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_off.as<uint64_t>(),
+                                                                (uint32_t)n_tiles, ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len,
                                                                 ctx->b_norm_out.as<NormOut>());
       t_end(ctx);
     } else {
-      // fast integer pass over every position, then the exact pass over the listed sites
-      const size_t smem = sizeof(FastStage) * HF_NSTAGE;
-      static bool attr_set = false;
-      if (!attr_set) {
-        CU(cudaFuncSetAttribute(k_norm_fast, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-      }
-      const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles_fast, (uint64_t)n_sm);
+      // bit-vector pass over every position, then the exact pass over the listed sites
       unsigned long long* d_nsites = ctx->b_counters.as<unsigned long long>() + 4;
-      unsigned long long site_cap = std::max<unsigned long long>(1ull << 16, total_span / 16);
-      if (const char* g = getenv("HIMUT_B200_NORM_SITE_CAP")) site_cap = std::max(1ll, atoll(g));
       unsigned long long n_sites = 0;
-      if (use_bits) {
-        const double md = ctx->params.md_threshold;
-        const int md_k = !(md == md) ? 256 : md < 0.0 ? 0 : md >= 255.0 ? 256 : (int)floor(md) + 1; // depth >= md_k <=> depth > md_threshold
-        const unsigned bgrid = (unsigned)std::min<uint64_t>((n_spans + NB_BITS_WARPS - 1) / NB_BITS_WARPS, (uint64_t)n_sm * (ctx->params.phase ? 4 : 6));
-        CU(ctx->b_tile_info.ensure((size_t)n_spans * 16 + 16));
-        if (n_spans) {
-          t_begin(ctx, "k_span_ranges");
-          k_span_ranges<<<(unsigned)((n_spans + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
-                                                                                ctx->b_span_off.as<uint64_t>(), n_spans, ctx->b_tile_info.as<uint4>());
-          t_end(ctx);
-          CU(cudaGetLastError());
-        }
-        if (n_spans) {
-          // every span leaves its 32 site words and its count; the counts are scanned and the keys written span by span:
-          // the site list comes out in (chunk, position) order and in exactly the room it needs
-          CU(ctx->b_push.ensure((size_t)n_spans * 128 + 16));
-          CU(ctx->b_span_cnt.ensure(((size_t)n_spans + 1) * 8 + 16));
-          uint32_t* span_cnt = ctx->b_span_cnt.as<uint32_t>();
-          uint32_t* span_dst = span_cnt + n_spans;
-          t_begin(ctx, "k_norm_bits");
-          (ctx->params.phase ? k_norm_bits<true> : k_norm_bits<false>)<<<bgrid, 32 * NB_BITS_WARPS, 0, ctx->stream>>>(
-              ctx->db, ctx->dp, ctx->b_thr.as<uint16_t>(), (int)ctx->cert.n_min, md_k, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
-              ctx->b_pair_off.as<uint64_t>(), ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_info.as<uint4>(), n_spans, ctx->b_cw_off.as<uint32_t>(),
-              ctx->b_calw.as<uint32_t>(), ctx->b_impure.as<uint32_t>(), ctx->b_tri8.as<uint8_t>(), ctx->b_norm_out.as<NormOut>(),
-              ctx->b_push.as<uint32_t>(), span_cnt);
-          t_end(ctx);
-          CU(cudaGetLastError());
-          t_begin(ctx, "k_emit_sites");
-          k_span_scan<<<1, 1024, 0, ctx->stream>>>(span_cnt, n_spans, span_dst, d_nsites);
-          CU(cudaMemcpyAsync(&n_sites, d_nsites, 8, cudaMemcpyDeviceToHost, ctx->stream));
-          CU(cudaStreamSynchronize(ctx->stream));
-          CU(ctx->b_sites.ensure((size_t)std::max<unsigned long long>(n_sites, 1) * 8));
-          if (n_sites)
-            k_emit_sites<<<(unsigned)((n_spans * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->b_tile_info.as<uint4>(), n_spans, ctx->b_push.as<uint32_t>(),
-                                                                                       span_dst, ctx->b_sites.as<unsigned long long>());
-          t_end(ctx);
-          CU(cudaGetLastError());
-        }
-      } else {
-      CU(ctx->b_tix.ensure((size_t)ctx->n_tix * 16 + 16));
-      CU(ctx->b_tile_info.ensure((size_t)n_tiles_fast * 16 + 16));
-      t_begin(ctx, "k_tile_index");
-      k_tile_ranges<<<(unsigned)((n_tiles_fast + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
-                                                                                  ctx->b_tile_off.as<uint64_t>() + 2 * (n_chunks + 1),
-                                                                                  (uint32_t)n_tiles_fast, ctx->b_tile_info.as<uint4>());
-      k_tile_index<<<(unsigned)((ctx->n_reads * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->dp.mismatch_window,
-                                                                                         ctx->b_tix_off.as<uint32_t>(), ctx->b_tix.as<uint4>());
-      t_end(ctx);
-      CU(cudaGetLastError());
-      for (int attempt = 0; attempt < 2; attempt++) {
-        CU(ctx->b_sites.ensure(site_cap * 8));
-        if (attempt) { // the list overflowed: start over with the exact size
-          CU(cudaMemsetAsync(ctx->b_norm_out.p, 0, sizeof(NormOut), ctx->stream));
-          CU(cudaMemsetAsync(d_nsites, 0, 8, ctx->stream));
-        }
-        t_begin(ctx, "k_norm_fast");
-        k_norm_fast<<<grid, HF_CONS + 32 * HF_NPROD, smem, ctx->stream>>>(
-            ctx->db, ctx->dp, ctx->cert, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(),
-            ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_info.as<uint4>(), (uint32_t)n_tiles_fast,
-            ctx->b_tix_off.as<uint32_t>(), ctx->b_tix.as<uint4>(), ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len, ctx->b_norm_out.as<NormOut>(), ctx->b_sites.as<unsigned long long>(), site_cap,
-            d_nsites);
+      const double md = ctx->params.md_threshold;
+      const int md_k = !(md == md) ? 256 : md < 0.0 ? 0 : md >= 255.0 ? 256 : (int)floor(md) + 1; // depth >= md_k <=> depth > md_threshold
+      const unsigned bgrid = (unsigned)std::min<uint64_t>((n_spans + NB_BITS_WARPS - 1) / NB_BITS_WARPS, (uint64_t)n_sm * (ctx->params.phase ? 4 : 6));
+      CU(ctx->b_tile_info.ensure((size_t)n_spans * 16 + 16));
+      if (n_spans) {
+        t_begin(ctx, "k_span_ranges");
+        k_span_ranges<<<(unsigned)((n_spans + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
+                                                                              ctx->b_span_off.as<uint64_t>(), n_spans, ctx->b_tile_info.as<uint4>());
         t_end(ctx);
         CU(cudaGetLastError());
+        // every span leaves its 32 site words and its count; the counts are scanned and the keys written span by span:
+        // the site list comes out in (chunk, position) order and in exactly the room it needs
+        CU(ctx->b_push.ensure((size_t)n_spans * 128 + 16));
+        CU(ctx->b_span_cnt.ensure(((size_t)n_spans + 1) * 8 + 16));
+        uint32_t* span_cnt = ctx->b_span_cnt.as<uint32_t>();
+        uint32_t* span_dst = span_cnt + n_spans;
+        t_begin(ctx, "k_norm_bits");
+        (ctx->params.phase ? k_norm_bits<true> : k_norm_bits<false>)<<<bgrid, 32 * NB_BITS_WARPS, 0, ctx->stream>>>(
+            ctx->db, ctx->dp, ctx->b_thr.as<uint16_t>(), (int)ctx->cert.n_min, md_k, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
+            ctx->b_pair_off.as<uint64_t>(), ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_info.as<uint4>(), n_spans, ctx->b_cw_off.as<uint32_t>(),
+            ctx->b_calw.as<uint32_t>(), ctx->b_impure.as<uint32_t>(), ctx->b_tri8.as<uint8_t>(), ctx->b_norm_out.as<NormOut>(),
+            ctx->b_push.as<uint32_t>(), span_cnt);
+        t_end(ctx);
+        CU(cudaGetLastError());
+        t_begin(ctx, "k_emit_sites");
+        k_span_scan<<<1, 1024, 0, ctx->stream>>>(span_cnt, n_spans, span_dst, d_nsites);
         CU(cudaMemcpyAsync(&n_sites, d_nsites, 8, cudaMemcpyDeviceToHost, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
-        if (n_sites <= site_cap) break;
-        site_cap = n_sites;
-      }
+        CU(ctx->b_sites.ensure((size_t)std::max<unsigned long long>(n_sites, 1) * 8));
+        if (n_sites)
+          k_emit_sites<<<(unsigned)((n_spans * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->b_tile_info.as<uint4>(), n_spans, ctx->b_push.as<uint32_t>(),
+                                                                                     span_dst, ctx->b_sites.as<unsigned long long>());
+        t_end(ctx);
+        CU(cudaGetLastError());
       }
       ctx->last_norm_sites = n_sites;
-      const bool by_site = getenv("HIMUT_B200_ENTRIES_BY_SITE") != nullptr; // thread-per-(site, read) gather (A/B)
       const unsigned long long* site_keys = ctx->b_sites.as<unsigned long long>();
-      if (n_sites && !by_site && use_bits) { // already in (chunk, position) order
+      if (n_sites) {
         CU(ctx->b_koff.ensure((n_chunks + 2) * 4));
         k_chunk_key_ranges<<<(unsigned)((n_chunks + 1 + 127) / 128), 128, 0, ctx->stream>>>(site_keys, d_nsites, (uint32_t)n_chunks, ctx->b_koff.as<uint32_t>());
-      } else if (n_sites && !by_site) {
-        // the list comes out in tile-completion order: sort it (chunk, position) so a read finds its sites by range
-        CU(ctx->b_keys_sorted.ensure(n_sites * 8));
-        int end_bit = 36;
-        for (size_t cc = n_chunks; cc > 0; cc >>= 1) end_bit++;
-        size_t tmp_sort = 0;
-        CU(cub::DeviceRadixSort::SortKeys(nullptr, tmp_sort, ctx->b_sites.as<unsigned long long>(), ctx->b_keys_sorted.as<unsigned long long>(),
-                                          (int64_t)n_sites, 4, std::min(end_bit, 64), ctx->stream));
-        CU(ctx->b_cub.ensure(tmp_sort));
-        CU(ctx->b_koff.ensure((n_chunks + 2) * 4));
-        t_begin(ctx, "cub_sort_site_list");
-        CU(cub::DeviceRadixSort::SortKeys(ctx->b_cub.p, tmp_sort, ctx->b_sites.as<unsigned long long>(), ctx->b_keys_sorted.as<unsigned long long>(),
-                                          (int64_t)n_sites, 4, std::min(end_bit, 64), ctx->stream));
-        site_keys = ctx->b_keys_sorted.as<unsigned long long>();
-        k_chunk_key_ranges<<<(unsigned)((n_chunks + 1 + 127) / 128), 128, 0, ctx->stream>>>(site_keys, d_nsites, (uint32_t)n_chunks, ctx->b_koff.as<uint32_t>());
-        t_end(ctx);
       }
       // sites per round of the exact pass: the entry table (slots x sites x 4 B) stays at 0.5 GB
-      const unsigned long long SITE_BATCH = std::max<unsigned long long>(1ull << 16, (1ull << 27) / std::max<uint32_t>(by_site ? (uint32_t)HM_SITE_SLOTS : ctx->site_slots, 1u));
+      const uint32_t n_slots = ctx->site_slots; // as the call path: about twice the mean depth
+      const unsigned long long SITE_BATCH = std::max<unsigned long long>(1ull << 16, (1ull << 27) / std::max<uint32_t>(n_slots, 1u));
       for (unsigned long long s0 = 0; s0 < n_sites; s0 += SITE_BATCH) {
         const uint64_t nb = (uint64_t)std::min<unsigned long long>(SITE_BATCH, n_sites - s0);
         const uint64_t stride = (nb + 31) & ~31ull;
-        const uint32_t n_slots = by_site ? (uint32_t)HM_SITE_SLOTS : ctx->site_slots; // as the call path: about twice the mean depth
         CU(ctx->b_agg.ensure(stride * n_slots * 4 + nb * 8));
         uint32_t* entries = ctx->b_agg.as<uint32_t>();
         uint32_t* site_lo = entries + stride * n_slots;
@@ -2072,28 +2004,14 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
         t_begin(ctx, "k_norm_site_range");
         k_norm_site_range<<<(unsigned)((nb + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->b_chunks.as<hm_chunk>(), keys, nb, site_lo, site_n);
         t_end(ctx);
-        if (by_site) {
-          t_begin(ctx, "k_norm_entries");
-          k_norm_entries<<<(unsigned)((nb + 15) / 16), 1024, 0, ctx->stream>>>(ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(),
-                                                                              ctx->b_pair_off.as<uint64_t>(), ctx->b_pair_hap.as<uint8_t>(),
-                                                                              keys, nb, site_lo, site_n, entries, stride);
-          t_end(ctx);
-        } else {
-          t_begin(ctx, use_bits ? "k_norm_entries_bits" : "k_norm_entries_by_read");
-          CU(cudaMemsetAsync(entries, 0xff, stride * n_slots * 4, ctx->stream));
-          if (use_bits)
-            k_norm_entries_bits<<<(unsigned)((n_pairs * 32 + 255) / 256), 256, 0, ctx->stream>>>(
-                ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(), n_pairs,
-                ctx->b_pair_hap.as<uint8_t>(), site_keys, ctx->b_koff.as<uint32_t>(), (uint64_t)s0, nb, site_lo, site_n, entries, stride,
-                ctx->b_cw_off.as<uint32_t>(), ctx->b_calw.as<uint32_t>(), ctx->b_cal_ok.as<uint8_t>(), ctx->b_sdiff.as<uint32_t>(),
-                ctx->b_ref2.as<uint32_t>(), ctx->compact_resident && !getenv("HIMUT_B200_NORM_BYTES") ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->modal,
-                n_slots);
-          else
-          k_norm_entries_by_read<<<(unsigned)((n_pairs * 32 + 255) / 256), 256, 0, ctx->stream>>>(
-              ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(), n_pairs,
-              ctx->b_pair_hap.as<uint8_t>(), site_keys, ctx->b_koff.as<uint32_t>(), (uint64_t)s0, nb, site_lo, site_n, entries, stride, n_slots);
-          t_end(ctx);
-        }
+        t_begin(ctx, "k_norm_entries_bits");
+        CU(cudaMemsetAsync(entries, 0xff, stride * n_slots * 4, ctx->stream));
+        k_norm_entries_bits<<<(unsigned)((n_pairs * 32 + 255) / 256), 256, 0, ctx->stream>>>(
+            ctx->db, ctx->dp, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(), n_pairs,
+            ctx->b_pair_hap.as<uint8_t>(), site_keys, ctx->b_koff.as<uint32_t>(), (uint64_t)s0, nb, site_lo, site_n, entries, stride,
+            ctx->b_cw_off.as<uint32_t>(), ctx->b_calw.as<uint32_t>(), ctx->b_cal_ok.as<uint8_t>(), ctx->b_sdiff.as<uint32_t>(),
+            ctx->b_ref2.as<uint32_t>(), ctx->compact_resident ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->modal, n_slots);
+        t_end(ctx);
         t_begin(ctx, "k_norm_reduce");
         k_norm_reduce<<<(unsigned)((nb + 127) / 128), 128, 0, ctx->stream>>>(
             ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(), ctx->b_pair_off.as<uint64_t>(),
@@ -2114,19 +2032,6 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
   }
   CU(cudaStreamSynchronize(ctx->stream));
   t_collect(ctx);
-#ifdef HM_NORM_DEBUG
-  {
-    unsigned long long fd[8];
-    cudaMemcpyFromSymbol(fd, g_fill_dbg, sizeof(fd));
-    fprintf(stderr, "[fill dbg, cycles summed over CTA 0's producer warps] meta %llu scans %llu scratch %llu walk %llu classify %llu tma %llu\n", fd[0], fd[1], fd[2], fd[3], fd[4], fd[5]);
-    memset(fd, 0, sizeof(fd));
-    cudaMemcpyToSymbol(g_fill_dbg, fd, sizeof(fd));
-  }
-  fprintf(stderr, "[norm dbg, CTA 0] producer: wait %.0f fill %.0f cycles per batch (%llu batches) | consumer warp 0: wait %.0f compute %.0f cycles per batch, %.1f slots per batch | epilogue %.0f cycles per tile (%llu tiles)\n",
-          (double)h.dbg[0] / (double)std::max<unsigned long long>(h.dbg[2], 1), (double)h.dbg[1] / (double)std::max<unsigned long long>(h.dbg[2], 1), h.dbg[2],
-          (double)h.dbg[3] / (double)std::max<unsigned long long>(h.dbg[2], 1), (double)h.dbg[4] / (double)std::max<unsigned long long>(h.dbg[2], 1),
-          (double)h.dbg[5] / (double)std::max<unsigned long long>(h.dbg[2], 1), (double)h.dbg[6] / (double)std::max<unsigned long long>(h.dbg[7], 1), h.dbg[7]);
-#endif
   if (h.err == HM_ERR_BQ_ZERO) return fail(ctx, HM_ERR_BQ_ZERO, "a base quality of 0 reached the genotype model (the reference raises ValueError: math.log10(0))");
   for (int i = 0; i < HM_TRI_BINS; i++) { ccs_tri[i] = (int64_t)h.ccs_tri[i]; ref_tri[i] = (int64_t)h.ref_tri[i]; }
   for (int i = 1; i < HM_NORM_LOG_LEN; i++) log[i] = (int64_t)h.log[i];

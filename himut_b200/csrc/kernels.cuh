@@ -9,10 +9,10 @@
 //                   then trim + mismatch-window filter of every substitution
 //                   (bamlib.get_tsbs_candidates, src/himut/bamlib.py:69-86,222-282;
 //                    haplib.get_ccs_hap, src/himut/haplib.py:46-83)
-//   k_site_range / k_site_entries / k_site_reduce
+//   k_site_range / k_site_entries_by_read / k_site_reduce
 //                   per distinct candidate: the pileup column of the chunk's reads at the site
-//                   (caller.update_allelecounts, caller.py:44-72) gathered with one thread per
-//                   (site, read), then per site in file order: counts, ordered fp64 sums,
+//                   (caller.update_allelecounts, caller.py:44-72) gathered with one warp per
+//                   (chunk, read), then per site in file order: counts, ordered fp64 sums,
 //                   10-genotype PL / GQ (gtlib.py:72-174), germline restatement test and the
 //                   filter cascade (caller.py:324-621) -> record
 //
@@ -648,9 +648,10 @@ __device__ __noinline__ int read_allele_walk(const DevBatch& b, uint32_t r, int3
 // the order-sensitive part stays sequential per site:
 //   k_site_range    1 thread / distinct candidate: the file-order index range [lo, lo + n) of the
 //                   chunk's reads that can touch the site (two 8-ary searches);
-//   k_site_entries  1 thread / (candidate, read slot < 64): allele, BQ, insertion count, haplotype
-//                   of that read at the site, packed into one u32, stored slot-major so both this
-//                   kernel's writes and the next kernel's reads are coalesced;
+//   k_site_entries_by_read
+//                   1 warp / (chunk, read): allele, BQ, insertion count, haplotype of that read at
+//                   each site it covers, packed into one u32 per (site, read slot), stored slot-major
+//                   so the next kernel's reads are coalesced;
 //   k_site_reduce   1 thread / candidate: walks the slots in file order — 6 counts, BQ sums, the
 //                   12 ordered fp64 sums (caller.update_allelecounts appends in fetch order,
 //                   caller.py:44-72), haplotype tallies — then 10-genotype PL / GQ
@@ -696,25 +697,9 @@ __global__ void __launch_bounds__(256) k_site_range(DevBatch b, const hm_chunk* 
   site_n[ki] = hi > lo ? hi - lo : 0u;
 }
 
-// block = 16 sites x 64 slots; thread (site = tid & 15, slot = tid >> 4)
-__global__ void __launch_bounds__(1024) k_site_entries(DevBatch b, DevParams p, const hm_chunk* chunks, const uint64_t* pair_off,
-                                                       const uint8_t* pair_hap, const unsigned long long* keys,
-                                                       const unsigned long long* n_keys_dev, const uint32_t* site_lo,
-                                                       const uint32_t* site_n, uint32_t* entries, uint64_t stride) {
-  const uint64_t ki = (uint64_t)blockIdx.x * 16 + (threadIdx.x & 15);
-  const uint32_t slot = threadIdx.x >> 4;
-  if (ki >= *n_keys_dev) return;
-  if (slot >= __ldg(site_n + ki)) return;
-  const unsigned long long key = keys[ki];
-  const uint32_t c = (uint32_t)(key >> 36);
-  const int32_t rpos = (int32_t)((key >> 4) & 0xffffffffull) - 1;
-  const hm_chunk ch = chunks[c];
-  entries[(uint64_t)slot * stride + ki] = site_entry(b, p, ch, c, pair_off, pair_hap, __ldg(site_lo + ki) + slot, rpos, (int)((key >> 2) & 3));
-}
-
 // ---- gather by read ------------------------------------------------------------------------------
-// k_site_entries asks, for every (site, read) pair, "which op of this read holds the site" with a search over
-// the read's op arrays in global memory.  k_site_entries_by_read turns the loop around: one warp per
+// Rather than asking, for every (site, read) pair, "which op of this read holds the site" with a search over
+// the read's op arrays in global memory, k_site_entries_by_read turns the loop around: one warp per
 // (chunk, read) pair stages the read's op arrays in shared memory once and then serves all the chunk's sites
 // the read covers (about 60 per 15 kb read), 32 sites at a time; the only scattered global loads left are the
 // site's quality byte and its 2-bit base.  Entries nobody writes (reads that do not reach a site) keep the

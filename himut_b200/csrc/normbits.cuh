@@ -1,11 +1,11 @@
-// normbits.cuh — the callable-base half of `himut normcounts` as bit vectors (sm_100a); replaces the byte-per-base tile
-// kernel k_norm_fast (normfast.cuh) as the integer pass in front of the exact pass.
+// normbits.cuh — the callable-base half of `himut normcounts` as bit vectors (sm_100a): the integer pass in front of the
+// exact pass (normfast.cuh).
 //
 // The reference asks two things of every aligned base (normcounts.py:65-110, 292-314): "does this read count here"
 // (matched base, BQ >= min_bq, no mismatch within the window of its block, not trimmed) and "what does the pileup
 // column look like" (gtlib.get_germ_gt over every base of the column).  At a *pure* position — every primary read that
 // covers it shows the FASTA base through a plain cs match — the second question has a certified answer that needs the
-// depth n and a lower bound of the column's quality sum only (NormCert, normfast.cuh).  And a lower bound is at hand
+// depth n and a lower bound of the column's quality sum only (NormCert, himut_b200.cu).  And a lower bound is at hand
 // without touching a single quality byte again: every counted base has BQ >= min_bq, every other base has BQ >= 1, so
 //     sum BQ  >=  min_bq * callable + (n - callable).
 // So each read is turned ONCE, by the warp that streams its qualities anyway, into one bit per reference position
@@ -25,7 +25,7 @@
 //                 logic ops per read and counter); depth, callable count and haplotype tallies of all 32 positions of
 //                 a lane never leave 8 + 8 (+ 16) registers.  Then, bit-parallel: certified -> the cascade's depth /
 //                 ref-count gates and the 33-bin tallies (normcounts.py:317-400); impure or not certified -> the site
-//                 list of the exact pass (k_norm_entries_by_read / k_norm_reduce, normfast.cuh), which evaluates the
+//                 list of the exact pass (k_norm_entries_bits below, k_norm_reduce in normfast.cuh), which evaluates the
 //                 position with the reference's own ordered fp64 arithmetic.  Both passes add into the same tallies.
 //
 // The verdict at a certified position is the exact verdict (tests/test_norm_cert.py holds the bound against the
@@ -71,6 +71,8 @@ __global__ void __launch_bounds__(256) k_ref_pack(const uint8_t* refseq, uint64_
   ref2[w] = code;
   reinterpret_cast<uint4*>(tri8)[w] = make_uint4(tb[0], tb[1], tb[2], tb[3]);
 }
+
+__device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; } // bit k -> bit 8k
 
 // the k lowest bits (k <= 0: none, k >= 32: all): one BMSK with its width clamped to [0, 32] (k_norm_prep 1.25 -> 1.20 ms,
 // k_norm_bits 0.28 -> 0.27 ms against the compare-and-shift form, NB_NO_BMSK)
@@ -474,9 +476,11 @@ __global__ void __launch_bounds__(32 * NB_PREP_WARPS, 8) k_norm_prep(DevBatch b,
 }
 
 // ============================================================================ k_norm_entries_bits
-// k_norm_entries_by_read (normfast.cuh) for the bit-vector path: "is this base counted by update_tri2count" is the
-// read's cal bit (no window / trim arithmetic), the base of a match run is the FASTA's unless k_norm_prep saw it
-// differ (sdiff), and on a compact upload the quality is the modal value wherever the bitmap says so — the byte
+// The exact pass's gather, one warp per (chunk, read) pair as k_site_entries_by_read (kernels.cuh) does it for `call`.
+// It stages the read's op arrays in shared memory and serves every listed site of the chunk the read covers; `keys` is
+// in (chunk, position) order and [s0, s0 + nb) is the slice of it this launch fills (entries are slice relative).
+// "Is this base counted by update_tri2count" is the read's cal bit (no window / trim arithmetic), the base of a match
+// run is the FASTA's unless k_norm_prep saw it differ (sdiff), and on a compact upload the quality is the modal value wherever the bitmap says so — the byte
 // stream is touched for the exceptions only.  Reads k_norm_prep could not stage go the general way (norm_entry).
 __global__ void __launch_bounds__(256) k_norm_entries_bits(DevBatch b, DevParams p, const hm_chunk* chunks, uint32_t n_chunks,
                                                            const uint64_t* pair_off, uint64_t n_pairs, const uint8_t* pair_flag,

@@ -3,29 +3,24 @@
 //
 //   k_pair_info        per (chunk, read) pair: fetch rule, [--phase] read haplotype, read gates,
 //                      distinct-qname mark (normcounts.py:292-314)
-//   k_norm_tiles       one CTA per 256-position tile of one chunk, one thread per reference
-//                      position.  The tile's reads are walked in file order, so each thread sees
-//                      "its" column of the pileup in the reference's append order: 6 allele
-//                      counts, the 12 ordered fp64 sums of the genotype model (registers), the
-//                      callable-read count of update_tri2count (normcounts.py:65-110) and the
-//                      haplotype counts; then the thread genotypes its position and runs the
-//                      filter cascade (normcounts.py:317-400).  Only 33+33 trinucleotide bins
-//                      and 14 counters leave the SM (shared-memory tallies, one global atomic
-//                      per bin per CTA).
+//   k_norm_tiles_tma   single pass that genotypes every covered position from ordered fp64 adds,
+//                      one thread per reference position of a 512-position tile (see below).  It
+//                      runs where the bit-vector pass of normbits.cuh does not apply: parameters
+//                      outside the certified domain, a chunk that starts below position 0, 2^32
+//                      or more cal words in one batch.  Only 33+33 trinucleotide bins and 14
+//                      counters leave the SM (shared-memory tallies, one global atomic per bin
+//                      per CTA).
+//   k_ref_tricounts    reference trinucleotide counts (reflib.get_chrom_tricount)
 //
-// Every covered position is genotyped from ordered fp64 adds, so this kernel is bound by
-// instruction issue / the fp64 pipe rather than by HBM; see DESIGN.md.
+// k_norm_tiles_tma is bound by instruction issue / the fp64 pipe rather than by HBM; see DESIGN.md.
 #pragma once
 #include "kernels.cuh"
-
-#define HM_TILE_W 256
 
 struct NormOut { // device tallies
   unsigned long long ccs_tri[HM_TRI_BINS];
   unsigned long long ref_tri[HM_TRI_BINS];
   unsigned long long log[HM_NORM_LOG_LEN];
   unsigned long long alt_tie;
-  unsigned long long dbg[8]; // HM_NORM_DEBUG cycle counters
   int err;
 };
 
@@ -70,211 +65,11 @@ __device__ __forceinline__ int tri_bin_dev(const uint8_t* seq, uint64_t n, int64
   return t0 * 8 + (t1 == 3 ? 4 : 0) + t2;
 }
 
-__global__ void __launch_bounds__(HM_TILE_W) k_norm_tiles(DevBatch b, DevParams p, DevSets sets, DevLut lut, const hm_chunk* chunks,
-                                                          uint32_t n_chunks, const uint64_t* pair_off, const uint8_t* pair_flag,
-                                                          const uint64_t* tile_off, const uint8_t* refseq, uint64_t ref_len,
-                                                          NormOut* out) {
-  __shared__ double s_lut[3][256];
-  __shared__ unsigned long long s_ccs[HM_TRI_BINS], s_ref[HM_TRI_BINS], s_log[HM_NORM_LOG_LEN], s_tie;
-  __shared__ uint32_t s_rng[2];
-  for (int i = threadIdx.x; i < 768; i += blockDim.x) s_lut[i >> 8][i & 255] = __ldg(lut.lut + i);
-  if (threadIdx.x < HM_TRI_BINS) { s_ccs[threadIdx.x] = 0; s_ref[threadIdx.x] = 0; }
-  if (threadIdx.x < HM_NORM_LOG_LEN) s_log[threadIdx.x] = 0;
-  if (threadIdx.x == 0) s_tie = 0;
-
-  const uint32_t c = upper_bound_dev(tile_off, n_chunks + 1, (uint64_t)blockIdx.x) - 1;
-  const hm_chunk ch = chunks[c];
-  const int32_t t0 = ch.start + (int32_t)(blockIdx.x - tile_off[c]) * HM_TILE_W;
-  const int32_t t1 = min(t0 + HM_TILE_W, ch.end);
-  const int32_t pos = t0 + (int32_t)threadIdx.x;
-  const bool live = pos < t1 && pos >= 0 && (uint64_t)pos < ref_len;
-  if (threadIdx.x == 0) {
-    // reads that can touch [t0, t1]: running-max(tend) >= t0, tstart < t1, inside the chunk's range
-    uint32_t lo = lower_bound_dev(b.pmax_tend, (uint32_t)b.n_reads, t0);
-    uint32_t hi = lower_bound_dev(b.tstart, (uint32_t)b.n_reads, t1);
-    s_rng[0] = max(lo, ch.read_lo);
-    s_rng[1] = min(hi, ch.read_hi);
-  }
-  __syncthreads();
-  const uint32_t r_lo = s_rng[0], r_hi = s_rng[1];
-  const int lane = threadIdx.x & 31;
-  const int32_t wp0 = t0 + (int32_t)(threadIdx.x & ~31); // first position of this warp
-  const int w = p.mismatch_window;
-
-  int cnt[6] = {0, 0, 0, 0, 0, 0};
-  double S[4][3];
-#pragma unroll
-  for (int a = 0; a < 4; a++) { S[a][0] = 0.0; S[a][1] = 0.0; S[a][2] = 0.0; }
-  int callable = 0, h0 = 0, h1 = 0;
-  bool bq_zero = false;
-
-  for (uint32_t r = r_lo; r < r_hi; r++) {
-    const uint32_t pf = pair_flag[pair_off[c] + (r - ch.read_lo)];
-    if (!(pf & HM_PF_FETCHED)) continue;
-    const int32_t ts = b.tstart[r], te = b.tend[r];
-    if (ts > wp0 + 31 || te < wp0) continue; // warp-uniform: the read misses these 32 positions
-    const uint64_t o0 = b.op_off[r];
-    const uint32_t nops = b.n_ops[r];
-    if (nops == 0) continue;
-    // warp-uniform: first op that can matter for the warp (last op with op_t <= offset of wp0)
-    const uint32_t woff = (uint32_t)max(wp0 - ts, 0);
-    uint32_t klo = 0, khi = nops;
-    while (klo < khi) {
-      const uint32_t mid = (klo + khi) >> 1;
-      if (__ldg(b.op_t + o0 + mid) <= woff) klo = mid + 1; else khi = mid;
-    }
-    uint32_t k = klo - 1;
-    // an insertion recorded at offset woff precedes op k: step back over equal offsets
-    while (k > 0 && __ldg(b.op_t + o0 + k - 1) == woff) k--;
-    // warp-uniform mismatch-list slice near these positions (window <= 2w either side, 1-based list)
-    const int32_t* mm = b.mm_pos + o0;
-    const uint32_t nmm = (uint32_t)b.n_mm[r];
-    const uint32_t m_lo = lower_bound_dev(mm, nmm, wp0 - 2 * w - 1);
-    const uint32_t m_hi = upper_bound_dev(mm, nmm, wp0 + 31 + 2 * w + 2);
-
-    if (!live || pos < ts || pos > te) continue;
-    const uint32_t off = (uint32_t)(pos - ts);
-    // advance to the last op with op_t <= off, counting insertions at off on the way
-    int ins = 0;
-    uint32_t kk = k;
-    uint32_t w_op = __ldg(b.ops + o0 + kk), t_op = __ldg(b.op_t + o0 + kk);
-    for (;;) {
-      if (t_op == off && (w_op & 3u) == HM_OP_INS) ins++;
-      if (kk + 1 >= nops) break;
-      const uint32_t t_next = __ldg(b.op_t + o0 + kk + 1);
-      if (t_next > off) break;
-      kk++; w_op = __ldg(b.ops + o0 + kk); t_op = t_next;
-    }
-    cnt[4] += ins;
-    const uint32_t kind = w_op & 3u, v = w_op >> 2;
-    const uint32_t rl = (uint32_t)op_ref_len(w_op);
-    if (rl == 0 || off >= t_op + rl) continue; // position tend with a trailing insertion only
-    if (kind == HM_OP_DEL) { cnt[5]++; continue; }
-    const uint32_t q0 = __ldg(b.op_q + o0 + kk);
-    const uint32_t q = q0 + (kind == HM_OP_MATCH ? off - t_op : 0u);
-    const int bq = b.bq[b.bq_off[r] + q];
-    const int a = kind == HM_OP_SUB ? (int)((v >> 3) & 3u) : (int)((b.seq[b.seq_off[r] + (q >> 2)] >> (2 * (q & 3u))) & 3u);
-    if (bq == 0) bq_zero = true;
-    const double x0 = s_lut[0][bq], x1 = s_lut[1][bq], x2 = s_lut[2][bq];
-#pragma unroll
-    for (int x = 0; x < 4; x++) {
-      if (a == x) {
-        cnt[x]++;
-        S[x][0] = __dadd_rn(S[x][0], x0); S[x][1] = __dadd_rn(S[x][1], x1); S[x][2] = __dadd_rn(S[x][2], x2);
-      }
-    }
-    const int hap = (int)(pf >> HM_PF_HAP_SHIFT) & 3;
-    if (hap == 0) h0++; else if (hap == 1) h1++;
-    if (!(pf & HM_PF_PASS)) continue;
-    // update_tri2count (normcounts.py:65-110)
-    if (kind == HM_OP_SUB) { callable++; continue; }
-    if (bq < p.min_bq) continue;
-    const int32_t qlen = b.qlen[r];
-    {
-      const double trim_s = floor(__dmul_rn(p.min_trim, (double)qlen));
-      const double trim_e = ceil(__dmul_rn(__dsub_rn(1.0, p.min_trim), (double)qlen));
-      if ((double)q < trim_s || (double)q > trim_e) continue;
-    }
-    if (m_lo < m_hi) {
-      // window of the match block, anchored at its start and shifted by j (0-based rpos, 1-based list)
-      const int32_t rpos0 = ts + (int32_t)t_op, qpos0 = (int32_t)q0, j = (int32_t)(off - t_op);
-      const int qs = qpos0 - w, qe = qpos0 + w;
-      int u, d;
-      if (qs < 0) { u = w + qs; d = w + (-qs); }
-      else if (qe > qlen) { u = w + (qe - qlen); d = qlen - qpos0; }
-      else { u = w; d = w; }
-      const int32_t lo = rpos0 - u + j, hi = rpos0 + d + j;
-      int mc = 0;
-      for (uint32_t m = m_lo; m < m_hi; m++) { const int32_t x = __ldg(mm + m); mc += (x >= lo && x <= hi); }
-      if (mc > p.max_mismatch_count) continue;
-    }
-    callable++;
-  }
-
-  // ---- position loop body (normcounts.py:317-400) ----
-  unsigned long long lg[HM_NORM_LOG_LEN];
-#pragma unroll
-  for (int i = 0; i < HM_NORM_LOG_LEN; i++) lg[i] = 0;
-  int tri = -1;
-  bool tie_alt = false;
-  const int ridx = live ? (refseq[pos] == 'A' ? 0 : refseq[pos] == 'T' ? 1 : refseq[pos] == 'G' ? 2 : refseq[pos] == 'C' ? 3 : -1) : -1;
-  if (ridx >= 0 && callable > 0) {
-    const unsigned long long ts_ = (unsigned long long)callable;
-    lg[1] = ts_;
-    bool go = true;
-    if (p.phase && !(h0 >= p.min_hap_count && h1 >= p.min_hap_count)) { lg[2] = ts_; go = false; }
-    if (go) {
-      double pl[10];
-#pragma unroll
-      for (int g = 0; g < 10; g++) pl[g] = gt_pl_dev(S, g, ridx, -1);
-      int gq; bool tie;
-      const int best = argmin_gt_dev(pl, &gq, &tie);
-      const int state = gt_state_dev(c_gt_b1[best], c_gt_b2[best], ridx);
-      const int depth = cnt[0] + cnt[1] + cnt[2] + cnt[3] + cnt[5];
-      const int ref_count = cnt[ridx];
-      if (state == 1) lg[3] = ts_;
-      else if (state == 2) lg[4] = ts_;
-      else if (state == 3) lg[5] = ts_;
-      else {
-        lg[6] = ts_;
-        if (cnt[5] != 0 || cnt[4] != 0) lg[7] = ts_;
-        else if ((double)depth > p.md_threshold) lg[8] = ts_;
-        else if (depth == ref_count) {
-          if (gq < p.min_gq) lg[10] = ts_;
-          else if (ref_count < p.min_ref_count) lg[9] = ts_;
-          else tri = tri_bin_dev(refseq, ref_len, pos);
-        } else {
-          // alts in canonical A,T,G,C order (the reference iterates a set: order flagged, not guessed)
-          bool filtered = false;
-          int alt = -1, amax = -1, nmax = 0;
-#pragma unroll
-          for (int x = 0; x < 4; x++) {
-            if (x == ridx || filtered) continue;
-            if (cnt[x] > 0) {
-              const uint64_t key = ((uint64_t)(uint32_t)(pos + 1) << 4) | ((uint64_t)ridx << 2) | (uint64_t)x;
-              if (!p.non_human_sample && key_in_dev(sets.pon, sets.n_pon, key)) { lg[11] = ts_; filtered = true; }
-              else if (!p.non_human_sample && key_in_dev(sets.common, sets.n_common, key)) { lg[12] = ts_; filtered = true; }
-            }
-            if (cnt[x] > amax) { amax = cnt[x]; alt = x; nmax = 1; }
-            else if (cnt[x] == amax) nmax++;
-          }
-          if (!filtered) {
-            tie_alt = nmax > 1;
-#pragma unroll
-            for (int g = 0; g < 10; g++) pl[g] = gt_pl_dev(S, g, ridx, alt); // get_germ_gq(alt 1-char)
-            int gq2; bool tie2;
-            argmin_gt_dev(pl, &gq2, &tie2);
-            if (gq2 < p.min_gq) lg[10] = ts_;
-            else if (!(ref_count >= p.min_ref_count && cnt[alt] >= p.min_alt_count)) lg[9] = ts_;
-            else tri = tri_bin_dev(refseq, ref_len, pos);
-          }
-        }
-      }
-    }
-    if (tri >= 0) lg[13] = ts_;
-  }
-  // ---- CTA tallies: warp reduce the counters, shared atomics for the bins ----
-#pragma unroll
-  for (int i = 1; i < HM_NORM_LOG_LEN; i++) {
-    unsigned long long v = lg[i];
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(HM_FULL, v, d);
-    if (lane == 0 && v) atomicAdd(&s_log[i], v);
-  }
-  if (tri >= 0) { atomicAdd(&s_ref[tri], 1ull); atomicAdd(&s_ccs[tri], (unsigned long long)callable); }
-  if (tie_alt) atomicAdd(&s_tie, 1ull);
-  if (bq_zero && ridx >= 0 && callable > 0) out->err = HM_ERR_BQ_ZERO;
-  __syncthreads();
-  if (threadIdx.x < HM_TRI_BINS) {
-    if (s_ccs[threadIdx.x]) atomicAdd(&out->ccs_tri[threadIdx.x], s_ccs[threadIdx.x]);
-    if (s_ref[threadIdx.x]) atomicAdd(&out->ref_tri[threadIdx.x], s_ref[threadIdx.x]);
-  }
-  if (threadIdx.x < HM_NORM_LOG_LEN && s_log[threadIdx.x]) atomicAdd(&out->log[threadIdx.x], s_log[threadIdx.x]);
-  if (threadIdx.x == 0 && s_tie) atomicAdd(&out->alt_tie, s_tie);
-}
-
 // ============================================================================ k_norm_tiles_tma
-// Warp-specialised, persistent version of k_norm_tiles.
+// Warp-specialised and persistent.  The tile's reads are walked in file order, so each thread sees "its" column of
+// the pileup in the reference's append order (6 allele counts, the ordered fp64 sums of the genotype model, the
+// callable-read count of update_tri2count, normcounts.py:65-110, and the haplotype counts); then the thread genotypes
+// its position and runs the filter cascade (normcounts.py:317-400).
 //   producer warp: for the tile's reads, 32 at a time (one lane per read), finds the slice of the
 //     op stream and of the mismatch list that touches the tile (8-ary searches), writes a compact
 //     descriptor into shared memory and stages the read's quality bytes and 2-bit bases for the
@@ -537,13 +332,7 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
       do {
         if (batch_no % HM_NPROD != pw) { batch_no++; r0 += HM_SLOTS; continue; }
         const uint32_t st = batch_no % HM_NSTAGE, ph = (batch_no / HM_NSTAGE) & 1;
-#ifdef HM_NORM_DEBUG
-        const long long c0 = clock64();
-#endif
         mbar_wait_backoff(&empty_bar[st], ph ^ 1);
-#ifdef HM_NORM_DEBUG
-        const long long c1 = clock64();
-#endif
         TileStage* T = &stages[st];
         const uint32_t r = r0 + lane;
         const uint32_t nb = min(r_hi > r0 ? r_hi - r0 : 0u, (uint32_t)HM_SLOTS);
@@ -554,9 +343,6 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
         } else {
           mbar_arrive(&full_bar[st]);
         }
-#ifdef HM_NORM_DEBUG
-        if (lane == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[0], (unsigned long long)(c1 - c0)); atomicAdd(&out->dbg[1], (unsigned long long)(clock64() - c1)); atomicAdd(&out->dbg[2], 1ull); }
-#endif
         batch_no++;
         r0 += HM_SLOTS;
       } while (r0 < r_hi);
@@ -589,13 +375,7 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
 
     for (;;) {
       const uint32_t st = batch_no % HM_NSTAGE, ph = (batch_no / HM_NSTAGE) & 1;
-#ifdef HM_NORM_DEBUG
-      const long long d0 = clock64();
-#endif
       mbar_wait(&full_bar[st], ph);
-#ifdef HM_NORM_DEBUG
-      const long long d1 = clock64();
-#endif
       const TileStage* T = &stages[st];
       const int nslots = T->n_slots;
       const int last = T->last;
@@ -710,16 +490,10 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(&empty_bar[st]);
-#ifdef HM_NORM_DEBUG
-      if (tid == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[3], (unsigned long long)(d1 - d0)); atomicAdd(&out->dbg[4], (unsigned long long)(clock64() - d1)); atomicAdd(&out->dbg[5], (unsigned long long)nslots); }
-#endif
       batch_no++;
       if (last) break;
     }
 
-#ifdef HM_NORM_DEBUG
-    const long long e0 = clock64();
-#endif
     // ---- position loop body (normcounts.py:317-400) ----
     // every counted position adds its callable count to log[1] and to exactly one more counter
     // (cat1 in 2..6); homref positions (cat1 == 6) to one of 7..13 as well (cat2)
@@ -839,9 +613,6 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
       atomicAdd(&s_ccs[32], (unsigned long long)atomicExch(&s_wccs[tid >> 5][32], 0u));
       atomicAdd(&s_ref[32], (unsigned long long)atomicExch(&s_wref[tid >> 5][32], 0u));
     }
-#ifdef HM_NORM_DEBUG
-    if (tid == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[6], (unsigned long long)(clock64() - e0)); atomicAdd(&out->dbg[7], 1ull); }
-#endif
   }
   // fold the per-warp bins
   for (int i = lane; i < HM_TRI_BINS; i += 32) {

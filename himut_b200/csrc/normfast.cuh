@@ -1,652 +1,20 @@
-// normfast.cuh — two-pass callable-base half of `himut normcounts` on sm_100a
-// (normcounts.get_callable_tricounts, src/himut/normcounts.py:240-419).
+// normfast.cuh — exact pass of the callable-base half of `himut normcounts` on sm_100a
+// (normcounts.get_callable_tricounts, src/himut/normcounts.py:240-419), and `himut phase` edge counting.
 //
-// The reference genotypes every covered position from ordered fp64 sums (gtlib.py:72-135).  At
-// the vast majority of positions every read shows the reference base through a plain cs match
-// and the verdict of that arithmetic is never in doubt.  So the work is split:
+// The integer pass in front of it (k_norm_bits, normbits.cuh) settles every pure position whose verdict is certified
+// and lists the others (about 1-2 % of the positions) as sites:
 //
-//   k_norm_fast     streaming pass, integer only.  One thread owns 4 consecutive reference
-//                   positions; reads of a 2048-position tile are staged by producer warps (TMA
-//                   1-D bulk copies of the quality bytes and 2-bit bases + a descriptor with two
-//                   2048-bit masks) and walked in file order.  Per position it keeps, packed four
-//                   to a register: depth n, sum of BQ, callable count (update_tri2count,
-//                   normcounts.py:65-110) and the two haplotype tallies.  A position is *pure*
-//                   when every covering read is a plain matched base equal to the FASTA base.
-//                   For a pure position the ten PL collapse to four values that depend on
-//                   (n, sum BQ, sum log10(1 - eps)) only; the kernel decides homref + GQ >= min_gq
-//                   from certified bounds (see norm_cert below).  Whatever is not pure, or not
-//                   certified, is appended to a site list.
-//   k_norm_entries / k_norm_reduce
-//                   exact pass over the listed sites (about 1-2 % of the positions): the pileup
-//                   column gathered with one thread per (site, read), then per site in file
-//                   order the ordered fp64 sums, ten PL, argmin, GQ and the cascade exactly as
-//                   k_norm_tiles does it.
+//   k_norm_site_range   per site: the file-order range of the chunk's reads that can touch it;
+//   k_norm_entries_bits (normbits.cuh) gathers the pileup column, one warp per (chunk, read); a read it cannot
+//                       stage is answered by norm_entry;
+//   k_norm_reduce       per site in file order: the ordered fp64 sums, ten PL, argmin, GQ and the cascade exactly as
+//                       k_norm_tiles_tma does it.
 //
-// Both passes add into the same NormOut tallies, so the result is bit-identical to evaluating
-// every position exactly (k_norm_tiles_tma, kept as the fallback for parameters outside the
-// certified domain and as the A/B baseline: HIMUT_B200_NORM_V2=1).
+// Both passes add into the same NormOut tallies, so the result is bit-identical to evaluating every position exactly
+// (k_norm_tiles_tma, normcounts.cuh, which runs instead where the bit vectors do not apply: parameters outside the
+// certified domain, a chunk that starts below position 0, 2^32 or more cal words in one batch).
 #pragma once
 #include "normcounts.cuh"
-
-#define HF_TW 2048                         // positions per tile
-#define HF_CONS (HF_TW / 4)                // consumer threads, 4 positions each
-#define HF_NSTAGE 4
-#define HF_NSPLIT 2                        // producer warps that share one stage (each fills HF_SLOTS / HF_NSPLIT slots)
-#define HF_NPROD (HF_NSTAGE * HF_NSPLIT)   // producer warps: a lane's work is serial, so throughput comes from the warp count
-#define HF_SLOTS 16                        // reads per stage
-#define HF_PAD 16                          // bytes of slack in front of the staged data (64 bases)
-#define HF_BQ_BUF (HF_PAD + HF_TW + 128)   // staged quality bytes per read
-#define HF_SEQ_BUF (HF_PAD + HF_TW / 4 + 48)
-#define HF_MAX_SEG 6                       // runs of constant (query - reference) offset per read and tile
-#ifndef HF_WAIT_NS
-#define HF_WAIT_NS 128
-#endif
-#define HF_MAX_WALK 1024                   // ops x mismatches a producer lane is willing to fold
-
-// Certified verdict of the genotype model at a pure position (host-computed from hm_params, see
-// make_norm_cert in himut_b200.cu).  With n reads of the reference allele r and qualities b_i:
-//   PL_rr     = -10 (M0 + lp_homref)        M0 = sum lut_hom[b_i]
-//   PL_het    = -10 (M1 + lp_het)           M1 = sum lut_het[b_i]   (= M0 - n log10 2 up to 1e-13)
-//   PL_hetalt = -10 (M2 + lp_hetalt)        M2 = sum lut_err[b_i]   (= -sum b_i / 30 up to 1e-13)
-//   PL_homalt = -10 (M2 + lp_homalt)
-// every other genotype equals one of these four (adding exact zeros is exact).  Homref is the
-// argmin and GQ = int(second - best) >= min_gq iff both differences are >= max(min_gq, 0) and > 0:
-//   PL_het - PL_rr      = 10 n log10 2 + 10 (lp_homref - lp_het)                    -> n >= n_min
-//   PL_other - PL_rr   >= 10 (sum b_i / 30 - f1 * x / 254) + 10 (lp_homref - max(lp_hetalt, lp_homalt))
-//     with x = min(254 n, 255 n - sum b_i), f1 = -lut_hom[1]: -lut_hom is convex and decreasing,
-//     so -M0 <= f1 * (255 n - sum b_i) / 254 and trivially <= f1 * n  (all b_i >= 1).
-// `margin` keeps the comparison away from the fp64 rounding of the reference's own sums (1e-9 at
-// most for depth <= 255); a position that fails the test is simply evaluated exactly.
-struct NormCert {
-  int32_t enabled;
-  int32_t n_min;       // smallest depth whose het - homref difference is certified
-  double a_bq;         // 10 / 30
-  double a_x;          // 10 * f1 / 254
-  double c_oth;        // 10 (lp_homref - max(lp_hetalt, lp_homalt))
-  double need;         // max(min_gq, 0) + margin
-  long long ia_bq, ia_x, i_need; // floor(a_bq 2^20), ceil(a_x 2^20), ceil((need - c_oth) 2^20)
-};
-
-struct __align__(16) FastSlot {
-  uint8_t bq[HF_BQ_BUF];
-  uint8_t seq[HF_SEQ_BUF];
-  uint2 mask[HF_TW / 32];              // x special, y blocked
-  uint4 head;                          // x flags | n_seg << 16, y cov_lo | cov_hi << 16, z q_base, w delta of run 0
-  int32_t seg_start[HF_MAX_SEG + 2];
-  int32_t seg_delta[HF_MAX_SEG + 2];
-  // per consumer warp (128 positions): x = class | flags << 8, y = delta - q_base + 64 of the run the chunk lies in.
-  // class 0: the read neither covers the chunk nor has special bits there; 1: plain — fully covered, no special and
-  // no blocked position, one run; 2: everything else (general path)
-  uint2 chunk[HF_CONS / 32];
-};
-struct __align__(16) FastStage {
-  FastSlot slot[HF_SLOTS];
-  int32_t n_slots, last, deep, pad;
-};
-
-// set bits [lo, hi) of mask word `which` (0 special, 1 blocked); single writer.  *touch collects which
-// 128-position chunks received bits
-__device__ __forceinline__ void fmask_set(uint2* m, int which, int32_t lo, int32_t hi, uint32_t* touch) {
-  if (lo < 0) lo = 0;
-  if (hi > HF_TW) hi = HF_TW;
-  if (lo >= hi) return;
-  *touch |= (2u << ((hi - 1) >> 7)) - (1u << (lo >> 7));
-  uint32_t* w = reinterpret_cast<uint32_t*>(m) + which;
-  while (lo < hi) {
-    const int32_t wi = lo >> 5, b0 = lo & 31, n = min(32 - b0, hi - lo);
-    w[2 * wi] |= (n == 32 ? 0xffffffffu : ((1u << n) - 1u)) << b0;
-    lo += n;
-  }
-}
-__device__ __forceinline__ void fmask_clear(uint2* m, int which, int32_t lo, int32_t hi) {
-  if (lo < 0) lo = 0;
-  if (hi > HF_TW) hi = HF_TW;
-  uint32_t* w = reinterpret_cast<uint32_t*>(m) + which;
-  while (lo < hi) {
-    const int32_t wi = lo >> 5, b0 = lo & 31, n = min(32 - b0, hi - lo);
-    w[2 * wi] &= ~((n == 32 ? 0xffffffffu : ((1u << n) - 1u)) << b0);
-    lo += n;
-  }
-}
-
-// ============================================================================ k_tile_index
-// Per read, for every 2048-aligned tile g it can touch (g = tstart >> 11 .. tend >> 11): the slice of its op
-// stream and of its mismatch list that matters for the tile, so the producers of k_norm_fast fetch it with one
-// 16-byte load instead of four searches.  x = first op, y = one past the last op, z / w = mismatch-list slice
-// (entries within 2 * window + 2 of the tile).  One warp per read, lanes over tiles.
-__global__ void __launch_bounds__(256) k_tile_index(DevBatch b, int32_t window, const uint32_t* tix_off, uint4* tix) {
-  const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (r >= b.n_reads) return;
-  const int32_t ts = b.tstart[r], te = b.tend[r];
-  const uint32_t n = b.n_ops[r];
-  const uint64_t o0 = b.op_off[r];
-  const uint32_t nmm = (uint32_t)b.n_mm[r];
-  const uint32_t reflen = (uint32_t)(te - ts);
-  const int32_t g0 = ts >> 11, g1 = te >> 11;
-  for (int32_t g = g0 + lane; g <= g1; g += 32) {
-    const int32_t t0 = g << 11;
-    uint4 e = make_uint4(0u, 0u, 0u, 0u);
-    if (n > 0) {
-      const uint32_t woff = (uint32_t)max(t0 - ts, 0);
-      const uint32_t eoff = min((uint32_t)(t0 + HF_TW - 1 - ts), reflen);
-      uint32_t k0 = count_le_kary(b.op_t + o0, n, woff) - 1;
-      while (k0 > 0 && __ldg(b.op_t + o0 + k0 - 1) == woff) k0--;
-      e.x = k0;
-      e.y = count_le_kary(b.op_t + o0, n, eoff);
-      e.z = count_le_kary_i32(b.mm_pos + o0, nmm, t0 - 2 * window - 2);
-      e.w = count_le_kary_i32(b.mm_pos + o0, nmm, t0 + HF_TW + 2 * window + 2);
-    }
-    tix[(uint64_t)tix_off[r] + (uint32_t)(g - g0)] = e;
-  }
-}
-
-// Per tile of the fast pass: its chunk, origin on the 2048 grid and the file-order range of reads that can touch
-// it (running-max(tend) >= first position, tstart < end), so that neither the producer nor the consumer warps of
-// k_norm_fast search for them.  One thread per tile.
-__global__ void __launch_bounds__(256) k_tile_ranges(DevBatch b, const hm_chunk* chunks, uint32_t n_chunks, const uint64_t* tile_off,
-                                                     uint32_t n_tiles, uint4* tile_info) {
-  const uint32_t tile = blockIdx.x * blockDim.x + threadIdx.x;
-  if (tile >= n_tiles) return;
-  const uint32_t c = upper_bound_dev(tile_off, n_chunks + 1, (uint64_t)tile) - 1;
-  const hm_chunk ch = chunks[c];
-  const int32_t t0 = ((ch.start >> 11) + (int32_t)(tile - tile_off[c])) << 11;
-  const int32_t lo_pos = max(t0, ch.start), t1 = min(t0 + HF_TW, ch.end);
-  const uint32_t n_in = ch.read_hi - ch.read_lo;
-  const uint32_t r_lo = ch.read_lo + count_le_kary_i32(b.pmax_tend + ch.read_lo, n_in, lo_pos - 1);
-  const uint32_t r_hi = ch.read_lo + count_le_kary_i32(b.tstart + ch.read_lo, n_in, t1 - 1);
-  tile_info[tile] = make_uint4(c, (uint32_t)t0, r_lo, r_hi);
-}
-
-#define HF_SCR_OPS 128   // ops of one read inside one tile the producer stages (3 words each) ...
-#define HF_SCR_MM 128    // ... and mismatch-list entries near the tile; both live in the slot's bq buffer until the TMA lands
-
-// producer lane: descriptor + bulk copies of read r for tile [t0, t1).
-// Global loads are grouped into three dependent rounds (read metadata; op_t / mismatch list scans; the tile's
-// op triples and mismatch entries, parked in the slot's own staging buffer), because a lane's time is load latency.
-#ifdef HM_NORM_DEBUG
-__device__ unsigned long long g_fill_dbg[8];
-#define FILL_T(i) do { const long long t_ = clock64(); if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) atomicAdd(&g_fill_dbg[i], (unsigned long long)(t_ - tp_)); tp_ = t_; } while (0)
-#else
-#define FILL_T(i)
-#endif
-__device__ __forceinline__ void fast_fill_slot(const DevBatch& b, const DevParams& p, const uint32_t* tix_off, const uint4* tix,
-                                               FastSlot* S, uint64_t* full_bar, uint32_t r, uint32_t pf, int32_t t0, int32_t lo_pos,
-                                               int32_t t1) {
-  // The lanes of a producer warp walk different reads; every phase below ends in a __syncwarp over the lanes that
-  // entered, so the warp executes the longest path of a phase once instead of one lane group after the other.
-  const unsigned fm = __activemask();
-#ifdef HM_NORM_DEBUG
-  long long tp_ = clock64();
-#endif
-  // round 1: everything addressed by r
-  const int32_t ts = __ldg(b.tstart + r), te = __ldg(b.tend + r);
-  const uint32_t n = __ldg(b.n_ops + r);
-  const uint64_t o0 = __ldg(b.op_off + r);
-  const int32_t qlen = __ldg(b.qlen + r);
-  const uint64_t bq_off = __ldg(b.bq_off + r), seq_off = __ldg(b.seq_off + r);
-  const uint32_t tx0 = __ldg(tix_off + r);
-  uint32_t sp_touch = 0, bl_touch = 0;
-  uint32_t nb_bq = 0, nb_seq = 0, cov = 1u, q_base = 0, nseg = 0;
-  int32_t delta0 = 0;
-  const uint8_t *src_bq = nullptr, *src_seq = nullptr;
-  const bool act = (pf & HM_PF_FETCHED) && ts < t1 && te >= lo_pos && n > 0;
-  const uint32_t flags = act ? (pf & 0xffu) : 0u;
-  const int32_t* mm = b.mm_pos + o0;
-  const int w = p.mismatch_window;
-  FILL_T(0);
-  // round 2: the read's slice for this tile (k_tile_index)
-  uint4 te4 = make_uint4(0u, 0u, 0u, 0u);
-  if (act) te4 = __ldg(tix + (uint64_t)tx0 + (uint32_t)((t0 >> 11) - (ts >> 11)));
-  const uint32_t k0 = te4.x, m_lo = te4.z;
-  uint32_t ns = te4.y - te4.x, nmv = te4.w - te4.z;
-  bool slow = act && (ns > HF_SCR_OPS || nmv > HF_SCR_MM || (uint64_t)ns * (uint64_t)(nmv + 1) > HF_MAX_WALK);
-  if (slow) { ns = 0; nmv = 0; }
-  // round 3: park the op triples and the mismatch entries in shared memory
-  uint32_t* scr = reinterpret_cast<uint32_t*>(S->bq);
-  int32_t* smm = reinterpret_cast<int32_t*>(S->bq) + 3 * HF_SCR_OPS;
-#pragma unroll 4
-  for (uint32_t i = 0; i < ns; i++) {
-    scr[3 * i] = __ldg(b.ops + o0 + k0 + i); scr[3 * i + 1] = __ldg(b.op_t + o0 + k0 + i); scr[3 * i + 2] = __ldg(b.op_q + o0 + k0 + i);
-  }
-#pragma unroll 4
-  for (uint32_t m = 0; m < nmv; m++) smm[m] = __ldg(mm + m_lo + m);
-  uint4* mz = reinterpret_cast<uint4*>(S->mask);
-  if (act) {
-#pragma unroll 4
-    for (int i = 0; i < (int)(sizeof(S->mask) / 16); i++) mz[i] = make_uint4(0u, 0u, 0u, 0u);
-  }
-  __syncwarp(fm);
-  FILL_T(2);
-  const int32_t trim_s = (int32_t)floor(__dmul_rn(p.min_trim, (double)qlen));
-  const int32_t trim_e = (int32_t)ceil(__dmul_rn(__dsub_rn(1.0, p.min_trim), (double)qlen));
-  const int32_t W = HF_TW; // bits beyond the chunk's end land on positions the consumers never count
-  int32_t cur_delta = INT32_MIN, q_lo = 0, q_hi = 0, last_bgroup = -1;
-  bool have_q = false;
-  // a matched base is not callable when a mismatch lies within the window of its block (normcounts.py:82-94).
-  // For every block but those starting within `w` of a read end the window is (w, w): one range per mismatch,
-  // laid over the whole read here; the edge blocks are redone with their own (u, d) below.
-  if (p.max_mismatch_count == 0)
-    for (uint32_t m = 0; m < nmv; m++) { const int32_t x = smm[m]; fmask_set(S->mask, 1, x - w - t0, x + w - t0 + 1, &bl_touch); }
-  __syncwarp(fm);
-  const uint32_t ns_max = __reduce_max_sync(fm, ns);
-  for (uint32_t i = 0; i < ns_max; i++) {
-    if (i < ns && !slow) {
-      const uint32_t wd = scr[3 * i], ot = scr[3 * i + 1];
-      const uint32_t kind = wd & 3u;
-      const int32_t a = ts + (int32_t)ot - t0, rl = op_ref_len(wd);
-      if (kind == HM_OP_MATCH) {
-        const int32_t lo_p = max(a, 0), hi_p = min(a + rl, W);
-        if (lo_p < hi_p) {
-          const int32_t qpos0 = (int32_t)scr[3 * i + 2], delta = qpos0 - a;
-          if (delta != cur_delta) {
-            if (nseg == HF_MAX_SEG) slow = true;
-            else {
-              S->seg_start[nseg] = lo_p; S->seg_delta[nseg] = delta;
-              if (nseg == 0) delta0 = delta;
-              else if (lo_p & 3) {
-                // a run that starts inside a 4-position group: the consumer blends the two offsets (one boundary per
-                // group); a second boundary in the same group sends the rest of the group to the exact pass
-                if (last_bgroup == (lo_p >> 2)) fmask_set(S->mask, 0, lo_p, (lo_p + 3) & ~3, &sp_touch);
-                last_bgroup = lo_p >> 2;
-              }
-              nseg++; cur_delta = delta;
-            }
-          }
-          if (!have_q) { q_lo = lo_p + delta; have_q = true; }
-          q_hi = hi_p + delta;
-          // bamlib.get_mismatch_range anchored at the block start (normcounts.py:82)
-          const int qs = qpos0 - w, qe2 = qpos0 + w;
-          int u, d;
-          if (qs < 0) { u = w + qs; d = w + (-qs); }
-          else if (qe2 > qlen) { u = w + (qe2 - qlen); d = qlen - qpos0; }
-          else { u = w; d = w; }
-          if (p.max_mismatch_count == 0) {
-            if (u != w || d != w) {
-              fmask_clear(S->mask, 1, lo_p, hi_p);
-              for (uint32_t m = 0; m < nmv; m++) {
-                const int32_t x = smm[m];
-                fmask_set(S->mask, 1, max(x - d - t0, lo_p), min(x + u - t0 + 1, hi_p), &bl_touch);
-              }
-            }
-          } else if (nmv > (uint32_t)p.max_mismatch_count) {
-            // general threshold: count per position (rare setting; window reach is small)
-            if ((uint64_t)(hi_p - lo_p) * nmv > 4 * HF_MAX_WALK) slow = true;
-            else
-              for (int32_t pp = lo_p; pp < hi_p; pp++) {
-                int mc = 0;
-                for (uint32_t m = 0; m < nmv; m++) { const int32_t x = smm[m]; mc += (x >= t0 + pp - u && x <= t0 + pp + d); }
-                if (mc > p.max_mismatch_count) fmask_set(S->mask, 1, pp, pp + 1, &bl_touch);
-              }
-          }
-          if (lo_p + delta < trim_s) fmask_set(S->mask, 1, lo_p, min(hi_p, trim_s - delta), &bl_touch);         // q < trim_s
-          if (hi_p - 1 + delta > trim_e) fmask_set(S->mask, 1, max(lo_p, trim_e - delta + 1), hi_p, &bl_touch); // q > trim_e
-        }
-      } else if (kind == HM_OP_DEL) {
-        fmask_set(S->mask, 0, max(a, 0), min(a + rl, W), &sp_touch);
-      } else if (a >= 0 && a < W) {
-        fmask_set(S->mask, 0, a, a + 1, &sp_touch); // substitution, or the base an insertion precedes
-      }
-    }
-    __syncwarp(fm);
-  }
-  FILL_T(3);
-  if (act) {
-    cov = (uint32_t)max(ts - t0, 0) | ((uint32_t)max(min(te - 1 - t0, W - 1), 0) << 16);
-    if (te - 1 < t0) cov = 1u; // lo 1 > hi 0: nothing aligned inside the tile (trailing insertion only)
-    if (!slow && have_q) {
-      const uint32_t qb = (uint32_t)q_lo & ~63u;
-      const uint32_t qe = min(((uint32_t)q_hi + 15u) & ~15u, ((uint32_t)qlen + 15u) & ~15u);
-      const uint32_t sb0 = qb >> 2;
-      const uint32_t sb1 = min((((((uint32_t)q_hi + 3u) >> 2) + 15u) & ~15u), (((((uint32_t)qlen + 3u) >> 2) + 15u) & ~15u));
-      q_base = qb;
-      if (qe - qb > HF_BQ_BUF - HF_PAD - 8 || sb1 - sb0 > HF_SEQ_BUF - HF_PAD - 8) slow = true;
-      else { nb_bq = qe - qb; nb_seq = sb1 - sb0; src_bq = b.bq + bq_off + qb; src_seq = b.seq + seq_off + sb0; }
-    }
-    if (slow) { // pathological read: every position of the tile goes to the exact pass
-#pragma unroll 4
-      for (int i = 0; i < (int)(sizeof(S->mask) / 16); i++) mz[i] = make_uint4(0xffffffffu, 0u, 0xffffffffu, 0u);
-      nb_bq = nb_seq = 0; nseg = 0; sp_touch = 0xffffu;
-    }
-  }
-  __syncwarp(fm);
-  S->head = make_uint4(flags | (nseg << 16), cov, q_base, (uint32_t)delta0);
-  {
-    const int cov_lo = (int)(cov & 0xffffu), cov_hi = (int)(cov >> 16);
-    // chunks the read touches at all / covers completely, as 16-bit masks
-    uint32_t any = 0, full = 0;
-    if (act && cov_hi >= cov_lo) {
-      any = (2u << (cov_hi >> 7)) - (1u << (cov_lo >> 7));
-      const int f_lo = (cov_lo + 127) >> 7, f_hi = ((cov_hi + 1) >> 7) - 1;
-      if (f_hi >= f_lo) full = (2u << f_hi) - (1u << f_lo);
-    }
-    const uint32_t plain = full & ~sp_touch & ~bl_touch, none = act ? (~any & ~sp_touch) : 0xffffu;
-    const int32_t dbase = 64 - (int32_t)q_base;
-    uint32_t sg = 0;
-#pragma unroll 4
-    for (int wi = 0; wi < HF_CONS / 32; wi++) {
-      const uint32_t cls = ((plain >> wi) & 1u) ? 1u : ((none >> wi) & 1u) ? 0u : 2u;
-      if (nseg > 1) while (sg + 1 < nseg && S->seg_start[sg + 1] <= wi * 128) sg++;
-      const int32_t dl = nseg > 1 ? S->seg_delta[sg] : delta0;
-      S->chunk[wi] = make_uint2(cls | (flags << 8), (uint32_t)(dl + dbase));
-    }
-  }
-  __syncwarp(fm);
-  FILL_T(4);
-  // the descriptor is complete: arrive (release) last, then let the bulk copies land on the barrier
-  if (nb_bq + nb_seq == 0) mbar_arrive(full_bar);
-  else {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // the scratch reads above precede the TMA writes
-    mbar_arrive_expect_tx(full_bar, nb_bq + nb_seq);
-    bulk_g2s(S->bq + HF_PAD, src_bq, nb_bq, full_bar);
-    bulk_g2s(S->seq + HF_PAD, src_seq, nb_seq, full_bar);
-  }
-  FILL_T(5);
-}
-
-// consumer-side wait: a warp that finds the stage not ready sleeps between probes, so that the 16 waiting
-// consumer warps leave the issue slots to the 4 producer warps they are waiting for
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0;
-  for (;;) {
-    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    if (ok) break;
-    __nanosleep(HF_WAIT_NS);
-  }
-}
-
-__device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; } // bit k -> bit 8k
-
-__global__ void __launch_bounds__(HF_CONS + 32 * HF_NPROD, 1)
-k_norm_fast(DevBatch b, DevParams p, NormCert cert, const hm_chunk* chunks, uint32_t n_chunks, const uint64_t* pair_off,
-            const uint8_t* pair_flag, const uint4* tile_info, uint32_t n_tiles, const uint32_t* tix_off, const uint4* tix,
-            const uint8_t* refseq, uint64_t ref_len,
-            NormOut* out, unsigned long long* sites, unsigned long long site_cap, unsigned long long* n_sites) {
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  FastStage* stages = reinterpret_cast<FastStage*>(smem_raw);
-  __shared__ uint64_t full_bar[HF_NSTAGE], empty_bar[HF_NSTAGE];
-  __shared__ unsigned long long s_ccs[HM_TRI_BINS], s_ref[HM_TRI_BINS], s_log[HM_NORM_LOG_LEN];
-  __shared__ unsigned int s_wccs[HF_CONS / 32][HM_TRI_BINS + 1], s_wref[HF_CONS / 32][HM_TRI_BINS + 1]; // per-warp bins
-  const int tid = threadIdx.x, lane = tid & 31;
-  const bool is_producer = tid >= HF_CONS;
-  for (int i = tid; i < (HF_CONS / 32) * (HM_TRI_BINS + 1); i += blockDim.x) { (&s_wccs[0][0])[i] = 0; (&s_wref[0][0])[i] = 0; }
-  if (tid < HM_TRI_BINS) { s_ccs[tid] = 0; s_ref[tid] = 0; }
-  if (tid < HM_NORM_LOG_LEN) s_log[tid] = 0;
-  if (tid == 0) {
-    for (int i = 0; i < HF_NSTAGE; i++) { mbar_init(&full_bar[i], HF_SLOTS); mbar_init(&empty_bar[i], HF_CONS / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-
-  uint32_t batch_no = 0; // same sequence on both sides
-  if (is_producer) {
-    // ------------------------------------------------------------------ producer warps
-    const uint32_t pw = (uint32_t)(tid - HF_CONS) >> 5;
-    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const uint4 ti = __ldg(tile_info + tile); // chunk, origin on the 2048 grid, read range (k_tile_ranges)
-      const uint32_t c = ti.x, r_lo = ti.z, r_hi = ti.w;
-      const hm_chunk ch = chunks[c];
-      const int32_t t0 = (int32_t)ti.y;
-      const int32_t lo_pos = max(t0, ch.start);
-      const int32_t t1 = min(t0 + HF_TW, ch.end);
-      const bool deep = r_hi > r_lo && r_hi - r_lo > 255u; // the packed 8-bit tallies would overflow
-      const uint64_t pbase = pair_off[c];
-      const uint32_t n_batches = (deep || r_hi <= r_lo) ? 1u : (r_hi - r_lo + HF_SLOTS - 1) / HF_SLOTS;
-      for (uint32_t bi = 0; bi < n_batches; bi++, batch_no++) {
-        if (batch_no % HF_NSTAGE != pw / HF_NSPLIT) continue; // warps pw / HF_NSPLIT == stage fill it together
-        const uint32_t st = batch_no % HF_NSTAGE, ph = (batch_no / HF_NSTAGE) & 1;
-        const uint32_t part = pw % HF_NSPLIT;
-#ifdef HM_NORM_DEBUG
-        const long long c0 = clock64();
-#endif
-        mbar_wait_backoff(&empty_bar[st], ph ^ 1);
-#ifdef HM_NORM_DEBUG
-        const long long c1 = clock64();
-#endif
-        FastStage* T = &stages[st];
-        const uint32_t r0 = r_lo + bi * HF_SLOTS;
-        const uint32_t slot = part * (HF_SLOTS / HF_NSPLIT) + (uint32_t)lane;
-        const uint32_t r = r0 + slot;
-        const uint32_t nb = deep ? 0u : min(r_hi > r0 ? r_hi - r0 : 0u, (uint32_t)HF_SLOTS);
-        if (lane == 0 && part == 0) { T->n_slots = (int32_t)nb; T->last = (bi + 1 == n_batches) ? 1 : 0; T->deep = deep ? 1 : 0; }
-        if (lane < HF_SLOTS / HF_NSPLIT) {
-          if (slot < nb) {
-            const uint32_t pf = pair_flag[pbase + (r - ch.read_lo)];
-            fast_fill_slot(b, p, tix_off, tix, &T->slot[slot], &full_bar[st], r, pf, t0, lo_pos, t1);
-          } else {
-            mbar_arrive(&full_bar[st]);
-          }
-        }
-        __syncwarp(); // idle lanes must not run ahead into the next wait: their polling would stall the working lanes
-#ifdef HM_NORM_DEBUG
-        if (lane == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[0], (unsigned long long)(c1 - c0)); atomicAdd(&out->dbg[1], (unsigned long long)(clock64() - c1)); atomicAdd(&out->dbg[2], 1ull); }
-#endif
-      }
-    }
-    return;
-  }
-
-  // -------------------------------------------------------------------- consumer warps
-  const int p0 = tid * 4;                 // first tile-relative position of this thread
-  const uint32_t sh4 = (uint32_t)(tid & 7) * 4u;
-  const uint32_t kge = (uint32_t)(128 - p.min_bq) * 0x01010101u; // byte >= min_bq  <=>  bit 7 of (byte & 0x7f) + 128 - min_bq, or of byte
-  for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const uint4 ti = __ldg(tile_info + tile);
-    const uint32_t c = ti.x;
-    const hm_chunk ch = chunks[c];
-    const int32_t t0 = (int32_t)ti.y;
-    const int32_t t1 = min(t0 + HF_TW, ch.end);
-    // reference bases pos-1 .. pos+4 now, so the loads hide behind the read loop
-    uint8_t rb[6];
-#pragma unroll
-    for (int k = 0; k < 6; k++) {
-      const int64_t q = (int64_t)t0 + p0 + k - 1;
-      rb[k] = (q >= 0 && (uint64_t)q < ref_len) ? __ldg(refseq + q) : (uint8_t)0;
-    }
-    uint32_t ref8 = 0, dead = 0; // 2-bit codes of the four reference bases; positions that are never counted
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const uint8_t ch_ = rb[k + 1];
-      const int code = ch_ == 'A' ? 0 : ch_ == 'T' ? 1 : ch_ == 'G' ? 2 : ch_ == 'C' ? 3 : -1;
-      const int64_t pos = (int64_t)t0 + p0 + k;
-      if (code < 0 || pos >= (int64_t)t1 || pos < (int64_t)ch.start || pos < 0 || (uint64_t)pos >= ref_len) dead |= 1u << k;
-      else ref8 |= (uint32_t)code << (2 * k);
-    }
-
-    uint32_t n4 = 0, s_lo = 0, s_hi = 0, c4 = 0, h0_4 = 0, h1_4 = 0, imp = 0;
-    uint32_t n_plain = 0, h0_plain = 0, h1_plain = 0, zacc = 0, misacc = 0; // plain chunks: uniform counts, deferred checks
-    bool deep = false;
-    for (;;) {
-      const uint32_t st = batch_no % HF_NSTAGE, ph = (batch_no / HF_NSTAGE) & 1;
-#ifdef HM_NORM_DEBUG
-      const long long d0 = clock64();
-#endif
-      mbar_wait_sleep(&full_bar[st], ph);
-#ifdef HM_NORM_DEBUG
-      const long long d1 = clock64();
-#endif
-      const FastStage* T = &stages[st];
-      const int nslots = T->n_slots;
-      const int last = T->last;
-      deep |= T->deep != 0;
-      for (int si = 0; si < nslots; si++) {
-        const FastSlot* S = &T->slot[si];
-        const uint2 ck = S->chunk[tid >> 5];              // broadcast LDS.64
-        const uint32_t cls = ck.x & 3u;
-        if (cls == 0u) continue;                          // uniform
-        if (cls == 1u) {
-          // plain chunk: every position of the warp is a matched base of this read, none blocked
-          const uint32_t qq = (uint32_t)p0 + ck.y;
-          const uint32_t* bw = reinterpret_cast<const uint32_t*>(S->bq);
-          const uint32_t bi = qq - 48u;
-          const uint32_t w = __funnelshift_r(bw[bi >> 2], bw[(bi >> 2) + 1], (bi & 3u) * 8u);
-          const uint32_t* sw = reinterpret_cast<const uint32_t*>(S->seq);
-          const uint32_t s8 = __funnelshift_r(sw[qq >> 4], sw[(qq >> 4) + 1], (qq & 15u) * 2u);
-          misacc |= (s8 ^ ref8) & 0xffu;                  // read base != FASTA base under a cs match: checked at the end
-          zacc |= (w - 0x01010101u) & ~w;                 // a quality of 0 (bit 7 of a byte): checked at the end
-          s_lo += w & 0x00ff00ffu;
-          s_hi += (w >> 8) & 0x00ff00ffu;
-          if (ck.x & (HM_PF_PASS << 8)) c4 += ((((w & 0x7f7f7f7fu) + kge) | w) >> 7) & 0x01010101u;
-          n_plain++;
-          if (p.phase) {
-            const uint32_t hap = (ck.x >> (8 + HM_PF_HAP_SHIFT)) & 3u;
-            h0_plain += (hap == 0u); h1_plain += (hap == 1u);
-          }
-          continue;
-        }
-        const uint4 hd = S->head;                         // broadcast LDS.128
-        const uint32_t fl = hd.x;
-        const uint2 mk = S->mask[tid >> 3];               // LDS.64, 4 addresses per warp
-        const uint32_t sp = (mk.x >> sh4) & 15u;
-        imp |= sp;
-        const int lo = (int)(hd.y & 0xffffu) - p0, hi = (int)(hd.y >> 16) - p0;
-        if (hi < 0 || lo > 3) continue;
-        uint32_t cm = 15u;
-        if (lo > 0) cm = (15u << lo) & 15u;
-        if (hi < 3) cm &= 15u >> (3 - hi);
-        uint32_t good = cm & ~sp;
-        int delta = (int)hd.w;
-        const uint32_t nseg = fl >> 16;
-        int delta2 = 0, b2 = 4;                           // a run that starts inside this group: its offset, its first position
-        for (uint32_t s = 1; s < nseg; s++) {             // uniform trip count, almost always zero
-          const int st = S->seg_start[s];
-          if (p0 >= st) delta = S->seg_delta[s];
-          else if (st <= p0 + 3 && b2 == 4) { b2 = st - p0; delta2 = S->seg_delta[s]; }
-        }
-        // query position relative to the staged origin, + 64; clamped so special / uncovered groups stay inside the buffers
-        const uint32_t qq = min((uint32_t)(p0 + delta - (int)hd.z + 64), (uint32_t)(HF_BQ_BUF - HF_PAD - 8 + 64));
-        const uint32_t* bw = reinterpret_cast<const uint32_t*>(S->bq);
-        const uint32_t bi = qq - 48u;                     // byte index into bq[] (HF_PAD = 16 in front)
-        uint32_t w = __funnelshift_r(bw[bi >> 2], bw[(bi >> 2) + 1], (bi & 3u) * 8u);
-        const uint32_t* sw = reinterpret_cast<const uint32_t*>(S->seq);
-        uint32_t s8 = __funnelshift_r(sw[qq >> 4], sw[(qq >> 4) + 1], (qq & 15u) * 2u) & 0xffu;
-        if (b2 < 4) { // positions b2.. of the group follow an indel: take them with the next run's offset
-          const uint32_t qq2 = min((uint32_t)(p0 + delta2 - (int)hd.z + 64), (uint32_t)(HF_BQ_BUF - HF_PAD - 8 + 64));
-          const uint32_t bj = qq2 - 48u;
-          const uint32_t w2 = __funnelshift_r(bw[bj >> 2], bw[(bj >> 2) + 1], (bj & 3u) * 8u);
-          const uint32_t t8 = __funnelshift_r(sw[qq2 >> 4], sw[(qq2 >> 4) + 1], (qq2 & 15u) * 2u) & 0xffu;
-          const uint32_t bm = 0xffffffffu << (8 * b2), sm = (0xffu << (2 * b2)) & 0xffu;
-          w = (w & ~bm) | (w2 & bm);
-          s8 = (s8 & ~sm) | (t8 & sm);
-        }
-        const uint32_t mis = s8 ^ ref8;
-        if (mis) { // special / uncovered / dead positions in the group, or a read base that differs from the FASTA under a cs match
-          const uint32_t m2 = (mis | (mis >> 1)) & 0x55u;
-          const uint32_t m4 = (m2 & 1u) | ((m2 >> 1) & 2u) | ((m2 >> 2) & 4u) | ((m2 >> 3) & 8u);
-          imp |= m4 & good;
-          good &= ~m4;
-        }
-        const uint32_t g1 = spread4(good);
-        const uint32_t gm = g1 * 0xffu;
-        const uint32_t wv = w & gm;
-        if (((wv - g1) & ~wv & (g1 << 7)) != 0u) { imp |= good; continue; } // a quality of 0: the exact pass raises the error
-        n4 += g1;
-        s_lo += wv & 0x00ff00ffu;
-        s_hi += (wv >> 8) & 0x00ff00ffu;
-        if (fl & HM_PF_PASS) {                            // uniform
-          const uint32_t bl = (mk.y >> sh4) & 15u;
-          const uint32_t ge = ((((wv & 0x7f7f7f7fu) + kge) | wv) >> 7) & 0x01010101u;
-          c4 += ge & spread4(good & ~bl);
-        }
-        if (p.phase) {
-          const uint32_t hap = (fl >> HM_PF_HAP_SHIFT) & 3u;
-          if (hap == 0u) h0_4 += g1; else if (hap == 1u) h1_4 += g1;
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&empty_bar[st]);
-#ifdef HM_NORM_DEBUG
-      if (tid == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[3], (unsigned long long)(d1 - d0)); atomicAdd(&out->dbg[4], (unsigned long long)(clock64() - d1)); atomicAdd(&out->dbg[5], (unsigned long long)nslots); }
-#endif
-      batch_no++;
-      if (last) break;
-    }
-#ifdef HM_NORM_DEBUG
-    const long long e0 = clock64();
-#endif
-
-    // ---- per position: certified verdict or the site list (normcounts.py:317-400) ----
-    n4 += n_plain * 0x01010101u; h0_4 += h0_plain * 0x01010101u; h1_4 += h1_plain * 0x01010101u;
-    if (zacc & 0x80808080u) imp = 15u;
-    if (misacc) {
-      const uint32_t m2 = (misacc | (misacc >> 1)) & 0x55u;
-      imp |= (m2 & 1u) | ((m2 >> 1) & 2u) | ((m2 >> 2) & 4u) | ((m2 >> 3) & 8u);
-    }
-    unsigned t1_ = 0, t2_ = 0, t8_ = 0, t9_ = 0, t13_ = 0;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const bool alive = !((dead >> k) & 1u);
-      const int n = (int)((n4 >> (8 * k)) & 255u);
-      const int s1 = (int)(((k & 1) ? s_hi : s_lo) >> (16 * (k >> 1)) & 0xffffu);
-      const int cal = (int)((c4 >> (8 * k)) & 255u);
-      bool push = alive && (deep || ((imp >> k) & 1u));
-      if (alive && !push && cal > 0) {
-        const int h0 = (int)((h0_4 >> (8 * k)) & 255u), h1 = (int)((h1_4 >> (8 * k)) & 255u);
-        if (p.phase && !(h0 >= p.min_hap_count && h1 >= p.min_hap_count)) { t1_ += cal; t2_ += cal; }
-        else {
-          const int x = min(254 * n, 255 * n - s1);
-          // s1 * a_bq - x * a_x >= need - c_oth, in 2^-20 fixed point rounded against certification
-          if (n >= cert.n_min && (long long)s1 * cert.ia_bq - (long long)x * cert.ia_x >= cert.i_need) {
-            t1_ += cal;
-            if ((double)n > p.md_threshold) t8_ += cal;
-            else if (n < p.min_ref_count) t9_ += cal;
-            else {
-              t13_ += cal;
-              const int tri = tri_bin3(rb[k], rb[k + 1], rb[k + 2], (int64_t)t0 + p0 + k, ref_len);
-              atomicAdd(&s_wref[tid >> 5][tri], 1u);
-              atomicAdd(&s_wccs[tid >> 5][tri], (unsigned)cal);
-            }
-          } else push = true;
-        }
-      }
-      const uint32_t bal = __ballot_sync(HM_FULL, push);
-      if (bal) {
-        unsigned long long at = 0;
-        if (lane == 0) at = atomicAdd(n_sites, (unsigned long long)__popc(bal));
-        at = __shfl_sync(HM_FULL, at, 0);
-        if (push) {
-          const unsigned long long slot = at + __popc(bal & ((1u << lane) - 1u));
-          if (slot < site_cap) sites[slot] = ((unsigned long long)c << 36) | ((unsigned long long)(uint32_t)(t0 + p0 + k + 1) << 4);
-        }
-      }
-    }
-    {
-      unsigned v;
-      v = __reduce_add_sync(HM_FULL, t1_); if (lane == 0 && v) { atomicAdd(&s_log[1], (unsigned long long)v); }
-      v = __reduce_add_sync(HM_FULL, t2_); if (lane == 0 && v) atomicAdd(&s_log[2], (unsigned long long)v);
-      v = __reduce_add_sync(HM_FULL, t8_ + t9_ + t13_); if (lane == 0 && v) atomicAdd(&s_log[6], (unsigned long long)v);
-      v = __reduce_add_sync(HM_FULL, t8_); if (lane == 0 && v) atomicAdd(&s_log[8], (unsigned long long)v);
-      v = __reduce_add_sync(HM_FULL, t9_); if (lane == 0 && v) atomicAdd(&s_log[9], (unsigned long long)v);
-      v = __reduce_add_sync(HM_FULL, t13_); if (lane == 0 && v) atomicAdd(&s_log[13], (unsigned long long)v);
-    }
-#ifdef HM_NORM_DEBUG
-    if (tid == 0 && blockIdx.x == 0) { atomicAdd(&out->dbg[6], (unsigned long long)(clock64() - e0)); atomicAdd(&out->dbg[7], 1ull); }
-#endif
-    // move the warp's 32-bit bins into the CTA's 64-bit ones before they can overflow
-    __syncwarp();
-    if (s_wccs[tid >> 5][lane] > 0x40000000u) {
-      atomicAdd(&s_ccs[lane], (unsigned long long)atomicExch(&s_wccs[tid >> 5][lane], 0u));
-      atomicAdd(&s_ref[lane], (unsigned long long)atomicExch(&s_wref[tid >> 5][lane], 0u));
-    }
-    if (lane == 0 && s_wccs[tid >> 5][32] > 0x40000000u) {
-      atomicAdd(&s_ccs[32], (unsigned long long)atomicExch(&s_wccs[tid >> 5][32], 0u));
-      atomicAdd(&s_ref[32], (unsigned long long)atomicExch(&s_wref[tid >> 5][32], 0u));
-    }
-  }
-  // fold the per-warp bins
-  for (int i = lane; i < HM_TRI_BINS; i += 32) {
-    if (s_wccs[tid >> 5][i]) atomicAdd(&s_ccs[i], (unsigned long long)s_wccs[tid >> 5][i]);
-    if (s_wref[tid >> 5][i]) atomicAdd(&s_ref[i], (unsigned long long)s_wref[tid >> 5][i]);
-  }
-  // consumers only: named barrier over the consumer threads, then flush the CTA tallies
-  asm volatile("bar.sync 1, %0;" ::"n"(HF_CONS));
-  if (tid < HM_TRI_BINS) {
-    if (s_ccs[tid]) atomicAdd(&out->ccs_tri[tid], s_ccs[tid]);
-    if (s_ref[tid]) atomicAdd(&out->ref_tri[tid], s_ref[tid]);
-  }
-  if (tid < HM_NORM_LOG_LEN && s_log[tid]) atomicAdd(&out->log[tid], s_log[tid]);
-}
 
 // ============================================================================ exact pass
 // entry: bits 0-2 allele (0-3 base, 5 deleted, 7 none), 3-10 BQ, 11-18 insertions at the site,
@@ -698,112 +66,6 @@ __device__ __forceinline__ uint32_t norm_entry(const DevBatch& b, const DevParam
     }
   }
   return a | (bq << 3) | ((uint32_t)min(ins, 255) << 11) | (((pf >> HM_PF_HAP_SHIFT) & 3u) << 19) | (cnt << 21);
-}
-
-// block = 16 sites x 64 slots; thread (site = tid & 15, slot = tid >> 4)
-__global__ void __launch_bounds__(1024) k_norm_entries(DevBatch b, DevParams p, const hm_chunk* chunks, const uint64_t* pair_off,
-                                                       const uint8_t* pair_flag, const unsigned long long* keys, uint64_t n_keys,
-                                                       const uint32_t* site_lo, const uint32_t* site_n, uint32_t* entries,
-                                                       uint64_t stride) {
-  const uint64_t ki = (uint64_t)blockIdx.x * 16 + (threadIdx.x & 15);
-  const uint32_t slot = threadIdx.x >> 4;
-  if (ki >= n_keys) return;
-  if (slot >= __ldg(site_n + ki)) return;
-  const unsigned long long key = keys[ki];
-  const uint32_t c = (uint32_t)(key >> 36);
-  const int32_t pos = (int32_t)((key >> 4) & 0xffffffffull) - 1;
-  const hm_chunk ch = chunks[c];
-  const uint32_t r = __ldg(site_lo + ki) + slot;
-  entries[(uint64_t)slot * stride + ki] = norm_entry(b, p, ch, pair_flag[pair_off[c] + (r - ch.read_lo)], r, pos);
-}
-
-// The same gather turned around (see k_site_entries_by_read): one warp per (chunk, read) pair stages the read's op
-// arrays and mismatch list in shared memory and serves every listed site of the chunk the read covers.  `keys` must
-// be sorted (chunk, position); [s0, s0 + nb) is the slice of it this launch fills (entries are slice relative).
-__global__ void __launch_bounds__(256) k_norm_entries_by_read(DevBatch b, DevParams p, const hm_chunk* chunks, uint32_t n_chunks,
-                                                              const uint64_t* pair_off, uint64_t n_pairs, const uint8_t* pair_flag,
-                                                              const unsigned long long* keys, const uint32_t* koff, uint64_t s0, uint64_t nb,
-                                                              const uint32_t* site_lo, const uint32_t* site_n, uint32_t* entries,
-                                                              uint64_t stride, uint32_t n_slots) {
-  __shared__ uint32_t s_w[8][HM_BYREAD_MAX_OPS], s_t[8][HM_BYREAD_MAX_OPS], s_q[8][HM_BYREAD_MAX_OPS];
-  __shared__ int32_t s_m[8][HM_BYREAD_MAX_OPS];
-  const uint64_t pr = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (pr >= n_pairs) return;
-  const uint32_t pf = pair_flag[pr];
-  if (!(pf & HM_PF_FETCHED)) return;
-  const uint32_t c = upper_bound_dev(pair_off, n_chunks + 1, pr) - 1;
-  const hm_chunk ch = chunks[c];
-  const uint32_t r = ch.read_lo + (uint32_t)(pr - pair_off[c]);
-  const int32_t ts = __ldg(b.tstart + r), te = __ldg(b.tend + r);
-  const uint32_t n = __ldg(b.n_ops + r);
-  if (n == 0) return;
-  const uint32_t k_lo = max(koff[c], (uint32_t)s0), k_hi = min(koff[c + 1], (uint32_t)(s0 + nb));
-  if (k_lo >= k_hi) return;
-  const unsigned long long base = (unsigned long long)c << 36;
-  const uint32_t s_lo = warp_lower_bound_u64(keys, k_lo, k_hi, base | ((unsigned long long)(uint32_t)(ts + 1) << 4), lane);
-  const uint32_t s_hi = warp_lower_bound_u64(keys, s_lo, k_hi, base | ((unsigned long long)(uint32_t)(te + 2) << 4), lane);
-  if (s_lo >= s_hi) return;
-  const uint64_t o0 = __ldg(b.op_off + r);
-  const uint32_t nmm = (uint32_t)__ldg(b.n_mm + r);
-  const bool staged = n <= HM_BYREAD_MAX_OPS;
-  if (staged) {
-    for (uint32_t k = lane; k < n; k += 32) {
-      s_w[wid][k] = __ldg(b.ops + o0 + k); s_t[wid][k] = __ldg(b.op_t + o0 + k); s_q[wid][k] = __ldg(b.op_q + o0 + k);
-      if (k < nmm) s_m[wid][k] = __ldg(b.mm_pos + o0 + k);
-    }
-    __syncwarp();
-  }
-  const uint64_t bq0 = __ldg(b.bq_off + r), sq0 = __ldg(b.seq_off + r);
-  const int32_t qlen = __ldg(b.qlen + r);
-  const int32_t trim_s = (int32_t)floor(__dmul_rn(p.min_trim, (double)qlen));
-  const int32_t trim_e = (int32_t)ceil(__dmul_rn(__dsub_rn(1.0, p.min_trim), (double)qlen));
-  const int w = p.mismatch_window;
-  for (uint32_t ki = s_lo + lane; ki < s_hi; ki += 32) {
-    const uint32_t li = ki - (uint32_t)s0;
-    const uint32_t slot = r - __ldg(site_lo + li);
-    if (slot >= n_slots || slot >= __ldg(site_n + li)) continue; // pileups deeper than the slots: k_norm_reduce computes these itself
-    const int32_t pos = (int32_t)((__ldg(keys + ki) >> 4) & 0xffffffffull) - 1;
-    uint32_t e;
-    if (!staged) e = norm_entry(b, p, ch, pf, r, pos);
-    else {
-      const uint32_t off = (uint32_t)(pos - ts);
-      uint32_t lo = 0, hi = n; // last op with op_t <= off
-      while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if (s_t[wid][m] <= off) lo = m + 1; else hi = m; }
-      const int k = (int)lo - 1;
-      int ins = 0;
-      for (int j = k; j >= 0 && s_t[wid][j] == off; j--) ins += ((s_w[wid][j] & 3u) == HM_OP_INS);
-      const uint32_t wd = s_w[wid][k], kind = wd & 3u, t_op = s_t[wid][k], q0 = s_q[wid][k];
-      const uint32_t rl = (uint32_t)op_ref_len(wd);
-      uint32_t a = HM_ENT_NONE, bq = 0, cnt = 0;
-      if (rl != 0 && off < t_op + rl) {
-        if (kind == HM_OP_DEL) a = 5u;
-        else {
-          const uint32_t q = q0 + (kind == HM_OP_MATCH ? off - t_op : 0u);
-          bq = b.bq[bq0 + q];
-          a = kind == HM_OP_SUB ? ((wd >> 5) & 3u) : (uint32_t)((b.seq[sq0 + (q >> 2)] >> (2 * (q & 3u))) & 3u);
-          if (pf & HM_PF_PASS) {
-            if (kind == HM_OP_SUB) cnt = 1; // normcounts.py:95-108: always counted
-            else if ((int)bq >= p.min_bq && !((int32_t)q < trim_s || (int32_t)q > trim_e)) {
-              const int32_t qpos0 = (int32_t)q0;
-              const int qs = qpos0 - w, qe = qpos0 + w;
-              int u, d;
-              if (qs < 0) { u = w + qs; d = w + (-qs); }
-              else if (qe > qlen) { u = w + (qe - qlen); d = qlen - qpos0; }
-              else { u = w; d = w; }
-              // mismatches x with pos - u <= x <= pos + d (1-based list against the 0-based position, normcounts.py:82-87)
-              uint32_t l1 = 0, h1 = nmm, l2 = 0, h2 = nmm;
-              while (l1 < h1) { const uint32_t m = (l1 + h1) >> 1; if (s_m[wid][m] <= pos + d) l1 = m + 1; else h1 = m; }
-              while (l2 < h2) { const uint32_t m = (l2 + h2) >> 1; if (s_m[wid][m] <= pos - u - 1) l2 = m + 1; else h2 = m; }
-              cnt = !((int)l1 - (int)l2 > p.max_mismatch_count);
-            }
-          }
-        }
-      }
-      e = a | (bq << 3) | ((uint32_t)min(ins, 255) << 11) | (((pf >> HM_PF_HAP_SHIFT) & 3u) << 19) | (cnt << 21);
-    }
-    entries[(uint64_t)slot * stride + li] = e;
-  }
 }
 
 __global__ void __launch_bounds__(128) k_norm_reduce(DevBatch b, DevParams p, DevSets sets, DevLut lut, const hm_chunk* chunks,
@@ -932,7 +194,7 @@ __global__ void __launch_bounds__(128) k_norm_reduce(DevBatch b, DevParams p, De
   }
 }
 
-// k_site_range for a plain key array of known length (the site list of the fast pass)
+// k_site_range for a plain key array of known length (the site list of k_norm_bits)
 __global__ void __launch_bounds__(256) k_norm_site_range(DevBatch b, const hm_chunk* chunks, const unsigned long long* keys,
                                                          uint64_t n_keys, uint32_t* site_lo, uint32_t* site_n) {
   const uint64_t ki = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;

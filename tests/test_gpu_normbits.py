@@ -1,6 +1,6 @@
 """The bit-vector integer pass of `himut normcounts` (himut_b200/csrc/normbits.cuh: k_norm_prep + k_norm_bits) on its
-edges, against the CPU oracle, and against the byte-tile kernel it replaced (HIMUT_B200_NORM_V3=1) and the single-pass
-kernel that genotypes every column exactly (HIMUT_B200_NORM_V2=1).  GPU."""
+edges, against the CPU oracle; and on the same 300 kb batch the single pass k_norm_tiles_tma that genotypes every
+column exactly where the parameters lie outside the certified domain.  GPU."""
 import numpy as np
 import pytest
 
@@ -25,26 +25,22 @@ def same(g, o):
     return np.array_equal(g[0], o[0]) and np.array_equal(g[1], o[1]) and list(g[2]) == list(o[2]) and g[3] == o[3]
 
 
-def test_three_integer_passes_agree(ctx, monkeypatch):
+def test_bits_and_single_pass_on_300_kb(ctx):
     d = synth.generate(300_000, seed=41)
     p = gtmodel.make_params(**gtmodel.DEFAULT_CALL_ARGS)
     loci = cases.chunkloci(0, 300_000)
     g, o = run(ctx, p, d, loci)
     assert same(g, o)
     names = [n for n, _ in ctx.last_kernel_times()]
-    assert "k_norm_prep" in names and "k_norm_bits" in names and "k_norm_fast" not in names
-    exact_bits = ctx.last_norm_exact_sites()
-    monkeypatch.setenv("HIMUT_B200_NORM_V3", "1")
-    g3, _ = run(ctx, p, d, loci)
-    assert same(g3, o)
-    assert "k_norm_fast" in [n for n, _ in ctx.last_kernel_times()]
-    exact_tiles = ctx.last_norm_exact_sites()
-    monkeypatch.delenv("HIMUT_B200_NORM_V3")
-    monkeypatch.setenv("HIMUT_B200_NORM_V2", "1")
-    g2, _ = run(ctx, p, d, loci)
-    assert same(g2, o)
-    # the lower bound of the quality sum costs next to nothing: about as many positions reach the exact pass
-    assert exact_bits <= exact_tiles * 1.05 + 64
+    assert "k_norm_prep" in names and "k_norm_bits" in names and "k_norm_tiles_tma" not in names
+    # the bit-vector pass is deterministic: exactly these positions reach the exact pass
+    assert ctx.last_norm_exact_sites() == 2771
+    # min_bq 0 lies outside the certified domain: the single pass genotypes every column
+    p = gtmodel.make_params(**cases.call_args(min_bq=0))
+    g, o = run(ctx, p, d, loci)
+    assert same(g, o)
+    names = [n for n, _ in ctx.last_kernel_times()]
+    assert "k_norm_tiles_tma" in names and "k_norm_bits" not in names
 
 
 @pytest.mark.parametrize("over", [dict(max_mismatch_count=2), dict(max_mismatch_count=1, mismatch_window=40),
@@ -112,7 +108,7 @@ def test_phase_and_sets_cases_on_the_bit_path(ctx):
 
 
 @pytest.mark.parametrize("over", [dict(), dict(min_bq=20), dict(min_bq=94), dict(min_bq=60, min_trim=0.05), dict(min_qv=92)])
-def test_compact_upload_takes_the_bits_from_the_bitmap(ctx, over, monkeypatch):
+def test_compact_upload_takes_the_bits_from_the_bitmap(ctx, over):
     """a batch uploaded as modal bitmap + exceptions (what the workers upload): where every exception of a read lies
     below min_bq the bit "BQ >= min_bq" is the bitmap's and the quality sum is the one taken at expansion; a read with
     an exception at or above min_bq goes through its quality bytes; both must equal the plain upload and the oracle"""
@@ -128,10 +124,6 @@ def test_compact_upload_takes_the_bits_from_the_bitmap(ctx, over, monkeypatch):
     ctx.upload_compact(d.batch, cq)
     g = ctx.normcounts_chunks(d.ref, chunks)
     assert same(g, o)
-    monkeypatch.setenv("HIMUT_B200_NORM_BYTES", "1")
-    g2 = ctx.normcounts_chunks(d.ref, chunks)
-    assert same(g2, o)
-    monkeypatch.delenv("HIMUT_B200_NORM_BYTES")
     rec, log = ctx.call_chunks(chunks)  # the expanded stream is still what `call` reads
     o_rec, o_log = oracle.call_chunks(p, d.batch, chunks)
     assert list(log) == list(o_log)

@@ -80,11 +80,26 @@ def test_normcounts_additive_over_chunks(ctx):
     assert list(whole[2][1:]) == list(sum(x[2] for x in parts)[1:])  # num_ccs is a distinct count, not additive
 
 
+def test_normcounts_chunk_with_a_negative_start(ctx):
+    """a fetch window that starts before the contig: the bit-vector pass works on the absolute 1024-position grid and
+    leaves such a call to the single pass, whose tiles are chunk-relative; positions below 0 count for nothing"""
+    d = synth.generate(100_000, seed=37)
+    p = gtmodel.make_params(**gtmodel.DEFAULT_CALL_ARGS)
+    chunks = d.batch.chunk_table([(-500, 40_000), (40_000, 100_000)])
+    ctx.set_params(p)
+    ctx.set_site_sets()
+    ctx.upload(d.batch)
+    g = ctx.normcounts_chunks(d.ref, chunks)
+    o = oracle.normcounts_chunks(p, d.batch, d.ref, chunks)
+    assert np.array_equal(g[0], o[0]) and np.array_equal(g[1], o[1]) and list(g[2]) == list(o[2]) and g[3] == o[3]
+    assert "k_norm_tiles_tma" in [n for n, _ in ctx.last_kernel_times()]
+
+
 @pytest.mark.parametrize("over", [dict(min_gq=60), dict(min_gq=99), dict(min_gq=0, germline_snv_prior=0.3),
                                   dict(min_bq=1, min_gq=35, md_threshold=25), dict(min_ref_count=40)])
 def test_normcounts_certification_edges(ctx, over):
     """parameters that push many pure positions out of the certified domain (or make every one fail a gate):
-    whatever the fast pass cannot decide must come back through the exact pass with the oracle's answer"""
+    whatever the integer pass cannot decide must come back through the exact pass with the oracle's answer"""
     d = synth.generate(200_000, seed=33)
     p = gtmodel.make_params(**cases.call_args(**over))
     chunks = d.batch.chunk_table(cases.chunkloci(0, 200_000))
@@ -98,8 +113,8 @@ def test_normcounts_certification_edges(ctx, over):
 
 @pytest.mark.parametrize("slots", [None, "64"])
 def test_normcounts_deep_pileup(ctx, slots, monkeypatch):
-    """400x: more than 255 reads per 2048-position tile (the packed 8-bit tallies of the fast pass would overflow:
-    the whole tile goes to the exact pass) and more reads per position than the entry table has slots (512 at most;
+    """400x: more than 255 reads per 1024-position span (the 8-bit bit-sliced counters of k_norm_bits would overflow:
+    the whole span goes to the exact pass) and more reads per position than the entry table has slots (512 at most;
     64 when HIMUT_B200_SITE_SLOTS forces it): the reduce computes the slots beyond the table itself"""
     if slots is not None:
         monkeypatch.setenv("HIMUT_B200_SITE_SLOTS", slots)  # read at upload

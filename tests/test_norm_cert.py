@@ -1,6 +1,6 @@
-"""The certified verdict of k_norm_fast (DESIGN.md §4.1) against the reference's own genotype code: whenever the
-integer test of the kernel (restated here from make_norm_cert in himut_b200.cu and the consumer epilogue in
-normfast.cuh) certifies a pure position — n reads of the reference allele with qualities b_i — the unmodified
+"""The certified verdict of the normcounts integer pass (DESIGN.md §4.1) against the reference's own genotype code:
+whenever the integer test (restated here from make_norm_cert in himut_b200.cu, which turns it into the table thr that
+k_norm_bits looks up) certifies a pure position — n reads of the reference allele with qualities b_i — the unmodified
 `himut.gtlib.get_germ_gt` must call it hom-ref with GQ >= min_gq.  Random depths, quality mixes, priors and GQ
 thresholds.  The comparisons with the reference run where its unmodified sources are present (tests/refshim.py)."""
 import math
@@ -15,7 +15,7 @@ needs_reference = pytest.mark.skipif(not refshim.have_reference(), reason="refer
 
 
 def make_cert(prior, min_gq, min_bq=93):
-    """make_norm_cert (himut_b200/csrc/himut_b200.cu) restated -> dict or None (fast pass switched off)"""
+    """make_norm_cert (himut_b200/csrc/himut_b200.cu) restated -> dict or None (bit-vector pass switched off)"""
     p = gtmodel.make_params(**dict(gtmodel.DEFAULT_CALL_ARGS, germline_snv_prior=prior, min_gq=min_gq, min_bq=min_bq))
     L2 = 0.30102999566398119521
     f1 = -p.lut_hom[1]
@@ -59,7 +59,7 @@ def certified_sum(cert, n, s1):
 
 
 def certified(cert, bqs):
-    """the consumer epilogue's test (normfast.cuh: `n >= cert.n_min && s1 * ia_bq - x * ia_x >= i_need`)"""
+    """the fixed-point test of make_norm_cert (himut_b200.cu: `n >= c.n_min`, `s1 * c.ia_bq - x * c.ia_x >= c.i_need`)"""
     return len(bqs) >= cert["n_min"] and certified_sum(cert, len(bqs), sum(bqs))
 
 
