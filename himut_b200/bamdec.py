@@ -12,11 +12,11 @@ import os
 
 import numpy as np
 
-from . import abi, pack
+from . import abi, bamio, pack
 
 _LIB = None
 EXPORTS = ["hm_bam_open", "hm_bam_close", "hm_bam_error", "hm_bam_header_text", "hm_bam_n_refs", "hm_bam_ref_name",
-           "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bq_compact_build",
+           "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bam_write_batch_tags", "hm_bq_compact_build",
            "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames"]
 
 
@@ -48,6 +48,7 @@ def load():
         lib.hm_bam_last_compact.argtypes = [vp, C.POINTER(abi.hm_bq_compact)]
         lib.hm_bam_window_qlens.argtypes = [vp, C.c_int, C.c_int32, C.c_int32, C.c_int, vp, C.c_size_t, C.POINTER(C.c_size_t)]
         lib.hm_bam_write_batch.argtypes = [C.c_char_p, C.c_char_p, C.c_int32, C.c_char_p, C.POINTER(abi.hm_read_batch), C.c_int, C.c_int]
+        lib.hm_bam_write_batch_tags.argtypes = lib.hm_bam_write_batch.argtypes + [C.c_int]
         lib.hm_bq_compact_build.argtypes = [C.POINTER(abi.hm_read_batch), C.c_int, vp, vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint8)]
         lib.hm_bq_compact_free.argtypes = [vp]
         lib.hm_bq_compact_free.restype = None
@@ -80,10 +81,12 @@ def _view(ptr, n, dtype):
     return np.frombuffer(buf, dtype=dt, count=n)
 
 
-def write_batch_bam(path, chrom, contig_len, batch, sample="synth", level=1, threads=None):
-    """ReadBatch -> coordinate-sorted BAM + BAI, natively (same content as bamio.write_batch_bam)"""
-    rc = load().hm_bam_write_batch(os.fsencode(path), chrom.encode(), int(contig_len), sample.encode(), C.byref(batch.as_struct()),
-                                   int(level), int(threads or default_threads()))
+def write_batch_bam(path, chrom, contig_len, batch, sample="synth", level=1, threads=None, tags="cs"):
+    """ReadBatch -> coordinate-sorted BAM + BAI, natively (same content as bamio.write_batch_bam, tags alike)"""
+    if tags not in bamio.TAGS:
+        raise ValueError("tags must be one of %s" % (bamio.TAGS,))
+    rc = load().hm_bam_write_batch_tags(os.fsencode(path), chrom.encode(), int(contig_len), sample.encode(), C.byref(batch.as_struct()),
+                                        int(level), int(threads or default_threads()), bamio.TAGS.index(tags))
     if rc != 0:
         raise IOError("cannot write %s" % path)
 

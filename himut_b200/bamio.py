@@ -5,7 +5,8 @@ records of a region as a packed ReadBatch rather than as Python objects anyway. 
 implements what the reference touches through pysam (SURVEY.md §8b): header text, @SQ table,
 fetch(chrom, start, end) — records overlapping the 0-based half-open window, in file order,
 secondary / supplementary included — and the per-record fields reference_start/end,
-query_alignment_start/end, query_sequence, query_qualities, mapping_quality, flag, cs:Z, tp:A.
+query_alignment_start/end, query_sequence, query_qualities, mapping_quality, flag, cs:Z, tp:A, and
+beyond it the CIGAR and MD:Z (records without cs:Z are decoded from CIGAR + MD, pack.parse_md).
 The writer exists for tests and for the synthetic-data tools (coordinate-sorted BAM + .bai).
 """
 import struct
@@ -96,7 +97,7 @@ class Record:
     """decoded alignment (attribute names follow pysam.AlignedSegment)"""
     __slots__ = ("ref_id", "reference_start", "reference_end", "query_name", "flag", "mapping_quality",
                  "query_alignment_start", "query_alignment_end", "seq_nibbles", "l_seq", "qual", "tags",
-                 "hard_clipped")
+                 "hard_clipped", "cigar")
 
     @property
     def is_secondary(self):
@@ -127,7 +128,7 @@ class Record:
         return t in self.tags
 
 
-def _parse_tags(buf, p, end, want=("cs", "tp")):
+def _parse_tags(buf, p, end, want=("cs", "tp", "MD")):
     tags = {}
     while p < end:
         tag = buf[p:p + 2].decode()
@@ -167,6 +168,7 @@ def _parse_record(buf):
     cig = np.frombuffer(buf, dtype="<u4", count=n_cig, offset=p)
     p += 4 * n_cig
     ops, lens = cig & 15, cig >> 4
+    r.cigar = [(int(o), int(l)) for o, l in zip(ops, lens)]
     ref_span = int(sum(int(l) for o, l in zip(ops, lens) if _CIGAR_REF[o]))
     lead = trail = 0
     r.hard_clipped = bool(n_cig and (ops[0] == 5 or ops[-1] == 5))
@@ -291,12 +293,14 @@ def read_batch(reader, chrom, start, end, builder=None):
 
     Secondary records are dropped here: bamlib.BAM.__init__ skips them before anything else
     (src/himut/bamlib.py:17); supplementary records are kept, as the reference keeps them.
+    A record's ops come from its cs:Z tag; a record without cs:Z but with MD:Z is decoded from CIGAR + MD
+    (pack.parse_md: the same ops for the same alignment); a record with neither is rejected.
     """
     bb = builder or pack.BatchBuilder()
     for r in reader.fetch(chrom, start, end):
         if r.is_secondary:  # BAM.__init__ skips them everywhere (bamlib.py:17)
             continue
-        if "cs" not in r.tags:
+        if "cs" not in r.tags and "MD" not in r.tags:
             raise pack.BatchFormatError("%s has no cs:Z tag (the reference raises KeyError in BAM.__init__)" % r.query_name)
         # hard clips: pysam's query_sequence / query_alignment_start leave the clipped bases out (SEQ does not hold
         # them), so cs2tuple indexes consistently and the reference processes such records; so do we
@@ -305,7 +309,7 @@ def read_batch(reader, chrom, start, end, builder=None):
             raise pack.BatchFormatError("%s has no base qualities" % r.query_name)
         bb.add(tstart=r.reference_start, tend=r.reference_end, qstart=r.query_alignment_start, qend=r.query_alignment_end,
                qseq=r.query_sequence, bq=bytes(q), mapq=r.mapping_quality, is_secondary=False, qname=r.query_name,
-               cs=r.tags["cs"])
+               cs=r.tags.get("cs"), cigar=r.cigar, md=r.tags.get("MD"))
     return bb.finish()
 
 
@@ -416,20 +420,27 @@ class BamWriter:
             f.write(struct.pack("<Q", 0))
 
 
-def write_batch_bam(path, chrom, contig_len, batch, sample="synth"):
-    """ReadBatch -> coordinate-sorted BAM + BAI (cs:Z short form, tp:A:P), for tests and tools"""
-    write_batches_bam(path, [(chrom, contig_len, batch)], sample)
+TAGS = ("cs", "md", "md_eqx")
 
 
-def write_batches_bam(path, contigs, sample="synth"):
+def write_batch_bam(path, chrom, contig_len, batch, sample="synth", tags="cs"):
+    """ReadBatch -> coordinate-sorted BAM + BAI, tp:A:P, for tests and tools.  tags: "cs" writes cs:Z short form
+    with a =/X CIGAR; "md" writes MD:Z and no cs with an M CIGAR; "md_eqx" MD:Z with the =/X CIGAR"""
+    write_batches_bam(path, [(chrom, contig_len, batch)], sample, tags)
+
+
+def write_batches_bam(path, contigs, sample="synth", tags="cs"):
     """[(chrom, contig_len, ReadBatch), ...] -> one coordinate-sorted BAM + BAI"""
     w = BamWriter(path, [(c, n) for c, n, _ in contigs], header_extra="@RG\tID:rg\tSM:%s\n" % sample)
     for rid, (_c, _n, batch) in enumerate(contigs):
-        _add_batch(w, rid, batch)
+        _add_batch(w, rid, batch, tags)
     w.close()
 
 
-def _add_batch(w, rid, batch):
+def _add_batch(w, rid, batch, tags="cs"):
+    if tags not in TAGS:
+        raise ValueError("tags must be one of %s" % (TAGS,))
+    m_op, x_op = (0, 0) if tags == "md" else (7, 8)
     for r in range(batch.n_reads):
         ql = int(batch.qlen[r])
         so, bo, oo = int(batch.seq_off[r]), int(batch.bq_off[r]), int(batch.op_off[r])
@@ -439,18 +450,22 @@ def _add_batch(w, rid, batch):
         ops = batch.ops[oo:oo + int(batch.n_ops[r])]
         qstart = int(batch.qstart[r])
         cs, cigar, q = [], [], qstart
+        md, md_run = [], 0  # MD: the matched bases since the last event, then the event (deleted bases as N)
         if qstart:
             cigar.append((4, qstart))
         for wd in ops:
             kind, val = int(wd) & 3, int(wd) >> 2
             if kind == abi.OP_MATCH:
-                cs.append(":%d" % val); cigar.append((7, val)); q += val
+                cs.append(":%d" % val); cigar.append((m_op, val)); q += val
+                md_run += val
             elif kind == abi.OP_SUB:
-                cs.append("*%s%s" % ("atgcn"[val & 7], "atgcn"[(val >> 3) & 7])); cigar.append((8, 1)); q += 1
+                cs.append("*%s%s" % ("atgcn"[val & 7], "atgcn"[(val >> 3) & 7])); cigar.append((x_op, 1)); q += 1
+                md.append("%d%s" % (md_run, "ATGCN"[val & 7])); md_run = 0
             elif kind == abi.OP_INS:
                 cs.append("+" + qseq[q:q + val].lower()); cigar.append((1, val)); q += val
             else:
                 cs.append("-" + "n" * val); cigar.append((2, val))
+                md.append("%d^%s" % (md_run, "N" * val)); md_run = 0
         if ql - q:
             cigar.append((4, ql - q))
         merged = []
@@ -461,4 +476,5 @@ def _add_batch(w, rid, batch):
                 merged.append((o, l))
         flag = 0x100 if (batch.flags[r] & abi.READ_SECONDARY) else 0
         w.add(rid, int(batch.tstart[r]), "read%d" % int(batch.qname_id[r]), flag, int(batch.mapq[r]), merged, qseq,
-              batch.bq[bo:bo + ql].tobytes(), [("cs", "Z", "".join(cs)), ("tp", "A", "P")])
+              batch.bq[bo:bo + ql].tobytes(),
+              [("cs", "Z", "".join(cs)) if tags == "cs" else ("MD", "Z", "".join(md) + "%d" % md_run), ("tp", "A", "P")])

@@ -577,7 +577,8 @@ static inline int base_code(char c) {
 /* one selected record between the serial scan (phase A) and the parallel decode (phase B) */
 typedef struct {
   const uint8_t* rec;   /* start of the fixed part (after block_size) */
-  const char* cs;
+  const char* cs;       /* the cs:Z value, or NULL: the ops come from CIGAR + md */
+  const char* md;
   int32_t pos, l_seq, lead, trail, ref_span;
   size_t seq_off, bq_off, op_slot; /* where its outputs go; op_slot is an upper-bound slot, compacted afterwards */
   size_t exc_slot;                 /* compact qualities: upper-bound slot of the exceptions, compacted afterwards */
@@ -649,7 +650,97 @@ static int32_t nib_to_codes_simd(const uint8_t* seq4, int32_t l_seq, uint8_t* co
 static int32_t pack_codes_simd(const uint8_t* codes, int32_t l_seq, uint8_t* dst) { (void)codes; (void)l_seq; (void)dst; return 0; }
 #endif
 
-/* phase B for one record: SEQ -> 2-bit, QUAL copy, cs -> ops (cslib.cs2lst grammar) with span and base checks */
+static inline int is_digit(char c) { return c >= '0' && c <= '9'; }
+static inline int is_alpha(char c) { return (c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z'); }
+/* an MD number; saturates far above any reference span, so that a huge one is left over like an exact one */
+static long long md_num(const char** c) {
+  long long n = 0;
+  while (is_digit(**c)) { n = n * 10 + (**c - '0'); if (n > (1ll << 40)) n = 1ll << 40; (*c)++; }
+  return n;
+}
+
+/* CIGAR + MD:Z -> ops, the rules and the order of checks of pack.parse_md; 0 with R->err set on failure */
+static int md_walk(rec_t* R, const uint8_t* cig, uint32_t n_cig, const uint8_t* codes, int32_t l_seq, uint32_t* ops,
+                   uint32_t* n_out, int32_t* q_out, int32_t* rspan_out) {
+#define MD_FAIL(e, a) do { R->err = (e); R->err_arg = (long)(a); return 0; } while (0)
+  uint32_t first = n_cig, last = 0; /* the aligned ops: clips may only lie outside [first, last] */
+  for (uint32_t k = 0; k < n_cig; k++) { const uint32_t op = rd32(cig + 4 * k) & 15; if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; } }
+  int64_t qcore = 0, qclip = 0;
+  for (uint32_t k = 0; k < n_cig; k++) {
+    const uint32_t c = rd32(cig + 4 * k), op = c & 15, ln = c >> 4;
+    if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) MD_FAIL(E_CIGAR_OP, k); if (op == 4) qclip += ln; }
+    else if (op == 0 || op == 1 || op == 7 || op == 8) qcore += ln;
+    else if (op != 2) MD_FAIL(E_CIGAR_OP, k);
+  }
+  if (qcore + qclip != l_seq) MD_FAIL(E_SPAN_QRY, qcore);
+  const char* md = R->md;
+  const char* c = md;
+  const char* good = md; /* end of the longest prefix the grammar accepts */
+  if (is_digit(*c)) {
+    while (is_digit(*c)) c++;
+    good = c;
+    while (*c) {
+      if (*c == '^') { const char* s0 = ++c; while (is_alpha(*c)) c++; if (c == s0) break; }
+      else if (is_alpha(*c)) c++;
+      else break;
+      if (!is_digit(*c)) break;
+      while (is_digit(*c)) c++;
+      good = c;
+    }
+  }
+  if (*good || good == md) MD_FAIL(E_MD_TOKEN, good - md);
+  c = md;
+  long long mnum = md_num(&c);
+  int32_t q = R->lead, r = 0;
+  uint32_t n = 0, run = 0;
+#define MD_FLUSH() do { if (run) { ops[n++] = HM_MAKE_OP(HM_OP_MATCH, run); run = 0; } } while (0)
+  for (uint32_t k = 0; k < n_cig; k++) {
+    const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+    if (ln == 0 || op == 4 || op == 5) continue;
+    if (op == 0 || op == 7 || op == 8) {
+      uint32_t left = ln;
+      while (left) {
+        if (mnum) {
+          if (op == 8) MD_FAIL(E_MD_SPAN, r);
+          const uint32_t t = mnum < (long long)left ? (uint32_t)mnum : left;
+          const uint8_t* bad = (const uint8_t*)memchr(codes + q, 0xff, t);
+          if (bad) MD_FAIL(E_N_MATCH, bad - codes);
+          run += t; mnum -= t; q += (int32_t)t; r += (int32_t)t; left -= t;
+        } else {
+          if (!*c || *c == '^' || op == 7) MD_FAIL(E_MD_SPAN, r);
+          const int rc_ = base_code(*c++);
+          mnum = md_num(&c);
+          if (codes[q] > 3) MD_FAIL(E_SUB_N, q);
+          MD_FLUSH();
+          ops[n++] = HM_MAKE_SUB(rc_ < 0 ? HM_BASE_N : (uint32_t)rc_, (uint32_t)codes[q]);
+          q++; r++; left--;
+        }
+      }
+    } else if (op == 1) {
+      MD_FLUSH();
+      ops[n++] = HM_MAKE_OP(HM_OP_INS, ln);
+      q += (int32_t)ln;
+    } else { /* D */
+      if (mnum || *c != '^') MD_FAIL(E_MD_SPAN, r);
+      const char* s0 = ++c;
+      while (is_alpha(*c)) c++;
+      if ((uint32_t)(c - s0) != ln) MD_FAIL(E_MD_SPAN, r);
+      mnum = md_num(&c);
+      MD_FLUSH();
+      ops[n++] = HM_MAKE_OP(HM_OP_DEL, ln);
+      r += (int32_t)ln;
+    }
+  }
+  MD_FLUSH();
+  if (mnum || *c) MD_FAIL(E_MD_SPAN, r);
+#undef MD_FLUSH
+#undef MD_FAIL
+  *n_out = n; *q_out = q; *rspan_out = r;
+  return 1;
+}
+
+/* phase B for one record: SEQ -> 2-bit, QUAL copy, cs -> ops (cslib.cs2lst grammar) or CIGAR + MD -> ops (md_walk)
+ * with span and base checks */
 static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_cap) {
   const uint8_t* r = R->rec;
   const uint32_t l_name = r[8], n_cig = r[12] | (r[13] << 8);
@@ -669,7 +760,8 @@ static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_
   int32_t q = R->lead, rspan = 0;
   const char* cs = R->cs;
   const char* c = cs;
-  while (*c) {
+  if (!cs && !md_walk(R, r + 32 + l_name, n_cig, codes, l_seq, ops, &n_ops, &q, &rspan)) return;
+  while (cs && *c) {
     if (*c == ':') {
       long n = 0; c++;
       if (*c < '0' || *c > '9') { R->err = E_CS_TOKEN; R->err_arg = (long)(c - cs); return; }
@@ -849,6 +941,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         const uint8_t* tag = qual + (l_seq > 0 ? l_seq : 0);
         const uint8_t* rec_end = r + bs;
         const char* cs = NULL;
+        const char* md = NULL;
         while (tag + 3 <= rec_end) {
           char ty = (char)tag[2];
           const uint8_t* v = tag + 3;
@@ -859,6 +952,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
             if (!z) { rc = fail(b, REC_ERR[E_TAG_UNTERM], qname, (long)ty); break; }
             adv = (size_t)((const uint8_t*)z - v) + 1;
             if (tag[0] == 'c' && tag[1] == 's' && ty == 'Z') cs = (const char*)v;
+            if (tag[0] == 'M' && tag[1] == 'D' && ty == 'Z') md = (const char*)v;
           }
           else if (ty == 'A' || ty == 'c' || ty == 'C') adv = 1;
           else if (ty == 's' || ty == 'S') adv = 2;
@@ -873,7 +967,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
           tag = v + adv;
         }
         if (rc) break;
-        if (!cs) { rc = fail(b, REC_ERR[E_NO_CS], qname, 0); break; }
+        if (!cs && !md) { rc = fail(b, REC_ERR[E_NO_CS], qname, 0); break; } /* cs when it is there, else CIGAR + MD */
         /* hard clips: pysam's query_sequence and query_alignment_start leave them out (SEQ holds no hard-clipped base),
          * so cs2tuple indexes consistently and the reference processes such records (minimap2 writes them for
          * supplementary alignments without -Y); lead / trail above count soft clips only */
@@ -898,7 +992,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         if (id < 0) { rc = fail(b, "out of memory%s (%ld)", NULL, 0); break; }
         const size_t sb = ((size_t)l_seq + 3) / 4, sb16 = (sb + 15) & ~(size_t)15, qb16 = ((size_t)l_seq + 15) & ~(size_t)15;
         rec_t* R = &recs[nsel++];
-        R->rec = r; R->cs = cs; R->pos = pos; R->l_seq = l_seq; R->lead = lead; R->trail = trail; R->ref_span = ref_span;
+        R->rec = r; R->cs = cs; R->md = cs ? NULL : md; R->pos = pos; R->l_seq = l_seq; R->lead = lead; R->trail = trail; R->ref_span = ref_span;
         R->seq_off = n_seq; R->bq_off = n_bq; R->op_slot = n_ops + seg_ops; R->n_ops = 0; R->rspan = 0; R->err = 0; R->err_arg = 0;
         R->exc_slot = (size_t)n_exc + seg_exc; R->n_exc = 0;
         if (b->compact_bq) {
@@ -915,7 +1009,8 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         b->mapq[n_reads] = (uint8_t)mapq; b->flags[n_reads] = 0; b->qname_id[n_reads] = (uint32_t)id;
         b->seq_off[n_reads] = n_seq; b->bq_off[n_reads] = n_bq;
         if (!b->no_seq) n_seq += sb16;
-        n_bq += qb16; seg_ops += strlen(cs) / 2 + 2; n_reads++;
+        /* ops of CIGAR + MD: SUBs <= MD letters, INS + DEL <= CIGAR ops, match runs <= the other ops + 1 */
+        n_bq += qb16; seg_ops += cs ? strlen(cs) / 2 + 2 : 2 * (strlen(md) + n_cig) + 2; n_reads++;
       }
       if (rc) break;
       if (nsel) {
@@ -1284,9 +1379,9 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
 }
 
 /* ------------------------------------------------------------------ writer (tests, tools, bench) */
-/* A packed batch back to a coordinate-sorted BAM + BAI: cs:Z short form, tp:A:P, query names "read<id>",
- * deleted bases written as "n" (they are not stored).  Mirrors bamio.write_batch_bam; exists so that the
- * benchmark can put a contig-sized BAM on disk in seconds.  Not on the calling path. */
+/* A packed batch back to a coordinate-sorted BAM + BAI: cs:Z short form (or MD:Z, see HM_BAM_TAGS_*), tp:A:P, query
+ * names "read<id>", deleted bases written as "n" ("N" in MD; they are not stored).  Mirrors bamio.write_batch_bam;
+ * exists so that the benchmark can put a contig-sized BAM on disk in seconds.  Not on the calling path. */
 typedef struct { uint8_t* p; size_t n, cap; } wbuf_t;
 static int wb_need(wbuf_t* w, size_t add) {
   if (w->n + add <= w->cap) return 0;
@@ -1347,7 +1442,14 @@ static void* deflate_worker(void* arg) {
 
 int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                        int level, int threads) {
-  if (!path || !chrom || !b) return HM_ERR_ARG;
+  return hm_bam_write_batch_tags(path, chrom, contig_len, sample, b, level, threads, HM_BAM_TAGS_CS);
+}
+
+int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
+                            int level, int threads, int tags) {
+  if (!path || !chrom || !b || (tags != HM_BAM_TAGS_CS && tags != HM_BAM_TAGS_MD && tags != HM_BAM_TAGS_MD_EQX)) return HM_ERR_ARG;
+  const int use_md = tags != HM_BAM_TAGS_CS;
+  const uint32_t m_op = tags == HM_BAM_TAGS_MD ? 0 : 7, x_op = tags == HM_BAM_TAGS_MD ? 0 : 8;
   (void)hm_crc32_available(); /* probed before the deflate threads exist */
   wbuf_t w; memset(&w, 0, sizeof(w));
   char text[1024];
@@ -1370,21 +1472,29 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
     const uint32_t* ops = b->ops + b->op_off[r];
     const uint8_t* seq = b->seq + b->seq_off[r];
     size_t need_cs = 16;
-    for (uint32_t k = 0; k < nops; k++) { const uint32_t kind = ops[k] & 3u, v = ops[k] >> 2; need_cs += (kind == HM_OP_MATCH) ? 12 : (kind == HM_OP_SUB) ? 3 : (size_t)v + 1; }
+    for (uint32_t k = 0; k < nops; k++) { const uint32_t kind = ops[k] & 3u, v = ops[k] >> 2; need_cs += (kind == HM_OP_MATCH) ? 12 : (kind == HM_OP_SUB) ? 14 : (size_t)v + 14; }
     if (need_cs > cs_cap) { cs_cap = need_cs * 2; cs = (char*)realloc(cs, cs_cap); }
     if ((size_t)nops + 4 > cig_cap) { cig_cap = ((size_t)nops + 4) * 2; cig = (uint32_t*)realloc(cig, cig_cap * 4); }
     if (!cs || !cig) { rc = HM_ERR_ARG; break; }
     size_t lc = 0, ncig = 0;
     int32_t q = qstart, rspan = 0;
+    uint32_t md_run = 0; /* MD: matched bases since the last event */
 #define CIG(op, len) do { if (ncig && (cig[ncig - 1] & 15u) == (uint32_t)(op)) cig[ncig - 1] += (uint32_t)(len) << 4; else cig[ncig++] = ((uint32_t)(len) << 4) | (uint32_t)(op); } while (0)
     if (qstart) CIG(4, qstart);
     for (uint32_t k = 0; k < nops; k++) {
       const uint32_t kind = ops[k] & 3u, v = ops[k] >> 2;
-      if (kind == HM_OP_MATCH) { lc += (size_t)sprintf(cs + lc, ":%u", v); CIG(7, v); q += (int32_t)v; rspan += (int32_t)v; }
+      if (use_md) {
+        if (kind == HM_OP_MATCH) { md_run += v; CIG(m_op, v); q += (int32_t)v; rspan += (int32_t)v; }
+        else if (kind == HM_OP_SUB) { lc += (size_t)sprintf(cs + lc, "%u%c", md_run, (v & 7u) < 4 ? "ATGC"[v & 7u] : 'N'); md_run = 0; CIG(x_op, 1); q += 1; rspan += 1; }
+        else if (kind == HM_OP_INS) { CIG(1, v); q += (int32_t)v; }
+        else { lc += (size_t)sprintf(cs + lc, "%u^", md_run); md_run = 0; for (uint32_t i = 0; i < v; i++) cs[lc++] = 'N'; CIG(2, v); rspan += (int32_t)v; }
+      }
+      else if (kind == HM_OP_MATCH) { lc += (size_t)sprintf(cs + lc, ":%u", v); CIG(7, v); q += (int32_t)v; rspan += (int32_t)v; }
       else if (kind == HM_OP_SUB) { cs[lc++] = '*'; cs[lc++] = (v & 7u) < 4 ? DEC[v & 7u] : 'n'; cs[lc++] = DEC[(v >> 3) & 3u]; CIG(8, 1); q += 1; rspan += 1; }
       else if (kind == HM_OP_INS) { cs[lc++] = '+'; for (uint32_t i = 0; i < v; i++) { const int32_t qq = q + (int32_t)i; cs[lc++] = DEC[(seq[qq >> 2] >> (2 * (qq & 3))) & 3]; } CIG(1, v); q += (int32_t)v; }
       else { cs[lc++] = '-'; for (uint32_t i = 0; i < v; i++) cs[lc++] = 'n'; CIG(2, v); rspan += (int32_t)v; }
     }
+    if (use_md) lc += (size_t)sprintf(cs + lc, "%u", md_run);
     if (ql - q > 0) CIG(4, ql - q);
 #undef CIG
     cs[lc] = 0;
@@ -1411,7 +1521,7 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
       w.p[w.n++] = (uint8_t)((hi << 4) | lo);
     }
     memcpy(w.p + w.n, b->bq + b->bq_off[r], (size_t)ql); w.n += (size_t)ql;
-    w.p[w.n++] = 'c'; w.p[w.n++] = 's'; w.p[w.n++] = 'Z'; memcpy(w.p + w.n, cs, lc + 1); w.n += lc + 1;
+    w.p[w.n++] = use_md ? 'M' : 'c'; w.p[w.n++] = use_md ? 'D' : 's'; w.p[w.n++] = 'Z'; memcpy(w.p + w.n, cs, lc + 1); w.n += lc + 1;
     w.p[w.n++] = 't'; w.p[w.n++] = 'p'; w.p[w.n++] = 'A'; w.p[w.n++] = 'P';
   }
   free(cs); free(cig);

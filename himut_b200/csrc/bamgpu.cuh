@@ -6,7 +6,8 @@
 //   k_bgzf_inflate   one thread per BGZF block: raw DEFLATE (stored, fixed, dynamic), ISIZE and CRC32 checked
 //   k_bam_walk       one thread per entry point (BAI linear-index entry): follows block_size to the next one
 //   k_bam_select     one thread per record: hm_bam_read_batch's selection and checks, counts for the output scans
-//   k_bam_parse      one warp per selected record: qualities, 2-bit bases (if asked), cs -> ops, coordinates, the name
+//   k_bam_parse      one warp per selected record: qualities, 2-bit bases (if asked), cs (or CIGAR + MD) -> ops,
+//                    coordinates, the name
 //
 // Shape of k_bgzf_inflate: a BGZF block is an independent stream of at most 64 KB whose decode is one serial chain
 // (each symbol's length is known only once it is decoded), so one thread decodes one block, and it is the only
@@ -34,15 +35,16 @@ struct Err {                    // first failure, in file order, of each kind
   unsigned long long entry;     // first entry point that is not a record start (~0: none)
   unsigned long long rec;       // first record that fails selection (~0: none)
   unsigned long long stop;      // first record that ends the region (~0: none)
-  unsigned long long parse;     // first selected record that fails cs -> ops (~0: none)
+  unsigned long long parse;     // first selected record that fails cs (or CIGAR + MD) -> ops (~0: none)
 };
 
 struct RecInfo {  // k_bam_select -> k_bam_parse
   uint64_t p;     // offset of block_size in the inflated stream
-  uint32_t cs;    // offset of the cs:Z value from the fixed part
+  uint32_t cs;    // offset of the cs:Z value (md: of the MD:Z value) from the fixed part
   int32_t pos, l_seq, lead, trail, ref_span;
   uint32_t n_ops;
   uint8_t keep;
+  uint8_t md;     // the record has no cs:Z: its ops come from CIGAR + MD:Z
 };
 
 __device__ __forceinline__ uint32_t rd32(const uint8_t* p) {
@@ -301,6 +303,43 @@ __device__ uint32_t cs_count(const char* c) {
   return n;
 }
 
+__device__ __forceinline__ bool md_digit(char c) { return c >= '0' && c <= '9'; }
+__device__ __forceinline__ bool md_alpha(char c) { return (c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z'); }
+// an MD number; saturates far above any reference span (the host decoder's md_num)
+__device__ __forceinline__ long long md_num(const char*& c) {
+  long long n = 0;
+  while (md_digit(*c)) { n = n * 10 + (*c - '0'); if (n > (1ll << 40)) n = 1ll << 40; c++; }
+  return n;
+}
+
+// ops CIGAR + MD give: k_bam_parse's walk without its checks, exact where that walk succeeds, stops where it cannot go on
+__device__ uint32_t md_count(const uint8_t* cig, uint32_t n_cig, const char* c) {
+  long long mnum = md_num(c);
+  uint32_t n = 0, run = 0;
+  for (uint32_t k = 0; k < n_cig; k++) {
+    const uint32_t cg = rd32(cig + 4 * k), op = cg & 15;
+    long long left = cg >> 4;
+    if (left == 0 || op == 4 || op == 5) continue;
+    if (op == 0 || op == 7 || op == 8) {
+      while (left) {
+        if (mnum) { const long long t = mnum < left ? mnum : left; mnum -= t; left -= t; run = 1; continue; }
+        if (!md_alpha(*c)) return n;
+        c++;
+        mnum = md_num(c);
+        n += run + 1; run = 0; left--;
+      }
+    } else if (op == 1) { n += run + 1; run = 0; }
+    else if (op == 2) {
+      if (mnum || *c != '^') return n;
+      c++;
+      while (md_alpha(*c)) c++;
+      mnum = md_num(c);
+      n += run + 1; run = 0;
+    } else return n;
+  }
+  return n + run;
+}
+
 __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n_rec, uint64_t walk_end, int32_t rid,
                              int32_t start, int32_t end, RecInfo* info, unsigned long long* cnt, int n_cnt, uint8_t* code,
                              long long* arg, Err* err) {
@@ -347,6 +386,7 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
   const uint8_t* tag = qual + (l_seq > 0 ? l_seq : 0);
   const uint8_t* rec_end = R + bs;
   const uint8_t* cs = nullptr;
+  const uint8_t* md = nullptr;
   while (tag + 3 <= rec_end) {
     const char ty = (char)tag[2];
     const uint8_t* v = tag + 3;
@@ -358,6 +398,7 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
       if (z == left) { sel_fail(err, code, arg, r, E_TAG_UNTERM, ty); return; }
       adv = z + 1;
       if (tag[0] == 'c' && tag[1] == 's' && ty == 'Z') cs = v;
+      if (tag[0] == 'M' && tag[1] == 'D' && ty == 'Z') md = v;
     } else if (ty == 'A' || ty == 'c' || ty == 'C') adv = 1;
     else if (ty == 's' || ty == 'S') adv = 2;
     else if (ty == 'i' || ty == 'I' || ty == 'f') adv = 4;
@@ -370,12 +411,13 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
     if (adv > left) { sel_fail(err, code, arg, r, E_TAG_PAST, (long long)adv); return; }
     tag = v + adv;
   }
-  if (!cs) { sel_fail(err, code, arg, r, E_NO_CS, 0); return; }
+  if (!cs && !md) { sel_fail(err, code, arg, r, E_NO_CS, 0); return; }  // cs when it is there, else CIGAR + MD
   if (l_seq <= 0 || qual[0] == 0xff) { sel_fail(err, code, arg, r, E_NO_QUAL, 0); return; }
   I.keep = 1;
-  I.cs = (uint32_t)(cs - R);
+  I.md = !cs;
+  I.cs = (uint32_t)((cs ? cs : md) - R);
   I.pos = pos; I.l_seq = l_seq; I.lead = lead; I.trail = trail; I.ref_span = ref_span;
-  I.n_ops = cs_count((const char*)cs);
+  I.n_ops = cs ? cs_count((const char*)cs) : md_count(cig, n_cig, (const char*)md);
   info[r] = I;
   cnt[r] = 1;
   cnt[stride + r] = I.n_ops;
@@ -453,7 +495,86 @@ __global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_
   int64_t q = I.lead, rspan = 0;
   int ec = 0;
   long long ea = 0;
-  while (*c && !ec) {
+  if (I.md) {  // CIGAR + MD: the rules and the order of checks of the host decoder's md_walk (pack.parse_md)
+    const uint8_t* cig = R + 32 + l_name;
+    uint32_t first = n_cig, last = 0;
+    for (uint32_t k = 0; k < n_cig; k++) { const uint32_t op = rd32(cig + 4 * k) & 15; if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; } }
+    int64_t qcore = 0, qclip = 0;
+    for (uint32_t k = 0; k < n_cig && !ec; k++) {
+      const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+      if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) { ec = E_CIGAR_OP; ea = k; } if (op == 4) qclip += ln; }
+      else if (op == 0 || op == 1 || op == 7 || op == 8) qcore += ln;
+      else if (op != 2) { ec = E_CIGAR_OP; ea = k; }
+    }
+    if (!ec && qcore + qclip != l_seq) { ec = E_SPAN_QRY; ea = qcore; }
+    if (!ec) {  // grammar: the end of the longest prefix it accepts must be the end
+      const char* good = cs;
+      if (md_digit(*c)) {
+        while (md_digit(*c)) c++;
+        good = c;
+        while (*c) {
+          if (*c == '^') { const char* s0 = ++c; while (md_alpha(*c)) c++; if (c == s0) break; }
+          else if (md_alpha(*c)) c++;
+          else break;
+          if (!md_digit(*c)) break;
+          while (md_digit(*c)) c++;
+          good = c;
+        }
+      }
+      if (*good || good == cs) { ec = E_MD_TOKEN; ea = good - cs; }
+    }
+    c = cs;
+    long long mnum = md_num(c);
+    uint32_t run = 0;
+    for (uint32_t k = 0; k < n_cig && !ec; k++) {
+      const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+      if (ln == 0 || op == 4 || op == 5) continue;
+      if (op == 0 || op == 7 || op == 8) {
+        int64_t left = ln;
+        while (left && !ec) {
+          if (mnum) {
+            if (op == 8) { ec = E_MD_SPAN; ea = rspan; break; }
+            const int64_t t = mnum < left ? mnum : left;
+            for (int64_t k0 = 0; k0 < t; k0 += 32) {  // first base outside A/C/G/T under the match
+              const bool bad = k0 + lane < t && base_at(seq4, q + k0 + lane) == 0xff;
+              const unsigned m = __ballot_sync(0xffffffffu, bad);
+              if (m) { ec = E_N_MATCH; ea = q + k0 + __ffs(m) - 1; break; }
+            }
+            if (ec) break;
+            run += (uint32_t)t; mnum -= t; q += t; rspan += t; left -= t;
+          } else {
+            if (!*c || *c == '^' || op == 7) { ec = E_MD_SPAN; ea = rspan; break; }
+            const int rc_ = base_code(*c++);
+            mnum = md_num(c);
+            const uint8_t ac = base_at(seq4, q);
+            if (ac == 0xff) { ec = E_SUB_N; ea = q; break; }
+            if (run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; run = 0; }
+            if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_SUB(rc_ < 0 ? HM_BASE_N : (uint32_t)rc_, (uint32_t)ac);
+            n_ops++;
+            q += 1; rspan += 1; left -= 1;
+          }
+        }
+      } else if (op == 1) {
+        if (run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; run = 0; }
+        if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_INS, ln);
+        n_ops++;
+        q += ln;
+      } else {  // D: "^" and as many letters
+        if (mnum || *c != '^') { ec = E_MD_SPAN; ea = rspan; break; }
+        const char* s0 = ++c;
+        while (md_alpha(*c)) c++;
+        if ((uint32_t)(c - s0) != ln) { ec = E_MD_SPAN; ea = rspan; break; }
+        mnum = md_num(c);
+        if (run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; run = 0; }
+        if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_DEL, ln);
+        n_ops++;
+        rspan += ln;
+      }
+    }
+    if (!ec && run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; }
+    if (!ec && (mnum || *c)) { ec = E_MD_SPAN; ea = rspan; }
+  }
+  while (!I.md && *c && !ec) {
     if (*c == ':') {
       long long n = 0;
       c++;

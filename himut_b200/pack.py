@@ -6,6 +6,10 @@ token grammar of the reference's cslib.cs2lst / cs2tuple (src/himut/cslib.py:7-4
 Inputs the reference would crash on are rejected here, loudly, instead of reaching a kernel:
 read bases outside ACGT under a match / substitution (KeyError at caller.py:57,62), "~"
 introns, a cs tag whose spans disagree with the CIGAR-derived coordinates.
+
+parse_md gives the same ops from a CIGAR plus an MD:Z tag, for records without cs:Z (pbmm2 output,
+minimap2 without --cs; `samtools calmd` adds MD to any BAM).  The reference reads cs only and
+raises KeyError on such records; for the same alignment both tags give the same op stream.
 """
 import re
 
@@ -22,6 +26,109 @@ for _b, _c in abi.BASE2CODE.items():
 
 class BatchFormatError(ValueError):
     pass
+
+
+# CIGAR + MD:Z.  The messages are those of csrc/bamerr.h, which both native decoders use, so that the three
+# implementations reject a record with the same words.
+_MD_GRAMMAR = re.compile(r"[0-9]+(?:(?:[A-Za-z]|\^[A-Za-z]+)[0-9]+)*")
+_MD_PART = re.compile(r"[0-9]+|\^[A-Za-z]+|[A-Za-z]")
+MD_ERR = {
+    "md_token": "%s: unsupported MD:Z token (%d)",
+    "md_span": "%s: MD:Z and CIGAR disagree at reference offset %d",
+    "cigar_op": "%s: unsupported CIGAR op (N, P, or a clip inside the alignment) at CIGAR index %d",
+    "span_qry": "%s: cs query span != aligned query span (%d)",
+    "n_match": "%s: read base outside A/C/G/T under a cs match (reference: KeyError) (%d)",
+    "sub_n": "%s: substitution to a base outside A/C/G/T (the reference pileup raises KeyError) (%d)",
+}
+_M, _I, _D, _S, _H, _EQ, _X = 0, 1, 2, 4, 5, 7, 8
+
+
+def parse_md(cigar, md, qseq, qstart, qname="read"):
+    """CIGAR [(op, len), ...] (BAM op codes) + MD:Z -> (ops, ref_span, query_span), the ops cs gives for the
+    same alignment: one MATCH per maximal run of matched bases, SUB(MD letter, read base) per mismatch, INS / DEL
+    with the CIGAR length.  qseq is the full read (soft clips included), qstart its leading soft clip.
+
+    Checked in this order, each failure the first one the walk meets:
+      - CIGAR ops: N, P, codes past X, and S / H between the first and the last aligned op are unsupported
+        (cs writes introns as "~", which parse_cs rejects too);
+      - the CIGAR's query length must be len(qseq);
+      - MD grammar [0-9]+(([A-Za-z]|^[A-Za-z]+)[0-9]+)*;
+      - the walk: M, = and X take reference positions from MD; a match run goes on across M / = / X and across
+        MD numbers and ends at a mismatch, an I or a D.  An MD letter is a SUB whose ref base is the letter (not
+        A/C/G/T: N, as cs "*nx") and whose alt base is SEQ there (not A/C/G/T: rejected, as cs "*xn"); nothing
+        checks that they differ, as for cs "*xy".  Matched read bases must be A/C/G/T.  "=" over an MD letter,
+        "X" over an MD match, D without "^" and as many letters (any letters: only the length is kept), MD
+        running out, or MD left at the end (a trailing 0 is fine) mean MD and CIGAR disagree.
+    Ops of length 0 are skipped."""
+    def fail(key, arg):
+        raise BatchFormatError(MD_ERR[key] % (qname, arg))
+
+    core = [i for i, (o, _l) in enumerate(cigar) if o not in (_S, _H)]
+    qcore = qclip = 0
+    for i, (o, l) in enumerate(cigar):
+        if o in (_S, _H):
+            if core and core[0] < i < core[-1]:
+                fail("cigar_op", i)
+            qclip += l if o == _S else 0
+        elif o in (_M, _I, _EQ, _X):
+            qcore += l
+        elif o != _D:
+            fail("cigar_op", i)
+    if qcore + qclip != len(qseq):
+        fail("span_qry", qcore)
+    m = _MD_GRAMMAR.match(md)
+    if m is None or m.end() != len(md):
+        fail("md_token", m.end() if m else 0)
+    parts = _MD_PART.findall(md)
+    mnum, ti = int(parts[0]), 1
+    codes = _CODE[np.frombuffer(qseq.encode(), dtype=np.uint8)]
+    ops, run, q, r = [], 0, qstart, 0
+
+    def flush():
+        nonlocal run
+        if run:
+            ops.append(abi.make_op(abi.OP_MATCH, run))
+            run = 0
+
+    for o, l in cigar:
+        if l == 0 or o in (_S, _H):
+            continue
+        if o in (_M, _EQ, _X):
+            k = 0
+            while k < l:
+                if mnum:
+                    if o == _X:
+                        fail("md_span", r)
+                    t = min(mnum, l - k)
+                    bad = np.flatnonzero(codes[q:q + t] == 255)
+                    if bad.size:
+                        fail("n_match", q + int(bad[0]))
+                    run += t; mnum -= t; q += t; r += t; k += t
+                else:
+                    if ti >= len(parts) or parts[ti][0] == "^" or o == _EQ:
+                        fail("md_span", r)
+                    ref = abi.BASE2CODE.get(parts[ti].upper(), abi.BASE_N)
+                    mnum, ti = int(parts[ti + 1]), ti + 2
+                    if codes[q] == 255:
+                        fail("sub_n", q)
+                    flush()
+                    ops.append(abi.make_sub(ref, int(codes[q])))
+                    q += 1; r += 1; k += 1
+        elif o == _I:
+            flush()
+            ops.append(abi.make_op(abi.OP_INS, l))
+            q += l
+        else:
+            if mnum or ti >= len(parts) or parts[ti][0] != "^" or len(parts[ti]) - 1 != l:
+                fail("md_span", r)
+            mnum, ti = int(parts[ti + 1]), ti + 2
+            flush()
+            ops.append(abi.make_op(abi.OP_DEL, l))
+            r += l
+    flush()
+    if mnum or ti < len(parts):
+        fail("md_span", r)
+    return ops, r, q - qstart
 
 
 def parse_cs(cs, qseq, qstart):
@@ -96,9 +203,12 @@ class BatchBuilder:
         self.seq_n = self.bq_n = self.ops_n = 0
         self.qnames = {}
 
-    def add(self, *, tstart, tend, qstart, qend, qseq, bq, mapq, is_secondary, qname, cs=None, ops=None):
+    def add(self, *, tstart, tend, qstart, qend, qseq, bq, mapq, is_secondary, qname, cs=None, ops=None, cigar=None, md=None):
+        """the record's ops come from `ops`, else from `cs`, else from `cigar` + `md` (parse_md)"""
         qb = qseq.encode() if isinstance(qseq, str) else bytes(qseq)
-        if ops is None:
+        if ops is None and cs is None and md is not None:
+            ops, rspan, qspan = parse_md(cigar, md, qb.decode(), qstart, qname)
+        elif ops is None:
             ops, rspan, qspan = parse_cs(cs, qb.decode(), qstart)
         else:
             ops = [int(w) for w in ops]

@@ -40,9 +40,12 @@ int hm_bam_ref_len(const hm_bam* b, int i);
 /* the records of contig `rid` overlapping the 0-based half-open window [start, end), in file
  * order, each once (pysam fetch semantics, caller.py:299); secondary records (0x100) are
  * dropped as bamlib.BAM.__init__ drops them (bamlib.py:17), supplementary ones are kept.
- * Inputs the reference would crash on are rejected with HM_ERR_ARG and a message: no cs:Z tag,
- * missing qualities, a read base outside A/C/G/T under a cs match or as the substituted base, cs spans that
- * disagree with the CIGAR, records whose fields run past their block_size.  Hard-clipped records are decoded as pysam
+ * A record's ops come from its cs:Z tag; a record without cs:Z but with MD:Z is decoded from CIGAR + MD
+ * (pack.parse_md; the reference raises KeyError there), to the ops cs gives for the same alignment.
+ * Inputs the reference would crash on are rejected with HM_ERR_ARG and a message: neither cs:Z nor MD:Z (worded
+ * "no cs:Z tag"), missing qualities, a read base outside A/C/G/T under a match or as the substituted base, cs spans
+ * that disagree with the CIGAR, an MD:Z outside its grammar or disagreeing with the CIGAR, CIGAR ops N and P and
+ * clips inside the alignment (MD path), records whose fields run past their block_size.  Hard-clipped records are decoded as pysam
  * presents them (SEQ holds no hard-clipped base; lead / trail count soft clips only).  `threads` = inflate threads. */
 int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int threads, hm_read_batch* out);
 
@@ -75,6 +78,14 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
  * query names "read<qname_id>"), BGZF blocks deflated on `threads` threads at zlib `level` */
 int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                        int level, int threads);
+/* the same with the alignment written as `tags`: HM_BAM_TAGS_CS is hm_bam_write_batch (cs:Z, CIGAR =/X);
+ * HM_BAM_TAGS_MD writes MD:Z and no cs:Z with a CIGAR of M; HM_BAM_TAGS_MD_EQX MD:Z with the CIGAR of =/X.  MD
+ * separates adjacent events with 0 and writes deleted bases as N. */
+#define HM_BAM_TAGS_CS 0
+#define HM_BAM_TAGS_MD 1
+#define HM_BAM_TAGS_MD_EQX 2
+int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
+                            int level, int threads, int tags);
 
 /* compact quality stream of a packed batch (struct hm_bq_compact, himut_b200.h), for the host -> device copy: `mask` (bq_bytes / 8 bytes) and
  * `exc_off` (n_reads + 1 entries) are caller allocated, the exception bytes are allocated here (*exc_out, release

@@ -8,7 +8,9 @@ power limit are read in the same run.
 --seq: the same for normcounts, which decodes with the 2-bit base stream: host read_batch(seq=True, compact=True) against
 decode_region(seq=True), with the device decode without seq timed beside it (k_bam_parse with and without the base
 stream), then the normcounts worker's BAM -> tri counts with decode="host", "device" and "auto", whose outputs must agree.
-    python tools/decode_trace.py [--reps 3] [--seq] [--out profiles/decode_trace_r03.json | decode_trace_norm_r04.json]"""
+--tags md | md_eqx: the BAMs carry CIGAR + MD:Z instead of cs:Z (the decoders' MD path).
+--group S: only the decode group [S, S + GROUP_SPAN) of the 64 Mb contig, no worker runs (A/B of the decode kernels).
+    python tools/decode_trace.py [--reps 3] [--seq] [--tags cs] [--group S] [--out profiles/decode_trace_r03.json | decode_trace_norm_r04.json]"""
 import argparse
 import json
 import os
@@ -23,6 +25,8 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 ap = argparse.ArgumentParser()
 ap.add_argument("--reps", type=int, default=3)
 ap.add_argument("--seq", action="store_true", help="decode with the base stream and time the normcounts worker")
+ap.add_argument("--tags", default="cs", choices=["cs", "md", "md_eqx"], help="the alignment tag the BAMs are written with")
+ap.add_argument("--group", type=int, default=None, help="time only the decode group starting here, on the 64 Mb contig")
 ap.add_argument("--out", default=None)
 a = ap.parse_args()
 if a.out is None:
@@ -34,10 +38,10 @@ from himut_b200 import bamdec, caller, gtmodel, lib, normcounts, synth, worker  
 card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv"], stdout=subprocess.PIPE, text=True).stdout
 tmp = tempfile.mkdtemp()
 inputs, refs = {}, {}
-for label, n, seed in (("64mb", 64_000_000, 5), ("1mb", 1_000_000, None)):
+for label, n, seed in (("64mb", 64_000_000, 5), ("1mb", 1_000_000, None))[:1 if a.group is not None else 2]:
     d = synth.generate(n, **({"seed": seed} if seed is not None else {}), copy=False)
     path = os.path.join(tmp, label + ".bam")
-    bamdec.write_batch_bam(path, "chr1", n, d.batch)
+    bamdec.write_batch_bam(path, "chr1", n, d.batch, **({"tags": a.tags} if a.tags != "cs" else {}))
     inputs[label] = (path, n, os.path.getsize(path))
     if a.seq:
         refs[path] = bytes(d.ref)
@@ -47,6 +51,8 @@ G = worker.GROUP_SPAN
 
 def groups(n):
     """the worker's decode groups, then (64 Mb contig) smaller regions at its start: where the two decoders cross"""
+    if a.group is not None:
+        return [(a.group, min(a.group + G, n))]
     g = [(s, min(s + G, n)) for s in range(0, n, G)]
     return g + [(0, L) for L in (1_000_000, 2_000_000, 4_000_000, 8_000_000) if L < n]
 
@@ -100,7 +106,7 @@ def norm_worker_run(path, n, mode):
         normcounts.normcounts_region = real
 
 
-out = {"card": card.strip(), "group_span": G, "threads_host_decoder": bamdec.default_threads(), "inputs": {}, "decode": [], "worker": []}
+out = {"card": card.strip(), "tags": a.tags, "group_span": G, "threads_host_decoder": bamdec.default_threads(), "inputs": {}, "decode": [], "worker": []}
 if a.seq:
     out["seq"] = True
     out["device_decode_min_bytes"] = {"call": caller.DEVICE_DECODE_MIN_BYTES, "normcounts": normcounts.DEVICE_DECODE_MIN_BYTES}
@@ -129,6 +135,8 @@ for label, (path, n, size) in inputs.items():
                                                                                      td * 1e3, {k: round(v, 2) for k, v in kt.items()}),
                   file=sys.stderr)
     nb.close()
+    if a.group is not None:
+        continue
     nb = bamdec.NativeBam(path)
     whole_bases = nb.read_batch("chr1", 0, n, seq=False).aligned_bases
     nb.close()

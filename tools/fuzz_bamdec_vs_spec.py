@@ -3,7 +3,9 @@
 adversarial batches (dense substitutions / indels, N bases, soft clips, secondary records, duplicate names) written
 to multi-contig BAM files: random windows, thread counts, with and without the base stream — packed batches must be
 equal byte for byte, the window pre-pass must return the same read lengths.
-    python tools/fuzz_bamdec_vs_spec.py 0 200
+    python tools/fuzz_bamdec_vs_spec.py 0 200 [--tags md | md_eqx]
+--tags: the files carry CIGAR + MD:Z instead of cs:Z (the decoders' MD path; the Python side reads them with
+pack.parse_md).
 (400 seeds x 6 windows on 2026-10-18: no mismatch.)"""
 import os
 import random
@@ -30,7 +32,13 @@ def same(a, b, skip=()):
 
 
 def main():
-    lo, hi = int(sys.argv[1]), int(sys.argv[2])
+    import argparse
+    ap = argparse.ArgumentParser()
+    ap.add_argument("lo", type=int)
+    ap.add_argument("hi", type=int)
+    ap.add_argument("--tags", default="cs", choices=["cs", "md", "md_eqx"])
+    args = ap.parse_args()
+    lo, hi = args.lo, args.hi
     bad = 0
     with tempfile.TemporaryDirectory() as tmp:
         for seed in range(lo, hi):
@@ -42,7 +50,7 @@ def main():
                                                       max_len=rnd.choice([300, 2000, 9000]))
                 contigs.append(("c%d" % k, n, batch))
             path = os.path.join(tmp, "f%d.bam" % seed)
-            bamio.write_batches_bam(path, contigs)
+            bamio.write_batches_bam(path, contigs, tags=args.tags)
             nb = bamdec.NativeBam(path, threads=rnd.choice([1, 2, 5]))
             rd = bamio.BamReader(path)
             qnames = {}
