@@ -2,24 +2,22 @@
 //
 // The reference piles up every aligned base of every read (caller.update_allelecounts, caller.py:44-72) and then looks
 // at the pileup only where a read carries a candidate substitution (caller.py:324-336).  The first version of this
-// path (kernels.cuh: k_read_scan -> k_candidates -> library sort -> k_site_entries_by_read -> k_site_reduce) touched
-// the quality stream twice: once to sum it for the QV gate, and once more, one 32-byte sector per looked-up byte, to
-// gather the pileup columns.  Here the quality stream is read exactly once:
+// path (kernels.cuh: k_read_scan -> k_candidates -> library sort -> k_site_entries_by_read -> k_site_reduce) streamed
+// the whole quality stream on every call to sum it for the QV gate.  Here no call streams it: the QV gate reads the
+// per-read quality sum the batch carries since it became resident (DevBatch.bq_total: k_bq_expand or k_bq_sum), and
+// the pileup columns take one quality byte per (site, covering read):
 //
-//   k_call_pairs   (ops only)  one warp per (chunk, read) pair: cs op prefix scan, mismatch list, identity / MAPQ /
+//   k_call_pairs   (ops only)  one thread per (chunk, read) pair: cs op walk, mismatch list, QV / MAPQ / identity /
 //                  length gates, [--phase] read haplotype, then trim + mismatch-window test of every substitution
 //                  (bamlib.get_tsbs_candidates, bamlib.py:69-86) -> candidate keys into the chunk's own segment.
-//                  The QV gate needs every quality byte, so candidates are emitted *speculatively* with their read.
+//                  A read that passes every gate counts its query name (num_ccs).
 //   k_site_sort    one CTA per 2^17-position tile of a chunk: the chunk's keys -> sorted distinct sites without a
 //                  comparison sort: position bitmap in shared memory, popcount prefix = rank, 16-bit (ref, alt) mask
 //                  per distinct position (set(somatic_tsbs_candidate_lst), caller.py:324).
 //   k_tile_scan    exclusive scan of the per-tile site counts (one CTA); k_site_range2: final key array, the
 //                  file-order read range of every site, entry slots initialised.
-//   k_call_scan    the one pass over the quality stream.  One warp per (chunk, read) pair; the first pair of a read
-//                  streams the read's qualities through a 3-stage cp.async.bulk (TMA) ring in shared memory, sums
-//                  them (QV gate, bamlib.get_qv) and, while a block is in shared memory, answers the pileup lookups
-//                  of the sites its read covers from it.  No second touch of the stream, no sector gather.
-//   k_site_valid   only if some read failed the QV gate: sites keep only candidates of reads that passed.
+//   k_call_scan    the pileup entries.  One warp per (chunk, read) pair: the sites the read covers, its op prefixes
+//                  in shared memory, the allele of every site and one quality byte per site that has a base.
 //   k_site_reduce  (kernels.cuh) per site, reads in file order: counts, ordered fp64 sums, PL / GQ, cascade, record.
 //   k_compact_sites  records the host wants, stably compacted (no germline restatements when asked, no dropped sites).
 //
@@ -27,7 +25,6 @@
 // high-water estimate with an overflow flag (distinct sites), counts stay on the device.
 #pragma once
 #include "kernels.cuh"
-#include "normcounts.cuh" // mbarrier / cp.async.bulk helpers
 
 #ifndef HC_MAX_OPS
 #define HC_MAX_OPS 96                  // ops of a read staged per warp; longer lists use the batch's global op_t / op_q
@@ -37,13 +34,6 @@
 #define HC_TILE_WORDS (HC_TILE / 32u)
 #define HC_CAPD 4096u                  // distinct positions of a tile kept in shared memory (more: global scratch)
 #define HC_SORT_THREADS 512
-#ifndef HC_BLK
-#define HC_BLK 2048u                   // bytes per quality stage
-#endif
-#ifndef HC_NS
-#define HC_NS 2                        // stages per warp
-#endif
-#define HC_WARPS 8                     // warps per CTA of k_call_pairs / k_call_scan
 #define HC_KEY_POS_BITS 27             // a chunk may span < 2^27 positions on this path (else the first version runs)
 
 struct OpView { const uint32_t* w; const uint32_t* t; const uint32_t* q; uint32_t n; };
@@ -121,9 +111,8 @@ __device__ __forceinline__ int warp_read_hap_ops(const DevBatch& b, uint32_t r, 
 //
 // pair_c[pr]: the pair's chunk, or 0xffffffff when the chunk does not fetch the read (k_call_scan starts from it).
 // pair_hap (--phase only): 0 / 1 / 2 ("."), 3 = not fetched.
-// read_counted[r] = 1: some chunk fetched r, r passed the MAPQ / identity / length gates there and (--phase) got a
-//   haplotype: if its QV gate passes too (k_call_scan) it counts in num_ccs and its candidates are real.
-// first_pair[r]: the lowest pair index that fetches r; that pair's warp streams the read's qualities in k_call_scan.
+// num_ccs: a pair whose read passes the QV / MAPQ / identity / length gates and (--phase) has a haplotype marks the
+//   read's query name; the first to mark a name counts it (m.num_ccs counts distinct names, caller.py:318-320).
 // Candidates: the thread reserves one slot per substitution of its read in the chunk's segment (one atomic), fills
 //   the slots of the substitutions that pass and marks the others as holes (HC_KEY_HOLE).
 #define HC_KEY_HOLE 0xffffffffu
@@ -206,8 +195,8 @@ template <bool kSeq, bool kShared>
 __device__ __forceinline__ void call_pair_body(const DevBatch& b, const DevParams& p, const DevPhase& ph, const uint32_t* ops_any,
                                                const hm_chunk& ch, uint32_t c, uint32_t r, uint64_t pr, uint32_t n, uint64_t o0,
                                                int32_t ts, int32_t te, int32_t qlen, uint32_t qstart, int mapq, uint8_t* pair_hap,
-                                               uint8_t* read_counted, const uint64_t* seg_off, uint32_t* seg_cnt, uint32_t* seg_keys,
-                                               uint32_t* seg_read) {
+                                               uint32_t* qname_seen32, unsigned long long* num_ccs, const uint64_t* seg_off, uint32_t* seg_cnt,
+                                               uint32_t* seg_keys, uint32_t* seg_read) {
   struct Ops { // address-space-specific loads; the shared window address is taken once
     const uint32_t* p;
     uint32_t sbase;
@@ -241,8 +230,10 @@ __device__ __forceinline__ void call_pair_body(const DevBatch& b, const DevParam
     }
   }
 
-  // read gates of caller.py:310-317 except the QV gate (k_call_scan has the quality sum), same order of evaluation
+  // read gates of caller.py:310-317, same order of evaluation; the QV gate is bamlib.get_qv (np.mean of the read's
+  // qualities: the resident integer sum divided once)
   bool pre_ok = true;
+  if (__ddiv_rn((double)__ldg(b.bq_total + r), (double)qlen) < (double)p.min_qv) pre_ok = false;
   if (mapq < p.min_mapq) pre_ok = false;
   const double ident = __ddiv_rn((double)nm, (double)(nm + ns + il + dl));
   if (ident < p.min_sequence_identity) pre_ok = false;
@@ -253,7 +244,11 @@ __device__ __forceinline__ void call_pair_body(const DevBatch& b, const DevParam
     if (hap > 1) return;
   }
   if (!pre_ok) return;
-  read_counted[r] = 1;
+  { // one byte per query name, set through 32-bit atomics
+    const uint32_t qn = __ldg(b.qname_id + r);
+    const uint32_t bit = 1u << (8u * (qn & 3u));
+    if (!(atomicOr(qname_seen32 + (qn >> 2), bit) & bit)) atomicAdd(num_ccs + (r & 7u), 1ull);
+  }
   if (n_sub_in == 0) return;
 
   // walk 2: bamlib.get_tsbs_candidates (bamlib.py:69-86) for every substitution of the read that lies in the chunk.
@@ -316,7 +311,7 @@ __device__ __forceinline__ void call_pair_body(const DevBatch& b, const DevParam
 template <bool kSeq>
 __global__ void __launch_bounds__(128) k_call_pairs(DevBatch b, DevParams p, DevPhase ph, const hm_chunk* chunks, uint32_t n_chunks,
                                                     const uint64_t* pair_off, uint64_t n_pairs, uint32_t* pair_c, uint8_t* pair_hap,
-                                                    uint8_t* read_counted, uint32_t* first_pair, const uint64_t* seg_off,
+                                                    uint32_t* qname_seen32, unsigned long long* num_ccs, const uint64_t* seg_off,
                                                     uint32_t* seg_cnt, uint32_t* seg_keys, uint32_t* seg_read) {
   extern __shared__ uint32_t s_ops[]; // HC_A_CAP
   __shared__ unsigned long long s_span[2];
@@ -347,7 +342,6 @@ __global__ void __launch_bounds__(128) k_call_pairs(DevBatch b, DevParams p, Dev
       active = false;
     } else {
       pair_c[pr] = c;
-      atomicMin(first_pair + r, (uint32_t)pr);
     }
   }
   { // the run of the op stream this CTA's reads span: warp reduction, one shared atomic per warp
@@ -378,11 +372,11 @@ __global__ void __launch_bounds__(128) k_call_pairs(DevBatch b, DevParams p, Dev
   __syncthreads();
   if (!active) return;
   if (staged)
-    call_pair_body<kSeq, true>(b, p, ph, s_ops + (o0 - sp_lo), ch, c, r, pr, n, o0, ts, te, qlen, qstart, mapq, pair_hap, read_counted, seg_off,
-                               seg_cnt, seg_keys, seg_read);
+    call_pair_body<kSeq, true>(b, p, ph, s_ops + (o0 - sp_lo), ch, c, r, pr, n, o0, ts, te, qlen, qstart, mapq, pair_hap, qname_seen32, num_ccs,
+                               seg_off, seg_cnt, seg_keys, seg_read);
   else
-    call_pair_body<kSeq, false>(b, p, ph, b.ops + o0, ch, c, r, pr, n, o0, ts, te, qlen, qstart, mapq, pair_hap, read_counted, seg_off, seg_cnt,
-                                seg_keys, seg_read);
+    call_pair_body<kSeq, false>(b, p, ph, b.ops + o0, ch, c, r, pr, n, o0, ts, te, qlen, qstart, mapq, pair_hap, qname_seen32, num_ccs,
+                                seg_off, seg_cnt, seg_keys, seg_read);
 }
 
 // ============================================================================ k_site_sort
@@ -536,11 +530,11 @@ __global__ void __launch_bounds__(1024) k_tile_scan(const uint32_t* tile_cnt, ui
 }
 
 // final key array (chunk << 36 | tpos << 4 | ref << 2 | alt, sorted), the file-order read range of every site
-// (as k_site_range), its entry slots set to "unwritten", its validity flag cleared
+// (as k_site_range), its entry slots set to "unwritten"
 __global__ void __launch_bounds__(256) k_site_range2(DevBatch b, const hm_chunk* chunks, const uint32_t* tile_chunk, const uint32_t* tile_src,
                                                      const uint32_t* tile_dst, uint32_t n_tiles, const uint32_t* keys_tmp,
                                                      const unsigned long long* n_keys_dev, unsigned long long* keys, uint32_t* site_lo,
-                                                     uint32_t* site_n, uint32_t* entries, uint64_t stride, uint8_t* site_valid, uint32_t n_slots) {
+                                                     uint32_t* site_n, uint32_t* entries, uint64_t stride, uint32_t n_slots) {
   const uint64_t ki = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (ki >= *n_keys_dev) return;
   const uint32_t t = upper_bound_dev(tile_dst, n_tiles + 1, (uint32_t)ki) - 1; // last tile with tile_dst <= ki (empty tiles repeat a value)
@@ -556,103 +550,64 @@ __global__ void __launch_bounds__(256) k_site_range2(DevBatch b, const hm_chunk*
   const uint32_t n = hi > lo ? hi - lo : 0u;
   site_lo[ki] = ch.read_lo + lo;
   site_n[ki] = n;
-  site_valid[ki] = 0;
   const uint32_t ns = min(n, n_slots);
   for (uint32_t s = 0; s < ns; s++) entries[(uint64_t)s * stride + ki] = HM_ENT_UNWRITTEN;
 }
 
 // ============================================================================ k_call_scan
-// One warp per (chunk, read) pair, four warps per CTA.  Shared memory per warp: HC_NS quality stages with their
-// mbarriers, the read's ops with their prefixes, and the pair's site list (query position, entry without its quality,
-// entry address).  The pair that owns the read (first_pair) and whose read can still count (read_counted) streams the
-// read's qualities: lane 0 issues the first bulk copies as soon as the read is known — the site searches, the op scan
-// and the site list are built while they fly — and keeps HC_NS copies in flight; every block is summed from shared
-// memory and then serves the listed sites whose query position lies in it.  Other pairs fetch their few quality bytes
-// directly.
+// One warp per (chunk, read) pair, HC_SCAN_WARPS warps per CTA.  The warp finds the chunk's sites the read can touch,
+// stages the read's ops with their prefixes in shared memory, lists the first HC_SITES sites in registers (entry
+// without its quality, query position of the base, entry address) and then fetches their quality bytes, every load
+// of the list issued before any of its entries is written.  The QV gate is k_call_pairs' (the resident quality sum):
+// nothing here streams the qualities, a lookup costs one sector of the stream.
 #ifndef HC_SCAN_WARPS
 #define HC_SCAN_WARPS 4
 #endif
-// Ten CTAs of four warps per SM is where the kernel runs best (B200, 64 Mb contig at 30x: 0.365 ms; eight CTAs with a
-// 96-site list and 128 staged ops 0.397 ms; twelve CTAs need spills: 0.40 - 0.42 ms): 48 registers and 21 KB per CTA.
 #ifndef HC_SITES
 #define HC_SITES 64 // sites of a pair kept in the list (registers); the rest go the direct way
 #endif
 #ifndef HC_SCAN_MINB
 #define HC_SCAN_MINB 10 // resident CTAs per SM asked of the compiler (register budget)
 #endif
-#ifndef HC_PREFETCH
-#define HC_PREFETCH 1 // the rest of the read is requested into L2 when its first blocks are asked for
-#endif
 
 struct __align__(16) ScanWarp {
-  uint8_t bq[HC_NS][HC_BLK];
   uint32_t w[HC_MAX_OPS], t[HC_MAX_OPS], q[HC_MAX_OPS];
-  uint64_t bar[HC_NS];
-  uint64_t pad;
 };
 
 template <bool kSeq>
 __global__ void __launch_bounds__(32 * HC_SCAN_WARPS, HC_SCAN_MINB) k_call_scan(DevBatch b, DevParams p, const hm_chunk* chunks, const uint64_t* pair_off,
                                                                   uint64_t n_pairs, const uint32_t* pair_c, const uint8_t* pair_hap,
-                                                                  const uint8_t* read_counted, const uint32_t* first_pair,
                                                                   const uint32_t* tile_off, const uint32_t* tile_dst,
                                                                   const unsigned long long* keys, const uint32_t* site_lo,
                                                                   const uint32_t* site_n, uint32_t* entries, uint32_t stride,
-                                                                  uint8_t* qv_fail_read, unsigned int* qv_fail_any, uint32_t* qname_seen32,
-                                                                  unsigned long long* num_ccs, const unsigned long long* n_keys_dev, uint32_t n_slots) {
+                                                                  const unsigned long long* n_keys_dev, uint32_t n_slots) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   const uint64_t pr = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   if (pr >= n_pairs) return;
   const uint32_t c = __ldg(pair_c + pr);
   if (c == 0xffffffffu) return; // the chunk does not fetch the read
+  if (*n_keys_dev == 0) return; // no sites (also when the site list overflowed its buffers: the host runs the call again)
   ScanWarp* S = reinterpret_cast<ScanWarp*>(smem_raw) + wid;
-  const int32_t ch_read_lo = (int32_t)__ldg(&chunks[c].read_lo);
   const uint32_t to0 = __ldg(tile_off + c), to1 = __ldg(tile_off + c + 1);
-  const uint32_t r = (uint32_t)ch_read_lo + (uint32_t)(pr - __ldg(pair_off + c));
+  const uint32_t r = __ldg(&chunks[c].read_lo) + (uint32_t)(pr - __ldg(pair_off + c));
   const int32_t ts = __ldg(b.tstart + r), te = __ldg(b.tend + r);
   const uint32_t n = __ldg(b.n_ops + r);
-  const uint64_t o0 = __ldg(b.op_off + r);
-  const uint64_t bq0 = __ldg(b.bq_off + r);
-  const uint32_t qlen = (uint32_t)__ldg(b.qlen + r);
-  const uint32_t qstart = (uint32_t)__ldg(b.qstart + r);
-  const bool owner = __ldg(first_pair + r) == (uint32_t)pr && __ldg(read_counted + r) != 0;
-  const uint32_t hap = p.phase ? (uint32_t)__ldg(pair_hap + pr) : 2u;
   const uint32_t k_lo = __ldg(tile_dst + to0), k_hi = __ldg(tile_dst + to1);
-  const bool have_sites = *n_keys_dev != 0; // 0 also when the site list overflowed its buffers: the host runs the call again
-  const uint8_t* bqg = b.bq + bq0;
-  const uint32_t nbytes = (qlen + 15u) & ~15u; // the stream is padded to 16 bytes per read
-  const uint32_t nblk = owner ? (nbytes + HC_BLK - 1u) / HC_BLK : 0u;
-
-  // the first copies leave before anything else is looked at
-  if (owner) {
-    if (lane == 0) {
-#pragma unroll
-      for (int s = 0; s < HC_NS; s++) mbar_init(&S->bar[s], 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      for (uint32_t s = 0; s < (uint32_t)HC_NS && s < nblk; s++) {
-        const uint32_t bytes = min(HC_BLK, nbytes - s * HC_BLK);
-        mbar_arrive_expect_tx(&S->bar[s], bytes);
-        bulk_g2s(S->bq[s], bqg + (size_t)s * HC_BLK, bytes, &S->bar[s]);
-      }
-#if HC_PREFETCH
-      if (nbytes > HC_NS * HC_BLK) bulk_prefetch_l2(bqg + (size_t)HC_NS * HC_BLK, nbytes - HC_NS * HC_BLK);
-#endif
-    }
-    __syncwarp();
-  }
+  if (n == 0 || k_lo >= k_hi) return;
 
   // the chunk's sites the read can touch: rpos in [ts, te], i.e. tpos in [ts + 1, te + 1]
-  uint32_t s_lo = 0, s_hi = 0;
-  if (n && have_sites && k_lo < k_hi) {
-    const unsigned long long kb = (unsigned long long)c << 36;
-    s_lo = warp_lower_bound_u64(keys, k_lo, k_hi, kb | ((unsigned long long)(uint32_t)(ts + 1) << 4), lane);
-    s_hi = warp_lower_bound_u64(keys, s_lo, k_hi, kb | ((unsigned long long)(uint32_t)(te + 2) << 4), lane);
-  }
-  if (!owner && s_lo >= s_hi) return;
+  const unsigned long long kb = (unsigned long long)c << 36;
+  const uint32_t s_lo = warp_lower_bound_u64(keys, k_lo, k_hi, kb | ((unsigned long long)(uint32_t)(ts + 1) << 4), lane);
+  const uint32_t s_hi = warp_lower_bound_u64(keys, s_lo, k_hi, kb | ((unsigned long long)(uint32_t)(te + 2) << 4), lane);
+  if (s_lo >= s_hi) return;
+  const uint64_t o0 = __ldg(b.op_off + r);
+  const uint8_t* bqg = b.bq + __ldg(b.bq_off + r);
+  const uint32_t qlen = (uint32_t)__ldg(b.qlen + r);
+  const uint32_t hap = p.phase ? (uint32_t)__ldg(pair_hap + pr) : 2u;
   const bool staged = n <= HC_MAX_OPS;
-  if (staged && s_lo < s_hi) { // the prefix scan again (registers only): cheaper than keeping 8 B per op in HBM
-    uint32_t t_carry = 0, q_carry = qstart;
+  if (staged) { // the prefix scan again (registers only): cheaper than keeping 8 B per op in HBM
+    uint32_t t_carry = 0, q_carry = (uint32_t)__ldg(b.qstart + r);
     for (uint32_t base = 0; base < n; base += 32) {
       const uint32_t k = base + lane;
       const uint32_t w = k < n ? __ldg(b.ops + o0 + k) : 0u;
@@ -690,6 +645,8 @@ __global__ void __launch_bounds__(32 * HC_SCAN_WARPS, HC_SCAN_MINB) k_call_scan(
     if (has_base) { *q_out = q; *e_out = e; *at_out = at; }
     else entries[at] = e;
   };
+  // the quality byte of query position q (0 past the read's end: malformed ops)
+  auto qual = [&](uint32_t q) { return q < qlen ? (uint32_t)__ldg(bqg + q) : 0u; };
 
   // the pair's site list (the first HC_SITES sites), HC_SITES / 32 per lane, in registers
   const uint32_t n_list = min(s_hi - s_lo, (uint32_t)HC_SITES);
@@ -700,106 +657,19 @@ __global__ void __launch_bounds__(32 * HC_SCAN_WARPS, HC_SCAN_MINB) k_call_scan(
     lq[g] = 0xffffffffu; le[g] = 0; la[g] = 0;
     if (i < n_list) site(s_lo + i, &lq[g], &le[g], &la[g]);
   }
-
-  if (owner) {
-    uint32_t acc = 0;
-    for (uint32_t blk = 0; blk < nblk; blk++) {
-      const uint32_t st = blk % HC_NS, parity = (blk / HC_NS) & 1u;
-      mbar_wait(&S->bar[st], parity);
-      const uint32_t blk0 = blk * HC_BLK;
-      const uint32_t bytes = min(HC_BLK, nbytes - blk0);
-      const uint4* s4 = reinterpret_cast<const uint4*>(S->bq[st]);
-      if (bytes == HC_BLK && blk0 + HC_BLK <= qlen) { // a full block inside the read: four words per lane, no edge to mind
-        const uint4 v0 = s4[lane], v1 = s4[lane + 32], v2 = s4[lane + 64], v3 = s4[lane + 96];
-        acc = sum4(v0.x, acc); acc = sum4(v0.y, acc); acc = sum4(v0.z, acc); acc = sum4(v0.w, acc);
-        acc = sum4(v1.x, acc); acc = sum4(v1.y, acc); acc = sum4(v1.z, acc); acc = sum4(v1.w, acc);
-        acc = sum4(v2.x, acc); acc = sum4(v2.y, acc); acc = sum4(v2.z, acc); acc = sum4(v2.w, acc);
-        acc = sum4(v3.x, acc); acc = sum4(v3.y, acc); acc = sum4(v3.z, acc); acc = sum4(v3.w, acc);
-      } else {
-        for (uint32_t i = lane; i < (bytes >> 4); i += 32) {
-          uint4 v = s4[i];
-          const uint32_t g0 = blk0 + (i << 4); // bytes past the read's length are padding: not part of the sum
-          if (g0 + 16u > qlen) {
-            const uint32_t keep = qlen - g0; // 1 .. 15
-            uint32_t wv[4] = {v.x, v.y, v.z, v.w};
+  uint32_t lb[HC_SITES / 32];
 #pragma unroll
-            for (int j = 0; j < 4; j++) {
-              const int kb = (int)keep - 4 * j;
-              wv[j] = kb >= 4 ? wv[j] : kb <= 0 ? 0u : (wv[j] & ((1u << (8 * kb)) - 1u));
-            }
-            v = make_uint4(wv[0], wv[1], wv[2], wv[3]);
-          }
-          acc = sum4(v.x, acc); acc = sum4(v.y, acc); acc = sum4(v.z, acc); acc = sum4(v.w, acc);
-        }
-      }
-      // listed sites whose quality byte is in this block (0xffffffff — no byte wanted — and earlier blocks wrap to
-      // large values)
+  for (uint32_t g = 0; g < HC_SITES / 32; g++) lb[g] = lq[g] != 0xffffffffu ? qual(lq[g]) : 0u;
 #pragma unroll
-      for (uint32_t g = 0; g < HC_SITES / 32; g++) {
-        const uint32_t rel = lq[g] - blk0;
-        if (rel < bytes && lq[g] != 0xffffffffu) entries[la[g]] = le[g] | ((uint32_t)S->bq[st][rel] << 3);
-      }
-      __syncwarp(); // every lane is done with this stage
-      if (lane == 0 && blk + HC_NS < nblk) {
-        const uint32_t nb0 = (blk + HC_NS) * HC_BLK;
-        const uint32_t nbts = min(HC_BLK, nbytes - nb0);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_arrive_expect_tx(&S->bar[st], nbts);
-        bulk_g2s(S->bq[st], bqg + nb0, nbts, &S->bar[st]);
-      }
-    }
-    // the QV gate (bamlib.get_qv, caller.py:310): np.mean over every base of the read
-    unsigned long long tot = acc;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) tot += __shfl_xor_sync(HM_FULL, tot, d);
-    if (lane == 0) {
-      const double qv = __ddiv_rn((double)tot, (double)qlen);
-      if (qv < (double)p.min_qv) { qv_fail_read[r] = 1; *qv_fail_any = 1u; }
-      else { // m.num_ccs counts distinct query names (caller.py:318-320): one byte per name, the first setter counts
-        const uint32_t qn = __ldg(b.qname_id + r);
-        const uint32_t bit = 1u << (8u * (qn & 3u));
-        if (!(atomicOr(qname_seen32 + (qn >> 2), bit) & bit)) atomicAdd(num_ccs + (r & 7u), 1ull);
-      }
-    }
-    // a listed site whose query position lies past the read's end (malformed ops) never met a block
-#pragma unroll
-    for (uint32_t g = 0; g < HC_SITES / 32; g++)
-      if (lq[g] != 0xffffffffu && lq[g] >= nbytes) entries[la[g]] = le[g];
-  } else {
-#pragma unroll
-    for (uint32_t g = 0; g < HC_SITES / 32; g++)
-      if (lq[g] != 0xffffffffu) entries[la[g]] = le[g] | ((uint32_t)(lq[g] < qlen ? bqg[lq[g]] : 0) << 3);
-  }
+  for (uint32_t g = 0; g < HC_SITES / 32; g++)
+    if (lq[g] != 0xffffffffu) entries[la[g]] = le[g] | (lb[g] << 3);
   // sites past the list: the direct way
   for (uint32_t k0 = s_lo + HC_SITES; k0 < s_hi; k0 += 32) {
     const uint32_t ki = k0 + (uint32_t)lane;
     if (ki >= s_hi) continue;
     uint32_t q, e, at;
     site(ki, &q, &e, &at);
-    if (q != 0xffffffffu) entries[at] = e | ((uint32_t)(q < qlen ? bqg[q] : 0) << 3);
-  }
-}
-
-// sites keep only the candidates of reads that passed the QV gate; does something only when some read failed it
-// (then every emitted key looks its site up in the sorted key array)
-__global__ void __launch_bounds__(256) k_site_valid(const unsigned int* qv_fail_any, const uint8_t* qv_fail_read, const hm_chunk* chunks,
-                                                    const uint64_t* seg_off, const uint32_t* seg_cnt, const uint32_t* seg_keys,
-                                                    const uint32_t* seg_read, const uint32_t* tile_off, const uint32_t* tile_dst,
-                                                    const unsigned long long* keys, const unsigned long long* n_keys_dev,
-                                                    uint8_t* site_valid) {
-  if (!*qv_fail_any || !*n_keys_dev) return;
-  const uint32_t c = blockIdx.x;
-  const uint64_t seg0 = seg_off[c];
-  const uint32_t nk = seg_cnt[c];
-  const uint32_t k_lo = tile_dst[tile_off[c]], k_hi = tile_dst[tile_off[c + 1]];
-  const int32_t start = chunks[c].start;
-  for (uint32_t j = threadIdx.x; j < nk; j += blockDim.x) {
-    const uint32_t k32 = seg_keys[seg0 + j];
-    if (k32 == HC_KEY_HOLE || qv_fail_read[seg_read[seg0 + j]]) continue;
-    const unsigned long long want = ((unsigned long long)c << 36) | ((unsigned long long)(uint32_t)(start + (int32_t)(k32 >> 4)) << 4) | (k32 & 15u);
-    uint32_t lo = k_lo, hi = k_hi;
-    while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if (__ldg(keys + m) < want) lo = m + 1; else hi = m; }
-    if (lo < k_hi && __ldg(keys + lo) == want) site_valid[lo] = 1;
+    if (q != 0xffffffffu) entries[at] = e | (qual(q) << 3);
   }
 }
 

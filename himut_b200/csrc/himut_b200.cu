@@ -169,13 +169,13 @@ struct hm_ctx {
   char* h_geom_pin = nullptr;
   size_t h_geom_cap = 0;
   struct Pending { bool active = false; std::vector<hm_chunk> chunks; uint64_t site_cap = 0; size_t bcap = 0; int n_launched = 0, parity = 0; bool omit = false; } pend;
-  DevBuf b_cgeom, b_seg_keys, b_seg_read, b_keys_tmp, b_gscratch, b_czero, b_first_pair, b_tiles, b_site_valid, b_pair_c;
+  DevBuf b_cgeom, b_seg_keys, b_seg_read, b_keys_tmp, b_gscratch, b_czero, b_tiles, b_pair_c;
   // bit-vector normcounts path (normbits.cuh)
   PinVec<uint32_t> h_cw_off;                // per read: first word of its cal bit vector
   uint64_t n_cw = 0;                        // words of all cal bit vectors (>= 2^32: the path is not used)
   uint16_t cert_thr[256];                   // smallest callable count that certifies a pure position of depth n (0xffff: none)
   uint64_t packed_pos = 0;                  // positions b_ref2 / b_tri8 cover for the reference now in b_ref (0: not packed)
-  DevBuf b_cw_off, b_calw, b_impure, b_ref2, b_tri8, b_thr, b_span_off, b_exc_minmax, b_exp_total, b_sdiff, b_cal_ok;
+  DevBuf b_cw_off, b_calw, b_impure, b_ref2, b_tri8, b_thr, b_span_off, b_exc_minmax, b_sdiff, b_cal_ok;
   bool compact_resident = false;            // the resident batch came as bitmap + exceptions: both are still on the device
   uint32_t modal = 0;
   // device BAM decoder (hm_decode_bam_*, bamgpu.cuh)
@@ -334,6 +334,17 @@ int check_ready(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks) {
   return HM_OK;
 }
 
+// the resident batch's per-read quality sums from its one-byte-per-base stream (a compact upload has k_bq_expand)
+int launch_bq_sum(hm_ctx* ctx) {
+  if (ctx->n_reads == 0) return HM_OK;
+  t_reset(ctx);
+  t_begin(ctx, "k_bq_sum");
+  k_bq_sum<<<(unsigned)((ctx->n_reads * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->db);
+  t_end(ctx);
+  CU(cudaGetLastError());
+  return HM_OK;
+}
+
 // k_read_scan over the resident batch
 int launch_read_scan(hm_ctx* ctx) {
   if (ctx->n_reads == 0) return HM_OK;
@@ -418,8 +429,8 @@ void hm_destroy(hm_ctx* ctx) {
                     &ctx->b_hpos, &ctx->b_href, &ctx->b_halt, &ctx->b_hbit, &ctx->b_set_off, &ctx->b_chunks,
                     &ctx->b_pair_off, &ctx->b_pair_hap, &ctx->b_qseen, &ctx->b_keys, &ctx->b_keys_sorted, &ctx->b_cub,
                     &ctx->b_records, &ctx->b_counters, &ctx->b_ref, &ctx->b_norm_out, &ctx->b_lut, &ctx->b_tile_off, &ctx->b_agg, &ctx->b_geom, &ctx->b_bidx, &ctx->b_brecs, &ctx->b_sites, &ctx->b_push, &ctx->b_span_cnt, &ctx->b_koff, &ctx->b_tile_info, &ctx->b_edge_counts, &ctx->b_edge_hpos, &ctx->b_edge_href, &ctx->b_bqmask, &ctx->b_bqexc, &ctx->b_bqexc_off,
-                    &ctx->b_cgeom, &ctx->b_seg_keys, &ctx->b_seg_read, &ctx->b_keys_tmp, &ctx->b_gscratch, &ctx->b_czero, &ctx->b_first_pair, &ctx->b_tiles, &ctx->b_site_valid, &ctx->b_pair_c,
-                    &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_exp_total, &ctx->b_sdiff, &ctx->b_cal_ok,
+                    &ctx->b_cgeom, &ctx->b_seg_keys, &ctx->b_seg_read, &ctx->b_keys_tmp, &ctx->b_gscratch, &ctx->b_czero, &ctx->b_tiles, &ctx->b_pair_c,
+                    &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_sdiff, &ctx->b_cal_ok,
                     &ctx->b_comp, &ctx->b_pcoff, &ctx->b_pcsize, &ctx->b_pisize, &ctx->b_puoff, &ctx->b_pcrc, &ctx->b_pentry, &ctx->b_inflated,
                     &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt,
                     &ctx->b_scan, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off};
@@ -682,17 +693,16 @@ static int upload_batch_impl(hm_ctx* ctx, const hm_read_batch* b, const hm_bq_co
   CU(cudaEventRecord(ctx->ev_up, ctx->stream)); // every host buffer has been read once this fires
   if (cq && n) {
     CU(ctx->b_exc_minmax.ensure(2 * n + 16));
-    CU(ctx->b_exp_total.ensure(8 * n + 16));
     ctx->modal = (uint32_t)cq->modal;
     ctx->compact_resident = true;
     t_reset(ctx);
     t_begin(ctx, "k_bq_expand");
     k_bq_expand<<<(unsigned)((n * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, ctx->b_bqmask.as<uint8_t>(), ctx->b_bqexc.as<uint8_t>(),
                                                                          ctx->b_bqexc_off.as<uint64_t>(), (uint32_t)cq->modal, ctx->b_bq.as<uint8_t>(),
-                                                                         ctx->b_exc_minmax.as<uint8_t>(), ctx->b_exp_total.as<unsigned long long>());
+                                                                         ctx->b_exc_minmax.as<uint8_t>(), ctx->db.bq_total);
     t_end(ctx);
     CU(cudaGetLastError());
-  }
+  } else if ((rc = launch_bq_sum(ctx))) return rc;
   if (wait) CU(cudaEventSynchronize(ctx->ev_up)); // the caller may reuse its buffers after return; k_bq_expand may still be running
   ctx->upload_pending = !wait;
   ctx->have_batch = true;
@@ -949,7 +959,6 @@ struct FusedGeom { // device pointers into the one geometry block of a call
 int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const std::vector<uint64_t>& pair_off, const int32_t* geom,
                   uint64_t total_cap, uint64_t n_tiles, uint64_t site_cap, int parity, bool omit, size_t boundary_cap, FusedGeom* G_out) {
   const uint64_t n_pairs = pair_off.back();
-  const size_t n_reads = (size_t)ctx->n_reads;
   // ---- geometry: one pinned block, one copy ----
   const size_t o_chunks = 0, o_pair = align16(o_chunks + n_chunks * sizeof(hm_chunk)), o_seg = align16(o_pair + (n_chunks + 1) * 8),
                o_tile = align16(o_seg + (n_chunks + 1) * 8), o_geom = align16(o_tile + (n_chunks + 1) * 4),
@@ -993,10 +1002,8 @@ int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const st
   const size_t capk = (size_t)std::max<uint64_t>(total_cap, 1);
   CU(ctx->b_seg_keys.ensure(capk * 4 + 16)); CU(ctx->b_seg_read.ensure(capk * 4 + 16));
   CU(ctx->b_keys_tmp.ensure(capk * 4 + 16)); CU(ctx->b_gscratch.ensure(capk * 8 + 16));
-  const size_t z_cnt = 0, z_cur = z_cnt + n_chunks * 4, z_cur2 = z_cur + n_chunks * 4, z_counted = align16(z_cur2 + n_chunks * 4),
-               z_qvfail = align16(z_counted + n_reads), z_bytes = align16(z_qvfail + n_reads) + 16;
+  const size_t z_cnt = 0, z_cur = z_cnt + n_chunks * 4, z_cur2 = z_cur + n_chunks * 4, z_bytes = align16(z_cur2 + n_chunks * 4) + 16;
   CU(ctx->b_czero.ensure(z_bytes));
-  CU(ctx->b_first_pair.ensure(n_reads * 4 + 16));
   CU(ctx->b_pair_c.ensure((size_t)n_pairs * 4 + 16));
   CU(ctx->b_tiles.ensure(((size_t)n_tiles * 3 + 4) * 4));
   const uint64_t stride = (site_cap + 31) & ~31ull;
@@ -1004,7 +1011,6 @@ int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const st
   if (stride * n_slots + site_cap >= (1ull << 32)) return fail(ctx, HM_ERR_ARG, "%llu candidate sites in one call: split the chunk list", (unsigned long long)site_cap);
   CU(ctx->b_keys.ensure(site_cap * 8 + 16));
   CU(ctx->b_agg.ensure(stride * n_slots * 4 + site_cap * 8 + 16));
-  CU(ctx->b_site_valid.ensure(site_cap + 16));
   CU(ctx->b_compact[parity].ensure(site_cap * sizeof(hm_site_record)));
   const unsigned n_red = (unsigned)((site_cap + 127) / 128);
   CU(ctx->b_bidx.ensure(boundary_cap * 4 + HM_BOUNDARY_FIRST * 4));
@@ -1018,8 +1024,6 @@ int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const st
   uint32_t* seg_cnt = reinterpret_cast<uint32_t*>(z + z_cnt);
   uint32_t* cursor = reinterpret_cast<uint32_t*>(z + z_cur);
   uint32_t* cursor2 = reinterpret_cast<uint32_t*>(z + z_cur2);
-  uint8_t* read_counted = reinterpret_cast<uint8_t*>(z + z_counted);
-  uint8_t* qv_fail_read = reinterpret_cast<uint8_t*>(z + z_qvfail);
   uint32_t* tile_src = ctx->b_tiles.as<uint32_t>();
   uint32_t* tile_cnt = tile_src + n_tiles;
   uint32_t* tile_dst = tile_cnt + n_tiles; // n_tiles + 1 entries
@@ -1048,16 +1052,15 @@ int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const st
   CU(cudaMemsetAsync(ctx->b_counters.p, 0, 256, ctx->stream));
   CU(cudaMemsetAsync(ctx->b_qseen.p, 0, qseen_bytes, ctx->stream));
   CU(cudaMemsetAsync(ctx->b_czero.p, 0, z_bytes, ctx->stream));
-  CU(cudaMemsetAsync(ctx->b_first_pair.p, 0xff, n_reads * 4, ctx->stream));
   const unsigned pair_blocks_a = (unsigned)((n_pairs + 127) / 128);
   t_begin(ctx, "k_call_pairs");
   if (has_seq)
     k_call_pairs<true><<<pair_blocks_a, 128, pairs_smem, ctx->stream>>>(ctx->db, ctx->dp, ctx->dphase, G.chunks, (uint32_t)n_chunks, G.pair_off, n_pairs, pair_c, pair_hap,
-                                                              read_counted, ctx->b_first_pair.as<uint32_t>(), G.seg_off, seg_cnt,
+                                                              ctx->b_qseen.as<uint32_t>(), d_cnt + 24, G.seg_off, seg_cnt,
                                                               ctx->b_seg_keys.as<uint32_t>(), ctx->b_seg_read.as<uint32_t>());
   else
     k_call_pairs<false><<<pair_blocks_a, 128, pairs_smem, ctx->stream>>>(ctx->db, ctx->dp, ctx->dphase, G.chunks, (uint32_t)n_chunks, G.pair_off, n_pairs, pair_c, pair_hap,
-                                                               read_counted, ctx->b_first_pair.as<uint32_t>(), G.seg_off, seg_cnt,
+                                                               ctx->b_qseen.as<uint32_t>(), d_cnt + 24, G.seg_off, seg_cnt,
                                                                ctx->b_seg_keys.as<uint32_t>(), ctx->b_seg_read.as<uint32_t>());
   t_end(ctx);
   CU(cudaGetLastError());
@@ -1068,38 +1071,30 @@ int fused_enqueue(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, const st
                                                                                tile_src, tile_cnt);
   k_tile_scan<<<1, 1024, 0, ctx->stream>>>(tile_cnt, (uint32_t)n_tiles, tile_dst, (unsigned long long)site_cap, d_cnt);
   k_site_range2<<<(unsigned)((site_cap + 255) / 256), 256, 0, ctx->stream>>>(ctx->db, G.chunks, G.tile_chunk, tile_src, tile_dst, (uint32_t)n_tiles,
-                                                                            ctx->b_keys_tmp.as<uint32_t>(), d_cnt + 1, keys, site_lo, site_n, entries, stride,
-                                                                            ctx->b_site_valid.as<uint8_t>(), n_slots);
+                                                                            ctx->b_keys_tmp.as<uint32_t>(), d_cnt + 1, keys, site_lo, site_n, entries, stride, n_slots);
   t_end(ctx);
   CU(cudaGetLastError());
-  int rc = flush_deferred(ctx, true); // the previous call's records start moving now, under the quality scan
+  int rc = flush_deferred(ctx, true); // the previous call's records start moving now, under k_call_scan
   if (rc) return rc;
-  unsigned int* qv_any = reinterpret_cast<unsigned int*>(d_cnt + 7);
   const unsigned pair_blocks_b = (unsigned)((n_pairs + HC_SCAN_WARPS - 1) / HC_SCAN_WARPS);
   t_begin(ctx, "k_call_scan");
   if (has_seq)
-    k_call_scan<true><<<pair_blocks_b, 32 * HC_SCAN_WARPS, scan_smem, ctx->stream>>>(ctx->db, ctx->dp, G.chunks, G.pair_off, n_pairs, pair_c, pair_hap, read_counted,
-                                                                                    ctx->b_first_pair.as<uint32_t>(), G.tile_off, tile_dst, keys, site_lo, site_n,
-                                                                                    entries, (uint32_t)stride, qv_fail_read, qv_any, ctx->b_qseen.as<uint32_t>(),
-                                                                                    d_cnt + 24, d_cnt + 1, n_slots);
+    k_call_scan<true><<<pair_blocks_b, 32 * HC_SCAN_WARPS, scan_smem, ctx->stream>>>(ctx->db, ctx->dp, G.chunks, G.pair_off, n_pairs, pair_c, pair_hap,
+                                                                                    G.tile_off, tile_dst, keys, site_lo, site_n, entries, (uint32_t)stride,
+                                                                                    d_cnt + 1, n_slots);
   else
-    k_call_scan<false><<<pair_blocks_b, 32 * HC_SCAN_WARPS, scan_smem, ctx->stream>>>(ctx->db, ctx->dp, G.chunks, G.pair_off, n_pairs, pair_c, pair_hap, read_counted,
-                                                                                     ctx->b_first_pair.as<uint32_t>(), G.tile_off, tile_dst, keys, site_lo, site_n,
-                                                                                     entries, (uint32_t)stride, qv_fail_read, qv_any, ctx->b_qseen.as<uint32_t>(),
-                                                                                     d_cnt + 24, d_cnt + 1, n_slots);
+    k_call_scan<false><<<pair_blocks_b, 32 * HC_SCAN_WARPS, scan_smem, ctx->stream>>>(ctx->db, ctx->dp, G.chunks, G.pair_off, n_pairs, pair_c, pair_hap,
+                                                                                     G.tile_off, tile_dst, keys, site_lo, site_n, entries, (uint32_t)stride,
+                                                                                     d_cnt + 1, n_slots);
   t_end(ctx);
   CU(cudaGetLastError());
   CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy_done[parity], 0)); // the copy that last read this record buffer
   t_begin(ctx, "k_site_reduce");
-  if (n_chunks)
-    k_site_valid<<<(unsigned)n_chunks, 256, 0, ctx->stream>>>(qv_any, qv_fail_read, G.chunks, G.seg_off, seg_cnt, ctx->b_seg_keys.as<uint32_t>(),
-                                                            ctx->b_seg_read.as<uint32_t>(), G.tile_off, tile_dst, keys, d_cnt + 1,
-                                                            ctx->b_site_valid.as<uint8_t>());
   k_site_reduce<<<n_red, 128, 0, ctx->stream>>>(ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->dphase, ctx->dup_names ? 1 : 0, G.chunks, G.pair_off, pair_hap,
                                                 G.geom, G.geom + n_chunks, keys, d_cnt + 1, site_lo, site_n, entries, stride,
                                                 nullptr, d_cnt + 8, ctx->b_bidx.as<uint32_t>(), ctx->b_brecs.as<hm_site_record>(),
-                                                (uint32_t)boundary_cap, d_cnt + 4, reinterpret_cast<int*>(d_cnt + 3), ctx->b_site_valid.as<uint8_t>(),
-                                                qv_any, ctx->b_compact[parity].as<hm_site_record>(), d_cnt + 6, ctx->b_bpos.as<uint32_t>(), omit ? 1 : 0, n_slots);
+                                                (uint32_t)boundary_cap, d_cnt + 4, reinterpret_cast<int*>(d_cnt + 3),
+                                                ctx->b_compact[parity].as<hm_site_record>(), d_cnt + 6, ctx->b_bpos.as<uint32_t>(), omit ? 1 : 0, n_slots);
   t_end(ctx);
   CU(cudaGetLastError());
   return HM_OK;
@@ -1150,7 +1145,7 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
 
   // counters (u64): [0] n_keys (first version), [1] n_unique, [2] num_ccs, [3] error flag, [4] n_boundary,
   // [5] sites needed when the fused path's site buffers overflowed, [6] records kept by k_compact_sites,
-  // [7] some read failed the QV gate, [8..23] status histogram
+  // [8..23] status histogram, [24..31] num_ccs of the fused path in eight slots
   const size_t CNT_BYTES = 256;
   CU(ctx->b_counters.ensure(CNT_BYTES));
   if (!ctx->h_cnt_pin) CU(cudaHostAlloc((void**)&ctx->h_cnt_pin, CNT_BYTES + HM_BOUNDARY_FIRST * (8 + sizeof(hm_site_record)), cudaHostAllocMapped));
@@ -1189,9 +1184,9 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
                                                    ctx->b_bpos.as<uint32_t>(), ctx->b_brecs.as<uint32_t>(), (uint32_t)std::min<size_t>(HM_BOUNDARY_FIRST, bcap),
                                                    d_cnt + 4, reinterpret_cast<uint32_t*>(ctx->h_cnt_pin), h_bidx, h_bpos, reinterpret_cast<uint32_t*>(h_brecs));
         CU(cudaGetLastError());
-        // own kernels launched by this attempt: k_fetch_block, k_call_pairs, k_site_sort, k_tile_scan, k_site_range2, k_call_scan, k_site_valid,
-        // k_site_reduce, k_publish_call (+ k_bq_expand when the batch came compact, counted by the upload)
-        n_launched += 7 + (n_tiles ? 1 : 0) + (n_chunks ? 1 : 0);
+        // own kernels launched by this attempt: k_fetch_block, k_call_pairs, k_site_sort, k_tile_scan, k_site_range2, k_call_scan,
+        // k_site_reduce, k_publish_call (+ k_bq_expand / k_bq_sum, counted by the upload)
+        n_launched += 7 + (n_tiles ? 1 : 0);
       }
       if (stage == 1) { // submitted: the rest happens at collect
         ctx->pend.active = true;
@@ -1312,7 +1307,7 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
           ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->dphase, ctx->dup_names ? 1 : 0, ctx->b_chunks.as<hm_chunk>(), ctx->b_pair_off.as<uint64_t>(),
           ctx->b_pair_hap.as<uint8_t>(), ctx->b_geom.as<int32_t>(), ctx->b_geom.as<int32_t>() + n_chunks, k_in, d_cnt + 1, site_lo,
           site_n, entries, stride, rec_buf.as<hm_site_record>(), d_cnt + 8, ctx->b_bidx.as<uint32_t>(),
-          ctx->b_brecs.as<hm_site_record>(), (uint32_t)HM_BOUNDARY_CAP, d_cnt + 4, reinterpret_cast<int*>(d_cnt + 3), nullptr, nullptr, nullptr, nullptr, nullptr, 0,
+          ctx->b_brecs.as<hm_site_record>(), (uint32_t)HM_BOUNDARY_CAP, d_cnt + 4, reinterpret_cast<int*>(d_cnt + 3), nullptr, nullptr, nullptr, 0,
           (uint32_t)HM_SITE_SLOTS);
       if (omit) { // records of germline restatements stay here: flags -> scan -> stable compaction
         CU(ctx->b_keep.ensure(n_unique * 4 + 16)); CU(ctx->b_kpos.ensure(n_unique * 4 + 16));
@@ -1358,7 +1353,7 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
   // ---- from here on both versions: counters are on the host, records still on the device ----
   size_t n_unique = (size_t)h_cnt[1], n_boundary = 0;
   // compacted: the records the host copies sit in b_compact (germline restatements left out when asked; the fused
-  // path always compacts, it may have dropped speculative sites); boundary records are addressed through their
+  // path always compacts); boundary records are addressed through their
   // position there (h_bpos)
   const bool compacted = fused || omit;
   hm_site_record* recs = nullptr; // where the device records land on the host
@@ -1394,8 +1389,7 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
       CU(cudaStreamSynchronize(ctx->stream));
       border.clear();
       for (size_t i = 0; i < n_unique; i++)
-        if (recs[i].status != HM_ST_INTERNAL_DROPPED &&
-            (recs[i].tpos <= prev_max_end[recs[i].chunk] || recs[i].tpos >= next_min_start[recs[i].chunk])) border.push_back(Border{(uint32_t)i, 0u, recs[i]});
+        if (recs[i].tpos <= prev_max_end[recs[i].chunk] || recs[i].tpos >= next_min_start[recs[i].chunk]) border.push_back(Border{(uint32_t)i, 0u, recs[i]});
       n_boundary = border.size();
       have_all = true;
     } else if (n_boundary) {
@@ -1457,11 +1451,11 @@ static int call_chunks_impl(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks
       n_final += to - from;
       from = to + 1;
     }
-    if (omit || fused) { // the slow path has everything on the host: drop here what the compaction would have
+    if (omit) { // the slow path has everything on the host: drop here what the compaction would have
       size_t w = 0;
       for (size_t i = 0; i < n_final; i++) {
         const uint8_t st = recs[i].status;
-        if (st == HM_ST_INTERNAL_DROPPED || (omit && st >= HM_ST_GERM_HET && st <= HM_ST_GERM_HOMREF)) continue;
+        if (omit && st >= HM_ST_GERM_HET && st <= HM_ST_GERM_HOMREF) continue;
         if (w != i) recs[w] = recs[i];
         w++;
       }
@@ -1772,6 +1766,7 @@ int hm_decode_bam_end(hm_ctx* ctx, const uint32_t* qname_id) {
   }
   if ((rc = upload(ctx, ctx->b_qname, qname_id, n))) return rc;
   if ((rc = bind_batch(ctx, &b, has_seq))) return rc;
+  if ((rc = launch_bq_sum(ctx))) return rc;
   ctx->compact_resident = false;
   CU(cudaStreamSynchronize(ctx->stream));
   ctx->have_batch = true;
@@ -1906,7 +1901,7 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     k_norm_prep<<<(unsigned)((ctx->n_reads + NB_PREP_WARPS - 1) / NB_PREP_WARPS), 32 * NB_PREP_WARPS, sizeof(PrepWarp) * NB_PREP_WARPS, ctx->stream>>>(
         ctx->db, ctx->dp, ctx->b_ref2.as<uint32_t>(), ctx->b_cw_off.as<uint32_t>(), ctx->b_calw.as<uint32_t>(), ctx->b_impure.as<uint32_t>(), imp_words,
         ctx->compact_resident ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->b_exc_minmax.as<uint8_t>(),
-        ctx->b_exp_total.as<unsigned long long>(), ctx->modal, ctx->b_sdiff.as<uint32_t>(), ctx->b_cal_ok.as<uint8_t>());
+        ctx->modal, ctx->b_sdiff.as<uint32_t>(), ctx->b_cal_ok.as<uint8_t>());
     t_end(ctx);
     CU(cudaGetLastError());
   } else if ((rc = launch_read_scan(ctx))) return rc;

@@ -112,9 +112,35 @@ __device__ __forceinline__ int op_qry_len(uint32_t w) {
   return kind == HM_OP_MATCH ? (int)v : kind == HM_OP_SUB ? 1 : kind == HM_OP_INS ? (int)v : 0;
 }
 
+// whole-read quality sum of read r for a warp (np.mean(bq_int_lst) is an exact integer sum divided once): the read's
+// qualities as 16-byte words, 4 in flight per lane, summed with dp4a; every lane returns the total
+__device__ __forceinline__ unsigned long long warp_bq_sum(const DevBatch& b, uint64_t r, int32_t qlen, int lane) {
+  const uint8_t* bq = b.bq + b.bq_off[r];
+  const uint4* q4 = reinterpret_cast<const uint4*>(bq);
+  const int n16 = qlen >> 4;
+  uint32_t acc = 0;
+  int i = lane;
+  for (; i + 96 < n16; i += 128) {
+    uint4 a0 = ldg_stream16(q4 + i), a1 = ldg_stream16(q4 + i + 32), a2 = ldg_stream16(q4 + i + 64), a3 = ldg_stream16(q4 + i + 96);
+    acc = sum4(a0.x, acc); acc = sum4(a0.y, acc); acc = sum4(a0.z, acc); acc = sum4(a0.w, acc);
+    acc = sum4(a1.x, acc); acc = sum4(a1.y, acc); acc = sum4(a1.z, acc); acc = sum4(a1.w, acc);
+    acc = sum4(a2.x, acc); acc = sum4(a2.y, acc); acc = sum4(a2.z, acc); acc = sum4(a2.w, acc);
+    acc = sum4(a3.x, acc); acc = sum4(a3.y, acc); acc = sum4(a3.z, acc); acc = sum4(a3.w, acc);
+  }
+  for (; i < n16; i += 32) {
+    uint4 a0 = ldg_stream16(q4 + i);
+    acc = sum4(a0.x, acc); acc = sum4(a0.y, acc); acc = sum4(a0.z, acc); acc = sum4(a0.w, acc);
+  }
+  for (int j = (n16 << 4) + lane; j < qlen; j += 32) acc += bq[j];
+  unsigned long long tot = acc;
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) tot += __shfl_xor_sync(HM_FULL, tot, d);
+  return tot;
+}
+
 // ============================================================================ k_read_scan
 // One warp per read.  Phase 1: 32 ops at a time, warp inclusive scan of (ref_len, qry_len).
-// Phase 2: the read's qualities as 16-byte words, 4 in flight per lane, summed with dp4a.
+// Phase 2: the read's quality sum (warp_bq_sum).
 __global__ void __launch_bounds__(256) k_read_scan(DevBatch b, DevParams p) {
   const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
@@ -157,27 +183,7 @@ __global__ void __launch_bounds__(256) k_read_scan(DevBatch b, DevParams p) {
   il = __reduce_add_sync(HM_FULL, il);
   dl = __reduce_add_sync(HM_FULL, dl);
 
-  // whole-read quality sum (np.mean(bq_int_lst) is an exact integer sum divided once)
-  const uint8_t* bq = b.bq + b.bq_off[r];
-  const uint4* q4 = reinterpret_cast<const uint4*>(bq);
-  const int n16 = qlen >> 4;
-  uint32_t acc = 0;
-  int i = lane;
-  for (; i + 96 < n16; i += 128) {
-    uint4 a0 = ldg_stream16(q4 + i), a1 = ldg_stream16(q4 + i + 32), a2 = ldg_stream16(q4 + i + 64), a3 = ldg_stream16(q4 + i + 96);
-    acc = sum4(a0.x, acc); acc = sum4(a0.y, acc); acc = sum4(a0.z, acc); acc = sum4(a0.w, acc);
-    acc = sum4(a1.x, acc); acc = sum4(a1.y, acc); acc = sum4(a1.z, acc); acc = sum4(a1.w, acc);
-    acc = sum4(a2.x, acc); acc = sum4(a2.y, acc); acc = sum4(a2.z, acc); acc = sum4(a2.w, acc);
-    acc = sum4(a3.x, acc); acc = sum4(a3.y, acc); acc = sum4(a3.z, acc); acc = sum4(a3.w, acc);
-  }
-  for (; i < n16; i += 32) {
-    uint4 a0 = ldg_stream16(q4 + i);
-    acc = sum4(a0.x, acc); acc = sum4(a0.y, acc); acc = sum4(a0.z, acc); acc = sum4(a0.w, acc);
-  }
-  for (int j = (n16 << 4) + lane; j < qlen; j += 32) acc += bq[j];
-  unsigned long long tot = acc;
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) tot += __shfl_xor_sync(HM_FULL, tot, d);
+  const unsigned long long tot = warp_bq_sum(b, r, qlen, lane);
 
   if (lane == 0) {
     b.bq_total[r] = tot;
@@ -194,14 +200,26 @@ __global__ void __launch_bounds__(256) k_read_scan(DevBatch b, DevParams p) {
   }
 }
 
+// ============================================================================ k_bq_sum
+// The resident batch's per-read quality sums (bq_total, the input of the QV gate) when it came with one quality byte
+// per base: one warp per read.  A compact upload has k_bq_expand write them instead.
+__global__ void __launch_bounds__(256) k_bq_sum(DevBatch b) {
+  const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= b.n_reads) return;
+  const unsigned long long tot = warp_bq_sum(b, r, b.qlen[r], lane);
+  if (lane == 0) b.bq_total[r] = tot;
+}
+
 // ============================================================================ k_bq_expand
 // hm_bq_compact -> the one-byte-per-base quality stream.  One warp per read, 16 bases per lane and step: the lane's
 // 16 mask bits, a warp scan of the clear-bit counts to find its first exception, then the exceptions dropped into
-// the modal-filled 16-byte word.  Bytes past the read's length (padding) are written as 0.
+// the modal-filled 16-byte word.  Bytes past the read's length (padding) are written as 0.  The read's quality sum
+// goes to bq_total.
 // exc_minmax[2 r], [2 r + 1]: the smallest / largest exception of read r (255 / 0 when it has none): what lets the
 // normcounts pass take "BQ >= min_bq" straight from the bitmap (normbits.cuh).
 __global__ void __launch_bounds__(256) k_bq_expand(DevBatch b, const uint8_t* mask, const uint8_t* exc, const uint64_t* exc_off,
-                                                   uint32_t modal, uint8_t* bq_out, uint8_t* exc_minmax, unsigned long long* exp_total) {
+                                                   uint32_t modal, uint8_t* bq_out, uint8_t* exc_minmax, unsigned long long* bq_total) {
   const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (r >= b.n_reads) return;
@@ -255,7 +273,7 @@ __global__ void __launch_bounds__(256) k_bq_expand(DevBatch b, const uint8_t* ma
   unsigned long long tot = acc; // the read's quality sum (bamlib.get_qv divides it once)
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) tot += __shfl_xor_sync(HM_FULL, tot, d);
-  if (lane == 0) { exc_minmax[2 * r] = (uint8_t)e_min; exc_minmax[2 * r + 1] = (uint8_t)e_max; exp_total[r] = tot; }
+  if (lane == 0) { exc_minmax[2 * r] = (uint8_t)e_min; exc_minmax[2 * r + 1] = (uint8_t)e_max; bq_total[r] = tot; }
 }
 
 // ============================================================================ lookups
@@ -801,14 +819,9 @@ __global__ void __launch_bounds__(256) k_site_entries_by_read(DevBatch b, DevPar
   }
 }
 
-// status of a record that is not one: a speculative candidate none of whose supporting reads passed the QV gate
-// (fused path, callfused.cuh); never leaves the device
-#define HM_ST_INTERNAL_DROPPED 31
-
 // ph / dup_names: two primary records of the batch share a query name.  The reference classifies the records it
 //   re-fetches at a phase-checked site by *name* (wt_ccs_set / alt_ccs_set, caller.py:556-567); with unique names
 //   that is the record's own allele (the entries' haplotype tallies), with shared names the exact walk below.
-// site_valid / qv_fail (fused path, else NULL): *qv_fail != 0 -> only sites with site_valid[ki] exist.
 // compact_out / n_kept / boundary_pos (fused path, else NULL): the records the host wants (not dropped; not a germline
 //   restatement when omit != 0) are written to compact_out only — a block reserves its range with one atomic on
 //   *n_kept, inside the block the order is the key order — and a boundary record carries its position there
@@ -825,7 +838,7 @@ __global__ void __launch_bounds__(128, HM_REDUCE_MINB) k_site_reduce(DevBatch b,
                                                      hm_site_record* out, unsigned long long* status_hist, uint32_t* boundary_idx,
                                                      hm_site_record* boundary_recs, uint32_t boundary_cap,
                                                      unsigned long long* n_boundary, int* err_flag,
-                                                     const uint8_t* site_valid, const unsigned int* qv_fail, hm_site_record* compact_out,
+                                                     hm_site_record* compact_out,
                                                      unsigned long long* n_kept, uint32_t* boundary_pos, int omit, uint32_t n_slots) {
   __shared__ unsigned int s_hist[16];
   __shared__ unsigned int s_wkeep[4], s_kbase;
@@ -837,10 +850,8 @@ __global__ void __launch_bounds__(128, HM_REDUCE_MINB) k_site_reduce(DevBatch b,
   bool have_rec = false, keep = false, bnd = false;
   const uint64_t ki = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const uint64_t n_keys = *n_keys_dev;
-  const bool fused = site_valid != nullptr; // no op prefix arrays in HBM then
-  if (ki < n_keys && site_valid && *qv_fail && !site_valid[ki]) {
-    // a speculative site none of whose supporting reads passed the QV gate: no record, no tally
-  } else if (ki < n_keys) {
+  const bool fused = compact_out != nullptr; // no op prefix arrays in HBM then
+  if (ki < n_keys) {
     const unsigned long long key = keys[ki];
     const uint32_t c = (uint32_t)(key >> 36);
     const int32_t tpos = (int32_t)((key >> 4) & 0xffffffffull);

@@ -110,7 +110,7 @@ __device__ __forceinline__ void mark_impure_range(uint32_t* impure, uint64_t imp
 __global__ void __launch_bounds__(32 * NB_PREP_WARPS, 8) k_norm_prep(DevBatch b, DevParams p, const uint32_t* ref2, const uint32_t* cw_off,
                                                                    uint32_t* calw, uint32_t* impure, uint64_t imp_words,
                                                                    const uint16_t* mask16, const uint8_t* exc_minmax,
-                                                                   const unsigned long long* exp_total, uint32_t modal, uint32_t* sdiff,
+                                                                   uint32_t modal, uint32_t* sdiff,
                                                                    uint8_t* cal_ok) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -455,7 +455,7 @@ __global__ void __launch_bounds__(32 * NB_PREP_WARPS, 8) k_norm_prep(DevBatch b,
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) tot += __shfl_xor_sync(HM_FULL, tot, d);
   bool has_zero = __any_sync(HM_FULL, (zacc & 0x80808080u) != 0u);
-  if (use_mask) { tot = __ldg(exp_total + r); has_zero = e_min == 0u; }
+  if (use_mask) { tot = b.bq_total[r]; has_zero = e_min == 0u; } // the resident sum (the bytes were not all read)
   if (lane == 0) {
     cal_ok[r] = do_bits ? 1 : 0; // the read's cal words are what update_tri2count counts (the exact pass takes them from there)
     b.bq_total[r] = tot;
