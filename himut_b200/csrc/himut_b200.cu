@@ -933,7 +933,7 @@ namespace {
 
 inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
-// can the fused path run this call?  (else the first version does: chunk spans of 2^28 positions and more, more than
+// can the fused path run this call?  (else the first version does: chunk spans of 2^27 positions and more, more than
 // 2^32 (chunk, read) pairs or candidate slots — nothing a reference-style chunk list produces)
 bool fused_eligible(hm_ctx* ctx, const hm_chunk* chunks, size_t n_chunks, uint64_t n_pairs, uint64_t* total_cap, uint64_t* n_tiles) {
   const bool force_v1 = getenv("HIMUT_B200_CALL_V1") != nullptr; // read per call: tests switch it

@@ -428,8 +428,8 @@ int hm_batch_read_back_seq(hm_ctx* ctx, uint64_t* seq_off, uint8_t* seq, uint64_
 int hm_inflate_device_test(hm_ctx* ctx, const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len, uint32_t crc);
 
 int hm_last_timing(hm_ctx* ctx, float* total_ms, int* n_launches);
-/* which device path the last hm_call_chunks took: 2 the fused one (one pass over the quality stream, no library
- * sort, one synchronisation), 1 the first version (chunk spans of 2^28 positions and more, or HIMUT_B200_CALL_V1 set),
+/* which device path the last hm_call_chunks took: 2 the fused one (no pass over the quality stream, no library
+ * sort, one synchronisation), 1 the first version (chunk spans of 2^27 positions and more, or HIMUT_B200_CALL_V1 set),
  * 0 none yet.  Same records either way; for tests and bench.py.                                              */
 int hm_last_call_path(hm_ctx* ctx);
 int hm_last_kernel_times(hm_ctx* ctx, const char** names, float* ms, size_t cap, size_t* n);

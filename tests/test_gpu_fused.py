@@ -1,8 +1,8 @@
 """The fused `himut call` device path (csrc/callfused.cuh) against the oracle on the shapes that exercise its own
 machinery — several sort tiles per chunk, more distinct positions per tile than fit in shared memory, op lists longer
-than a warp stages, the site-buffer overflow retry, reads that fail the QV gate after their candidates were emitted —
-and the first version of the path (HIMUT_B200_CALL_V1=1), which stays as the route for chunk spans of 2^28 and more,
-on every fixed case.  GPU."""
+than a warp stages, the site-buffer overflow retry, reads that fail the QV gate (k_call_pairs emits no candidate for
+them) — and the first version of the path (HIMUT_B200_CALL_V1=1), which stays as the route for chunk spans of 2^27
+and more, on every fixed case.  GPU."""
 import numpy as np
 import pytest
 
@@ -73,9 +73,9 @@ def test_dense_candidates(ctx):
     _same_as_oracle(ctx, p, d.batch.without_seq(), d.batch.chunk_table([(0, 75_000), (75_000, 150_000)]), full=d.batch)
 
 
-def test_reads_that_fail_the_qv_gate_take_their_candidates_with_them(ctx):
-    """candidates are emitted before the quality sum of their read is known; a site none of whose supporting reads
-    passes the QV gate must vanish (records, counters, num_ccs)"""
+def test_reads_that_fail_the_qv_gate_emit_no_candidates(ctx):
+    """the QV gate (the read's resident quality sum) decides before any candidate of the read is emitted; a site none
+    of whose supporting reads passes it must vanish (records, counters, num_ccs)"""
     d = synth.generate(200_000, seed=11)
     b = d.batch
     for r in range(0, b.n_reads, 3):  # every third read: qualities 20 everywhere (mean < min_qv = 30)
