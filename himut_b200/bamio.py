@@ -128,6 +128,10 @@ class Record:
         return t in self.tags
 
 
+_B_SIZE = {"c": 1, "C": 1, "s": 2, "S": 2, "i": 4, "I": 4, "f": 4}
+_TAG_FMT = {"c": "b", "C": "B", "s": "h", "S": "H", "i": "i", "I": "I", "f": "f"}
+
+
 def _parse_tags(buf, p, end, want=("cs", "tp", "MD")):
     tags = {}
     while p < end:
@@ -151,8 +155,10 @@ def _parse_tags(buf, p, end, want=("cs", "tp", "MD")):
             p += 4
         elif ty == "B":
             sub = chr(buf[p])
+            if sub not in _B_SIZE:  # htslib rejects the record too
+                raise BamError("unknown B subtype %r" % sub)
             n = struct.unpack_from("<I", buf, p + 1)[0]
-            p += 5 + n * {"c": 1, "C": 1, "s": 2, "S": 2, "i": 4, "I": 4, "f": 4}[sub]
+            p += 5 + n * _B_SIZE[sub]
         else:
             raise BamError("unknown tag type %r" % ty)
     return tags
@@ -365,7 +371,8 @@ class BamWriter:
         self.buf += b
 
     def add(self, ref_id, pos, qname, flag, mapq, cigar, seq, qual, tags):
-        """cigar: list of (op, len); seq: ASCII str; qual: bytes; tags: list of (tag, type, value)"""
+        """cigar: list of (op, len); seq: ASCII str; qual: bytes; tags: list of (tag, type, value), type one of
+        A Z H c C s S i I f, or B with value (subtype, list of numbers)"""
         v0 = (self.coff << 16) | len(self.buf)
         ref_span = sum(l for o, l in cigar if _CIGAR_REF[o])
         end = pos + max(ref_span, 1)
@@ -377,12 +384,18 @@ class BamWriter:
         body = struct.pack("<iiBBHHHiiii", ref_id, pos, len(qname) + 1, mapq, _reg2bin(pos, end), len(cigar), flag, l_seq, -1, -1, 0)
         body += qname.encode() + b"\0" + b"".join(struct.pack("<I", (l << 4) | o) for o, l in cigar) + packed + bytes(qual)
         for tag, ty, val in tags:
-            if ty == "Z":
-                body += tag.encode() + b"Z" + val.encode() + b"\0"
+            body += tag.encode() + ty.encode()
+            if ty in ("Z", "H"):
+                body += val.encode() + b"\0"
             elif ty == "A":
-                body += tag.encode() + b"A" + val.encode()
-            elif ty == "i":
-                body += tag.encode() + b"i" + struct.pack("<i", val)
+                body += val.encode()
+            elif ty == "B":
+                sub, vals = val
+                body += sub.encode() + struct.pack("<I%d%s" % (len(vals), _TAG_FMT[sub]), len(vals), *vals)
+            elif ty in _TAG_FMT:
+                body += struct.pack("<" + _TAG_FMT[ty], val)
+            else:
+                raise ValueError("unknown tag type %r" % ty)
         rec = struct.pack("<i", len(body)) + body
         self.buf += rec
         self._flush(everything=False)  # pending tail < 0xFF00, so offsets stay exact

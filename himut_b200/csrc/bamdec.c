@@ -178,6 +178,10 @@ static int64_t qt_get(qtab_t* t, const char* s, size_t n) {
   return t->n++;
 }
 
+/* bytes per element of a B array tag; 0: a subtype htslib does not know (it rejects the record) */
+static inline size_t b_elem_size(char sub) {
+  return (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : (sub == 'i' || sub == 'I' || sub == 'f') ? 4 : 0;
+}
 static inline uint32_t rd32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
 
 /* ------------------------------------------------------------------ BGZF */
@@ -959,8 +963,9 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
           else if (ty == 'i' || ty == 'I' || ty == 'f') adv = 4;
           else if (ty == 'B') {
             if (left < 5) { rc = fail(b, REC_ERR[E_TAG_B], qname, (long)left); break; }
-            char sub = (char)v[0]; uint32_t cnt = rd32(v + 1);
-            adv = 5 + (size_t)cnt * ((sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4);
+            const size_t esz = b_elem_size((char)v[0]);
+            if (!esz) { rc = fail(b, REC_ERR[E_TAG_B], qname, (long)v[0]); break; }
+            adv = 5 + (size_t)rd32(v + 1) * esz;
           }
           else { rc = fail(b, REC_ERR[E_TAG_TYPE], qname, ty); break; }
           if (adv > left) { rc = fail(b, REC_ERR[E_TAG_PAST], qname, (long)adv); break; }
@@ -1358,8 +1363,9 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
       else if (ty == 'i' || ty == 'I' || ty == 'f') adv = 4;
       else if (ty == 'B') {
         if (left < 5) { rc = fail(b, REC_ERR[E_TAG_B], (const char*)(r + 32), (long)left); break; }
-        char sub = (char)v[0]; uint32_t cnt = rd32(v + 1);
-        adv = 5 + (size_t)cnt * ((sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4);
+        const size_t esz = b_elem_size((char)v[0]);
+        if (!esz) { rc = fail(b, REC_ERR[E_TAG_B], (const char*)(r + 32), (long)v[0]); break; }
+        adv = 5 + (size_t)rd32(v + 1) * esz;
       }
       else { rc = fail(b, REC_ERR[E_TAG_TYPE], (const char*)(r + 32), ty); break; }
       if (adv > left) { rc = fail(b, REC_ERR[E_TAG_PAST], (const char*)(r + 32), (long)adv); break; }

@@ -23,7 +23,7 @@ static const char* const REC_ERR[E_N_CODES] = {
     "%s: unsupported MD:Z token (%ld)", "%s: MD:Z and CIGAR disagree at reference offset %ld",
     "%s: unsupported CIGAR op (N, P, or a clip inside the alignment) at CIGAR index %ld",
     "malformed BAM record in %s: block_size %ld", "malformed BAM record in %s: fields run past block_size %ld",
-    "malformed BAM record %s: unterminated %ld tag", "malformed BAM record %s: truncated B tag (%ld)",
+    "malformed BAM record %s: unterminated %ld tag", "malformed BAM record %s: truncated B tag or unknown B subtype (%ld)",
     "unknown tag type in record %s (%ld)", "malformed BAM record %s: a tag runs past the record (%ld)",
     "%s has no cs:Z tag (the reference raises KeyError in BAM.__init__) (%ld)", "%s has no base qualities (%ld)",
     "truncated BAM record in %s (%ld)",

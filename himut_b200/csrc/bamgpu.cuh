@@ -405,8 +405,9 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
     else if (ty == 'B') {
       if (left < 5) { sel_fail(err, code, arg, r, E_TAG_B, (long long)left); return; }
       const char sub = (char)v[0];
-      const uint32_t cnt = rd32(v + 1);
-      adv = 5 + (size_t)cnt * ((sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4);
+      const size_t esz = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : (sub == 'i' || sub == 'I' || sub == 'f') ? 4 : 0;
+      if (!esz) { sel_fail(err, code, arg, r, E_TAG_B, (long long)v[0]); return; }  // htslib rejects it too
+      adv = 5 + (size_t)rd32(v + 1) * esz;
     } else { sel_fail(err, code, arg, r, E_TAG_TYPE, ty); return; }
     if (adv > left) { sel_fail(err, code, arg, r, E_TAG_PAST, (long long)adv); return; }
     tag = v + adv;

@@ -294,7 +294,7 @@ def test_malformed_records_are_rejected_not_read_past(tmp_path):
     import struct
     import zlib
     path = str(tmp_path / "ok.bam")
-    _write(path, [_rec(pos=10, qname="first"), _rec(pos=20, qname="second", extra=[("xb", "B", ("c", [1, 2, 3]))] if False else [])])
+    _write(path, [_rec(pos=10, qname="first"), _rec(pos=20, qname="second", extra=[("xb", "B", ("c", [1, 2, 3]))])])
     raw = bytearray(gzip.open(path, "rb").read())  # BGZF members are gzip members
     first = raw.find(b"first\x00") - 36  # block_size field of the first record
     assert first > 0
@@ -302,18 +302,7 @@ def test_malformed_records_are_rejected_not_read_past(tmp_path):
     rng = np.random.default_rng(5)
 
     def rewrite(mut, name):
-        out = str(tmp_path / name)
-        blocks = []
-        for i in range(0, len(mut), 60000):
-            piece = bytes(mut[i:i + 60000])
-            c = zlib.compressobj(6, zlib.DEFLATED, -15)
-            comp = c.compress(piece) + c.flush()
-            blocks.append(b"\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00" + struct.pack("<H", len(comp) + 25) + comp +
-                          struct.pack("<II", zlib.crc32(piece) & 0xffffffff, len(piece)))
-        blocks.append(bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000"))
-        with open(out, "wb") as f:
-            f.write(b"".join(blocks))
-        return out
+        return _rebgzf(mut, str(tmp_path / name))
 
     cases_ = []
     m = bytearray(raw); struct.pack_into("<i", m, first + 4 + 16, 1 << 20); cases_.append(m)       # l_seq far past the record
@@ -342,3 +331,49 @@ def test_malformed_records_are_rejected_not_read_past(tmp_path):
             n_bad += 1
         nb.close()
     assert n_bad >= 5  # the five structural mutations at least
+
+
+def _rebgzf(raw, out):
+    """an inflated BAM stream -> BGZF blocks (zlib) at `out`, without a BAI"""
+    import struct
+    import zlib
+    blocks = []
+    for i in range(0, len(raw), 60000):
+        piece = bytes(raw[i:i + 60000])
+        c = zlib.compressobj(6, zlib.DEFLATED, -15)
+        comp = c.compress(piece) + c.flush()
+        blocks.append(b"\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00" + struct.pack("<H", len(comp) + 25) + comp +
+                      struct.pack("<II", zlib.crc32(piece) & 0xffffffff, len(piece)))
+    blocks.append(bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000"))
+    with open(out, "wb") as f:
+        f.write(b"".join(blocks))
+    return out
+
+
+def bad_b_subtype(tmp_path):
+    """a record with a B array tag of subtype 'x' between cs:Z and another tag: htslib rejects such a record as
+    corrupted aux data; a walker that took 'x' for 4-byte elements would step into the next tag"""
+    import gzip
+    path = str(tmp_path / "sub.bam")
+    _write(path, [_rec(pos=10, qname="badsub", extra=[("xb", "B", ("C", [7])), ("yz", "Z", "abcdefgh")])])
+    raw = gzip.open(path, "rb").read()
+    assert raw.count(b"xbBC\x01\x00\x00\x00") == 1
+    return _rebgzf(raw.replace(b"xbBC\x01\x00\x00\x00", b"xbBx\x01\x00\x00\x00"), str(tmp_path / "badsub.bam"))
+
+
+B_SUBTYPE_MSG = "malformed BAM record badsub: truncated B tag or unknown B subtype (120)"
+
+
+def test_unknown_b_subtype_is_rejected_by_every_walker(tmp_path):
+    path = bad_b_subtype(tmp_path)
+    nb = bamdec.NativeBam(path, threads=1)
+    for kw in (dict(), dict(seq=False, compact=True)):
+        with pytest.raises(pack.BatchFormatError) as ex:
+            nb.read_batch("chr1", 0, 1000, **kw)
+        assert str(ex.value) == B_SUBTYPE_MSG
+    with pytest.raises(pack.BatchFormatError) as ex:
+        nb.window_qlens("chr1", 0, 1000)
+    assert str(ex.value) == B_SUBTYPE_MSG
+    nb.close()
+    with pytest.raises(bamio.BamError, match="unknown B subtype 'x'"):
+        bamio.read_batch(bamio.BamReader(path), "chr1", 0, 1000)

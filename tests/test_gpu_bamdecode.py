@@ -184,6 +184,11 @@ def test_device_rejections_match_the_host(ctx, tmp_path, bad):
     assert _device_error(ctx, path) == _host_error(path)
 
 
+def test_device_rejects_an_unknown_b_subtype_as_the_host_does(ctx, tmp_path):
+    path = tb.bad_b_subtype(tmp_path)
+    assert _device_error(ctx, path) == _host_error(path) == tb.B_SUBTYPE_MSG
+
+
 def test_device_reports_the_record_the_host_reports(ctx, tmp_path):
     """a bad cs string (found when records are decoded) before a record without cs (found when they are selected): the
     host decoder selects every record of its buffer before it decodes any, so it names the second record; so does the
