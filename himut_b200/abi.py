@@ -9,6 +9,7 @@ import numpy as np
 
 HM_OK, HM_ERR_ARG, HM_ERR_CUDA, HM_ERR_CAPACITY, HM_ERR_BQ_ZERO, HM_ERR_NO_DEVICE, HM_ERR_STATE = range(7)
 HM_DECODE_SEQ = 1  # hm_decode_bam_begin_opts: decode the 2-bit base stream too
+HM_DECODE_REF = 2  # hm_decode_bam_begin_opts: records with neither cs:Z nor MD:Z decode against the resident reference
 
 OP_MATCH, OP_SUB, OP_INS, OP_DEL = 0, 1, 2, 3
 BASE_N = 4

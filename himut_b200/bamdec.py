@@ -17,7 +17,7 @@ from . import abi, bamio, pack
 _LIB = None
 EXPORTS = ["hm_bam_open", "hm_bam_close", "hm_bam_error", "hm_bam_header_text", "hm_bam_n_refs", "hm_bam_ref_name",
            "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bam_write_batch_tags", "hm_bq_compact_build",
-           "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames"]
+           "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames", "hm_bam_set_reference"]
 
 
 def lib_path():
@@ -59,6 +59,7 @@ def load():
         lib.hm_bam_qname.restype = C.c_char_p
         lib.hm_bam_region_plan.argtypes = [vp, C.c_int, C.c_int32, C.c_int32, C.POINTER(abi.hm_bgzf_plan)]
         lib.hm_bam_intern_qnames.argtypes = [vp, vp, vp, C.c_size_t, vp]
+        lib.hm_bam_set_reference.argtypes = [vp, C.c_int, C.c_char_p, C.c_size_t]
         _LIB = lib
     return _LIB
 
@@ -159,6 +160,19 @@ class NativeBam:
         exc = cp(_view(q.exc, (n_exc + 31) & ~15, np.uint8))  # the decoder keeps 32 readable bytes past the last exception
         exc_off = cp(_view(q.exc_off, n + 1, np.uint64))
         return batch, abi.BqCompact(mask, exc, exc_off, int(q.modal), n_exc)
+
+    def set_reference(self, chrom, seq):
+        """the sequence of `chrom` (bytes or str, the whole contig: its length must be the @SQ LN), for its records with
+        neither cs:Z nor MD:Z, which read_batch then decodes from CIGAR + reference (pack.parse_ref); None clears it.
+        The handle keeps a reference to the bytes it reads."""
+        if chrom not in self.references:
+            raise KeyError(chrom)
+        seq = seq.encode() if isinstance(seq, str) else (None if seq is None else bytes(seq))
+        rc = self.lib.hm_bam_set_reference(self.h, self.references.index(chrom), seq, 0 if seq is None else len(seq))
+        if rc != 0:
+            self._ref = None
+            raise pack.BatchFormatError(self.lib.hm_bam_error(self.h).decode())
+        self._ref = seq
 
     def plan(self, chrom, start, end):
         """abi.hm_bgzf_plan of the records read_batch(chrom, start, end) visits, for Context.decode_region: the

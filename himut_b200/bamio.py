@@ -6,7 +6,8 @@ implements what the reference touches through pysam (SURVEY.md §8b): header tex
 fetch(chrom, start, end) — records overlapping the 0-based half-open window, in file order,
 secondary / supplementary included — and the per-record fields reference_start/end,
 query_alignment_start/end, query_sequence, query_qualities, mapping_quality, flag, cs:Z, tp:A, and
-beyond it the CIGAR and MD:Z (records without cs:Z are decoded from CIGAR + MD, pack.parse_md).
+beyond it the CIGAR and MD:Z (records without cs:Z are decoded from CIGAR + MD, pack.parse_md, and records with
+neither tag from CIGAR + the contig's reference sequence when the caller gives it, pack.parse_ref).
 The writer exists for tests and for the synthetic-data tools (coordinate-sorted BAM + .bai).
 """
 import struct
@@ -294,19 +295,20 @@ def _load_bai(path, n_ref):
 
 
 # ------------------------------------------------------------------------------ region -> batch
-def read_batch(reader, chrom, start, end, builder=None):
+def read_batch(reader, chrom, start, end, builder=None, refseq=None):
     """all records of `chrom` overlapping [start, end), packed (each record once, file order).
 
     Secondary records are dropped here: bamlib.BAM.__init__ skips them before anything else
     (src/himut/bamlib.py:17); supplementary records are kept, as the reference keeps them.
     A record's ops come from its cs:Z tag; a record without cs:Z but with MD:Z is decoded from CIGAR + MD
-    (pack.parse_md: the same ops for the same alignment); a record with neither is rejected.
+    (pack.parse_md: the same ops for the same alignment); a record with neither is decoded from CIGAR + refseq, the
+    whole sequence of `chrom` (pack.parse_ref), when it is given, and rejected otherwise.
     """
     bb = builder or pack.BatchBuilder()
     for r in reader.fetch(chrom, start, end):
         if r.is_secondary:  # BAM.__init__ skips them everywhere (bamlib.py:17)
             continue
-        if "cs" not in r.tags and "MD" not in r.tags:
+        if "cs" not in r.tags and "MD" not in r.tags and refseq is None:
             raise pack.BatchFormatError("%s has no cs:Z tag (the reference raises KeyError in BAM.__init__)" % r.query_name)
         # hard clips: pysam's query_sequence / query_alignment_start leave the clipped bases out (SEQ does not hold
         # them), so cs2tuple indexes consistently and the reference processes such records; so do we
@@ -315,7 +317,7 @@ def read_batch(reader, chrom, start, end, builder=None):
             raise pack.BatchFormatError("%s has no base qualities" % r.query_name)
         bb.add(tstart=r.reference_start, tend=r.reference_end, qstart=r.query_alignment_start, qend=r.query_alignment_end,
                qseq=r.query_sequence, bq=bytes(q), mapq=r.mapping_quality, is_secondary=False, qname=r.query_name,
-               cs=r.tags.get("cs"), cigar=r.cigar, md=r.tags.get("MD"))
+               cs=r.tags.get("cs"), cigar=r.cigar, md=r.tags.get("MD"), refseq=refseq)
     return bb.finish()
 
 
@@ -433,12 +435,13 @@ class BamWriter:
             f.write(struct.pack("<Q", 0))
 
 
-TAGS = ("cs", "md", "md_eqx")
+TAGS = ("cs", "md", "md_eqx", "eqx", "m")
 
 
 def write_batch_bam(path, chrom, contig_len, batch, sample="synth", tags="cs"):
     """ReadBatch -> coordinate-sorted BAM + BAI, tp:A:P, for tests and tools.  tags: "cs" writes cs:Z short form
-    with a =/X CIGAR; "md" writes MD:Z and no cs with an M CIGAR; "md_eqx" MD:Z with the =/X CIGAR"""
+    with a =/X CIGAR; "md" writes MD:Z and no cs with an M CIGAR; "md_eqx" MD:Z with the =/X CIGAR; "eqx" the =/X
+    CIGAR and neither tag; "m" the M CIGAR and neither tag (these two decode with the contig's reference sequence)"""
     write_batches_bam(path, [(chrom, contig_len, batch)], sample, tags)
 
 
@@ -453,7 +456,8 @@ def write_batches_bam(path, contigs, sample="synth", tags="cs"):
 def _add_batch(w, rid, batch, tags="cs"):
     if tags not in TAGS:
         raise ValueError("tags must be one of %s" % (TAGS,))
-    m_op, x_op = (0, 0) if tags == "md" else (7, 8)
+    m_op, x_op = (0, 0) if tags in ("md", "m") else (7, 8)
+    aln_tag = {"cs": "cs", "md": "MD", "md_eqx": "MD"}.get(tags)
     for r in range(batch.n_reads):
         ql = int(batch.qlen[r])
         so, bo, oo = int(batch.seq_off[r]), int(batch.bq_off[r]), int(batch.op_off[r])
@@ -490,4 +494,5 @@ def _add_batch(w, rid, batch, tags="cs"):
         flag = 0x100 if (batch.flags[r] & abi.READ_SECONDARY) else 0
         w.add(rid, int(batch.tstart[r]), "read%d" % int(batch.qname_id[r]), flag, int(batch.mapq[r]), merged, qseq,
               batch.bq[bo:bo + ql].tobytes(),
-              [("cs", "Z", "".join(cs)) if tags == "cs" else ("MD", "Z", "".join(md) + "%d" % md_run), ("tp", "A", "P")])
+              ([("cs", "Z", "".join(cs)) if aln_tag == "cs" else ("MD", "Z", "".join(md) + "%d" % md_run)] if aln_tag else [])
+              + [("tp", "A", "P")])

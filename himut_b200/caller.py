@@ -73,7 +73,7 @@ def carry_som_seen(parts, later_starts):
     return out
 
 
-def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_names=False, ctx2=None, decode="auto"):
+def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_names=False, ctx2=None, decode="auto", refseq=None):
     """the device path over a contig's chunk list (or a run of it), pipelined: group k + 1 is decoded on a thread of its
     own while group k is uploaded; with a second context (configured like the first) the two alternate from group to
     group, so upload(k + 1) also overlaps kernels(k) and the record copy of k - 1:
@@ -83,11 +83,15 @@ def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_nam
     group k do.  It needs a context with the device decoder and a BAM with a BAI; without either the host decoder runs.
     "host" is the pipeline above (the native host decoder).  "auto" takes the device decoder when it can run and the
     groups average at least DEVICE_DECODE_MIN_BYTES of compressed BAM (below that the host decoder is faster).
+    refseq: the sequence of `chrom`, for records with neither cs:Z nor MD:Z, which whichever decoder runs then decodes
+    from CIGAR + reference (every context that decodes gets it); None: such records are rejected.
     -> (records incl. germline restatements, number of distinct query names that passed the read gates,
         names blob (want_names) or None)"""
     if decode not in ("auto", "host", "device"):
         raise ValueError("decode must be 'auto', 'host' or 'device'")
     src = worker.RegionSource(bam_file)
+    if refseq is not None:
+        src.reader.set_reference(chrom, refseq)
     tally = worker.QnameTally()
     kept, laters = [], []
     starts = [s for _, s, _e in chunkloci_lst]
@@ -120,7 +124,8 @@ def call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, want_nam
             for idx in groups:
                 loci = [chunkloci_lst[i] for i in idx]
                 c = ctxs[k % len(ctxs)]  # never the context whose call is pending
-                region = c.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci) + (1 if phase else 0))
+                region = c.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci) + (1 if phase else 0),
+                                         ref=refseq)
                 lap("device decode")
                 if region.n_reads == 0:
                     continue
@@ -217,7 +222,7 @@ def get_somatic_substitutions(
     if len(worker.group_chunks(chunkloci_lst)) > 1 and hasattr(ctx, "call_chunks_submit"):
         ctx2 = worker.second_context()  # long contigs: two contexts alternate between decode groups
         configure(ctx2, *conf)
-    rec, num_ccs, _ = call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, ctx2=ctx2)
+    rec, num_ccs, _ = call_region(ctx, bam_file, chrom, chunkloci_lst, chunk_sets, phase, ctx2=ctx2, refseq=worker.env_reference(chrom))
     chrom2tsbs_lst[chrom] = records.records_to_tsbs_lst(chrom, rec)
     chrom2tsbs_log[chrom] = [int(v) for v in _log_from_records(rec, num_ccs)]
     return int((rec["flags"] & abi.SITE_PL_TIE).astype(bool).sum())

@@ -116,6 +116,10 @@ typedef struct hm_bam {
   size_t cap_plan_blocks, cap_plan_entry;
   uint8_t* p_comp;
   size_t cap_p_comp;
+  /* hm_bam_set_reference: the caller's sequence of contig ref_rid (NULL: none), for records with neither cs:Z nor MD:Z */
+  const uint8_t* ref_seq;
+  size_t ref_len;
+  int ref_rid;
 } hm_bam;
 
 /* swap the active output buffers with the parked set */
@@ -543,6 +547,18 @@ const char* hm_bam_header_text(const hm_bam* b) { return b->header; }
 int hm_bam_n_refs(const hm_bam* b) { return b->n_ref; }
 const char* hm_bam_ref_name(const hm_bam* b, int i) { return (i >= 0 && i < b->n_ref) ? b->refs[i].name : NULL; }
 int hm_bam_ref_len(const hm_bam* b, int i) { return (i >= 0 && i < b->n_ref) ? b->refs[i].len : -1; }
+int hm_bam_set_reference(hm_bam* b, int rid, const uint8_t* seq, size_t len) {
+  if (!b) return HM_ERR_ARG;
+  b->ref_seq = NULL; b->ref_len = 0; b->ref_rid = -1;
+  if (!seq) return HM_OK;
+  if (rid < 0 || rid >= b->n_ref) return fail(b, "invalid contig index%s %ld", NULL, rid);
+  if ((uint64_t)len != (uint64_t)b->refs[rid].len) {
+    snprintf(b->err, sizeof(b->err), "the reference sequence of %s has %zu bases, its @SQ LN %d", b->refs[rid].name, len, b->refs[rid].len);
+    return HM_ERR_ARG;
+  }
+  b->ref_seq = seq; b->ref_len = len; b->ref_rid = rid;
+  return HM_OK;
+}
 uint32_t hm_bam_n_qnames(const hm_bam* b) { return b->qt.n; }
 const char* hm_bam_qname(const hm_bam* b, uint32_t id) { return id < b->qt.n ? b->qt.names[id] : NULL; }
 /* the names whose flag is set, each followed by '\n', in id order: what a worker that owns only a run of a contig's
@@ -582,7 +598,8 @@ static inline int base_code(char c) {
 typedef struct {
   const uint8_t* rec;   /* start of the fixed part (after block_size) */
   const char* cs;       /* the cs:Z value, or NULL: the ops come from CIGAR + md */
-  const char* md;
+  const char* md;       /* the MD:Z value, or NULL with cs NULL too: the ops come from CIGAR + the reference (ref_walk) */
+  uint32_t* ext;        /* CIGAR + reference: the ops, allocated by the decode (no slot is reserved for them) */
   int32_t pos, l_seq, lead, trail, ref_span;
   size_t seq_off, bq_off, op_slot; /* where its outputs go; op_slot is an upper-bound slot, compacted afterwards */
   size_t exc_slot;                 /* compact qualities: upper-bound slot of the exceptions, compacted afterwards */
@@ -663,20 +680,118 @@ static long long md_num(const char** c) {
   return n;
 }
 
-/* CIGAR + MD:Z -> ops, the rules and the order of checks of pack.parse_md; 0 with R->err set on failure */
-static int md_walk(rec_t* R, const uint8_t* cig, uint32_t n_cig, const uint8_t* codes, int32_t l_seq, uint32_t* ops,
-                   uint32_t* n_out, int32_t* q_out, int32_t* rspan_out) {
-#define MD_FAIL(e, a) do { R->err = (e); R->err_arg = (long)(a); return 0; } while (0)
+/* the CIGAR checks of md_walk and ref_walk (pack._check_cigar): N, P, codes past X and clips between aligned ops are
+ * unsupported, the CIGAR's query length must be l_seq; 0 with R->err set on failure */
+static int cigar_check(rec_t* R, const uint8_t* cig, uint32_t n_cig, int32_t l_seq) {
   uint32_t first = n_cig, last = 0; /* the aligned ops: clips may only lie outside [first, last] */
   for (uint32_t k = 0; k < n_cig; k++) { const uint32_t op = rd32(cig + 4 * k) & 15; if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; } }
   int64_t qcore = 0, qclip = 0;
   for (uint32_t k = 0; k < n_cig; k++) {
     const uint32_t c = rd32(cig + 4 * k), op = c & 15, ln = c >> 4;
-    if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) MD_FAIL(E_CIGAR_OP, k); if (op == 4) qclip += ln; }
+    if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) { R->err = E_CIGAR_OP; R->err_arg = (long)k; return 0; } if (op == 4) qclip += ln; }
     else if (op == 0 || op == 1 || op == 7 || op == 8) qcore += ln;
-    else if (op != 2) MD_FAIL(E_CIGAR_OP, k);
+    else if (op != 2) { R->err = E_CIGAR_OP; R->err_arg = (long)k; return 0; }
   }
-  if (qcore + qclip != l_seq) MD_FAIL(E_SPAN_QRY, qcore);
+  if (qcore + qclip != l_seq) { R->err = E_SPAN_QRY; R->err_arg = (long)qcore; return 0; }
+  return 1;
+}
+
+/* a reference byte -> A0 T1 G2 C3 (either case), 0xfe anything else: never equal to a read code (0..3, 0xff) */
+static inline uint8_t ref_code(uint8_t c) {
+  switch (c & 0xdf) { case 'A': return 0; case 'T': return 1; case 'G': return 2; case 'C': return 3; default: return 0xfe; }
+}
+/* w <= 16 bases from reference bytes rp and read codes cp: bit i of *m set when read base i equals an A/C/G/T
+ * reference base, of *bad when read base i is outside A/C/G/T.  16 at a time with SSE2 (only whole windows: the
+ * reference may end right after the alignment), the plain loop for the rest. */
+static inline void ref_masks(const uint8_t* rp, const uint8_t* cp, int w, uint32_t* m, uint32_t* bad) {
+#if defined(__SSE2__)
+  if (w == 16) {
+    const __m128i u = _mm_and_si128(_mm_loadu_si128((const __m128i*)rp), _mm_set1_epi8((char)0xdf));
+    const __m128i c = _mm_loadu_si128((const __m128i*)cp);
+    const __m128i a = _mm_cmpeq_epi8(u, _mm_set1_epi8('A')), t = _mm_cmpeq_epi8(u, _mm_set1_epi8('T'));
+    const __m128i g = _mm_cmpeq_epi8(u, _mm_set1_epi8('G')), cc = _mm_cmpeq_epi8(u, _mm_set1_epi8('C'));
+    const __m128i acgt = _mm_or_si128(_mm_or_si128(a, t), _mm_or_si128(g, cc));
+    const __m128i code = _mm_or_si128(_mm_or_si128(_mm_and_si128(t, _mm_set1_epi8(1)), _mm_and_si128(g, _mm_set1_epi8(2))),
+                                      _mm_or_si128(_mm_and_si128(cc, _mm_set1_epi8(3)), _mm_andnot_si128(acgt, _mm_set1_epi8((char)0xfe))));
+    *m = (uint32_t)_mm_movemask_epi8(_mm_cmpeq_epi8(code, c));
+    *bad = (uint32_t)_mm_movemask_epi8(_mm_cmpeq_epi8(c, _mm_set1_epi8((char)0xff)));
+    return;
+  }
+#endif
+  uint32_t mm = 0, bb = 0;
+  for (int i = 0; i < w; i++) { mm |= (uint32_t)(ref_code(rp[i]) == cp[i]) << i; bb |= (uint32_t)(cp[i] == 0xff) << i; }
+  *m = mm; *bad = bb;
+}
+
+/* CIGAR + the reference sequence set with hm_bam_set_reference -> ops, the rules and the order of checks of
+ * pack.parse_ref; ops needs room for 2 l_seq + n_cig + 1; 0 with R->err set on failure */
+static int ref_walk(const hm_bam* b, rec_t* R, const uint8_t* cig, uint32_t n_cig, const uint8_t* codes, int32_t l_seq,
+                    uint32_t* ops, uint32_t* n_out, int32_t* q_out, int32_t* rspan_out) {
+#define REF_FAIL(e, a) do { R->err = (e); R->err_arg = (long)(a); return 0; } while (0)
+  if (!cigar_check(R, cig, n_cig, l_seq)) return 0;
+  int64_t span = 0;
+  for (uint32_t k = 0; k < n_cig; k++) { const uint32_t c = rd32(cig + 4 * k), op = c & 15; if (op == 0 || op == 2 || op == 7 || op == 8) span += c >> 4; }
+  if (R->pos < 0 || (uint64_t)R->pos + (uint64_t)span > (uint64_t)b->ref_len) REF_FAIL(E_REF_END, (int64_t)R->pos + span);
+  const uint8_t* ref = b->ref_seq + R->pos;
+  int32_t q = R->lead, r = 0;
+  uint32_t n = 0, run = 0;
+#define REF_FLUSH() do { if (run) { ops[n++] = HM_MAKE_OP(HM_OP_MATCH, run); run = 0; } } while (0)
+  for (uint32_t k = 0; k < n_cig; k++) {
+    const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+    if (ln == 0 || op == 4 || op == 5) continue;
+    if (op == 0 || op == 7 || op == 8) {
+      for (uint32_t k0 = 0; k0 < ln; k0 += 16) {
+        const int w = ln - k0 < 16 ? (int)(ln - k0) : 16;
+        const uint32_t full = (1u << w) - 1;
+        uint32_t m, bad, sub;
+        ref_masks(ref + r, codes + q, w, &m, &bad);
+        if (op == 0) { /* M: mismatches are SUBs, of read bases inside A/C/G/T only */
+          if (bad) REF_FAIL(E_SUB_N, q + __builtin_ctz(bad));
+          sub = ~m & full;
+        } else { /* =: every base matches; X: none does */
+          const uint32_t stop = op == 7 ? (~m & full) : (m | bad);
+          if (stop) {
+            const int j = __builtin_ctz(stop);
+            if ((bad >> j) & 1) REF_FAIL(op == 7 ? E_N_MATCH : E_SUB_N, q + j);
+            REF_FAIL(E_REF_SPAN, r + j);
+          }
+          sub = op == 7 ? 0 : full;
+        }
+        int last = -1;
+        while (sub) {
+          const int j = __builtin_ctz(sub);
+          sub &= sub - 1;
+          run += (uint32_t)(j - last - 1);
+          REF_FLUSH();
+          const uint8_t rc_ = ref_code(ref[r + j]);
+          ops[n++] = HM_MAKE_SUB(rc_ > 3 ? HM_BASE_N : (uint32_t)rc_, (uint32_t)codes[q + j]);
+          last = j;
+        }
+        run += (uint32_t)(w - last - 1);
+        q += w; r += w;
+      }
+    } else if (op == 1) {
+      REF_FLUSH();
+      ops[n++] = HM_MAKE_OP(HM_OP_INS, ln);
+      q += (int32_t)ln;
+    } else { /* D: the deleted bases are not read */
+      REF_FLUSH();
+      ops[n++] = HM_MAKE_OP(HM_OP_DEL, ln);
+      r += (int32_t)ln;
+    }
+  }
+  REF_FLUSH();
+#undef REF_FLUSH
+#undef REF_FAIL
+  *n_out = n; *q_out = q; *rspan_out = r;
+  return 1;
+}
+
+/* CIGAR + MD:Z -> ops, the rules and the order of checks of pack.parse_md; 0 with R->err set on failure */
+static int md_walk(rec_t* R, const uint8_t* cig, uint32_t n_cig, const uint8_t* codes, int32_t l_seq, uint32_t* ops,
+                   uint32_t* n_out, int32_t* q_out, int32_t* rspan_out) {
+#define MD_FAIL(e, a) do { R->err = (e); R->err_arg = (long)(a); return 0; } while (0)
+  if (!cigar_check(R, cig, n_cig, l_seq)) return 0;
   const char* md = R->md;
   const char* c = md;
   const char* good = md; /* end of the longest prefix the grammar accepts */
@@ -743,9 +858,9 @@ static int md_walk(rec_t* R, const uint8_t* cig, uint32_t n_cig, const uint8_t* 
   return 1;
 }
 
-/* phase B for one record: SEQ -> 2-bit, QUAL copy, cs -> ops (cslib.cs2lst grammar) or CIGAR + MD -> ops (md_walk)
- * with span and base checks */
-static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_cap) {
+/* phase B for one record: SEQ -> 2-bit, QUAL copy, cs -> ops (cslib.cs2lst grammar), CIGAR + MD -> ops (md_walk) or
+ * CIGAR + reference -> ops (ref_walk, into the worker's scratch, then R->ext) with span and base checks */
+static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_cap, uint32_t** scratch, size_t* scratch_cap) {
   const uint8_t* r = R->rec;
   const uint32_t l_name = r[8], n_cig = r[12] | (r[13] << 8);
   const int32_t l_seq = R->l_seq;
@@ -764,7 +879,17 @@ static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_
   int32_t q = R->lead, rspan = 0;
   const char* cs = R->cs;
   const char* c = cs;
-  if (!cs && !md_walk(R, r + 32 + l_name, n_cig, codes, l_seq, ops, &n_ops, &q, &rspan)) return;
+  const int by_ref = !cs && !R->md;
+  if (by_ref) {
+    const size_t need = 2 * (size_t)l_seq + n_cig + 2;
+    if (need > *scratch_cap) {
+      uint32_t* np_ = (uint32_t*)realloc(*scratch, need * sizeof(uint32_t));
+      if (!np_) { R->err = E_NO_MEM; R->err_arg = (long)(need * sizeof(uint32_t)); return; }
+      *scratch = np_; *scratch_cap = need;
+    }
+    ops = *scratch;
+    if (!ref_walk(b, R, r + 32 + l_name, n_cig, codes, l_seq, ops, &n_ops, &q, &rspan)) return;
+  } else if (!cs && !md_walk(R, r + 32 + l_name, n_cig, codes, l_seq, ops, &n_ops, &q, &rspan)) return;
   while (cs && *c) {
     if (*c == ':') {
       long n = 0; c++;
@@ -802,6 +927,11 @@ static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_
   }
   if (rspan != R->ref_span) { R->err = E_SPAN_REF; R->err_arg = rspan; return; }
   if (q - R->lead != l_seq - R->trail - R->lead) { R->err = E_SPAN_QRY; R->err_arg = q - R->lead; return; }
+  if (by_ref) {
+    R->ext = (uint32_t*)malloc((n_ops ? n_ops : 1) * sizeof(uint32_t));
+    if (!R->ext) { R->err = E_NO_MEM; R->err_arg = (long)((n_ops ? n_ops : 1) * sizeof(uint32_t)); return; }
+    memcpy(R->ext, ops, (size_t)n_ops * sizeof(uint32_t));
+  }
   R->n_ops = n_ops; R->rspan = rspan;
   const size_t sb = ((size_t)l_seq + 3) / 4, sb16 = (sb + 15) & ~(size_t)15, qb16 = ((size_t)l_seq + 15) & ~(size_t)15;
   if (!b->no_seq) {
@@ -842,15 +972,16 @@ static void decode_record(hm_bam* b, rec_t* R, uint8_t** codes_p, size_t* codes_
 static void* decode_worker(void* arg) {
   decode_job_t* j = (decode_job_t*)arg;
   uint8_t* codes = NULL; size_t cap = 0;
+  uint32_t* scratch = NULL; size_t scap = 0;
   for (;;) {
     pthread_mutex_lock(&j->mu);
     size_t i0 = j->next;
     j->next += 64;
     pthread_mutex_unlock(&j->mu);
     if (i0 >= j->n) break;
-    for (size_t i = i0; i < i0 + 64 && i < j->n; i++) decode_record(j->b, &j->recs[i], &codes, &cap);
+    for (size_t i = i0; i < i0 + 64 && i < j->n; i++) decode_record(j->b, &j->recs[i], &codes, &cap, &scratch, &scap);
   }
-  free(codes);
+  free(codes); free(scratch);
   return NULL;
 }
 
@@ -909,7 +1040,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         if (stream_need(&s, 4 + (size_t)bs0)) { rc = fail(b, REC_ERR[E_TRUNC_REC], b->path, 0); break; }
       }
       double tA = now_s();
-      size_t nsel = 0, seg_ops = 0, seg_exc = 0;
+      size_t nsel = 0, seg_ops = 0, seg_exc = 0, seg_ref = 0;
       const size_t first_read = n_reads;
       while (s.len - s.pos >= 4) {
         uint32_t bs = rd32(s.buf + s.pos);
@@ -972,7 +1103,9 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
           tag = v + adv;
         }
         if (rc) break;
-        if (!cs && !md) { rc = fail(b, REC_ERR[E_NO_CS], qname, 0); break; } /* cs when it is there, else CIGAR + MD */
+        /* cs when it is there, else CIGAR + MD, else CIGAR + the reference when the caller set this contig's */
+        const int by_ref = !cs && !md && b->ref_seq && b->ref_rid == rid;
+        if (!cs && !md && !by_ref) { rc = fail(b, REC_ERR[E_NO_CS], qname, 0); break; }
         /* hard clips: pysam's query_sequence and query_alignment_start leave them out (SEQ holds no hard-clipped base),
          * so cs2tuple indexes consistently and the reference processes such records (minimap2 writes them for
          * supplementary alignments without -Y); lead / trail above count soft clips only */
@@ -997,7 +1130,7 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         if (id < 0) { rc = fail(b, "out of memory%s (%ld)", NULL, 0); break; }
         const size_t sb = ((size_t)l_seq + 3) / 4, sb16 = (sb + 15) & ~(size_t)15, qb16 = ((size_t)l_seq + 15) & ~(size_t)15;
         rec_t* R = &recs[nsel++];
-        R->rec = r; R->cs = cs; R->md = cs ? NULL : md; R->pos = pos; R->l_seq = l_seq; R->lead = lead; R->trail = trail; R->ref_span = ref_span;
+        R->rec = r; R->cs = cs; R->md = cs ? NULL : md; R->ext = NULL; R->pos = pos; R->l_seq = l_seq; R->lead = lead; R->trail = trail; R->ref_span = ref_span;
         R->seq_off = n_seq; R->bq_off = n_bq; R->op_slot = n_ops + seg_ops; R->n_ops = 0; R->rspan = 0; R->err = 0; R->err_arg = 0;
         R->exc_slot = (size_t)n_exc + seg_exc; R->n_exc = 0;
         if (b->compact_bq) {
@@ -1014,8 +1147,11 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         b->mapq[n_reads] = (uint8_t)mapq; b->flags[n_reads] = 0; b->qname_id[n_reads] = (uint32_t)id;
         b->seq_off[n_reads] = n_seq; b->bq_off[n_reads] = n_bq;
         if (!b->no_seq) n_seq += sb16;
-        /* ops of CIGAR + MD: SUBs <= MD letters, INS + DEL <= CIGAR ops, match runs <= the other ops + 1 */
-        n_bq += qb16; seg_ops += cs ? strlen(cs) / 2 + 2 : 2 * (strlen(md) + n_cig) + 2; n_reads++;
+        /* ops of CIGAR + MD: SUBs <= MD letters, INS + DEL <= CIGAR ops, match runs <= the other ops + 1; CIGAR +
+         * reference: no slot (R->ext) */
+        n_bq += qb16; n_reads++;
+        if (by_ref) seg_ref++;
+        else seg_ops += cs ? strlen(cs) / 2 + 2 : 2 * (strlen(md) + n_cig) + 2;
       }
       if (rc) break;
       if (nsel) {
@@ -1041,12 +1177,26 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
         for (int t = 1; t < use; t++) pthread_join(th[t], NULL);
         pthread_mutex_destroy(&job.mu);
         g_phase[5] += now_s() - tA; tA = now_s();
-        /* serial tail: first error in file order, op compaction */
-        for (size_t i = 0; i < nsel; i++) {
+        /* serial tail: first error in file order, op compaction.  Ops of CIGAR + reference records (R->ext) are counted
+         * only by their decode, so with any of them the segment's ops are gathered past the slots and moved down. */
+        size_t gather = 0;
+        const size_t ops0 = n_ops;
+        if (seg_ref) {
+          size_t tot = 0;
+          for (size_t i = 0; i < nsel; i++) tot += recs[i].n_ops;
+          gather = n_ops + seg_ops;
+          if (gather + tot + 4 > b->cap_ops) {
+            uint32_t* np_ = (uint32_t*)realloc(b->ops, (gather + tot + 4) * sizeof(uint32_t));
+            if (!np_) rc = fail(b, "out of memory%s (%ld)", NULL, (long)(gather + tot + 4));
+            else { b->ops = np_; b->cap_ops = gather + tot + 4; }
+          }
+        }
+        for (size_t i = 0; i < nsel && !rc; i++) {
           rec_t* R = &recs[i];
           if (R->err) { rc = fail(b, REC_ERR[R->err], (const char*)(R->rec + 32), R->err_arg); break; }
           const size_t rd = first_read + i;
-          if (R->op_slot != n_ops) memmove(b->ops + n_ops, b->ops + R->op_slot, (size_t)R->n_ops * sizeof(uint32_t));
+          if (seg_ref) memcpy(b->ops + gather + (n_ops - ops0), R->ext ? R->ext : b->ops + R->op_slot, (size_t)R->n_ops * sizeof(uint32_t));
+          else if (R->op_slot != n_ops) memmove(b->ops + n_ops, b->ops + R->op_slot, (size_t)R->n_ops * sizeof(uint32_t));
           b->op_off[rd] = n_ops; b->n_ops[rd] = R->n_ops; b->tend[rd] = R->pos + R->rspan;
           n_ops += R->n_ops;
           if (b->compact_bq) {
@@ -1055,6 +1205,8 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
             n_exc += R->n_exc;
           }
         }
+        if (seg_ref && !rc) memmove(b->ops + ops0, b->ops + gather, (n_ops - ops0) * sizeof(uint32_t));
+        if (seg_ref) for (size_t i = 0; i < nsel; i++) { free(recs[i].ext); recs[i].ext = NULL; }
       }
     }
     if (getenv("HIMUT_B200_DECODE_TIMING"))
@@ -1453,9 +1605,11 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
 
 int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                             int level, int threads, int tags) {
-  if (!path || !chrom || !b || (tags != HM_BAM_TAGS_CS && tags != HM_BAM_TAGS_MD && tags != HM_BAM_TAGS_MD_EQX)) return HM_ERR_ARG;
-  const int use_md = tags != HM_BAM_TAGS_CS;
-  const uint32_t m_op = tags == HM_BAM_TAGS_MD ? 0 : 7, x_op = tags == HM_BAM_TAGS_MD ? 0 : 8;
+  if (!path || !chrom || !b || tags < HM_BAM_TAGS_CS || tags > HM_BAM_TAGS_M) return HM_ERR_ARG;
+  const int use_md = tags != HM_BAM_TAGS_CS;                             /* the walk below writes MD (unused without a tag) */
+  const int no_tag = tags == HM_BAM_TAGS_EQX || tags == HM_BAM_TAGS_M;  /* no alignment tag: CIGAR + reference decodes it */
+  const int m_cigar = tags == HM_BAM_TAGS_MD || tags == HM_BAM_TAGS_M;
+  const uint32_t m_op = m_cigar ? 0 : 7, x_op = m_cigar ? 0 : 8;
   (void)hm_crc32_available(); /* probed before the deflate threads exist */
   wbuf_t w; memset(&w, 0, sizeof(w));
   char text[1024];
@@ -1507,7 +1661,7 @@ int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_
     char qname[32];
     const int lq = snprintf(qname, sizeof(qname), "read%u", b->qname_id[r]) + 1;
     const int32_t pos = b->tstart[r], endp = pos + (rspan > 0 ? rspan : 1);
-    const size_t body = 32 + (size_t)lq + 4 * ncig + ((size_t)ql + 1) / 2 + (size_t)ql + (3 + lc + 1) + 4;
+    const size_t body = 32 + (size_t)lq + 4 * ncig + ((size_t)ql + 1) / 2 + (size_t)ql + (no_tag ? 0 : 3 + lc + 1) + 4;
     if (wb_need(&w, body + 8)) { rc = HM_ERR_ARG; break; }
     rec_off[r] = w.n; rec_end[r] = endp;
     wb_u32(&w, (uint32_t)body);
@@ -1527,7 +1681,7 @@ int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_
       w.p[w.n++] = (uint8_t)((hi << 4) | lo);
     }
     memcpy(w.p + w.n, b->bq + b->bq_off[r], (size_t)ql); w.n += (size_t)ql;
-    w.p[w.n++] = use_md ? 'M' : 'c'; w.p[w.n++] = use_md ? 'D' : 's'; w.p[w.n++] = 'Z'; memcpy(w.p + w.n, cs, lc + 1); w.n += lc + 1;
+    if (!no_tag) { w.p[w.n++] = use_md ? 'M' : 'c'; w.p[w.n++] = use_md ? 'D' : 's'; w.p[w.n++] = 'Z'; memcpy(w.p + w.n, cs, lc + 1); w.n += lc + 1; }
     w.p[w.n++] = 't'; w.p[w.n++] = 'p'; w.p[w.n++] = 'A'; w.p[w.n++] = 'P';
   }
   free(cs); free(cig);

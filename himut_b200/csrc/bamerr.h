@@ -9,6 +9,8 @@
 enum {
   E_CS_TOKEN = 1, E_CS_PAST, E_N_MATCH, E_CS_LONG, E_SUB_N, E_SPAN_REF, E_SPAN_QRY, /* cs -> ops (record decode) */
   E_MD_TOKEN, E_MD_SPAN, E_CIGAR_OP,         /* CIGAR + MD:Z -> ops (record decode, records without cs:Z) */
+  E_REF_END, E_REF_SPAN,                     /* CIGAR + reference -> ops (record decode, records with neither tag) */
+  E_NO_MEM,                                  /* host decoder only: no memory for a record's ops */
   E_BLOCK_SIZE, E_FIELDS, E_TAG_UNTERM, E_TAG_B, E_TAG_TYPE, E_TAG_PAST, E_NO_CS, E_NO_QUAL, /* record selection */
   E_TRUNC_REC,                               /* a record runs past the end of the data */
   E_INFLATE, E_CRC, E_BAI_ENTRY,             /* device decoder only: BGZF block / index problems */
@@ -22,6 +24,9 @@ static const char* const REC_ERR[E_N_CODES] = {
     "%s: cs reference span != CIGAR span (%ld)", "%s: cs query span != aligned query span (%ld)",
     "%s: unsupported MD:Z token (%ld)", "%s: MD:Z and CIGAR disagree at reference offset %ld",
     "%s: unsupported CIGAR op (N, P, or a clip inside the alignment) at CIGAR index %ld",
+    "%s: alignment runs past the end of the reference sequence (%ld)",
+    "%s: CIGAR and the reference sequence disagree at reference offset %ld",
+    "out of memory decoding record %s (%ld bytes)",
     "malformed BAM record in %s: block_size %ld", "malformed BAM record in %s: fields run past block_size %ld",
     "malformed BAM record %s: unterminated %ld tag", "malformed BAM record %s: truncated B tag or unknown B subtype (%ld)",
     "unknown tag type in record %s (%ld)", "malformed BAM record %s: a tag runs past the record (%ld)",

@@ -6,8 +6,10 @@
 //   k_bgzf_inflate   one thread per BGZF block: raw DEFLATE (stored, fixed, dynamic), ISIZE and CRC32 checked
 //   k_bam_walk       one thread per entry point (BAI linear-index entry): follows block_size to the next one
 //   k_bam_select     one thread per record: hm_bam_read_batch's selection and checks, counts for the output scans
-//   k_bam_parse      one warp per selected record: qualities, 2-bit bases (if asked), cs (or CIGAR + MD) -> ops,
-//                    coordinates, the name
+//   k_bam_ref_count  one warp per record with neither cs:Z nor MD:Z (HM_DECODE_REF): its exact op count from CIGAR +
+//                    the resident reference, 32 bases per step
+//   k_bam_parse      one warp per selected record: qualities, 2-bit bases (if asked), cs (or CIGAR + MD, or CIGAR +
+//                    reference) -> ops, coordinates, the name
 //
 // Shape of k_bgzf_inflate: a BGZF block is an independent stream of at most 64 KB whose decode is one serial chain
 // (each symbol's length is known only once it is decoded), so one thread decodes one block, and it is the only
@@ -35,7 +37,8 @@ struct Err {                    // first failure, in file order, of each kind
   unsigned long long entry;     // first entry point that is not a record start (~0: none)
   unsigned long long rec;       // first record that fails selection (~0: none)
   unsigned long long stop;      // first record that ends the region (~0: none)
-  unsigned long long parse;     // first selected record that fails cs (or CIGAR + MD) -> ops (~0: none)
+  unsigned long long parse;     // first selected record that fails cs (or CIGAR + MD, or CIGAR + reference) -> ops (~0: none)
+  unsigned long long n_ref;     // records k_bam_select listed for k_bam_ref_count (starts at 0, not ~0)
 };
 
 struct RecInfo {  // k_bam_select -> k_bam_parse
@@ -45,6 +48,7 @@ struct RecInfo {  // k_bam_select -> k_bam_parse
   uint32_t n_ops;
   uint8_t keep;
   uint8_t md;     // the record has no cs:Z: its ops come from CIGAR + MD:Z
+  uint8_t ref;    // the record has neither tag: its ops come from CIGAR + the resident reference (n_ops: k_bam_ref_count)
 };
 
 __device__ __forceinline__ uint32_t rd32(const uint8_t* p) {
@@ -340,9 +344,11 @@ __device__ uint32_t md_count(const uint8_t* cig, uint32_t n_cig, const char* c) 
   return n + run;
 }
 
+// ref_list (HM_DECODE_REF; nullptr: without): records with neither cs:Z nor MD:Z are kept and listed there, in no
+// particular order, for k_bam_ref_count; their op count is left to it
 __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n_rec, uint64_t walk_end, int32_t rid,
                              int32_t start, int32_t end, RecInfo* info, unsigned long long* cnt, int n_cnt, uint8_t* code,
-                             long long* arg, Err* err) {
+                             long long* arg, Err* err, uint32_t* ref_list) {
   const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const uint64_t stride = n_rec + 1;  // cnt: n_cnt (4 or 5) arrays of n_rec + 1 (the last entry 0: the scan's total)
   if (r == 0)
@@ -412,19 +418,135 @@ __global__ void k_bam_select(const uint8_t* buf, const uint64_t* rec, uint64_t n
     if (adv > left) { sel_fail(err, code, arg, r, E_TAG_PAST, (long long)adv); return; }
     tag = v + adv;
   }
-  if (!cs && !md) { sel_fail(err, code, arg, r, E_NO_CS, 0); return; }  // cs when it is there, else CIGAR + MD
+  // cs when it is there, else CIGAR + MD, else CIGAR + the resident reference when the caller asked for it
+  if (!cs && !md && !ref_list) { sel_fail(err, code, arg, r, E_NO_CS, 0); return; }
   if (l_seq <= 0 || qual[0] == 0xff) { sel_fail(err, code, arg, r, E_NO_QUAL, 0); return; }
   I.keep = 1;
-  I.md = !cs;
-  I.cs = (uint32_t)((cs ? cs : md) - R);
+  I.md = !cs && md;
+  I.ref = !cs && !md;
+  I.cs = (uint32_t)(cs ? cs - R : md ? md - R : 0);
   I.pos = pos; I.l_seq = l_seq; I.lead = lead; I.trail = trail; I.ref_span = ref_span;
-  I.n_ops = cs ? cs_count((const char*)cs) : md_count(cig, n_cig, (const char*)md);
+  I.n_ops = cs ? cs_count((const char*)cs) : md ? md_count(cig, n_cig, (const char*)md) : 0;
   info[r] = I;
+  if (I.ref) ref_list[atomicAdd(&err->n_ref, 1ull)] = (uint32_t)r;
   cnt[r] = 1;
   cnt[stride + r] = I.n_ops;
   cnt[2 * stride + r] = ((uint64_t)l_seq + 15) & ~(uint64_t)15;
   cnt[3 * stride + r] = l_name;
   if (n_cnt == 5) cnt[4 * stride + r] = (((uint64_t)l_seq + 3) / 4 + 15) & ~(uint64_t)15;
+}
+
+// ------------------------------------------------------------------------------------------ CIGAR + reference
+// the CIGAR checks of the MD and reference paths (the host decoder's cigar_check): 0, or the code with *ea set.
+// *span: the reference span of M / D / = / X in 64 bits.  RecInfo::ref_span is an int32 sum that D lengths (which no
+// query length bounds) can wrap, so the bounds check that guards the reference reads takes this one.
+__device__ __forceinline__ int cigar_check(const uint8_t* cig, uint32_t n_cig, int32_t l_seq, long long* ea, int64_t* span) {
+  uint32_t first = n_cig, last = 0;
+  for (uint32_t k = 0; k < n_cig; k++) { const uint32_t op = rd32(cig + 4 * k) & 15; if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; } }
+  int64_t qcore = 0, qclip = 0, rs = 0;
+  for (uint32_t k = 0; k < n_cig; k++) {
+    const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+    if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) { *ea = k; return E_CIGAR_OP; } if (op == 4) qclip += ln; }
+    else if (op == 0 || op == 7 || op == 8) { qcore += ln; rs += ln; }
+    else if (op == 1) qcore += ln;
+    else if (op == 2) rs += ln;
+    else { *ea = k; return E_CIGAR_OP; }
+  }
+  if (qcore + qclip != l_seq) { *ea = qcore; return E_SPAN_QRY; }
+  *span = rs;
+  return 0;
+}
+
+// the code of read base q (A0 T1 G2 C3, 0xff anything else)
+__device__ __forceinline__ uint8_t base_at(const uint8_t* seq4, int64_t q) {
+  const int8_t nib2code[16] = {-1, 0, 3, -1, 2, -1, -1, -1, 1, -1, -1, -1, -1, -1, -1, -1};
+  const uint8_t by = seq4[q >> 1];
+  return (uint8_t)nib2code[(q & 1) ? (by & 15) : (by >> 4)];
+}
+// a reference byte -> A0 T1 G2 C3 (either case), 0xfe anything else: never equal to a read code (0..3, 0xff)
+__device__ __forceinline__ uint8_t ref_code(uint8_t c) {
+  switch (c & 0xdf) { case 'A': return 0; case 'T': return 1; case 'G': return 2; case 'C': return 3; default: return 0xfe; }
+}
+
+// One window of w <= 32 bases of an M (0), = (7) or X (8) op: lane i compares read base q + i with reference byte
+// rp[i] (coalesced loads).  -> 0 and the lanes that are SUBs (*sub), or the code of the first failing base with *ea
+// set: the rules of the host decoder's ref_walk.  *rc / *ac: this lane's reference and read codes.
+__device__ __forceinline__ int ref_window(uint32_t op, const uint8_t* rp, const uint8_t* seq4, int64_t q, int64_t r, int w,
+                                          int lane, unsigned* sub, uint8_t* rc, uint8_t* ac, long long* ea) {
+  const bool in = lane < w;
+  *rc = in ? ref_code(rp[lane]) : 0xfe;
+  *ac = in ? base_at(seq4, q + lane) : 0xff;
+  const unsigned full = w == 32 ? 0xffffffffu : (1u << w) - 1;
+  const unsigned m = __ballot_sync(0xffffffffu, in && *rc == *ac);
+  const unsigned bad = __ballot_sync(0xffffffffu, in && *ac == 0xff);
+  if (op == 0) {  // M: mismatches are SUBs, of read bases inside A/C/G/T only
+    if (bad) { *ea = q + __ffs(bad) - 1; return E_SUB_N; }
+    *sub = ~m & full;
+    return 0;
+  }
+  const unsigned stop = op == 7 ? (~m & full) : (m | bad);  // =: every base matches; X: none does
+  if (stop) {
+    const int j = __ffs(stop) - 1;
+    if ((bad >> j) & 1) { *ea = q + j; return op == 7 ? E_N_MATCH : E_SUB_N; }
+    *ea = r + j;
+    return E_REF_SPAN;
+  }
+  *sub = op == 7 ? 0u : full;
+  return 0;
+}
+
+// the SUB lanes of a window that a MATCH precedes: the base before is matched (the carried run for lane 0)
+__device__ __forceinline__ unsigned ref_match_before(unsigned sub, int w, uint32_t run) {
+  const unsigned full = w == 32 ? 0xffffffffu : (1u << w) - 1;
+  return sub & (((~sub & full) << 1) | (run ? 1u : 0u));
+}
+
+// One warp per listed record (k_bam_select's ref_list): the ops k_bam_parse's reference walk writes, counted with the
+// same windows, into the record's op count and its entry of the op scan.  Exact where that walk succeeds; where it
+// fails it stops (k_bam_parse reports the failure before it compares the counts).
+__global__ void k_bam_ref_count(const uint8_t* buf, RecInfo* info, const uint32_t* ref_list, uint64_t n_list,
+                                const uint8_t* ref, uint64_t ref_len, unsigned long long* cnt_ops) {
+  const uint64_t w_id = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (w_id >= n_list) return;
+  const uint32_t r = ref_list[w_id];
+  const RecInfo I = info[r];
+  const uint8_t* R = buf + I.p + 4;
+  const uint32_t l_name = R[8], n_cig = R[12] | (R[13] << 8);
+  const uint8_t* cig = R + 32 + l_name;
+  const uint8_t* seq4 = cig + 4 * (size_t)n_cig;
+  long long ea = 0;
+  int64_t span = 0;
+  uint32_t n = 0, run = 0;
+  if (!cigar_check(cig, n_cig, I.l_seq, &ea, &span) && I.pos >= 0 && (uint64_t)I.pos + (uint64_t)span <= ref_len) {
+    const uint8_t* rp = ref + I.pos;
+    int64_t q = I.lead, rs = 0;
+    bool ok = true;
+    for (uint32_t k = 0; k < n_cig && ok; k++) {
+      const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+      if (ln == 0 || op == 4 || op == 5) continue;
+      if (op == 0 || op == 7 || op == 8) {
+        for (uint32_t k0 = 0; k0 < ln; k0 += 32) {
+          const int w = (int)min(32u, ln - k0);
+          unsigned sub;
+          uint8_t rc, ac;
+          if (ref_window(op, rp + rs, seq4, q, rs, w, lane, &sub, &rc, &ac, &ea)) { ok = false; break; }
+          n += __popc(sub) + __popc(ref_match_before(sub, w, run));
+          run = sub ? (uint32_t)(w - 32 + __clz(sub)) : run + (uint32_t)w;
+          q += w; rs += w;
+        }
+      } else {
+        n += (run != 0) + 1;
+        run = 0;
+        if (op == 1) q += ln; else rs += ln;
+      }
+    }
+    if (ok) n += run != 0;
+  }
+  if (lane == 0) {
+    info[r].n_ops = n;
+    cnt_ops[r] = n;
+  }
 }
 
 // ------------------------------------------------------------------------------------------ k_bam_parse
@@ -438,14 +560,10 @@ struct ParseOut {
   char* names;
   uint64_t* seq_off;  // both nullptr: no base stream (the batch of `call` and the phase edges)
   uint8_t* seq;
+  const uint8_t* ref;  // the resident reference (HM_DECODE_REF), for records with neither tag
+  uint64_t ref_len;
 };
 
-// the code of read base q (A0 T1 G2 C3, 0xff anything else)
-__device__ __forceinline__ uint8_t base_at(const uint8_t* seq4, int64_t q) {
-  const int8_t nib2code[16] = {-1, 0, 3, -1, 2, -1, -1, -1, 1, -1, -1, -1, -1, -1, -1, -1};
-  const uint8_t by = seq4[q >> 1];
-  return (uint8_t)nib2code[(q & 1) ? (by & 15) : (by >> 4)];
-}
 __device__ __forceinline__ int base_code(char c) {
   switch (c) { case 'A': case 'a': return 0; case 'T': case 't': return 1; case 'G': case 'g': return 2; case 'C': case 'c': return 3; default: return -1; }
 }
@@ -498,16 +616,8 @@ __global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_
   long long ea = 0;
   if (I.md) {  // CIGAR + MD: the rules and the order of checks of the host decoder's md_walk (pack.parse_md)
     const uint8_t* cig = R + 32 + l_name;
-    uint32_t first = n_cig, last = 0;
-    for (uint32_t k = 0; k < n_cig; k++) { const uint32_t op = rd32(cig + 4 * k) & 15; if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; } }
-    int64_t qcore = 0, qclip = 0;
-    for (uint32_t k = 0; k < n_cig && !ec; k++) {
-      const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
-      if (op == 4 || op == 5) { if (first < n_cig && k > first && k < last) { ec = E_CIGAR_OP; ea = k; } if (op == 4) qclip += ln; }
-      else if (op == 0 || op == 1 || op == 7 || op == 8) qcore += ln;
-      else if (op != 2) { ec = E_CIGAR_OP; ea = k; }
-    }
-    if (!ec && qcore + qclip != l_seq) { ec = E_SPAN_QRY; ea = qcore; }
+    int64_t span;
+    ec = cigar_check(cig, n_cig, l_seq, &ea, &span);
     if (!ec) {  // grammar: the end of the longest prefix it accepts must be the end
       const char* good = cs;
       if (md_digit(*c)) {
@@ -574,8 +684,48 @@ __global__ void k_bam_parse(const uint8_t* buf, const RecInfo* info, uint64_t n_
     }
     if (!ec && run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; }
     if (!ec && (mnum || *c)) { ec = E_MD_SPAN; ea = rspan; }
+  } else if (I.ref) {  // CIGAR + the resident reference: the host decoder's ref_walk (pack.parse_ref), 32 bases per step
+    const uint8_t* cig = R + 32 + l_name;
+    int64_t span = 0;
+    ec = cigar_check(cig, n_cig, l_seq, &ea, &span);
+    if (!ec && (I.pos < 0 || (uint64_t)I.pos + (uint64_t)span > o.ref_len)) { ec = E_REF_END; ea = (long long)I.pos + span; }
+    const uint8_t* rp = o.ref + I.pos;
+    uint32_t run = 0;
+    for (uint32_t k = 0; k < n_cig && !ec; k++) {
+      const uint32_t cg = rd32(cig + 4 * k), op = cg & 15, ln = cg >> 4;
+      if (ln == 0 || op == 4 || op == 5) continue;
+      if (op == 0 || op == 7 || op == 8) {
+        for (uint32_t k0 = 0; k0 < ln; k0 += 32) {
+          const int w = (int)min(32u, ln - k0);
+          unsigned sub;
+          uint8_t rc, ac;
+          if ((ec = ref_window(op, rp + rspan, seq4, q, rspan, w, lane, &sub, &rc, &ac, &ea))) break;
+          // the window's ops in order, each SUB lane placed by ranks: the MATCH of the bases since the previous SUB (or
+          // of the carried run), then the SUB
+          const unsigned fl = ref_match_before(sub, w, run), below = (1u << lane) - 1;
+          if ((sub >> lane) & 1) {
+            const unsigned prev = sub & below;
+            uint32_t at = n_ops + __popc(prev) + __popc(fl & below);
+            if ((fl >> lane) & 1) {
+              if (at < I.n_ops) ops[at] = HM_MAKE_OP(HM_OP_MATCH, prev ? (uint32_t)(__clz(prev) - 32 + lane) : run + lane);
+              at++;
+            }
+            if (at < I.n_ops) ops[at] = HM_MAKE_SUB(rc > 3 ? HM_BASE_N : (uint32_t)rc, (uint32_t)ac);
+          }
+          n_ops += __popc(sub) + __popc(fl);
+          run = sub ? (uint32_t)(w - 32 + __clz(sub)) : run + (uint32_t)w;
+          q += w; rspan += w;
+        }
+      } else {  // I / D: the run ends; deleted reference bases are not read
+        if (run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; run = 0; }
+        if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(op == 1 ? HM_OP_INS : HM_OP_DEL, ln);
+        n_ops++;
+        if (op == 1) q += ln; else rspan += ln;
+      }
+    }
+    if (!ec && run) { if (lane == 0 && n_ops < I.n_ops) ops[n_ops] = HM_MAKE_OP(HM_OP_MATCH, run); n_ops++; }
   }
-  while (!I.md && *c && !ec) {
+  while (!I.md && !I.ref && *c && !ec) {
     if (*c == ':') {
       long long n = 0;
       c++;

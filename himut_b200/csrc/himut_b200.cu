@@ -180,7 +180,7 @@ struct hm_ctx {
   uint32_t modal = 0;
   // device BAM decoder (hm_decode_bam_*, bamgpu.cuh)
   DevBuf b_comp, b_pcoff, b_pcsize, b_pisize, b_puoff, b_pcrc, b_pentry, b_inflated, b_blk_code, b_derr, b_seg_cnt,
-      b_seg_off, b_recoff, b_recinfo, b_cnt, b_scan, b_ecode, b_earg, b_names, b_name_off;
+      b_seg_off, b_recoff, b_recinfo, b_cnt, b_scan, b_ecode, b_earg, b_names, b_name_off, b_reflist;
   PinVec<int32_t> hd_tstart, hd_tend, hd_qstart, hd_qlen;   // per-read arrays of the last hm_decode_bam_begin
   PinVec<uint32_t> hd_n_ops;
   PinVec<uint64_t> hd_bq_off, hd_op_off, hd_name_off, hd_seq_off, hd_scal; // hd_scal: walk / scan totals read back
@@ -433,7 +433,7 @@ void hm_destroy(hm_ctx* ctx) {
                     &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_sdiff, &ctx->b_cal_ok,
                     &ctx->b_comp, &ctx->b_pcoff, &ctx->b_pcsize, &ctx->b_pisize, &ctx->b_puoff, &ctx->b_pcrc, &ctx->b_pentry, &ctx->b_inflated,
                     &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt,
-                    &ctx->b_scan, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off};
+                    &ctx->b_scan, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off, &ctx->b_reflist};
   for (DevBuf* b : bufs) b->release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_cnt_pin) cudaFreeHost(ctx->h_cnt_pin);
@@ -729,7 +729,7 @@ static int decode_record_error(hm_ctx* ctx, const hm_bgzf_plan* pl, unsigned lon
 }
 
 static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32_t start, int32_t end, bool want_seq,
-                             uint64_t* n_reads) {
+                             bool use_ref, uint64_t* n_reads) {
   using namespace bamgpu;
   const uint64_t nb = pl->n_blocks, ne = pl->n_entry;
   ctx->dec_n = ctx->dec_ops = 0;
@@ -764,6 +764,7 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   CU(ctx->b_blk_code.ensure(nb));
   CU(ctx->b_derr.ensure(sizeof(Err)));
   CU(cudaMemsetAsync(ctx->b_derr.p, 0xff, sizeof(Err), ctx->stream));
+  CU(cudaMemsetAsync(&ctx->b_derr.as<Err>()->n_ref, 0, sizeof(unsigned long long), ctx->stream));
   if (!ctx->hd_err.resize(1) || !ctx->hd_scal.resize(5)) return fail(ctx, HM_ERR_ARG, "out of page-locked host memory");
   Err* derr = ctx->b_derr.as<Err>();
   Err& herr = ctx->hd_err[0];
@@ -814,10 +815,12 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   CU(ctx->b_scan.ensure(n_cnt * stride * 8));
   CU(ctx->b_ecode.ensure(n_rec));
   CU(ctx->b_earg.ensure(n_rec * 8));
+  if (use_ref) CU(ctx->b_reflist.ensure(n_rec * 4));
   t_begin(ctx, "k_bam_select");
   k_bam_select<<<(unsigned)((n_rec + 127) / 128), 128, 0, ctx->stream>>>(buf, ctx->b_recoff.as<uint64_t>(), n_rec, pl->walk_end, rid, start, end,
                                                                           ctx->b_recinfo.as<RecInfo>(), ctx->b_cnt.as<unsigned long long>(), n_cnt,
-                                                                          ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
+                                                                          ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr,
+                                                                          use_ref ? ctx->b_reflist.as<uint32_t>() : nullptr);
   t_end(ctx);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(&herr, derr, sizeof(Err), cudaMemcpyDeviceToHost, ctx->stream));
@@ -825,9 +828,17 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   const uint64_t stop = std::min<uint64_t>(herr.stop, n_rec);  // records from here on are never looked at by the host
   if (herr.rec < stop) return decode_record_error(ctx, pl, herr.rec);
   if (stop == 0) return HM_OK;
+  // records with neither tag: their op counts, one warp per record, before the scans read them
+  unsigned long long* cnt = ctx->b_cnt.as<unsigned long long>();
+  if (herr.n_ref) {
+    t_begin(ctx, "k_bam_ref_count");
+    k_bam_ref_count<<<(unsigned)((herr.n_ref * 32 + 255) / 256), 256, 0, ctx->stream>>>(buf, ctx->b_recinfo.as<RecInfo>(), ctx->b_reflist.as<uint32_t>(),
+                                                                                     herr.n_ref, ctx->b_ref.as<uint8_t>(), (uint64_t)ctx->ref_len, cnt + stride);
+    t_end(ctx);
+    CU(cudaGetLastError());
+  }
   // output offsets: exclusive scans of the counts (read index, first op, first quality byte, first name byte, and with
   // the base stream its first byte)
-  unsigned long long* cnt = ctx->b_cnt.as<unsigned long long>();
   unsigned long long* scan = ctx->b_scan.as<unsigned long long>();
   tmp = 0;
   CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, scan, (int)stride, ctx->stream));
@@ -849,7 +860,8 @@ static int decode_begin_impl(hm_ctx* ctx, const hm_bgzf_plan* pl, int rid, int32
   ParseOut o{ctx->b_tstart.as<int32_t>(), ctx->b_tend.as<int32_t>(), ctx->b_qstart.as<int32_t>(), ctx->b_qlen.as<int32_t>(),
              ctx->b_mapq.as<uint8_t>(), ctx->b_flags.as<uint8_t>(), ctx->b_n_ops.as<uint32_t>(), ctx->b_bq_off.as<uint64_t>(),
              ctx->b_op_off.as<uint64_t>(), ctx->b_name_off.as<uint64_t>(), ctx->b_bq.as<uint8_t>(), ctx->b_ops.as<uint32_t>(),
-             ctx->b_names.as<char>(), want_seq ? ctx->b_seq_off.as<uint64_t>() : nullptr, want_seq ? ctx->b_seq.as<uint8_t>() : nullptr};
+             ctx->b_names.as<char>(), want_seq ? ctx->b_seq_off.as<uint64_t>() : nullptr, want_seq ? ctx->b_seq.as<uint8_t>() : nullptr,
+             ctx->b_ref.as<uint8_t>(), use_ref ? (uint64_t)ctx->ref_len : 0};
   t_begin(ctx, "k_bam_parse");
   k_bam_parse<<<(unsigned)((stop * 32 + 255) / 256), 256, 0, ctx->stream>>>(buf, ctx->b_recinfo.as<RecInfo>(), stop, scan, stride, o,
                                                                              ctx->b_ecode.as<uint8_t>(), ctx->b_earg.as<long long>(), derr);
@@ -1706,7 +1718,9 @@ int hm_decode_bam_begin_opts(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int
                              uint64_t* n_reads) {
   if (!ctx || !plan || !n_reads) return HM_ERR_ARG;
   *n_reads = 0;
-  if (opts & ~HM_DECODE_SEQ) return fail(ctx, HM_ERR_ARG, "unknown decode option bits 0x%x", opts & ~HM_DECODE_SEQ);
+  if (opts & ~(HM_DECODE_SEQ | HM_DECODE_REF)) return fail(ctx, HM_ERR_ARG, "unknown decode option bits 0x%x", opts & ~(HM_DECODE_SEQ | HM_DECODE_REF));
+  if ((opts & HM_DECODE_REF) && !ctx->ref_len)
+    return fail(ctx, HM_ERR_STATE, "HM_DECODE_REF: no reference sequence is resident (hm_set_reference)");
   CU(cudaSetDevice(ctx->device));
   if (ctx->upload_pending) { // the copies of an upload that was not waited for still read their host buffers
     CU(cudaEventSynchronize(ctx->ev_up));
@@ -1716,7 +1730,7 @@ int hm_decode_bam_begin_opts(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int
   ctx->dec_ready = false;
   t_reset(ctx);
   if (start < 0) start = 0;
-  const int rc = decode_begin_impl(ctx, plan, rid, start, end, (opts & HM_DECODE_SEQ) != 0, n_reads);
+  const int rc = decode_begin_impl(ctx, plan, rid, start, end, (opts & HM_DECODE_SEQ) != 0, (opts & HM_DECODE_REF) != 0, n_reads);
   if (rc) { cudaStreamSynchronize(ctx->stream); return rc; }
   t_collect(ctx);
   ctx->dec_ready = true;

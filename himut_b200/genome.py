@@ -19,7 +19,7 @@ import time
 
 import numpy as np
 
-from . import abi, caller, records, shard, worker
+from . import abi, caller, fasta, records, shard, worker
 
 
 class Run:
@@ -114,12 +114,14 @@ def _dist():
 
 
 def call_genome(bam_file, chrom2chunkloci, args, phase_tables=None, common_snps=None, panel_of_normals=None, pieces_per_rank=4,
-                ctx=None):
+                ctx=None, ref=None):
     """`himut call` over every contig of chrom2chunkloci (contig -> its chunkloci list, as util.load_loci /
     vcflib.load_phased_hetsnps build it), sharded over the ranks of the initialised process group.
 
     args: the worker's scalar arguments by name (gtmodel.DEFAULT_CALL_ARGS keys + phase / non_human_sample /
           create_panel_of_normals);  phase_tables: contig -> (hbit, hpos, hetsnp dicts) in --phase mode.
+    ref: a FASTA of the reference the reads were aligned to, for records with neither cs:Z nor MD:Z (each run reads
+    its contig from it).
     Returns on rank 0 (chrom2tsbs_lst, chrom2tsbs_log, stats) — the dictionaries the reference's dump_call_log /
     dump_sbs / dump_phased_sbs take (vcflib.py:820-1060) — and (None, None, stats) on the other ranks."""
     dist = _dist()
@@ -133,6 +135,7 @@ def call_genome(bam_file, chrom2chunkloci, args, phase_tables=None, common_snps=
     ctx = ctx or worker.context()
     phase = bool(args.get("phase"))
     local, t0, my_weight = [], time.perf_counter(), 0
+    ref_contig = (None, None)
     for r in runs:
         if r.rank != rank:
             continue
@@ -149,7 +152,11 @@ def call_genome(bam_file, chrom2chunkloci, args, phase_tables=None, common_snps=
             ctx2 = worker.second_context()
             caller.configure(ctx2, *conf)
         split = len(per_contig[r.chrom]) > 1
-        rec, num_ccs, names = caller.call_region(ctx, bam_file, r.chrom, chunks, chunk_sets, phase, want_names=split, ctx2=ctx2)
+        if ref and r.chrom != ref_contig[0]:  # read once per contig: its runs on this rank reuse it, uploads included
+            ref_contig = (r.chrom, fasta.load_contig(ref, r.chrom))
+        refseq = ref_contig[1] if ref else None
+        rec, num_ccs, names = caller.call_region(ctx, bam_file, r.chrom, chunks, chunk_sets, phase, want_names=split, ctx2=ctx2,
+                                                 refseq=refseq)
         local.append((r.index, rec, num_ccs, names))
         my_weight += r.weight
     seconds = time.perf_counter() - t0
@@ -225,6 +232,7 @@ def main(argv=None):
     ap.add_argument("--panel_of_normals")
     ap.add_argument("--non_human_sample", action="store_true")
     ap.add_argument("--pieces_per_rank", type=int, default=4)
+    ap.add_argument("--ref", help="FASTA of the reference the reads were aligned to: decodes records with neither cs:Z nor MD:Z")
     a = ap.parse_args(argv)
     if "RANK" in os.environ and "WORLD_SIZE" in os.environ and int(os.environ["WORLD_SIZE"]) > 1:
         import torch
@@ -243,7 +251,7 @@ def main(argv=None):
                 non_human_sample=a.non_human_sample)
     loci = {c: chunkloci(c, n) for c, n in contigs}
     lst, log, stats = call_genome(a.bam, loci, args, common_snps=a.common_snps, panel_of_normals=a.panel_of_normals,
-                                  pieces_per_rank=a.pieces_per_rank)
+                                  pieces_per_rank=a.pieces_per_rank, ref=a.ref)
     if lst is not None:
         from .natsort_compat import natsorted
         chroms = natsorted(list(lst))

@@ -201,18 +201,31 @@ class Context:
             self._uploading = (batch, cq)  # alive until the copies are done
             self._chk(self.lib.hm_upload_batch_compact_begin(self.h, C.byref(batch.as_struct()), C.byref(cq.struct)))
 
-    def decode_region(self, reader, chrom, start, end, seq=False):
+    def decode_region(self, reader, chrom, start, end, seq=False, ref=False):
         """the records reader.read_batch(chrom, start, end, seq=seq) returns, decoded on the device from the
         compressed file (reader: bamdec.NativeBam) and left resident as upload() would leave that batch: seq=True
-        with the 2-bit base stream normcounts reads, seq=False without it (`call`, phase edges).  Query-name ids come
-        from the reader's table.  Rejected input raises pack.BatchFormatError with the host decoder's text.
+        with the 2-bit base stream normcounts reads, seq=False without it (`call`, phase edges).  ref: records with
+        neither cs:Z nor MD:Z are decoded from CIGAR + the sequence of `chrom`, as the reader does after its own
+        set_reference: True reads the one set_reference made resident, bytes are made resident first (set_reference);
+        False / None rejects such records.  A resident sequence whose length is not the contig's @SQ LN (another
+        contig's, another build's) raises ValueError.  Query-name ids come from the reader's table.  Rejected input
+        raises pack.BatchFormatError with the host decoder's text.
         -> DecodedRegion (n_reads, tstart, tend, chunk_table)"""
         rid = reader.references.index(chrom)
         start, end = int(max(start, 0)), int(min(end, reader.lengths[rid]))
+        if isinstance(ref, (bytes, bytearray)):
+            self.set_reference(ref)
+        elif ref is not True and ref is not False and ref is not None:
+            raise TypeError("ref must be True, False, None or the contig's sequence as bytes, not %s" % type(ref).__name__)
+        resident = getattr(self, "_ref_obj", None)
+        if ref is not None and ref is not False and resident is not None and len(resident) != reader.lengths[rid]:
+            raise ValueError("the resident reference sequence has %d bases, contig %s of the BAM %d (@SQ LN)"
+                             % (len(resident), chrom, reader.lengths[rid]))
         plan = reader.plan(chrom, start, end)
         n = C.c_uint64(0)
-        if seq:
-            rc = self.lib.hm_decode_bam_begin_opts(self.h, C.byref(plan), rid, start, end, abi.HM_DECODE_SEQ, C.byref(n))
+        opts = (abi.HM_DECODE_SEQ if seq else 0) | (abi.HM_DECODE_REF if ref is not None and ref is not False else 0)
+        if opts:
+            rc = self.lib.hm_decode_bam_begin_opts(self.h, C.byref(plan), rid, start, end, opts, C.byref(n))
         else:
             rc = self.lib.hm_decode_bam_begin(self.h, C.byref(plan), rid, start, end, C.byref(n))
         if rc == abi.HM_ERR_ARG:
@@ -356,13 +369,20 @@ class Context:
         """upload + call (host buffers in, records out): the end-to-end path"""
         return self._call(self.lib.hm_call_batch, (C.byref(batch.as_struct()),), chunks, cap, view)
 
-    def normcounts_chunks(self, refseq, chunks):
-        """callable-base half of `himut normcounts` -> (ccs_tri[33], ref_tri[33], log[14], n_alt_tie)"""
-        chunks = np.ascontiguousarray(chunks, dtype=abi.CHUNK_DTYPE)
-        if refseq is not getattr(self, "_ref_obj", None):  # upload a contig's reference once
+    def set_reference(self, refseq):
+        """make a contig's sequence (bytes) resident: normcounts_chunks(None, ...) and decode_region(..., ref=True) read
+        it.  Uploaded once per object: the same bytes again cost nothing."""
+        if refseq is not getattr(self, "_ref_obj", None):
             ref = np.frombuffer(refseq, dtype=np.uint8)
             self._chk(self.lib.hm_set_reference(self.h, _p(ref), ref.size))
             self._ref_obj = refseq
+
+    def normcounts_chunks(self, refseq, chunks):
+        """callable-base half of `himut normcounts` -> (ccs_tri[33], ref_tri[33], log[14], n_alt_tie); refseq None:
+        the sequence set_reference made resident"""
+        chunks = np.ascontiguousarray(chunks, dtype=abi.CHUNK_DTYPE)
+        if refseq is not None:  # upload a contig's reference once
+            self.set_reference(refseq)
         ref = np.zeros(0, np.uint8)
         ccs = np.zeros(abi.TRI_BINS, np.int64)
         rt = np.zeros(abi.TRI_BINS, np.int64)

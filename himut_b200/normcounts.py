@@ -25,10 +25,12 @@ def normcounts_region(ctx, bam_file, chrom, refseq, chunkloci_lst, chunk_sets, d
     decode: "device" inflates and parses each group on the GPU from the compressed file with the 2-bit base stream
     (Context.decode_region(..., seq=True)); "host" decodes with the native host decoder one group ahead of the device;
     "auto" takes the device decoder when the groups average at least DEVICE_DECODE_MIN_BYTES of compressed BAM.  Either
-    needs a context with the device decoder and a BAM with a BAI; without them the host decoder runs.
+    needs a context with the device decoder and a BAM with a BAI; without them the host decoder runs.  Records with
+    neither cs:Z nor MD:Z are decoded from CIGAR + refseq by either decoder.
     -> (ccs_tri[33], ref_tri[33], log[14], n_alt_tie, distinct query names that passed the read gates); log[0] is
     that count"""
     src = worker.RegionSource(bam_file)
+    src.reader.set_reference(chrom, refseq)
     tally = worker.QnameTally()
     ccs = np.zeros(abi.TRI_BINS, np.int64)
     ref = np.zeros(abi.TRI_BINS, np.int64)
@@ -37,9 +39,9 @@ def normcounts_region(ctx, bam_file, chrom, refseq, chunkloci_lst, chunk_sets, d
     groups = worker.group_chunks(chunkloci_lst)
     lo, hi = (min(s for _, s, _e in chunkloci_lst), max(e for _, _s, e in chunkloci_lst)) if chunkloci_lst else (None, None)
 
-    def add(table):
+    def add(table, seq=refseq):
         nonlocal ties
-        c, r, l, t = ctx.normcounts_chunks(refseq, table)
+        c, r, l, t = ctx.normcounts_chunks(seq, table)
         tally.add(ctx.qname_seen())
         ccs[:] += c; ref[:] += r; log[:] += l
         ties += t
@@ -49,10 +51,13 @@ def normcounts_region(ctx, bam_file, chrom, refseq, chunkloci_lst, chunk_sets, d
         if decode == "device":
             for idx in groups:
                 loci = [chunkloci_lst[i] for i in idx]
-                region = ctx.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci), seq=True)
+                # the contig is made resident once: the decoder and normcounts_chunks(None, ...) both read it
+                region = ctx.decode_region(src.reader, chrom, min(s for _, s, _e in loci), max(e for _, _s, e in loci), seq=True,
+                                           ref=refseq)
                 if region.n_reads == 0:
                     continue
-                add(region.chunk_table([(s, e) for _, s, e in loci], None if chunk_sets is None else [chunk_sets[i] for i in idx]))
+                add(region.chunk_table([(s, e) for _, s, e in loci], None if chunk_sets is None else [chunk_sets[i] for i in idx]),
+                    None)
         else:
             pins = worker.PinCache(ctx, enabled=len(groups) > 1)
             try:

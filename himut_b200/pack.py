@@ -10,6 +10,9 @@ introns, a cs tag whose spans disagree with the CIGAR-derived coordinates.
 parse_md gives the same ops from a CIGAR plus an MD:Z tag, for records without cs:Z (pbmm2 output,
 minimap2 without --cs; `samtools calmd` adds MD to any BAM).  The reference reads cs only and
 raises KeyError on such records; for the same alignment both tags give the same op stream.
+
+parse_ref gives the same ops from the CIGAR and the contig's reference sequence, for records with
+neither tag (what minimap2 writes without --cs or --MD, and what pbmm2 writes).
 """
 import re
 
@@ -41,6 +44,106 @@ MD_ERR = {
     "sub_n": "%s: substitution to a base outside A/C/G/T (the reference pileup raises KeyError) (%d)",
 }
 _M, _I, _D, _S, _H, _EQ, _X = 0, 1, 2, 4, 5, 7, 8
+# CIGAR + reference: the messages of the two checks only this path makes (csrc/bamerr.h); the others are MD_ERR's
+REF_ERR = {
+    "ref_end": "%s: alignment runs past the end of the reference sequence (%d)",
+    "ref_span": "%s: CIGAR and the reference sequence disagree at reference offset %d",
+}
+# reference bytes -> codes, case-insensitive; anything outside A/C/G/T (N, IUPAC codes) is BASE_N, as minimap2 writes it
+_REF_CODE = np.full(256, abi.BASE_N, np.uint8)
+for _b, _c in abi.BASE2CODE.items():
+    _REF_CODE[ord(_b)] = _c
+    _REF_CODE[ord(_b.lower())] = _c
+
+
+def _fail(key, qname, arg):
+    raise BatchFormatError((MD_ERR.get(key) or REF_ERR[key]) % (qname, arg))
+
+
+def _check_cigar(cigar, qseq, qname):
+    """the CIGAR checks parse_md and parse_ref share: N, P, codes past X and S / H between the first and the last
+    aligned op are unsupported; the CIGAR's query length must be len(qseq)"""
+    core = [i for i, (o, _l) in enumerate(cigar) if o not in (_S, _H)]
+    qcore = qclip = 0
+    for i, (o, l) in enumerate(cigar):
+        if o in (_S, _H):
+            if core and core[0] < i < core[-1]:
+                _fail("cigar_op", qname, i)
+            qclip += l if o == _S else 0
+        elif o in (_M, _I, _EQ, _X):
+            qcore += l
+        elif o != _D:
+            _fail("cigar_op", qname, i)
+    if qcore + qclip != len(qseq):
+        _fail("span_qry", qname, qcore)
+
+
+def parse_ref(cigar, refseq, tstart, qseq, qstart, qname="read"):
+    """CIGAR [(op, len), ...] (BAM op codes) + the contig's reference sequence -> (ops, ref_span, query_span), the ops
+    cs gives for the same alignment when the BAM agrees with its reference: one MATCH per maximal run of matched bases,
+    SUB(reference base, read base) per mismatch, INS / DEL with the CIGAR length.  refseq: the whole contig (bytes or
+    str), tstart the record's 0-based position; qseq the full read (soft clips included), qstart its leading soft clip.
+
+    Checked in this order, each failure the first one the walk meets:
+      - the CIGAR checks of parse_md (cigar_op, span_qry);
+      - the alignment must lie inside the reference: tstart + reference span <= len(refseq) (ref_end), before any
+        reference byte is read;
+      - the walk.  Reference bases are case-insensitive, anything outside A/C/G/T is N.  M: a read base equal to an
+        A/C/G/T reference base is matched, every other base is a SUB(reference base or N, read base), and a read base
+        outside A/C/G/T there is rejected (sub_n, as cs "*xn").  =: the read base must be A/C/G/T (n_match) and equal
+        to an A/C/G/T reference base (ref_span).  X: a read base outside A/C/G/T is rejected (sub_n), one equal to an
+        A/C/G/T reference base disagrees with the CIGAR (ref_span); every other base is a SUB.
+    A match run goes on across M / = / X and ends at a SUB, an I or a D; ops of length 0 are skipped.  Deleted
+    reference bases are not read."""
+    _check_cigar(cigar, qseq, qname)
+    rspan = sum(l for o, l in cigar if o in (_M, _D, _EQ, _X))
+    if tstart < 0 or tstart + rspan > len(refseq):
+        _fail("ref_end", qname, tstart + rspan)
+    rb = refseq.encode() if isinstance(refseq, str) else refseq
+    rcodes = _REF_CODE[np.frombuffer(rb, dtype=np.uint8, count=rspan, offset=tstart)] if rspan else np.zeros(0, np.uint8)
+    codes = _CODE[np.frombuffer(qseq.encode(), dtype=np.uint8)]
+    ops, run, q, r = [], 0, qstart, 0
+
+    def flush():
+        nonlocal run
+        if run:
+            ops.append(abi.make_op(abi.OP_MATCH, run))
+            run = 0
+
+    for o, l in cigar:
+        if l == 0 or o in (_S, _H):
+            continue
+        if o in (_M, _EQ, _X):
+            rc, ac = rcodes[r:r + l], codes[q:q + l]
+            match, bad = rc == ac, ac == 255  # rc is never 255: equal codes are A/C/G/T on both sides
+            if o == _M:
+                if bad.any():
+                    _fail("sub_n", qname, q + int(np.argmax(bad)))
+                subs = np.flatnonzero(~match)
+            else:
+                stop = (~match) if o == _EQ else (match | bad)
+                if stop.any():
+                    j = int(np.argmax(stop))
+                    _fail(("n_match" if o == _EQ else "sub_n") if bad[j] else "ref_span", qname, (q + j) if bad[j] else (r + j))
+                subs = np.arange(l) if o == _X else np.zeros(0, np.int64)
+            last = -1
+            for j in subs.tolist():
+                run += j - last - 1
+                flush()
+                ops.append(abi.make_sub(int(rc[j]), int(ac[j])))
+                last = j
+            run += l - last - 1
+            q += l; r += l
+        elif o == _I:
+            flush()
+            ops.append(abi.make_op(abi.OP_INS, l))
+            q += l
+        else:
+            flush()
+            ops.append(abi.make_op(abi.OP_DEL, l))
+            r += l
+    flush()
+    return ops, r, q - qstart
 
 
 def parse_md(cigar, md, qseq, qstart, qname="read"):
@@ -61,21 +164,9 @@ def parse_md(cigar, md, qseq, qstart, qname="read"):
         running out, or MD left at the end (a trailing 0 is fine) mean MD and CIGAR disagree.
     Ops of length 0 are skipped."""
     def fail(key, arg):
-        raise BatchFormatError(MD_ERR[key] % (qname, arg))
+        _fail(key, qname, arg)
 
-    core = [i for i, (o, _l) in enumerate(cigar) if o not in (_S, _H)]
-    qcore = qclip = 0
-    for i, (o, l) in enumerate(cigar):
-        if o in (_S, _H):
-            if core and core[0] < i < core[-1]:
-                fail("cigar_op", i)
-            qclip += l if o == _S else 0
-        elif o in (_M, _I, _EQ, _X):
-            qcore += l
-        elif o != _D:
-            fail("cigar_op", i)
-    if qcore + qclip != len(qseq):
-        fail("span_qry", qcore)
+    _check_cigar(cigar, qseq, qname)
     m = _MD_GRAMMAR.match(md)
     if m is None or m.end() != len(md):
         fail("md_token", m.end() if m else 0)
@@ -203,11 +294,15 @@ class BatchBuilder:
         self.seq_n = self.bq_n = self.ops_n = 0
         self.qnames = {}
 
-    def add(self, *, tstart, tend, qstart, qend, qseq, bq, mapq, is_secondary, qname, cs=None, ops=None, cigar=None, md=None):
-        """the record's ops come from `ops`, else from `cs`, else from `cigar` + `md` (parse_md)"""
+    def add(self, *, tstart, tend, qstart, qend, qseq, bq, mapq, is_secondary, qname, cs=None, ops=None, cigar=None, md=None,
+            refseq=None):
+        """the record's ops come from `ops`, else from `cs`, else from `cigar` + `md` (parse_md), else from `cigar` + the
+        contig's `refseq` (parse_ref)"""
         qb = qseq.encode() if isinstance(qseq, str) else bytes(qseq)
         if ops is None and cs is None and md is not None:
             ops, rspan, qspan = parse_md(cigar, md, qb.decode(), qstart, qname)
+        elif ops is None and cs is None and refseq is not None:
+            ops, rspan, qspan = parse_ref(cigar, refseq, tstart, qb.decode(), qstart, qname)
         elif ops is None:
             ops, rspan, qspan = parse_cs(cs, qb.decode(), qstart)
         else:

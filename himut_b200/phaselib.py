@@ -17,15 +17,18 @@ from . import caller, natsort_compat, worker
 BASE2CODE = {"A": 0, "T": 1, "G": 2, "C": 3}
 
 
-def edge_table(ctx, bam_file, chrom, hpos, href, min_bq, min_mapq, decode="auto"):
+def edge_table(ctx, bam_file, chrom, hpos, href, min_bq, min_mapq, decode="auto", refseq=None):
     """the pair tables of the hetSNPs (hpos, href) over the whole contig, decoded window by window (worker.GROUP_SPAN)
     -> uint32[n_hetsnp, band, 4] (Context.phase_edges_end).
     decode: "device" decodes each window on the GPU from the compressed file (Context.decode_region, no base stream);
     "host" with the native host decoder; "auto" takes the device decoder when the windows average at least
     caller.DEVICE_DECODE_MIN_BYTES of compressed BAM (the same no-seq decode that threshold was measured on).  Either
-    needs a context with the device decoder and a BAM with a BAI; without them the host decoder runs."""
+    needs a context with the device decoder and a BAM with a BAI; without them the host decoder runs.
+    refseq: the sequence of `chrom`, for records with neither cs:Z nor MD:Z (decoded from CIGAR + reference)."""
     src = worker.RegionSource(bam_file)
     try:
+        if refseq is not None:
+            src.reader.set_reference(chrom, refseq)
         length = src.reader.lengths[src.reader.references.index(chrom)]
         n_windows = -(-length // worker.GROUP_SPAN)
         decode = worker.choose_decode(decode, ctx, src.reader, chrom, 0 if length else None, length, n_windows,
@@ -37,7 +40,7 @@ def edge_table(ctx, bam_file, chrom, hpos, href, min_bq, min_mapq, decode="auto"
             while lo < length and not need:
                 hi = min(length, lo + worker.GROUP_SPAN)
                 if decode == "device":
-                    n_reads = ctx.decode_region(src.reader, chrom, lo, hi).n_reads
+                    n_reads = ctx.decode_region(src.reader, chrom, lo, hi, ref=refseq).n_reads
                 else:
                     batch, _ = src.batch(chrom, [(chrom, lo, hi)], seq=False)  # a cs match at a hetSNP carries its reference allele
                     n_reads = batch.n_reads
@@ -65,7 +68,7 @@ def get_edges(chrom, bam_file, min_bq, min_mapq, hpos_lst, hetsnp_lst, hetsnp2hi
         hpos = np.asarray(hpos_lst, np.int32)
         href = np.array([BASE2CODE.get(h[1], 4) for h in hetsnp_lst], np.uint8)
         hidx = np.array([hetsnp2hidx[h] for h in hetsnp_lst], np.int64)
-        table = edge_table(worker.context(), bam_file, chrom, hpos, href, min_bq, min_mapq)
+        table = edge_table(worker.context(), bam_file, chrom, hpos, href, min_bq, min_mapq, refseq=worker.env_reference(chrom))
         a_idx, d_idx = np.nonzero(table.any(axis=2))
         for a, d in zip(a_idx.tolist(), d_idx.tolist()):
             edge2counts[(int(hidx[a]), int(hidx[a + d + 1]))] += table[a, d].astype(np.float64)

@@ -4,7 +4,7 @@ import os
 
 import numpy as np
 
-from . import abi, bamdec, lib
+from . import abi, bamdec, fasta, lib
 
 _CTX = None
 _CTX_PID = None
@@ -50,6 +50,14 @@ def second_context():
 def _device_count():
     """visible CUDA devices, asked of the library itself (cudaGetDeviceCount): no torch import in a pool worker"""
     return max(1, lib.device_count())
+
+
+def env_reference(chrom):
+    """the sequence of `chrom` from the FASTA HIMUT_B200_REF names, for BAMs whose records carry neither cs:Z nor MD:Z
+    (the drop-in workers take no FASTA argument); None when the variable is unset, and then nothing is read.  Its
+    length is checked against the BAM's @SQ LN where the decoder takes it (bamdec.NativeBam.set_reference)."""
+    path = os.environ.get("HIMUT_B200_REF")
+    return fasta.load_contig(path, chrom) if path else None
 
 
 def group_chunks(chunkloci_lst, span=None):

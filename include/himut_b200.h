@@ -341,7 +341,9 @@ int hm_upload_batch_compact_begin(hm_ctx* ctx, const hm_read_batch* batch, const
 int hm_upload_wait(hm_ctx* ctx);
 
 /* keep a contig's reference sequence (the `seq` argument of get_callable_tricounts,
- * normcounts.py:208) resident on the device; hm_normcounts_chunks then accepts refseq = NULL */
+ * normcounts.py:208) resident on the device; hm_normcounts_chunks then accepts refseq = NULL, and
+ * hm_decode_bam_begin_opts(HM_DECODE_REF) decodes the contig's records without an alignment tag against it.
+ * hm_ref_tricounts and hm_normcounts_chunks with a refseq replace it (none resident afterwards). */
 int hm_set_reference(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len);
 
 /* callable-base half of `himut normcounts` over chunks of the resident batch (replaces the
@@ -402,13 +404,18 @@ int hm_read_stats(hm_ctx* ctx, int64_t* bq_total, int32_t* n_match, int32_t* n_s
  *   ISIZE checked), walks the records from the entry points, selects and parses them with hm_bam_read_batch's rules
  *   (file order, same messages for rejected input: HM_ERR_ARG) and brings back the query names and the per-read
  *   coordinates; *n_reads = the batch's reads.  `end` is clamped to the contig by the caller.  It decodes without the
- *   base stream; hm_decode_bam_begin_opts takes option bits (HM_DECODE_SEQ; others: HM_ERR_ARG).
+ *   base stream; hm_decode_bam_begin_opts takes option bits (HM_DECODE_SEQ, HM_DECODE_REF; others: HM_ERR_ARG).
  *   hm_decode_bam_names: views of those host arrays (valid until the next begin): NUL-terminated names at
  *   names + name_off[i], tstart / tend per read.
  *   hm_decode_bam_end takes the query-name ids (interned by the BAM handle: hm_bam_intern_qnames) and makes the batch
  *   resident; afterwards every call behaves as after hm_upload_batch of hm_bam_read_batch's batch without seq, or
  *   with HM_DECODE_SEQ of its batch with seq (one quality byte per base either way). */
 #define HM_DECODE_SEQ 1u /* hm_decode_bam_begin_opts: pack the 2-bit base stream too (seq / seq_off of hm_read_batch) */
+/* hm_decode_bam_begin_opts: records with neither cs:Z nor MD:Z are decoded from CIGAR + the reference sequence resident
+ * from hm_set_reference (which must be the contig `rid` names; none resident: HM_ERR_STATE), as hm_bam_read_batch does
+ * after hm_bam_set_reference, with its messages for rejected records.  Records with either tag never read it.  Without
+ * the bit such records are rejected ("no cs:Z tag"). */
+#define HM_DECODE_REF 2u
 int hm_decode_bam_begin(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint64_t* n_reads);
 int hm_decode_bam_begin_opts(hm_ctx* ctx, const hm_bgzf_plan* plan, int rid, int32_t start, int32_t end, uint32_t opts,
                              uint64_t* n_reads);

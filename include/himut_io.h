@@ -41,13 +41,23 @@ int hm_bam_ref_len(const hm_bam* b, int i);
  * order, each once (pysam fetch semantics, caller.py:299); secondary records (0x100) are
  * dropped as bamlib.BAM.__init__ drops them (bamlib.py:17), supplementary ones are kept.
  * A record's ops come from its cs:Z tag; a record without cs:Z but with MD:Z is decoded from CIGAR + MD
- * (pack.parse_md; the reference raises KeyError there), to the ops cs gives for the same alignment.
- * Inputs the reference would crash on are rejected with HM_ERR_ARG and a message: neither cs:Z nor MD:Z (worded
- * "no cs:Z tag"), missing qualities, a read base outside A/C/G/T under a match or as the substituted base, cs spans
+ * (pack.parse_md; the reference raises KeyError there), to the ops cs gives for the same alignment; a record with
+ * neither from CIGAR + the contig's sequence when hm_bam_set_reference gave it (pack.parse_ref).
+ * Inputs the reference would crash on are rejected with HM_ERR_ARG and a message: neither cs:Z nor MD:Z nor a
+ * reference sequence (worded "no cs:Z tag"), missing qualities, a read base outside A/C/G/T under a match or as the substituted base, cs spans
  * that disagree with the CIGAR, an MD:Z outside its grammar or disagreeing with the CIGAR, CIGAR ops N and P and
  * clips inside the alignment (MD path), records whose fields run past their block_size.  Hard-clipped records are decoded as pysam
  * presents them (SEQ holds no hard-clipped base; lead / trail count soft clips only).  `threads` = inflate threads. */
 int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int threads, hm_read_batch* out);
+
+/* the reference sequence of contig `rid` (ASCII, either case), for its records with neither cs:Z nor MD:Z: from then
+ * on hm_bam_read_batch decodes them from CIGAR + reference (pack.parse_ref) to the ops cs gives for the same alignment
+ * when the BAM agrees with its reference.  Reference bases outside A/C/G/T are N.  Rejected there with HM_ERR_ARG and a
+ * message: an alignment that runs past the end of the sequence, "=" over a mismatch and "X" over a match, a read base
+ * outside A/C/G/T under M / = / X, CIGAR ops N and P and clips inside the alignment.  Records of other contigs and
+ * records with either tag never read it.  The handle keeps the pointer, not a copy: the buffer must stay valid until
+ * the next call or hm_bam_close.  len must be the contig's @SQ LN (else HM_ERR_ARG); seq NULL clears it. */
+int hm_bam_set_reference(hm_bam* b, int rid, const uint8_t* seq, size_t len);
 
 /* HM_BAM_OPT_NO_SEQ = 1: batches come without the 2-bit base stream (seq = NULL, seq_off = NULL, seq_bytes = 0; see
  * hm_read_batch in himut_b200.h) — `call` and the phase edges do not need it; every check on the bases (A/C/G/T under
@@ -84,6 +94,10 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
 #define HM_BAM_TAGS_CS 0
 #define HM_BAM_TAGS_MD 1
 #define HM_BAM_TAGS_MD_EQX 2
+/* HM_BAM_TAGS_EQX writes the CIGAR of =/X and no alignment tag, HM_BAM_TAGS_M a CIGAR of M and no alignment tag: what
+ * aligners write without --cs or --MD; they decode with the contig's sequence (hm_bam_set_reference) */
+#define HM_BAM_TAGS_EQX 3
+#define HM_BAM_TAGS_M 4
 int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                             int level, int threads, int tags);
 

@@ -8,7 +8,9 @@ power limit are read in the same run.
 --seq: the same for normcounts, which decodes with the 2-bit base stream: host read_batch(seq=True, compact=True) against
 decode_region(seq=True), with the device decode without seq timed beside it (k_bam_parse with and without the base
 stream), then the normcounts worker's BAM -> tri counts with decode="host", "device" and "auto", whose outputs must agree.
---tags md | md_eqx: the BAMs carry CIGAR + MD:Z instead of cs:Z (the decoders' MD path).
+--tags md | md_eqx: the BAMs carry CIGAR + MD:Z instead of cs:Z (the decoders' MD path); eqx | m: the =/X or M CIGAR
+and neither tag, decoded with the synthetic contig (written next to the BAM as a FASTA) by both decoders (the CIGAR +
+reference path).  A comma-separated list (with --group) writes one BAM per form and alternates them region by region.
 --group S: only the decode group [S, S + GROUP_SPAN) of the 64 Mb contig, no worker runs (A/B of the decode kernels).
     python tools/decode_trace.py [--reps 3] [--seq] [--tags cs] [--group S] [--out profiles/decode_trace_r03.json | decode_trace_norm_r04.json]"""
 import argparse
@@ -25,26 +27,33 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 ap = argparse.ArgumentParser()
 ap.add_argument("--reps", type=int, default=3)
 ap.add_argument("--seq", action="store_true", help="decode with the base stream and time the normcounts worker")
-ap.add_argument("--tags", default="cs", choices=["cs", "md", "md_eqx"], help="the alignment tag the BAMs are written with")
+ap.add_argument("--tags", default="cs", help="the alignment form(s) the BAMs are written with: cs, md, md_eqx, eqx, m")
 ap.add_argument("--group", type=int, default=None, help="time only the decode group starting here, on the 64 Mb contig")
 ap.add_argument("--out", default=None)
 a = ap.parse_args()
+TAGS = a.tags.split(",")
+if any(t not in ("cs", "md", "md_eqx", "eqx", "m") for t in TAGS) or (len(TAGS) > 1 and a.group is None):
+    ap.error("--tags: cs, md, md_eqx, eqx or m; several only with --group")
+BY_REF = ("eqx", "m")
 if a.out is None:
     a.out = os.path.join(ROOT, "profiles", "decode_trace_norm_r04.json" if a.seq else "decode_trace_r03.json")
 
 import cases  # noqa: E402
-from himut_b200 import bamdec, caller, gtmodel, lib, normcounts, synth, worker  # noqa: E402
+from himut_b200 import bamdec, caller, fasta, gtmodel, lib, normcounts, synth, worker  # noqa: E402
 
 card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv"], stdout=subprocess.PIPE, text=True).stdout
 tmp = tempfile.mkdtemp()
-inputs, refs = {}, {}
+inputs, refs, forms = {}, {}, {}
 for label, n, seed in (("64mb", 64_000_000, 5), ("1mb", 1_000_000, None))[:1 if a.group is not None else 2]:
     d = synth.generate(n, **({"seed": seed} if seed is not None else {}), copy=False)
-    path = os.path.join(tmp, label + ".bam")
-    bamdec.write_batch_bam(path, "chr1", n, d.batch, **({"tags": a.tags} if a.tags != "cs" else {}))
-    inputs[label] = (path, n, os.path.getsize(path))
-    if a.seq:
+    for tags in TAGS:
+        path = os.path.join(tmp, "%s_%s.bam" % (label, tags))
+        bamdec.write_batch_bam(path, "chr1", n, d.batch, **({"tags": tags} if tags != "cs" else {}))
+        forms[path] = tags
+        inputs.setdefault(label, []).append((path, n, os.path.getsize(path)))
         refs[path] = bytes(d.ref)
+    if set(TAGS) & set(BY_REF):
+        fasta.write_fasta(os.path.join(tmp, label + ".fa"), [("chr1", d.ref)])
     del d
 G = worker.GROUP_SPAN
 
@@ -57,15 +66,22 @@ def groups(n):
     return g + [(0, L) for L in (1_000_000, 2_000_000, 4_000_000, 8_000_000) if L < n]
 
 
+def open_bam(path):
+    nb = bamdec.NativeBam(path)
+    if forms[path] in BY_REF:
+        nb.set_reference("chr1", refs[path])
+    return nb
+
+
 def host_decode(nb, s, e, seq=False):
     t0 = time.perf_counter()
     b, _cq = nb.read_batch("chr1", s, e, copy=False, seq=seq, compact=True)
     return time.perf_counter() - t0, b.n_reads
 
 
-def device_decode(ctx, nb, s, e, seq=False):
+def device_decode(ctx, nb, s, e, seq=False, ref=None):
     t0 = time.perf_counter()
-    r = ctx.decode_region(nb, "chr1", s, e, seq=seq)
+    r = ctx.decode_region(nb, "chr1", s, e, seq=seq, ref=ref)
     wall = time.perf_counter() - t0
     ab = ctx.read_back().aligned_bases
     return wall, r.n_reads, dict(ctx.last_decode_times), ab
@@ -106,38 +122,45 @@ def norm_worker_run(path, n, mode):
         normcounts.normcounts_region = real
 
 
-out = {"card": card.strip(), "tags": a.tags, "group_span": G, "threads_host_decoder": bamdec.default_threads(), "inputs": {}, "decode": [], "worker": []}
+out = {"card": card.strip(), "tags": TAGS, "group_span": G, "threads_host_decoder": bamdec.default_threads(), "inputs": {}, "decode": [], "worker": []}
 if a.seq:
     out["seq"] = True
     out["device_decode_min_bytes"] = {"call": caller.DEVICE_DECODE_MIN_BYTES, "normcounts": normcounts.DEVICE_DECODE_MIN_BYTES}
 ctx = lib.Context(0)
-for label, (path, n, size) in inputs.items():
-    out["inputs"][label] = {"contig_len": n, "bam_bytes": size}
-    nb = bamdec.NativeBam(path)
-    for s, e in groups(n):  # warm-up of every shape (module load, allocations)
-        host_decode(nb, s, e, a.seq)
-        device_decode(ctx, nb, s, e, a.seq)
-        if a.seq:
-            device_decode(ctx, nb, s, e)
+for label, files in inputs.items():
+    out["inputs"][label] = {"contig_len": files[0][1], "bam_bytes": {forms[p]: size for p, _n, size in files}}
+    nbs = [(open_bam(p), forms[p], refs[p] if forms[p] in BY_REF else None) for p, _n, _size in files]
+    n = files[0][1]
+    for s, e in groups(n):  # warm-up of every shape and form (module load, allocations)
+        for nb, _tags, ref in nbs:
+            host_decode(nb, s, e, a.seq)
+            device_decode(ctx, nb, s, e, a.seq, ref)
+            if a.seq:
+                device_decode(ctx, nb, s, e, ref=ref)
     for rep in range(a.reps):
         for s, e in groups(n):
-            th, nh = host_decode(nb, s, e, a.seq)
-            td, nd, kt, ab = device_decode(ctx, nb, s, e, a.seq)
-            assert nh == nd
-            pl = nb.plan("chr1", s, e)
-            row = {"input": label, "rep": rep, "start": s, "end": e, "reads": nd, "aligned_bases": ab,
-                   "compressed_bytes": int(pl.comp_bytes), "host_s": th, "device_s": td, "device_ms": kt,
-                   "host_bases_per_s": ab / th, "device_bases_per_s": ab / td}
-            if a.seq:  # the same region without the base stream, right after: k_bam_parse with and without it
-                row["device_noseq_s"], _, row["device_noseq_ms"], _ = device_decode(ctx, nb, s, e)
-            out["decode"].append(row)
-            print("%s [%d, %d) %.0f MB rep %d: host %.1f ms, device %.1f ms %s" % (label, s, e, pl.comp_bytes / 1e6, rep, th * 1e3,
-                                                                                     td * 1e3, {k: round(v, 2) for k, v in kt.items()}),
-                  file=sys.stderr)
-    nb.close()
+            for nb, tags, ref in nbs:  # the forms alternate: their spread is measured on the same conditions
+                th, nh = host_decode(nb, s, e, a.seq)
+                td, nd, kt, ab = device_decode(ctx, nb, s, e, a.seq, ref)
+                assert nh == nd
+                pl = nb.plan("chr1", s, e)
+                row = {"input": label, "tags": tags, "rep": rep, "start": s, "end": e, "reads": nd, "aligned_bases": ab,
+                       "compressed_bytes": int(pl.comp_bytes), "host_s": th, "device_s": td, "device_ms": kt,
+                       "host_bases_per_s": ab / th, "device_bases_per_s": ab / td}
+                if a.seq:  # the same region without the base stream, right after: k_bam_parse with and without it
+                    row["device_noseq_s"], _, row["device_noseq_ms"], _ = device_decode(ctx, nb, s, e, ref=ref)
+                out["decode"].append(row)
+                print("%s %s [%d, %d) %.0f MB rep %d: host %.1f ms, device %.1f ms %s" % (
+                    label, tags, s, e, pl.comp_bytes / 1e6, rep, th * 1e3, td * 1e3, {k: round(v, 2) for k, v in kt.items()}),
+                    file=sys.stderr)
+    for nb, _tags, _ref in nbs:
+        nb.close()
     if a.group is not None:
         continue
-    nb = bamdec.NativeBam(path)
+    path = files[0][0]
+    if forms[path] in BY_REF:  # the call worker reads its FASTA from the environment
+        os.environ["HIMUT_B200_REF"] = os.path.join(tmp, label + ".fa")
+    nb = open_bam(path)
     whole_bases = nb.read_batch("chr1", 0, n, seq=False).aligned_bases
     nb.close()
     run = norm_worker_run if a.seq else worker_run
