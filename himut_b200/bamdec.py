@@ -16,8 +16,8 @@ from . import abi, bamio, pack
 
 _LIB = None
 EXPORTS = ["hm_bam_open", "hm_bam_close", "hm_bam_error", "hm_bam_header_text", "hm_bam_n_refs", "hm_bam_ref_name",
-           "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bam_write_batch_tags", "hm_bq_compact_build",
-           "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames", "hm_bam_set_reference"]
+           "hm_bam_ref_len", "hm_bam_read_batch", "hm_bam_set_option", "hm_bam_last_compact", "hm_bam_qnames_blob", "hm_bam_n_qnames", "hm_bam_qname", "hm_bam_window_qlens", "hm_bam_write_batch", "hm_bam_write_batch_tags", "hm_bam_write_batch_index", "hm_bq_compact_build",
+           "hm_bq_compact_free", "hm_bam_region_plan", "hm_bam_intern_qnames", "hm_bam_set_reference", "hm_bam_index_kind"]
 
 
 def lib_path():
@@ -49,6 +49,8 @@ def load():
         lib.hm_bam_window_qlens.argtypes = [vp, C.c_int, C.c_int32, C.c_int32, C.c_int, vp, C.c_size_t, C.POINTER(C.c_size_t)]
         lib.hm_bam_write_batch.argtypes = [C.c_char_p, C.c_char_p, C.c_int32, C.c_char_p, C.POINTER(abi.hm_read_batch), C.c_int, C.c_int]
         lib.hm_bam_write_batch_tags.argtypes = lib.hm_bam_write_batch.argtypes + [C.c_int]
+        lib.hm_bam_write_batch_index.argtypes = lib.hm_bam_write_batch_tags.argtypes + [C.c_int, C.c_int]
+        lib.hm_bam_index_kind.argtypes = [vp]
         lib.hm_bq_compact_build.argtypes = [C.POINTER(abi.hm_read_batch), C.c_int, vp, vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint8)]
         lib.hm_bq_compact_free.argtypes = [vp]
         lib.hm_bq_compact_free.restype = None
@@ -82,12 +84,19 @@ def _view(ptr, n, dtype):
     return np.frombuffer(buf, dtype=dt, count=n)
 
 
-def write_batch_bam(path, chrom, contig_len, batch, sample="synth", level=1, threads=None, tags="cs"):
-    """ReadBatch -> coordinate-sorted BAM + BAI, natively (same content as bamio.write_batch_bam, tags alike)"""
+def write_batch_bam(path, chrom, contig_len, batch, sample="synth", level=1, threads=None, tags="cs", index="bai", min_shift=14,
+                    depth=None):
+    """ReadBatch -> coordinate-sorted BAM + BAI, natively (same content as bamio.write_batch_bam, tags alike).
+    index="csi" writes <path>.csi instead, with min_shift and depth (None: the smallest that holds the contig)."""
     if tags not in bamio.TAGS:
         raise ValueError("tags must be one of %s" % (bamio.TAGS,))
-    rc = load().hm_bam_write_batch_tags(os.fsencode(path), chrom.encode(), int(contig_len), sample.encode(), C.byref(batch.as_struct()),
-                                        int(level), int(threads or default_threads()), bamio.TAGS.index(tags))
+    if index not in ("bai", "csi"):
+        raise ValueError("index must be 'bai' or 'csi'")
+    if index == "bai" and contig_len > bamio.BAI_MAX_LEN:
+        raise ValueError("a BAI cannot index a contig longer than 2^29 (%d): use index='csi'" % contig_len)
+    rc = load().hm_bam_write_batch_index(os.fsencode(path), chrom.encode(), int(contig_len), sample.encode(), C.byref(batch.as_struct()),
+                                         int(level), int(threads or default_threads()), bamio.TAGS.index(tags),
+                                         int(min_shift) if index == "csi" else 0, int(depth or 0))
     if rc != 0:
         raise IOError("cannot write %s" % path)
 
@@ -110,20 +119,27 @@ def compact_bq(batch, threads=None):
     return abi.BqCompact(mask, exc, exc_off, int(modal.value), n)
 
 
+def _pos32(pos):
+    """a region bound as the C ABI's int32: past 2^31 - 1 (the longest contig a BAM holds) it reads as the contig's end"""
+    return int(min(pos, 2**31 - 1))
+
+
 class NativeBam:
-    """one open BAM (+ .bai); read_batch() returns an abi.ReadBatch copied out of the handle"""
+    """one open BAM (+ its BAI or CSI); read_batch() returns an abi.ReadBatch copied out of the handle"""
 
     def __init__(self, path, threads=None):
         self.lib = load()
         self.h = C.c_void_p()
         rc = self.lib.hm_bam_open(os.fsencode(path), C.byref(self.h))
         if rc != 0:
-            raise IOError("cannot open %s as BAM" % path)
+            why = self.lib.hm_bam_error(None)
+            raise IOError("cannot open %s as BAM%s" % (path, ": " + why.decode() if why else ""))
         self.threads = threads or default_threads()
         self.references = [self.lib.hm_bam_ref_name(self.h, i).decode() for i in range(self.lib.hm_bam_n_refs(self.h))]
         self.lengths = [self.lib.hm_bam_ref_len(self.h, i) for i in range(len(self.references))]
         self.header_text = self.lib.hm_bam_header_text(self.h).decode()
-        self.has_index = os.path.exists(os.fsencode(path) + b".bai")
+        self.index_kind = ("none", "bai", "csi")[self.lib.hm_bam_index_kind(self.h)]
+        self.has_index = self.index_kind != "none"
 
     def read_batch(self, chrom, start, end, copy=True, seq=True, compact=False, buffer_set=0):
         """seq=False: the batch comes without its 2-bit base stream (HM_BAM_OPT_NO_SEQ), as `call` and the phase
@@ -139,7 +155,7 @@ class NativeBam:
             if self.lib.hm_bam_set_option(self.h, opt, val) != 0:
                 raise RuntimeError(self.lib.hm_bam_error(self.h).decode())
         s = abi.hm_read_batch()
-        rc = self.lib.hm_bam_read_batch(self.h, self.references.index(chrom), int(max(start, 0)), int(end), self.threads, C.byref(s))
+        rc = self.lib.hm_bam_read_batch(self.h, self.references.index(chrom), _pos32(max(start, 0)), _pos32(end), self.threads, C.byref(s))
         if rc != 0:
             raise pack.BatchFormatError(self.lib.hm_bam_error(self.h).decode())
         n = int(s.n_reads)
@@ -176,11 +192,11 @@ class NativeBam:
 
     def plan(self, chrom, start, end):
         """abi.hm_bgzf_plan of the records read_batch(chrom, start, end) visits, for Context.decode_region: the
-        compressed blocks and the record starts the BAI knows, nothing inflated.  Valid until the next plan()."""
+        compressed blocks and the record starts the index knows, nothing inflated.  Valid until the next plan()."""
         if chrom not in self.references:
             raise KeyError(chrom)
         p = abi.hm_bgzf_plan()
-        if self.lib.hm_bam_region_plan(self.h, self.references.index(chrom), int(max(start, 0)), int(end), C.byref(p)) != 0:
+        if self.lib.hm_bam_region_plan(self.h, self.references.index(chrom), _pos32(max(start, 0)), _pos32(end), C.byref(p)) != 0:
             raise pack.BatchFormatError(self.lib.hm_bam_error(self.h).decode())
         return p
 
@@ -201,7 +217,7 @@ class NativeBam:
         while True:
             out = np.empty(cap, np.int32)
             n = C.c_size_t(0)
-            rc = self.lib.hm_bam_window_qlens(self.h, rid, int(max(start, 0)), int(end), self.threads, out.ctypes.data_as(C.c_void_p), cap, C.byref(n))
+            rc = self.lib.hm_bam_window_qlens(self.h, rid, _pos32(max(start, 0)), _pos32(end), self.threads, out.ctypes.data_as(C.c_void_p), cap, C.byref(n))
             if rc == 3:  # HM_ERR_CAPACITY
                 cap = int(n.value)
                 continue

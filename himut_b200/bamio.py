@@ -1,4 +1,4 @@
-"""Minimal BAM / BGZF / BAI reader and writer (pure Python + zlib).
+"""Minimal BAM / BGZF / BAI / CSI reader and writer (pure Python + zlib).
 
 pysam / htslib are not available in this image (SURVEY.md §0.4), and the worker mirrors need the
 records of a region as a packed ReadBatch rather than as Python objects anyway.  The reader
@@ -8,8 +8,11 @@ secondary / supplementary included — and the per-record fields reference_start
 query_alignment_start/end, query_sequence, query_qualities, mapping_quality, flag, cs:Z, tp:A, and
 beyond it the CIGAR and MD:Z (records without cs:Z are decoded from CIGAR + MD, pack.parse_md, and records with
 neither tag from CIGAR + the contig's reference sequence when the caller gives it, pack.parse_ref).
-The writer exists for tests and for the synthetic-data tools (coordinate-sorted BAM + .bai).
+The reader seeks with the first index it finds of <bam>.bai, <bam>.csi, <stem>.bai and <stem>.csi (the names htslib
+finds).  The writer exists for tests and for the synthetic-data tools (coordinate-sorted BAM + .bai or .csi).
 """
+import io
+import os
 import struct
 import zlib
 
@@ -24,6 +27,9 @@ _NIB2CODE[1], _NIB2CODE[2], _NIB2CODE[4], _NIB2CODE[8] = 0, 3, 2, 1
 _CIGAR_REF = (1, 0, 1, 1, 0, 0, 0, 1, 1)    # M I D N S H P = X consume reference?
 _CIGAR_QRY = (1, 1, 0, 0, 1, 0, 0, 1, 1)    # ... consume query?
 _BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+BAI_MAX_LEN = 1 << 29  # the BAI binning scheme ends there: a longer contig can only be indexed with a CSI
 
 
 class BamError(IOError):
@@ -217,7 +223,12 @@ class BamReader:
             self.references.append(self.bg.read(l_name)[:-1].decode())
             self.lengths.append(struct.unpack("<i", self.bg.read(4))[0])
         self.first_record = self.bg.tell()
-        self.index = _load_bai(path + ".bai", n_ref)
+        self.index_kind, self.index = "none", None
+        for ip, kind in index_paths(path):
+            if os.path.exists(ip):
+                self.index_kind = kind
+                self.index = _load_bai(ip, n_ref) if kind == "bai" else _load_csi(ip, self.references, self.lengths, path)
+                break
 
     def close(self):
         self.bg.close()
@@ -231,6 +242,22 @@ class BamReader:
             size = struct.unpack("<i", head)[0]
             yield _parse_record(self.bg.read(size))
 
+    def seek_offset(self, rid, pos):
+        """the virtual offset a fetch from pos of contig rid reads from; None: the index knows no record of the contig"""
+        if self.index is None:
+            return self.first_record
+        if self.index_kind == "csi":
+            return self.index.seek(rid, pos)
+        lin = self.index[rid]
+        if lin is None:
+            return None
+        w = min(pos >> 14, len(lin) - 1) if len(lin) else -1
+        voff = None
+        while w >= 0 and voff is None:   # windows nothing overlaps have offset 0
+            voff = lin[w] or None
+            w -= 1
+        return self.first_record if voff is None else voff
+
     def fetch(self, chrom=None, start=None, end=None):
         """records overlapping [start, end) of chrom in file order (whole contig when start is None)"""
         if chrom is None:
@@ -241,18 +268,9 @@ class BamReader:
         rid = self.references.index(chrom)
         lo = 0 if start is None else max(int(start), 0)
         hi = self.lengths[rid] if end is None else int(end)
-        voff = self.first_record
-        if self.index is not None:
-            lin = self.index[rid]
-            if lin is None:
-                return
-            w = min(lo >> 14, len(lin) - 1) if len(lin) else -1
-            voff = None
-            while w >= 0 and voff is None:   # windows nothing overlaps have offset 0
-                voff = lin[w] or None
-                w -= 1
-            if voff is None:
-                voff = self.first_record
+        voff = self.seek_offset(rid, lo)
+        if voff is None:
+            return
         for r in self._records_from(voff):
             if r.ref_id != rid:
                 if r.ref_id > rid or r.ref_id < 0:
@@ -294,6 +312,135 @@ def _load_bai(path, n_ref):
     return out
 
 
+def index_paths(path):
+    """[(index path, "bai" | "csi"), ...] in the order the readers look for them"""
+    out = [(path + ".bai", "bai"), (path + ".csi", "csi")]
+    if len(path) > 4 and path.endswith(".bam"):
+        out += [(path[:-4] + ".bai", "bai"), (path[:-4] + ".csi", "csi")]
+    return out
+
+
+def _bin_first(level):
+    return ((1 << (3 * level)) - 1) // 7
+
+
+def _bin_level(b):
+    lv = 0
+    while b >= _bin_first(lv + 1):
+        lv += 1
+    return lv
+
+
+def bin_start(b, min_shift=14, depth=5):
+    """first reference position of bin b of the (min_shift, depth) binning scheme (SAM spec 5.3)"""
+    lv = _bin_level(b)
+    return (b - _bin_first(lv)) << (min_shift + 3 * (depth - lv))
+
+
+def pseudo_bin(depth):
+    return _bin_first(depth + 1) + 1
+
+
+class CsiIndex:
+    """a parsed CSI: min_shift, depth and per reference {bin: (loffset, [(beg, end), ...])} (None: no bins), the
+    pseudo-bin and bins without chunks left out"""
+
+    def __init__(self, min_shift, depth, refs):
+        self.min_shift, self.depth, self.refs = min_shift, depth, refs
+
+    def seek(self, rid, pos):
+        """htslib's hts_itr_query: the loffset of the leaf bin that holds pos, else of its nearest left sibling, else of
+        its parent, and so on up; without one, the contig's first chunk.  None: no record of the contig."""
+        bins = self.refs[rid] if rid < len(self.refs) else None
+        if not bins:
+            return None
+        top = (1 << (self.min_shift + 3 * self.depth)) - 1
+        b = _bin_first(self.depth) + (min(pos, top) >> self.min_shift)
+        while True:
+            if b in bins and bins[b][0]:
+                return bins[b][0]
+            if b == 0:
+                break
+            first = (((b - 1) >> 3) << 3) + 1
+            b = b - 1 if b > first else (b - 1) >> 3
+        return min(c[0] for _l, ch in bins.values() for c in ch)
+
+
+def _load_csi(path, names, lengths, bam_path):
+    """-> CsiIndex; BamError naming the file for anything that cannot be read"""
+    def bad(why):
+        return BamError("%s: %s" % (path, why))
+    raw = open(path, "rb").read()
+    f, data = io.BytesIO(raw), []
+    try:
+        while True:
+            at = f.tell()
+            size, payload = _read_block(f)
+            if size == 0:
+                break
+            if len(raw) < at + size or struct.unpack_from("<II", raw, at + size - 8) != (zlib.crc32(payload), len(payload)):
+                raise BamError("bad block")
+            data.append(payload)
+    except (BamError, struct.error, zlib.error) as e:
+        raise BamError("%s is not a BGZF-compressed CSI index (%s)" % (path, e))
+    data = b"".join(data)
+    bam_size = os.path.getsize(bam_path)
+    if len(data) < 16 or data[:4] != b"CSI\x01":
+        raise BamError("%s is not a CSI index" % path)
+    min_shift, depth, l_aux = struct.unpack_from("<iii", data, 4)
+    if min_shift < 1 or depth < 0 or depth > 10 or min_shift + 3 * depth > 62:
+        raise bad("unsupported min_shift %d / depth %d" % (min_shift, depth))
+    for name, ln in zip(names, lengths):
+        if ln > 1 << (min_shift + 3 * depth):
+            raise bad("min_shift %d and depth %d cover %d positions, %s has %d" % (min_shift, depth, 1 << (min_shift + 3 * depth), name, ln))
+    p = 16 + l_aux
+    if l_aux < 0 or p + 4 > len(data):
+        raise bad("l_aux %d runs past the end of the index" % l_aux)
+    pseudo = pseudo_bin(depth)
+
+    def take(fmt, what):
+        nonlocal p
+        if p + struct.calcsize(fmt) > len(data):
+            raise bad("truncated at byte %d (%s)" % (p, what))
+        v = struct.unpack_from(fmt, data, p)
+        p += struct.calcsize(fmt)
+        return v
+
+    n_ref, = take("<i", "n_ref")
+    if n_ref < 0:
+        raise bad("n_ref %d" % n_ref)
+    refs = []
+    for _ in range(n_ref):
+        n_bin, = take("<i", "n_bin")
+        if n_bin < 0 or n_bin * 16 > len(data) - p:
+            raise bad("n_bin %d runs past the end of the index" % n_bin)
+        bins = {}
+        for _b in range(n_bin):
+            b, loff, n_chunk = take("<IQi", "bin")
+            if b > pseudo or b == pseudo - 1:  # pseudo - 1 is past the last level
+                raise bad("bin %d past the pseudo-bin %d" % (b, pseudo))
+            if b != pseudo and loff >> 16 >= bam_size:
+                raise bad("loffset of bin %d points past the end of the BAM" % b)
+            if n_chunk < 0 or n_chunk * 16 > len(data) - p:
+                raise bad("n_chunk %d of bin %d runs past the end of the index" % (n_chunk, b))
+            chunks = [struct.unpack_from("<QQ", data, p + 16 * c) for c in range(n_chunk)]
+            p += 16 * n_chunk
+            if b == pseudo:
+                continue
+            for c, (beg, end) in enumerate(chunks):
+                if beg > end:
+                    raise bad("chunk %d of bin %d begins after its end" % (c, b))
+                if beg >> 16 >= bam_size:
+                    raise bad("chunk %d of bin %d points past the end of the BAM" % (c, b))
+            if chunks:
+                loff0, ch0 = bins.get(b, (loff, []))
+                bins[b] = (loff0, ch0 + chunks)
+        refs.append(bins or None)
+    while len(refs) < len(names):
+        refs.append(None)
+    return CsiIndex(min_shift, depth, refs)
+
+
 # ------------------------------------------------------------------------------ region -> batch
 def read_batch(reader, chrom, start, end, builder=None, refseq=None):
     """all records of `chrom` overlapping [start, end), packed (each record once, file order).
@@ -322,26 +469,48 @@ def read_batch(reader, chrom, start, end, builder=None, refseq=None):
 
 
 # ------------------------------------------------------------------------------ writer
-def _reg2bin(beg, end):
+def _reg2bin(beg, end, min_shift=14, depth=5):
+    """the smallest bin of the (min_shift, depth) scheme that holds [beg, end) (htslib's hts_reg2bin)"""
     end -= 1
-    if beg >> 14 == end >> 14:
-        return ((1 << 15) - 1) // 7 + (beg >> 14)
-    if beg >> 17 == end >> 17:
-        return ((1 << 12) - 1) // 7 + (beg >> 17)
-    if beg >> 20 == end >> 20:
-        return ((1 << 9) - 1) // 7 + (beg >> 20)
-    if beg >> 23 == end >> 23:
-        return ((1 << 6) - 1) // 7 + (beg >> 23)
-    if beg >> 26 == end >> 26:
-        return ((1 << 3) - 1) // 7 + (beg >> 26)
+    sh = min_shift
+    for lv in range(depth, 0, -1):
+        if beg >> sh == end >> sh:
+            return _bin_first(lv) + (beg >> sh)
+        sh += 3
     return 0
 
 
-class BamWriter:
-    """coordinate-sorted BAM + BAI writer; records must be added in sorted order"""
+def default_depth(lengths, min_shift=14):
+    """htslib's choice of CSI depth: the smallest whose span holds the longest contig plus 256"""
+    need, depth = max(lengths, default=0) + 256, 0
+    while (1 << (min_shift + 3 * depth)) < need:
+        depth += 1
+    return depth
 
-    def __init__(self, path, references, header_extra="@RG\tID:rg\tSM:synth\n", level=1):
+
+def _bgzf_block(chunk, level):
+    c = zlib.compressobj(level, zlib.DEFLATED, -15)
+    comp = c.compress(chunk) + c.flush()
+    return (b"\x1f\x8b\x08\x04\0\0\0\0\0\xff\x06\0BC\x02\0" + struct.pack("<H", len(comp) + 25)
+            + comp + struct.pack("<II", zlib.crc32(chunk), len(chunk)))
+
+
+class BamWriter:
+    """coordinate-sorted BAM + index writer; records must be added in sorted order.  index="bai" writes <path>.bai
+    (refused for a contig longer than 2^29); index="csi" writes <path>.csi as htslib writes it, with min_shift and
+    depth (None: default_depth)."""
+
+    def __init__(self, path, references, header_extra="@RG\tID:rg\tSM:synth\n", level=1, index="bai", min_shift=14, depth=None):
         self.path, self.refs, self.level = path, list(references), level
+        if index not in ("bai", "csi"):
+            raise ValueError("index must be 'bai' or 'csi'")
+        if index == "bai" and any(ln > BAI_MAX_LEN for _n, ln in self.refs):
+            raise ValueError("a BAI cannot index a contig longer than 2^29: use index='csi'")
+        self.index = index
+        self.min_shift = min_shift if index == "csi" else 14
+        self.depth = 5 if index == "bai" else (default_depth([ln for _n, ln in self.refs], min_shift) if depth is None else depth)
+        if (1 << (self.min_shift + 3 * self.depth)) < max([ln for _n, ln in self.refs], default=0):
+            raise ValueError("min_shift %d and depth %d do not cover the longest contig" % (self.min_shift, self.depth))
         self.f = open(path, "wb")
         self.coff = 0
         self.buf = bytearray()
@@ -353,12 +522,10 @@ class BamWriter:
         self._flush()
         self.bins = [dict() for _ in self.refs]
         self.lin = [[] for _ in self.refs]
+        self.n_mapped = [0] * len(self.refs)
 
     def _emit_block(self, chunk):
-        c = zlib.compressobj(self.level, zlib.DEFLATED, -15)
-        comp = c.compress(chunk) + c.flush()
-        block = (b"\x1f\x8b\x08\x04\0\0\0\0\0\xff\x06\0BC\x02\0" + struct.pack("<H", len(comp) + 25)
-                 + comp + struct.pack("<II", zlib.crc32(chunk), len(chunk)))
+        block = _bgzf_block(chunk, self.level)
         self.f.write(block)
         self.coff += len(block)
 
@@ -383,7 +550,8 @@ class BamWriter:
         if l_seq % 2:
             codes = np.concatenate([codes, np.zeros(1, np.uint8)])
         packed = ((codes[0::2] << 4) | codes[1::2]).astype(np.uint8).tobytes()
-        body = struct.pack("<iiBBHHHiiii", ref_id, pos, len(qname) + 1, mapq, _reg2bin(pos, end), len(cigar), flag, l_seq, -1, -1, 0)
+        bai_bin = _reg2bin(pos, end) if end - 1 < BAI_MAX_LEN else 4680  # no decoder here reads it: past 2^29 it cannot be right
+        body = struct.pack("<iiBBHHHiiii", ref_id, pos, len(qname) + 1, mapq, bai_bin, len(cigar), flag, l_seq, -1, -1, 0)
         body += qname.encode() + b"\0" + b"".join(struct.pack("<I", (l << 4) | o) for o, l in cigar) + packed + bytes(qual)
         for tag, ty, val in tags:
             body += tag.encode() + ty.encode()
@@ -403,9 +571,10 @@ class BamWriter:
         self._flush(everything=False)  # pending tail < 0xFF00, so offsets stay exact
         v1 = (self.coff << 16) | len(self.buf)
         if ref_id >= 0:
-            self.bins[ref_id].setdefault(_reg2bin(pos, end), []).append((v0, v1))
+            self.bins[ref_id].setdefault(_reg2bin(pos, end, self.min_shift, self.depth), []).append((v0, v1))
+            self.n_mapped[ref_id] += 1
             lin = self.lin[ref_id]
-            for w in range(pos >> 14, ((end - 1) >> 14) + 1):
+            for w in range(pos >> self.min_shift, ((end - 1) >> self.min_shift) + 1):
                 while len(lin) <= w:
                     lin.append(0)
                 if lin[w] == 0:
@@ -415,6 +584,9 @@ class BamWriter:
         self._flush()
         self.f.write(_BGZF_EOF)
         self.f.close()
+        if self.index == "csi":
+            self._write_csi()
+            return
         with open(self.path + ".bai", "wb") as f:
             f.write(b"BAI\x01" + struct.pack("<i", len(self.refs)))
             for bins, lin in zip(self.bins, self.lin):
@@ -434,20 +606,51 @@ class BamWriter:
                 f.write(struct.pack("<%dQ" % len(filled), *filled))
             f.write(struct.pack("<Q", 0))
 
+    def _write_csi(self):
+        ms, depth = self.min_shift, self.depth
+        out = bytearray(b"CSI\x01" + struct.pack("<iiii", ms, depth, 0, len(self.refs)))
+        for bins, lin, n_mapped in zip(self.bins, self.lin, self.n_mapped):
+            # htslib's linear index (update_loff): windows before the first entry take the contig's first record, later
+            # empty ones the entry to their left; a bin's loffset is the entry of its first window
+            first = min((ch[0][0] for ch in bins.values()), default=0)
+            filled, last = [], first
+            for v in lin:
+                last = v or last
+                filled.append(last)
+            out += struct.pack("<i", len(bins) + (1 if bins else 0))
+            for b, chunks in sorted(bins.items()):
+                merged = []  # adjacent records of one bin share a chunk, as htslib writes them
+                for beg, end in chunks:
+                    if merged and merged[-1][1] == beg:
+                        merged[-1] = (merged[-1][0], end)
+                    else:
+                        merged.append((beg, end))
+                bot = bin_start(b, ms, depth) >> ms
+                out += struct.pack("<IQi", b, filled[bot] if bot < len(filled) else 0, len(merged))
+                out += b"".join(struct.pack("<QQ", *c) for c in merged)
+            if bins:  # the pseudo-bin: first and last offsets of the contig, mapped and unmapped record counts
+                last_end = max(ch[-1][1] for ch in bins.values())
+                out += struct.pack("<IQi", pseudo_bin(depth), 0, 2) + struct.pack("<QQQQ", first, last_end, n_mapped, 0)
+        out += struct.pack("<Q", 0)  # n_no_coor
+        with open(self.path + ".csi", "wb") as f:
+            for k in range(0, len(out), 0xFF00):
+                f.write(_bgzf_block(bytes(out[k:k + 0xFF00]), self.level))
+            f.write(_BGZF_EOF)
+
 
 TAGS = ("cs", "md", "md_eqx", "eqx", "m")
 
 
-def write_batch_bam(path, chrom, contig_len, batch, sample="synth", tags="cs"):
+def write_batch_bam(path, chrom, contig_len, batch, sample="synth", tags="cs", **index):
     """ReadBatch -> coordinate-sorted BAM + BAI, tp:A:P, for tests and tools.  tags: "cs" writes cs:Z short form
     with a =/X CIGAR; "md" writes MD:Z and no cs with an M CIGAR; "md_eqx" MD:Z with the =/X CIGAR; "eqx" the =/X
     CIGAR and neither tag; "m" the M CIGAR and neither tag (these two decode with the contig's reference sequence)"""
-    write_batches_bam(path, [(chrom, contig_len, batch)], sample, tags)
+    write_batches_bam(path, [(chrom, contig_len, batch)], sample, tags, **index)
 
 
-def write_batches_bam(path, contigs, sample="synth", tags="cs"):
-    """[(chrom, contig_len, ReadBatch), ...] -> one coordinate-sorted BAM + BAI"""
-    w = BamWriter(path, [(c, n) for c, n, _ in contigs], header_extra="@RG\tID:rg\tSM:%s\n" % sample)
+def write_batches_bam(path, contigs, sample="synth", tags="cs", **index):
+    """[(chrom, contig_len, ReadBatch), ...] -> one coordinate-sorted BAM + BAI (index, min_shift, depth: BamWriter's)"""
+    w = BamWriter(path, [(c, n) for c, n, _ in contigs], header_extra="@RG\tID:rg\tSM:%s\n" % sample, **index)
     for rid, (_c, _n, batch) in enumerate(contigs):
         _add_batch(w, rid, batch, tags)
     w.close()

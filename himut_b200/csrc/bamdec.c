@@ -47,16 +47,21 @@ static uint32_t block_crc(const uint8_t* p, size_t n) {
 uint32_t hm_crc32_test(const uint8_t* p, size_t n) { return block_crc(p, n); }
 
 
+/* one bin of a BAI or CSI: its smallest chunk begin, its largest chunk end and (CSI) its loffset */
+typedef struct {
+  uint32_t id;
+  uint64_t beg, end, loff;
+} idx_bin_t;
+
 typedef struct {
   char* name;
   int32_t len;
-  uint64_t* lin; /* linear index */
+  uint64_t* lin; /* BAI linear index */
   int32_t n_lin;
   int has_index;
-  uint32_t* bin;     /* BAI bins (the pseudo-bin 37450 left out) ... */
-  uint64_t* bin_end; /* ... the largest chunk end of each ... */
-  uint64_t* bin_beg; /* ... and the smallest chunk begin */
+  idx_bin_t* bins; /* ascending ids, the pseudo-bin left out */
   int32_t n_bin;
+  uint64_t min_beg; /* smallest chunk begin of the contig */
 } bam_ref_t;
 
 typedef struct {
@@ -75,7 +80,9 @@ typedef struct hm_bam {
   int32_t n_ref;
   bam_ref_t* refs;
   uint64_t first_record; /* virtual offset */
-  int have_bai;
+  uint64_t file_size;
+  int index_kind;        /* HM_BAM_INDEX_NONE / _BAI / _CSI */
+  int min_shift, depth;  /* binning scheme of the index: (14, 5) for a BAI */
   qtab_t qt;
   char err[512];
   /* last decoded batch (owned) */
@@ -413,58 +420,249 @@ static int stream_seek(stream_t* s, uint64_t voffset) {
 }
 
 /* ------------------------------------------------------------------ open / close */
-static int load_bai(hm_bam* b) {
-  size_t n = strlen(b->path);
-  char* p = (char*)malloc(n + 5);
-  if (!p) return -1;
-  memcpy(p, b->path, n); memcpy(p + n, ".bai", 5);
-  FILE* f = fopen(p, "rb");
-  free(p);
-  if (!f) return 0;
-  fseeko(f, 0, SEEK_END);
-  size_t sz = (size_t)ftello(f);
-  fseeko(f, 0, SEEK_SET);
-  uint8_t* d = (uint8_t*)malloc(sz + 8);
-  if (!d || fread(d, 1, sz, f) != sz) { free(d); fclose(f); return -1; }
-  fclose(f);
-  if (sz < 8 || memcmp(d, "BAI\1", 4)) { free(d); return -1; }
-  size_t q = 8;
-  int32_t nref = (int32_t)rd32(d + 4);
-  for (int32_t r = 0; r < nref && r < b->n_ref; r++) {
-    int32_t nbin = (int32_t)rd32(d + q); q += 4;
-    b->refs[r].bin = (uint32_t*)malloc(((size_t)nbin + 1) * 4);
-    b->refs[r].bin_end = (uint64_t*)malloc(((size_t)nbin + 1) * 8);
-    b->refs[r].bin_beg = (uint64_t*)malloc(((size_t)nbin + 1) * 8);
-    if (!b->refs[r].bin || !b->refs[r].bin_end || !b->refs[r].bin_beg) { free(d); return -1; }
-    for (int32_t k = 0; k < nbin; k++) {
-      const uint32_t bin = rd32(d + q);
-      int32_t nchunk = (int32_t)rd32(d + q + 4);
-      uint64_t e = 0, bg = UINT64_MAX;
-      for (int32_t c = 0; c < nchunk; c++) {
-        uint64_t cb, ce;
-        memcpy(&cb, d + q + 8 + 16 * (size_t)c, 8); memcpy(&ce, d + q + 8 + 16 * (size_t)c + 8, 8);
-        if (ce > e) e = ce;
-        if (cb < bg) bg = cb;
+/* the binning scheme of SAM spec 5.3, for an index of min_shift and depth (a BAI is (14, 5)): level l has 8^l bins of
+ * 2^(min_shift + 3 (depth - l)) positions, numbered from bin_first(l); the pseudo-bin follows the last level */
+static inline uint32_t bin_first(int level) { return (uint32_t)(((1ull << (3 * level)) - 1) / 7); }
+static inline uint32_t pseudo_bin(int depth) { return bin_first(depth + 1) + 1; }
+static int bin_level(uint32_t bin) {
+  int l = 0;
+  while (bin >= bin_first(l + 1)) l++;
+  return l;
+}
+/* first reference position of a bin, and the number of positions it covers */
+static int64_t bin_start(uint32_t bin, int min_shift, int depth) {
+  const int l = bin_level(bin);
+  return (int64_t)(bin - bin_first(l)) << (min_shift + 3 * (depth - l));
+}
+static int64_t bin_size(uint32_t bin, int min_shift, int depth) { return (int64_t)1 << (min_shift + 3 * (depth - bin_level(bin))); }
+
+static char* path_with(const char* base, size_t n, const char* ext) {
+  char* p = (char*)malloc(n + strlen(ext) + 1);
+  if (p) { memcpy(p, base, n); strcpy(p + n, ext); }
+  return p;
+}
+
+/* the payload of a BGZF-compressed file (a CSI), NULL with b->err set when it is not one */
+static uint8_t* bgzf_slurp(hm_bam* b, const uint8_t* d, size_t sz, const char* ip, size_t* out_len) {
+  size_t cap = 1u << 16, n = 0, off = 0;
+  uint8_t* u = (uint8_t*)malloc(cap);
+  z_stream zs;
+  memset(&zs, 0, sizeof(zs));
+  if (!u || inflateInit2(&zs, -15) != Z_OK) { free(u); snprintf(b->err, sizeof(b->err), "out of memory reading %s", ip); return NULL; }
+  while (off < sz) {
+    const uint8_t* h = d + off;
+    int bsize = -1;
+    if (sz - off >= 18 && h[0] == 0x1f && h[1] == 0x8b && h[2] == 8 && (h[3] & 4)) {
+      const size_t xlen = (size_t)(h[10] | (h[11] << 8));
+      for (size_t q = 0; 12 + xlen <= sz - off && q + 4 <= xlen;) {
+        const size_t slen = (size_t)(h[12 + q + 2] | (h[12 + q + 3] << 8));
+        if (h[12 + q] == 66 && h[12 + q + 1] == 67 && slen == 2 && q + 6 <= xlen) bsize = h[12 + q + 4] | (h[12 + q + 5] << 8);
+        q += 4 + slen;
       }
-      if (bin != 37450) { b->refs[r].bin[b->refs[r].n_bin] = bin; b->refs[r].bin_beg[b->refs[r].n_bin] = bg; b->refs[r].bin_end[b->refs[r].n_bin++] = e; }
-      q += 8 + 16 * (size_t)nchunk;
+      if (bsize >= 0 && ((size_t)bsize + 1 < 12 + xlen + 8 || (size_t)bsize + 1 > sz - off)) bsize = -1;
+      if (bsize >= 0) {
+        const size_t csize = (size_t)bsize + 1, isize = rd32(h + csize - 4);
+        if (isize > 65536) goto bad;
+        if (n + isize > cap) {
+          while (n + isize > cap) cap *= 2;
+          uint8_t* nu = (uint8_t*)realloc(u, cap);
+          if (!nu) goto bad;
+          u = nu;
+        }
+        inflateReset(&zs);
+        zs.next_in = (Bytef*)(h + 12 + xlen); zs.avail_in = (uInt)(csize - 12 - xlen - 8);
+        zs.next_out = u + n; zs.avail_out = (uInt)isize;
+        if ((isize || csize - 12 - xlen - 8 > 2) && (inflate(&zs, Z_FINISH) != Z_STREAM_END || zs.avail_out || block_crc(u + n, isize) != rd32(h + csize - 8))) bsize = -1;
+        else { n += isize; off += csize; continue; }
+      }
     }
-    int32_t nintv = (int32_t)rd32(d + q); q += 4;
-    b->refs[r].lin = (uint64_t*)malloc(((size_t)nintv + 1) * 8);
-    b->refs[r].n_lin = nintv;
-    b->refs[r].has_index = (nbin || nintv);
-    for (int32_t k = 0; k < nintv; k++) { memcpy(&b->refs[r].lin[k], d + q, 8); q += 8; }
+  bad:
+    inflateEnd(&zs);
+    free(u);
+    snprintf(b->err, sizeof(b->err), "%s is not a BGZF-compressed CSI index (block at byte %zu)", ip, off);
+    return NULL;
   }
-  free(d);
-  b->have_bai = 1;
+  inflateEnd(&zs);
+  *out_len = n;
+  return u;
+}
+
+static int cmp_u64(const void* x, const void* y) {
+  const uint64_t a = *(const uint64_t*)x, c = *(const uint64_t*)y;
+  return a < c ? -1 : a > c;
+}
+static int cmp_bin(const void* x, const void* y) {
+  const uint32_t a = ((const idx_bin_t*)x)->id, c = ((const idx_bin_t*)y)->id;
+  return a < c ? -1 : a > c;
+}
+
+/* the bins of one reference at d + *q (n_bin, then per bin: bin, [loffset,] n_chunk, chunks), every count bounded by
+ * the bytes left; R NULL: parsed and checked, not kept (references past the BAM's) */
+static int load_bins(hm_bam* b, bam_ref_t* R, const uint8_t* d, size_t sz, size_t* qp, int csi, const char* ip) {
+  const uint32_t pseudo = pseudo_bin(b->depth);
+  const size_t fixed = csi ? 16 : 8; /* bin, loffset (CSI), n_chunk */
+  size_t q = *qp;
+#define IDX_BAD(...) do { int k_ = snprintf(b->err, sizeof(b->err), "%s: ", ip); snprintf(b->err + k_, sizeof(b->err) - (size_t)k_, __VA_ARGS__); return -1; } while (0)
+  if (sz - q < 4) IDX_BAD("truncated at byte %zu (n_bin)", q);
+  const int32_t nbin = (int32_t)rd32(d + q);
+  q += 4;
+  if (nbin < 0 || (size_t)nbin > (sz - q) / fixed) IDX_BAD("n_bin %d runs past the end of the index", nbin);
+  if (R) {
+    R->bins = (idx_bin_t*)malloc(((size_t)nbin + 1) * sizeof(idx_bin_t));
+    if (!R->bins) IDX_BAD("out of memory for %d bins", nbin);
+    R->min_beg = UINT64_MAX;
+  }
+  for (int32_t k = 0; k < nbin; k++) {
+    if (sz - q < fixed) IDX_BAD("truncated at byte %zu (bin)", q);
+    const uint32_t bin = rd32(d + q);
+    uint64_t loff = 0;
+    if (csi) memcpy(&loff, d + q + 4, 8);
+    const int32_t nchunk = (int32_t)rd32(d + q + fixed - 4);
+    q += fixed;
+    if (csi && (bin > pseudo || bin == pseudo - 1)) IDX_BAD("bin %u past the pseudo-bin %u", bin, pseudo); /* pseudo - 1: past the last level */
+    if (csi && bin != pseudo && (loff >> 16) >= b->file_size) IDX_BAD("loffset of bin %u points past the end of the BAM", bin);
+    if (nchunk < 0 || (size_t)nchunk > (sz - q) / 16) IDX_BAD("n_chunk %d of bin %u runs past the end of the index", nchunk, bin);
+    uint64_t e = 0, bg = UINT64_MAX;
+    for (int32_t c = 0; c < nchunk; c++) {
+      uint64_t cb, ce;
+      memcpy(&cb, d + q + 16 * (size_t)c, 8); memcpy(&ce, d + q + 16 * (size_t)c + 8, 8);
+      if (csi && bin != pseudo && cb > ce) IDX_BAD("chunk %d of bin %u begins after its end", c, bin);
+      if (csi && bin != pseudo && (cb >> 16) >= b->file_size) IDX_BAD("chunk %d of bin %u points past the end of the BAM", c, bin);
+      if (ce > e) e = ce;
+      if (cb < bg) bg = cb;
+    }
+    q += 16 * (size_t)nchunk;
+    if (R && bin < pseudo - 1 && nchunk) {
+      idx_bin_t* x = &R->bins[R->n_bin++];
+      x->id = bin; x->beg = bg; x->end = e; x->loff = loff;
+      if (bg < R->min_beg) R->min_beg = bg;
+    }
+  }
+#undef IDX_BAD
+  if (R) qsort(R->bins, (size_t)R->n_bin, sizeof(idx_bin_t), cmp_bin);
+  *qp = q;
   return 0;
+}
+
+/* the index of the BAM, by the names htslib finds: <bam>.bai, <bam>.csi, then <stem>.bai and <stem>.csi for x.bam.
+ * None found: b->index_kind stays 0 and every query scans from the first record.  -1 (b->err set): an index that
+ * cannot be read. */
+static int load_index(hm_bam* b) {
+  const size_t n = strlen(b->path);
+  const size_t stem = n > 4 && strcmp(b->path + n - 4, ".bam") == 0 ? n - 4 : 0;
+  const struct { size_t len; const char* ext; int kind; } cand[4] = {
+      {n, ".bai", HM_BAM_INDEX_BAI}, {n, ".csi", HM_BAM_INDEX_CSI}, {stem, ".bai", HM_BAM_INDEX_BAI}, {stem, ".csi", HM_BAM_INDEX_CSI}};
+  FILE* f = NULL;
+  char* ip = NULL;
+  int kind = 0;
+  for (int i = 0; i < 4 && !f; i++) {
+    if (!cand[i].len) continue;
+    free(ip);
+    ip = path_with(b->path, cand[i].len, cand[i].ext);
+    if (!ip) return -1;
+    f = fopen(ip, "rb");
+    kind = cand[i].kind;
+  }
+  if (!f) { free(ip); return 0; }
+  size_t sz = 0;
+  uint8_t* raw = NULL;
+  if (fseeko(f, 0, SEEK_END) == 0) {
+    const off_t end = ftello(f);
+    sz = end > 0 ? (size_t)end : 0;
+    raw = (uint8_t*)malloc(sz + 8);
+    if (raw && (fseeko(f, 0, SEEK_SET) || fread(raw, 1, sz, f) != sz)) { free(raw); raw = NULL; }
+  }
+  fclose(f);
+  int rc = -1;
+  uint8_t* d = raw;
+  if (!raw) { snprintf(b->err, sizeof(b->err), "cannot read %s", ip); goto out; }
+  b->min_shift = 14; b->depth = 5;
+  size_t q;
+  int32_t nref;
+  if (kind == HM_BAM_INDEX_BAI) {
+    if (sz < 8 || memcmp(d, "BAI\1", 4)) { snprintf(b->err, sizeof(b->err), "%s is not a BAI index", ip); goto out; }
+    nref = (int32_t)rd32(d + 4);
+    q = 8;
+  } else {
+    d = bgzf_slurp(b, raw, sz, ip, &sz);
+    if (!d) goto out;
+    if (sz < 16 || memcmp(d, "CSI\1", 4)) { snprintf(b->err, sizeof(b->err), "%s is not a CSI index", ip); goto out; }
+    const int32_t ms = (int32_t)rd32(d + 4), depth = (int32_t)rd32(d + 8), l_aux = (int32_t)rd32(d + 12);
+    if (ms < 1 || depth < 0 || depth > 10 || ms + 3 * depth > 62) {
+      snprintf(b->err, sizeof(b->err), "%s: unsupported min_shift %d / depth %d", ip, ms, depth);
+      goto out;
+    }
+    b->min_shift = ms; b->depth = depth;
+    for (int32_t r = 0; r < b->n_ref; r++)
+      if ((int64_t)b->refs[r].len > ((int64_t)1 << (ms + 3 * depth))) {
+        snprintf(b->err, sizeof(b->err), "%s: min_shift %d and depth %d cover %lld positions, %s has %d", ip, ms, depth,
+                 (long long)1 << (ms + 3 * depth), b->refs[r].name, b->refs[r].len);
+        goto out;
+      }
+    if (l_aux < 0 || (size_t)l_aux > sz - 16 || sz - 16 - (size_t)l_aux < 4) { snprintf(b->err, sizeof(b->err), "%s: l_aux %d runs past the end of the index", ip, l_aux); goto out; }
+    q = 16 + (size_t)l_aux;
+    nref = (int32_t)rd32(d + q);
+    q += 4;
+  }
+  if (nref < 0) { snprintf(b->err, sizeof(b->err), "%s: n_ref %d", ip, nref); goto out; }
+  for (int32_t r = 0; r < nref; r++) {
+    bam_ref_t* R = r < b->n_ref ? &b->refs[r] : NULL;
+    if (kind == HM_BAM_INDEX_BAI && !R) break; /* as before: references past the BAM's are not read */
+    if (load_bins(b, R, d, sz, &q, kind == HM_BAM_INDEX_CSI, ip)) goto out;
+    if (kind == HM_BAM_INDEX_CSI) { if (R) R->has_index = R->n_bin > 0; continue; }
+    if (sz - q < 4) { snprintf(b->err, sizeof(b->err), "%s: truncated at byte %zu (n_intv)", ip, q); goto out; }
+    const int32_t nintv = (int32_t)rd32(d + q);
+    q += 4;
+    if (nintv < 0 || (size_t)nintv > (sz - q) / 8) { snprintf(b->err, sizeof(b->err), "%s: n_intv %d runs past the end of the index", ip, nintv); goto out; }
+    R->lin = (uint64_t*)malloc(((size_t)nintv + 1) * 8);
+    if (!R->lin) { snprintf(b->err, sizeof(b->err), "out of memory reading %s", ip); goto out; }
+    R->n_lin = nintv;
+    R->has_index = (R->n_bin || nintv);
+    memcpy(R->lin, d + q, 8 * (size_t)nintv);
+    q += 8 * (size_t)nintv;
+  }
+  b->index_kind = kind;
+  rc = 0;
+out:
+  if (d != raw) free(d);
+  free(raw);
+  free(ip);
+  return rc;
+}
+
+/* the virtual offset the records of [start, ...) of contig rid are read from; 0: the index knows no record of the
+ * contig.  BAI: the linear-index entry of start's 16 kb window, or of the nearest window to its left that has one.
+ * CSI (htslib's hts_itr_query): the loffset of the leaf bin that holds start, else of its nearest left sibling, else
+ * of its parent, and so on up; without one, the contig's first chunk.  Without an index: the first record. */
+static uint64_t seek_voff(const hm_bam* b, int rid, int32_t start) {
+  if (!b->index_kind) return b->first_record;
+  const bam_ref_t* R = &b->refs[rid];
+  if (!R->has_index) return 0;
+  if (b->index_kind == HM_BAM_INDEX_BAI) {
+    int32_t w = start >> 14;
+    if (w >= R->n_lin) w = R->n_lin - 1;
+    uint64_t v = 0;
+    for (; w >= 0 && !v; w--) v = R->lin[w];
+    return v ? v : b->first_record;
+  }
+  const int64_t top = ((int64_t)1 << (b->min_shift + 3 * b->depth)) - 1;
+  uint32_t bin = bin_first(b->depth) + (uint32_t)(((int64_t)start < top ? (int64_t)start : top) >> b->min_shift);
+  for (;;) {
+    size_t lo = 0, hi = (size_t)R->n_bin;
+    while (lo < hi) { const size_t m = (lo + hi) / 2; if (R->bins[m].id < bin) lo = m + 1; else hi = m; }
+    if (lo < (size_t)R->n_bin && R->bins[lo].id == bin && R->bins[lo].loff) return R->bins[lo].loff;
+    if (bin == 0) break;
+    const uint32_t first = (((bin - 1) >> 3) << 3) + 1; /* the first child of the parent */
+    bin = bin > first ? bin - 1 : (bin - 1) >> 3;
+  }
+  return R->min_beg;
 }
 
 void hm_bam_close(hm_bam* b) {
   if (!b) return;
   if (b->map) munmap((void*)b->map, b->map_len);
   if (b->f) fclose(b->f);
-  for (int32_t i = 0; i < b->n_ref; i++) { free(b->refs[i].name); free(b->refs[i].lin); free(b->refs[i].bin); free(b->refs[i].bin_end); free(b->refs[i].bin_beg); }
+  for (int32_t i = 0; i < b->n_ref; i++) { free(b->refs[i].name); free(b->refs[i].lin); free(b->refs[i].bins); }
   free(b->refs); free(b->header); free(b->path);
   free(b->p_coff); free(b->p_uoff); free(b->p_entry); free(b->p_csize); free(b->p_isize); free(b->p_crc); free(b->p_comp);
   for (uint32_t i = 0; i < b->qt.n; i++) free(b->qt.names[i]);
@@ -482,9 +680,13 @@ void hm_bam_close(hm_bam* b) {
 static int have_ssse3(void); /* probed once in hm_bam_open, read by the record-decode threads */
 #endif
 
+/* why the last hm_bam_open of this thread failed: hm_bam_error(NULL) */
+static __thread char g_open_err[512];
+
 int hm_bam_open(const char* path, hm_bam** out) {
   if (!path || !out) return HM_ERR_ARG;
   *out = NULL;
+  g_open_err[0] = 0;
   (void)hi_use_run(); (void)hm_crc32_available(); /* one-time CPU probes and tables, before any worker thread exists */
 #if defined(__x86_64__) && defined(__GNUC__)
   (void)have_ssse3();
@@ -496,7 +698,8 @@ int hm_bam_open(const char* path, hm_bam** out) {
   if (!b->f) { hm_bam_close(b); return HM_ERR_ARG; }
   {
     struct stat st;
-    if (fstat(fileno(b->f), &st) == 0 && st.st_size > 0) {
+    if (fstat(fileno(b->f), &st) == 0) b->file_size = (uint64_t)st.st_size;
+    if (b->file_size > 0) {
       void* m = mmap(NULL, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, fileno(b->f), 0);
       if (m != MAP_FAILED) { b->map = (const uint8_t*)m; b->map_len = (size_t)st.st_size; }
     }
@@ -533,16 +736,21 @@ int hm_bam_open(const char* path, hm_bam** out) {
       left -= blk.usize; coff += blk.csize;
     }
   }
-  if (load_bai(b) < 0) goto done;
+  if (load_index(b) < 0) goto done;
   rc = HM_OK;
 done:
   free(s.buf);
-  if (rc) { hm_bam_close(b); return rc; }
+  if (rc) {
+    snprintf(g_open_err, sizeof(g_open_err), "%s", b->err);
+    hm_bam_close(b);
+    return rc;
+  }
   *out = b;
   return HM_OK;
 }
 
-const char* hm_bam_error(const hm_bam* b) { return b ? b->err : "null handle"; }
+const char* hm_bam_error(const hm_bam* b) { return b ? b->err : g_open_err; }
+int hm_bam_index_kind(const hm_bam* b) { return b ? b->index_kind : HM_BAM_INDEX_NONE; }
 const char* hm_bam_header_text(const hm_bam* b) { return b->header; }
 int hm_bam_n_refs(const hm_bam* b) { return b->n_ref; }
 const char* hm_bam_ref_name(const hm_bam* b, int i) { return (i >= 0 && i < b->n_ref) ? b->refs[i].name : NULL; }
@@ -1006,16 +1214,8 @@ int hm_bam_read_batch(hm_bam* b, int rid, int32_t start, int32_t end, int thread
   uint64_t n_exc = 0;
   memset(out, 0, sizeof(*out));
   b->n_qexc = 0;
-  uint64_t voff = b->first_record;
-  if (b->have_bai) {
-    const bam_ref_t* R = &b->refs[rid];
-    if (!R->has_index) goto finish; /* no reads on this contig */
-    int32_t w = start >> 14;
-    if (w >= R->n_lin) w = R->n_lin - 1;
-    uint64_t v = 0;
-    for (; w >= 0 && !v; w--) v = R->lin[w];
-    if (v) voff = v;
-  }
+  const uint64_t voff = seek_voff(b, rid, start);
+  if (!voff) goto finish; /* no reads on this contig */
   {
     stream_t s;
     memset(&s, 0, sizeof(s));
@@ -1252,29 +1452,6 @@ int hm_bam_last_compact(hm_bam* b, hm_bq_compact* out) {
 }
 
 /* ------------------------------------------------------------------ region plan for the device decoder */
-/* the bins of the UCSC binning scheme that overlap [beg, end) (SAM spec 5.3) */
-static int reg2bins(int64_t beg, int64_t end, uint32_t* list) {
-  int n = 0;
-  --end;
-  list[n++] = 0;
-  for (int64_t k = 1 + (beg >> 26); k <= 1 + (end >> 26); ++k) list[n++] = (uint32_t)k;
-  for (int64_t k = 9 + (beg >> 23); k <= 9 + (end >> 23); ++k) list[n++] = (uint32_t)k;
-  for (int64_t k = 73 + (beg >> 20); k <= 73 + (end >> 20); ++k) list[n++] = (uint32_t)k;
-  for (int64_t k = 585 + (beg >> 17); k <= 585 + (end >> 17); ++k) list[n++] = (uint32_t)k;
-  for (int64_t k = 4681 + (beg >> 14); k <= 4681 + (end >> 14); ++k) list[n++] = (uint32_t)k;
-  return n;
-}
-
-/* first reference position of a bin of the binning scheme */
-static int64_t bin_start(uint32_t bin) {
-  if (bin >= 4681) return (int64_t)(bin - 4681) << 14;
-  if (bin >= 585) return (int64_t)(bin - 585) << 17;
-  if (bin >= 73) return (int64_t)(bin - 73) << 20;
-  if (bin >= 9) return (int64_t)(bin - 9) << 23;
-  if (bin >= 1) return (int64_t)(bin - 1) << 26;
-  return 0;
-}
-
 /* the BGZF header at coff: 0 and *blk filled, 1 end of file, -1 not a BGZF block */
 static int block_at(hm_bam* b, uint64_t coff, blk_t* blk, uint32_t* crc) {
   if (!b->map) {
@@ -1315,42 +1492,52 @@ int hm_bam_region_plan(hm_bam* b, int rid, int32_t start, int32_t end, hm_bgzf_p
   uint64_t v_lo = b->first_record, v_hi = UINT64_MAX; /* UINT64_MAX: to the end of the file */
   uint64_t* ventry = NULL; /* virtual offsets of the later entry points */
   size_t n_ventry = 0;
-  if (b->have_bai) {
+  if (b->index_kind) {
     const bam_ref_t* R = &b->refs[rid];
-    if (!R->has_index) return HM_OK; /* no reads on this contig: an empty plan */
-    /* the window hm_bam_read_batch seeks to, then the linear-index entries of the windows the region covers */
-    int32_t w0 = start >> 14;
-    if (w0 >= R->n_lin) w0 = R->n_lin - 1;
-    int32_t w = w0;
-    uint64_t v = 0;
-    for (; w >= 0 && !v; w--) v = R->lin[w];
-    if (v) v_lo = v;
+    const int ms = b->min_shift, depth = b->depth;
+    /* where hm_bam_read_batch seeks to */
+    v_lo = seek_voff(b, rid, start);
+    if (!v_lo) return HM_OK; /* no reads on this contig: an empty plan */
     /* every record that overlaps the region (hm_bam_read_batch's rule: pos < end, reference end > start) lies in a
      * chunk of a bin that overlaps [min(start, end), max(start, end) + 1): the range ends at their largest end.  The
-     * large bins (64 and 512 Mb) overlap every region and their chunks reach to the far end of the contig, so the range
-     * also ends at the first chunk of any bin that starts at or past `end`: every record there has pos >= end, where
+     * large bins overlap every region and their chunks reach to the far end of the contig, so the range also ends at
+     * the first chunk of any bin that starts at or past `end`: every record there has pos >= end, where
      * hm_bam_read_batch stops, and it is a record start. */
-    const int64_t rb = start < end ? start : end, re = (start > end ? start : end) + 1;
-    uint8_t* in_region = (uint8_t*)calloc(37450, 1);
-    uint32_t* bins = (uint32_t*)malloc(37450 * sizeof(uint32_t));
-    if (!in_region || !bins) { free(in_region); free(bins); return fail(b, "out of memory%s (%ld)", NULL, 0); }
-    const int nbins = reg2bins(rb, re, bins);
-    for (int j = 0; j < nbins; j++) if (bins[j] < 37450) in_region[bins[j]] = 1;
-    free(bins);
+    const int64_t rb = start < end ? start : end, re = (int64_t)(start > end ? start : end) + 1; /* end may be 2^31 - 1 */
     v_hi = 0;
-    for (int32_t k = 0; k < R->n_bin; k++)
-      if (R->bin[k] < 37450 && in_region[R->bin[k]] && R->bin_end[k] > v_hi) v_hi = R->bin_end[k];
-    free(in_region);
-    for (int32_t k = 0; k < R->n_bin; k++)
-      if (R->bin[k] < 37450 && bin_start(R->bin[k]) >= (int64_t)end && R->bin_beg[k] < v_hi) v_hi = R->bin_beg[k];
-    if (v_hi <= v_lo) return HM_OK; /* no record overlaps the region */
-    const int32_t w_last = (int32_t)((re - 1) >> 14) < R->n_lin - 1 ? (int32_t)((re - 1) >> 14) : R->n_lin - 1;
-    if (w_last > w0) {
-      ventry = (uint64_t*)malloc((size_t)(w_last - w0) * sizeof(uint64_t));
-      if (!ventry) return fail(b, "out of memory%s (%ld)", NULL, 0);
+    for (int32_t k = 0; k < R->n_bin; k++) {
+      const int64_t bs = bin_start(R->bins[k].id, ms, depth);
+      if (bs < re && bs + bin_size(R->bins[k].id, ms, depth) > rb && R->bins[k].end > v_hi) v_hi = R->bins[k].end;
     }
-    for (int32_t k = w0 + 1; k <= w_last; k++)
-      if (R->lin[k] > v_lo && R->lin[k] < v_hi && (!n_ventry || R->lin[k] > ventry[n_ventry - 1])) ventry[n_ventry++] = R->lin[k];
+    for (int32_t k = 0; k < R->n_bin; k++)
+      if (bin_start(R->bins[k].id, ms, depth) >= (int64_t)end && R->bins[k].beg < v_hi) v_hi = R->bins[k].beg;
+    if (v_hi <= v_lo) return HM_OK; /* no record overlaps the region */
+    if (b->index_kind == HM_BAM_INDEX_BAI) {
+      /* the linear-index entries of the windows the region covers */
+      int32_t w0 = start >> 14;
+      if (w0 >= R->n_lin) w0 = R->n_lin - 1;
+      const int32_t w_last = (int32_t)((re - 1) >> 14) < R->n_lin - 1 ? (int32_t)((re - 1) >> 14) : R->n_lin - 1;
+      if (w_last > w0) {
+        ventry = (uint64_t*)malloc((size_t)(w_last - w0) * sizeof(uint64_t));
+        if (!ventry) return fail(b, "out of memory%s (%ld)", NULL, 0);
+      }
+      for (int32_t k = w0 + 1; k <= w_last; k++)
+        if (R->lin[k] > v_lo && R->lin[k] < v_hi && (!n_ventry || R->lin[k] > ventry[n_ventry - 1])) ventry[n_ventry++] = R->lin[k];
+    } else {
+      /* the loffsets of the bins of any level that start inside the region: each is a record start.  A read that
+       * crosses a window boundary goes to a larger bin, so the leaf bins alone would leave long serial segments. */
+      ventry = (uint64_t*)malloc(((size_t)R->n_bin + 1) * sizeof(uint64_t));
+      if (!ventry) return fail(b, "out of memory%s (%ld)", NULL, 0);
+      for (int32_t k = 0; k < R->n_bin; k++) {
+        const int64_t bs = bin_start(R->bins[k].id, ms, depth);
+        const uint64_t v = R->bins[k].loff;
+        if (bs >= rb && bs < re && v > v_lo && v < v_hi) ventry[n_ventry++] = v;
+      }
+      qsort(ventry, n_ventry, sizeof(uint64_t), cmp_u64);
+      size_t m = 0;
+      for (size_t k = 0; k < n_ventry; k++) if (!m || ventry[k] != ventry[m - 1]) ventry[m++] = ventry[k];
+      n_ventry = m;
+    }
   }
   const int rc = plan_range(b, v_lo, v_hi, ventry, n_ventry, out);
   free(ventry);
@@ -1392,7 +1579,9 @@ static int plan_range(hm_bam* b, uint64_t v_lo, uint64_t v_hi, const uint64_t* v
     size_t lo_ = 0, hi_ = nb;                                                                                    \
     while (lo_ < hi_) { const size_t m_ = (lo_ + hi_) / 2; if (b->p_coff[m_] < c_) lo_ = m_ + 1; else hi_ = m_; } \
     if (b->p_coff[lo_] != c_ || (lo_ < nb && ((v) & 0xffff) > b->p_isize[lo_]) || (lo_ == nb && ((v) & 0xffff)))  \
-      return fail(b, "BAI virtual offset outside the BGZF blocks of %s (%ld)", b->path, (long)((v) >> 16));      \
+      return fail(b, b->index_kind == HM_BAM_INDEX_CSI ? "CSI virtual offset outside the BGZF blocks of %s (%ld)"  \
+                                                        : "BAI virtual offset outside the BGZF blocks of %s (%ld)", b->path, \
+                  (long)((v) >> 16));                                                                            \
     (dst) = b->p_uoff[lo_] + ((v) & 0xffff);                                                                     \
   } while (0)
   uint64_t u_end = usum;
@@ -1453,16 +1642,8 @@ int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int thre
   if (start < 0) start = 0;
   if (end > b->refs[rid].len) end = b->refs[rid].len;
   if (start >= end) return HM_OK;
-  uint64_t voff = b->first_record;
-  if (b->have_bai) {
-    const bam_ref_t* R = &b->refs[rid];
-    if (!R->has_index) return HM_OK;
-    int32_t w = start >> 14;
-    if (w >= R->n_lin) w = R->n_lin - 1;
-    uint64_t v = 0;
-    for (; w >= 0 && !v; w--) v = R->lin[w];
-    if (v) voff = v;
-  }
+  const uint64_t voff = seek_voff(b, rid, start);
+  if (!voff) return HM_OK;
   stream_t s;
   memset(&s, 0, sizeof(s));
   s.b = b; s.threads = threads;
@@ -1551,13 +1732,11 @@ static int wb_need(wbuf_t* w, size_t add) {
   return 0;
 }
 static void wb_u32(wbuf_t* w, uint32_t v) { w->p[w->n++] = (uint8_t)v; w->p[w->n++] = (uint8_t)(v >> 8); w->p[w->n++] = (uint8_t)(v >> 16); w->p[w->n++] = (uint8_t)(v >> 24); }
-static int reg2bin(int32_t beg, int32_t end) {
+/* the smallest bin of the (min_shift, depth) scheme that holds [beg, end) (htslib's hts_reg2bin) */
+static uint32_t reg2bin(int64_t beg, int64_t end, int min_shift, int depth) {
   --end;
-  if (beg >> 14 == end >> 14) return ((1 << 15) - 1) / 7 + (beg >> 14);
-  if (beg >> 17 == end >> 17) return ((1 << 12) - 1) / 7 + (beg >> 17);
-  if (beg >> 20 == end >> 20) return ((1 << 9) - 1) / 7 + (beg >> 20);
-  if (beg >> 23 == end >> 23) return ((1 << 6) - 1) / 7 + (beg >> 23);
-  if (beg >> 26 == end >> 26) return ((1 << 3) - 1) / 7 + (beg >> 26);
+  for (int l = depth, sh = min_shift; l > 0; l--, sh += 3)
+    if (beg >> sh == end >> sh) return bin_first(l) + (uint32_t)(beg >> sh);
   return 0;
 }
 #define WBLK 0xff00u
@@ -1605,7 +1784,59 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
 
 int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                             int level, int threads, int tags) {
+  return hm_bam_write_batch_index(path, chrom, contig_len, sample, b, level, threads, tags, 0, 0);
+}
+
+/* BGZF blocks of 0xff00 bytes of src, deflated on `threads` threads, then the end-of-file block, to f; coff (NULL: not
+ * wanted) receives the file offset of every block, n_blocks + 1 entries */
+static int bgzf_write(FILE* f, const uint8_t* src, size_t n, int level, int threads, uint64_t** coff_out) {
+  deflate_job_t job; memset(&job, 0, sizeof(job));
+  job.src = src; job.n_src = n; job.n_blocks = (n + WBLK - 1) / WBLK; job.level = level < 0 ? 1 : level;
+  job.dst = (uint8_t*)malloc(job.n_blocks * 65536 + 1); job.csize = (uint32_t*)calloc(job.n_blocks + 1, 4);
+  uint64_t* coff = (uint64_t*)malloc((job.n_blocks + 2) * sizeof(uint64_t));
+  int rc = HM_OK;
+  if (!job.dst || !job.csize || !coff) rc = HM_ERR_ARG;
+  else {
+    pthread_mutex_init(&job.mu, NULL);
+    int nt = threads < 1 ? 1 : (threads > 64 ? 64 : threads);
+    pthread_t th[64];
+    for (int t = 1; t < nt; t++) pthread_create(&th[t], NULL, deflate_worker, &job);
+    deflate_worker(&job);
+    for (int t = 1; t < nt; t++) pthread_join(th[t], NULL);
+    pthread_mutex_destroy(&job.mu);
+    if (job.error) rc = HM_ERR_ARG;
+    coff[0] = 0;
+    for (size_t i = 0; i < job.n_blocks && !rc; i++) {
+      if (fwrite(job.dst + i * 65536, 1, job.csize[i], f) != job.csize[i]) rc = HM_ERR_ARG;
+      coff[i + 1] = coff[i] + job.csize[i];
+    }
+    static const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (!rc && fwrite(BGZF_EOF, 1, 28, f) != 28) rc = HM_ERR_ARG;
+  }
+  free(job.dst); free(job.csize);
+  if (rc || !coff_out) free(coff);
+  else *coff_out = coff;
+  return rc;
+}
+
+typedef struct { uint32_t bin; uint64_t beg, end; size_t i; } bchunk_t;
+static int cmp_chunk(const void* x, const void* y) {
+  const bchunk_t *a = (const bchunk_t*)x, *c = (const bchunk_t*)y;
+  return a->bin != c->bin ? (a->bin < c->bin ? -1 : 1) : (a->i < c->i ? -1 : a->i > c->i);
+}
+
+int hm_bam_write_batch_index(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
+                             int level, int threads, int tags, int min_shift, int depth) {
   if (!path || !chrom || !b || tags < HM_BAM_TAGS_CS || tags > HM_BAM_TAGS_M) return HM_ERR_ARG;
+  const int csi = min_shift != 0;
+  if (!csi && (int64_t)contig_len > ((int64_t)1 << 29)) return HM_ERR_ARG; /* past what a BAI can bin */
+  if (csi) {
+    if (depth <= 0) /* htslib's choice: the smallest depth whose span holds the contig plus 256 */
+      for (depth = 0; ((int64_t)1 << (min_shift + 3 * depth)) < (int64_t)contig_len + 256; depth++) {}
+    if (min_shift < 1 || depth > 10 || min_shift + 3 * depth > 62 || ((int64_t)1 << (min_shift + 3 * depth)) < (int64_t)contig_len) return HM_ERR_ARG;
+  } else {
+    min_shift = 14; depth = 5;
+  }
   const int use_md = tags != HM_BAM_TAGS_CS;                             /* the walk below writes MD (unused without a tag) */
   const int no_tag = tags == HM_BAM_TAGS_EQX || tags == HM_BAM_TAGS_M;  /* no alignment tag: CIGAR + reference decodes it */
   const int m_cigar = tags == HM_BAM_TAGS_MD || tags == HM_BAM_TAGS_M;
@@ -1667,7 +1898,8 @@ int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_
     wb_u32(&w, (uint32_t)body);
     wb_u32(&w, 0); wb_u32(&w, (uint32_t)pos);
     w.p[w.n++] = (uint8_t)lq; w.p[w.n++] = b->mapq[r];
-    const int bin = reg2bin(pos, endp);
+    /* the BAI bin, which no decoder here reads: past 2^29 no BAI bin exists, and 4680 there cannot be right */
+    const uint32_t bin = endp - 1 < (1 << 29) ? reg2bin(pos, endp, 14, 5) : 4680;
     w.p[w.n++] = (uint8_t)bin; w.p[w.n++] = (uint8_t)(bin >> 8);
     w.p[w.n++] = (uint8_t)ncig; w.p[w.n++] = (uint8_t)(ncig >> 8);
     const uint32_t flag = (b->flags[r] & HM_READ_SECONDARY) ? 0x100u : 0u;
@@ -1687,86 +1919,91 @@ int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_
   free(cs); free(cig);
   if (rc) { free(w.p); free(rec_off); free(rec_end); return rc; }
   rec_off[n] = w.n;
-  /* BGZF: fixed 0xff00-byte blocks, deflated in parallel */
-  deflate_job_t job; memset(&job, 0, sizeof(job));
-  job.src = w.p; job.n_src = w.n; job.n_blocks = (w.n + WBLK - 1) / WBLK; job.level = level < 0 ? 1 : level;
-  job.dst = (uint8_t*)malloc(job.n_blocks * 65536 + 1); job.csize = (uint32_t*)calloc(job.n_blocks + 1, 4);
-  uint64_t* coff = (uint64_t*)malloc((job.n_blocks + 2) * sizeof(uint64_t));
-  if (!job.dst || !job.csize || !coff) { free(w.p); free(rec_off); free(rec_end); free(job.dst); free(job.csize); free(coff); return HM_ERR_ARG; }
-  pthread_mutex_init(&job.mu, NULL);
-  int nt = threads < 1 ? 1 : (threads > 64 ? 64 : threads);
-  pthread_t th[64];
-  for (int t = 1; t < nt; t++) pthread_create(&th[t], NULL, deflate_worker, &job);
-  deflate_worker(&job);
-  for (int t = 1; t < nt; t++) pthread_join(th[t], NULL);
-  pthread_mutex_destroy(&job.mu);
-  FILE* f = job.error ? NULL : fopen(path, "wb");
-  if (!f) rc = HM_ERR_ARG;
-  coff[0] = 0;
-  for (size_t i = 0; i < job.n_blocks && !rc; i++) {
-    if (fwrite(job.dst + i * 65536, 1, job.csize[i], f) != job.csize[i]) rc = HM_ERR_ARG;
-    coff[i + 1] = coff[i] + job.csize[i];
-  }
-  static const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  if (!rc && fwrite(BGZF_EOF, 1, 28, f) != 28) rc = HM_ERR_ARG;
-  if (f) fclose(f);
-  /* BAI: bins (adjacent records of one bin merged into one chunk) + 16 kb linear index */
+  FILE* f = fopen(path, "wb");
+  uint64_t* coff = NULL;
+  rc = f ? bgzf_write(f, w.p, w.n, level, threads, &coff) : HM_ERR_ARG;
+  if (f && fclose(f)) rc = HM_ERR_ARG;
+  /* the index: bins (adjacent records of one bin merged into one chunk) + linear index of 2^min_shift windows.  A BAI
+   * keeps the linear index; a CSI keeps, per bin, the linear-index entry of its first window (its loffset, as htslib's
+   * update_loff sets it) and comes BGZF-compressed. */
+  bchunk_t* ch = NULL;
+  uint64_t* lin = NULL;
+  wbuf_t x; memset(&x, 0, sizeof(x));
   if (!rc) {
 #define VOFF(o) ((coff[(o) / WBLK] << 16) | (uint64_t)((o) % WBLK))
-    const int32_t n_lin = contig_len > 0 ? ((contig_len - 1) >> 14) + 1 : 0;
-    uint64_t* lin = (uint64_t*)calloc((size_t)n_lin + 1, 8);
-    typedef struct { uint32_t bin; uint64_t beg, end; } bchunk_t;
-    bchunk_t* ch = (bchunk_t*)malloc((n + 1) * sizeof(bchunk_t));
+    int64_t n_lin = 0;
+    for (size_t r = 0; r < n; r++) if (((int64_t)rec_end[r] - 1) >> min_shift >= n_lin) n_lin = (((int64_t)rec_end[r] - 1) >> min_shift) + 1;
+    if (!csi && contig_len > 0) n_lin = (((int64_t)contig_len - 1) >> 14) + 1;
+    lin = (uint64_t*)calloc((size_t)n_lin + 1, 8);
+    ch = (bchunk_t*)malloc((n + 1) * sizeof(bchunk_t));
+    if (!lin || !ch) rc = HM_ERR_ARG;
     size_t nch = 0;
-    for (size_t r = 0; r < n; r++) {
-      const int32_t pos = b->tstart[r], endp = rec_end[r];
+    for (size_t r = 0; r < n && !rc; r++) {
+      const int64_t pos = b->tstart[r], endp = rec_end[r];
       const uint64_t v0 = VOFF(rec_off[r]), v1 = VOFF(rec_off[r + 1]);
-      const uint32_t bin = (uint32_t)reg2bin(pos, endp);
+      const uint32_t bin = reg2bin(pos, endp, min_shift, depth);
       if (nch && ch[nch - 1].bin == bin && ch[nch - 1].end == v0) ch[nch - 1].end = v1;
-      else { ch[nch].bin = bin; ch[nch].beg = v0; ch[nch].end = v1; nch++; }
-      for (int32_t wv = pos >> 14; wv <= ((endp - 1) >> 14) && wv < n_lin; wv++) if (!lin[wv]) lin[wv] = v0;
+      else { ch[nch].bin = bin; ch[nch].beg = v0; ch[nch].end = v1; ch[nch].i = nch; nch++; }
+      for (int64_t wv = pos >> min_shift; wv <= ((endp - 1) >> min_shift) && wv < n_lin; wv++) if (!lin[wv]) lin[wv] = v0;
     }
-    /* group chunks by bin (stable insertion into per-bin lists via a sort on (bin, order)) */
-    size_t* order = (size_t*)malloc((nch + 1) * sizeof(size_t));
-    for (size_t i = 0; i < nch; i++) order[i] = i;
-    /* counting sort by bin (bins < 37450) */
-    uint32_t* cnt = (uint32_t*)calloc(37451, 4);
-    for (size_t i = 0; i < nch; i++) cnt[ch[i].bin + 1]++;
-    for (int i = 0; i < 37450; i++) cnt[i + 1] += cnt[i];
-    for (size_t i = 0; i < nch; i++) order[cnt[ch[i].bin]++] = i;
-    size_t lp = strlen(path);
-    char* ip = (char*)malloc(lp + 5); memcpy(ip, path, lp); memcpy(ip + lp, ".bai", 5);
-    FILE* g = fopen(ip, "wb");
-    free(ip);
-    if (!g) rc = HM_ERR_ARG;
-    else {
-      wbuf_t x; memset(&x, 0, sizeof(x));
-      wb_need(&x, 64 + nch * 28 + (size_t)n_lin * 8);
-      memcpy(x.p, "BAI\1", 4); x.n = 4; wb_u32(&x, 1);
+    if (!rc) {
+      /* windows no record overlaps: a CSI (htslib) takes the contig's first record before the first one that has an
+       * entry and the entry to the left after it; the BAI keeps 0 before the first entry */
+      uint64_t last = csi && n ? VOFF(rec_off[0]) : 0;
+      for (int64_t k = 0; k < n_lin; k++) { if (lin[k]) last = lin[k]; else lin[k] = last; }
+      qsort(ch, nch, sizeof(bchunk_t), cmp_chunk);
       uint32_t n_bins = 0;
-      for (size_t i = 0; i < nch; i++) if (i == 0 || ch[order[i]].bin != ch[order[i - 1]].bin) n_bins++;
-      wb_u32(&x, n_bins);
+      for (size_t i = 0; i < nch; i++) if (i == 0 || ch[i].bin != ch[i - 1].bin) n_bins++;
+      if (wb_need(&x, 128 + nch * 28 + (size_t)n_bins * 8 + (size_t)n_lin * 8)) rc = HM_ERR_ARG;
+    }
+    if (!rc) {
+      memcpy(x.p, csi ? "CSI\1" : "BAI\1", 4); x.n = 4;
+      if (csi) { wb_u32(&x, (uint32_t)min_shift); wb_u32(&x, (uint32_t)depth); wb_u32(&x, 0); }
+      wb_u32(&x, 1);
+      uint32_t n_bins = 0;
+      for (size_t i = 0; i < nch; i++) if (i == 0 || ch[i].bin != ch[i - 1].bin) n_bins++;
+      wb_u32(&x, n_bins + (csi && nch ? 1 : 0));
       for (size_t i = 0; i < nch;) {
         size_t j = i;
-        while (j < nch && ch[order[j]].bin == ch[order[i]].bin) j++;
-        wb_u32(&x, ch[order[i]].bin); wb_u32(&x, (uint32_t)(j - i));
+        while (j < nch && ch[j].bin == ch[i].bin) j++;
+        wb_u32(&x, ch[i].bin);
+        if (csi) {
+          const int64_t bot = bin_start(ch[i].bin, min_shift, depth) >> min_shift;
+          const uint64_t loff = bot < n_lin ? lin[bot] : 0;
+          wb_u32(&x, (uint32_t)loff); wb_u32(&x, (uint32_t)(loff >> 32));
+        }
+        wb_u32(&x, (uint32_t)(j - i));
         for (size_t k = i; k < j; k++) {
-          const uint64_t a = ch[order[k]].beg, e = ch[order[k]].end;
+          const uint64_t a = ch[k].beg, e = ch[k].end;
           wb_u32(&x, (uint32_t)a); wb_u32(&x, (uint32_t)(a >> 32)); wb_u32(&x, (uint32_t)e); wb_u32(&x, (uint32_t)(e >> 32));
         }
         i = j;
       }
-      wb_u32(&x, (uint32_t)n_lin);
-      uint64_t last = 0;
-      for (int32_t k = 0; k < n_lin; k++) { if (lin[k]) last = lin[k]; const uint64_t v = lin[k] ? lin[k] : last; wb_u32(&x, (uint32_t)v); wb_u32(&x, (uint32_t)(v >> 32)); }
-      wb_u32(&x, 0); wb_u32(&x, 0);
-      if (fwrite(x.p, 1, x.n, g) != x.n) rc = HM_ERR_ARG;
-      fclose(g); free(x.p);
-    }
-    free(lin); free(ch); free(order); free(cnt);
+      if (csi) {
+        if (nch) { /* the pseudo-bin: the contig's first and last offsets, then mapped and unmapped record counts */
+          const uint64_t pv[4] = {VOFF(rec_off[0]), VOFF(rec_off[n]), (uint64_t)n, 0};
+          wb_u32(&x, pseudo_bin(depth)); wb_u32(&x, 0); wb_u32(&x, 0); wb_u32(&x, 2);
+          for (int k = 0; k < 4; k++) { wb_u32(&x, (uint32_t)pv[k]); wb_u32(&x, (uint32_t)(pv[k] >> 32)); }
+        }
+      } else {
+        wb_u32(&x, (uint32_t)n_lin);
+        for (int64_t k = 0; k < n_lin; k++) { wb_u32(&x, (uint32_t)lin[k]); wb_u32(&x, (uint32_t)(lin[k] >> 32)); }
+      }
+      wb_u32(&x, 0); wb_u32(&x, 0); /* n_no_coor */
 #undef VOFF
+      char* ip = path_with(path, strlen(path), csi ? ".csi" : ".bai");
+      FILE* g = ip ? fopen(ip, "wb") : NULL;
+      free(ip);
+      if (!g) rc = HM_ERR_ARG;
+      else {
+        if (csi) rc = bgzf_write(g, x.p, x.n, level, 1, NULL);
+        else if (fwrite(x.p, 1, x.n, g) != x.n) rc = HM_ERR_ARG;
+        if (fclose(g)) rc = HM_ERR_ARG;
+      }
+    }
   }
-  free(w.p); free(rec_off); free(rec_end); free(job.dst); free(job.csize); free(coff);
+  free(lin); free(ch); free(x.p);
+  free(w.p); free(rec_off); free(rec_end); free(coff);
   return rc;
 }
 

@@ -605,7 +605,7 @@ __global__ void __launch_bounds__(256) k_span_ranges(DevBatch b, const hm_chunk*
   const uint32_t c = upper_bound_dev(span_off, n_chunks + 1, span) - 1;
   const hm_chunk ch = chunks[c];
   const int32_t s0 = (int32_t)(((uint32_t)(ch.start >> 10) + (uint32_t)(span - __ldg(span_off + c))) << 10);
-  const int32_t lo_pos = max(s0, ch.start), hi_pos = min(s0 + NB_SPAN, ch.end);
+  const int32_t lo_pos = max(s0, ch.start), hi_pos = (int32_t)min((int64_t)s0 + NB_SPAN, (int64_t)ch.end); // s0 + NB_SPAN reaches 2^31
   const uint32_t n_in = ch.read_hi - ch.read_lo;
   const uint32_t r_lo = ch.read_lo + count_le_kary_i32(b.pmax_tend + ch.read_lo, n_in, lo_pos);
   const uint32_t r_hi = ch.read_lo + count_le_kary_i32(b.tstart + ch.read_lo, n_in, hi_pos - 1);
@@ -635,7 +635,7 @@ __global__ void __launch_bounds__(32 * NB_BITS_WARPS, kPhase ? 4 : 6) k_norm_bit
     const uint32_t c = si.x, r_lo = si.z, r_hi = si.w;
     const hm_chunk ch = chunks[c];
     const int32_t s0 = (int32_t)si.y;
-    const int32_t lo_pos = max(s0, ch.start), hi_pos = min(s0 + NB_SPAN, ch.end);
+    const int32_t lo_pos = max(s0, ch.start), hi_pos = (int32_t)min((int64_t)s0 + NB_SPAN, (int64_t)ch.end); // s0 + NB_SPAN reaches 2^31
     const bool deep = r_hi > r_lo && r_hi - r_lo > 255u; // the 8-bit counters would overflow: every position to the exact pass
     const uint64_t pbase = __ldg(pair_off + c);
     const int32_t P0 = s0 + 32 * lane;

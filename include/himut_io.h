@@ -26,11 +26,21 @@ extern "C" {
 
 typedef struct hm_bam hm_bam;
 
-/* open <path> (and <path>.bai when it exists: without it every query scans from the first
- * record), read the header text and the @SQ table (bamlib.get_tname2tsize, bamlib.py:109-129) */
+/* open <path>, read the header text and the @SQ table (bamlib.get_tname2tsize, bamlib.py:109-129) and the first index
+ * found of <path>.bai, <path>.csi, then for x.bam x.bai and x.csi (the names htslib finds; a BAI first, so a file
+ * with both is read as before).  Without an index every query scans from the first record.  An index that cannot be
+ * read fails the open (HM_ERR_ARG) with a message that names it: a bad magic, a truncation, a count that runs past its
+ * data; for a CSI also a span 2^(min_shift + 3 depth) shorter than a contig's @SQ LN, a bin past the pseudo-bin and a
+ * chunk that begins after its end. */
 int hm_bam_open(const char* path, hm_bam** out);
 void hm_bam_close(hm_bam* b);
+/* the message of the handle's last failure; NULL: why the calling thread's last hm_bam_open failed */
 const char* hm_bam_error(const hm_bam* b);
+/* which index hm_bam_open read */
+#define HM_BAM_INDEX_NONE 0
+#define HM_BAM_INDEX_BAI 1
+#define HM_BAM_INDEX_CSI 2
+int hm_bam_index_kind(const hm_bam* b);
 
 const char* hm_bam_header_text(const hm_bam* b); /* SAM header text, as str(alignments.header) */
 int hm_bam_n_refs(const hm_bam* b);
@@ -84,7 +94,7 @@ int hm_bam_last_compact(hm_bam* b, hm_bq_compact* out);
  * record headers, CIGARs and tags are parsed.  HM_ERR_CAPACITY when cap is too small (*n_out = needed). */
 int hm_bam_window_qlens(hm_bam* b, int rid, int32_t start, int32_t end, int threads, int32_t* out, size_t cap, size_t* n_out);
 
-/* tests / tools / bench only: a packed batch back to a coordinate-sorted BAM + BAI (cs:Z short form, tp:A:P,
+/* tests / tools / bench only: a packed batch back to a single-contig coordinate-sorted BAM + BAI (cs:Z short form, tp:A:P,
  * query names "read<qname_id>"), BGZF blocks deflated on `threads` threads at zlib `level` */
 int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                        int level, int threads);
@@ -100,6 +110,13 @@ int hm_bam_write_batch(const char* path, const char* chrom, int32_t contig_len, 
 #define HM_BAM_TAGS_M 4
 int hm_bam_write_batch_tags(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
                             int level, int threads, int tags);
+/* the same with the index chosen: min_shift == 0 writes <path>.bai (HM_ERR_ARG for a contig longer than 2^29, which a
+ * BAI cannot bin); min_shift > 0 writes <path>.csi instead, BGZF-compressed, as htslib writes it (per bin the
+ * linear-index offset of its first window as loffset, the pseudo-bin, n_no_coor), with `depth` levels, or with the
+ * smallest depth whose span holds the contig plus 256 when depth <= 0.  The records' BAI bin field is 4680, which
+ * cannot be right, for records that end past 2^29. */
+int hm_bam_write_batch_index(const char* path, const char* chrom, int32_t contig_len, const char* sample, const hm_read_batch* b,
+                             int level, int threads, int tags, int min_shift, int depth);
 
 /* compact quality stream of a packed batch (struct hm_bq_compact, himut_b200.h), for the host -> device copy: `mask` (bq_bytes / 8 bytes) and
  * `exc_off` (n_reads + 1 entries) are caller allocated, the exception bytes are allocated here (*exc_out, release
@@ -109,10 +126,12 @@ int hm_bq_compact_build(const hm_read_batch* b, int threads, uint8_t* mask, uint
 void hm_bq_compact_free(uint8_t* exc);
 
 /* plan of the records hm_bam_read_batch would visit for [start, end) of contig `rid`, for the device decoder
- * (hm_decode_bam_begin of himut_b200.h): nothing is inflated.  The range starts at the BAI linear-index entry
- * hm_bam_read_batch seeks to and ends at the largest chunk end of the BAI bins that overlap the region; the entry
- * points are the linear-index entries of the windows the region covers.  Without a BAI: one entry point at the first
- * record and the range runs to the end of the file.  An empty contig gives n_entry = 0.  The arrays (and the
+ * (hm_decode_bam_begin of himut_b200.h): nothing is inflated.  The range starts where hm_bam_read_batch seeks to (BAI:
+ * the linear-index entry of start's window; CSI: the loffset of the bin htslib's query starts from) and ends at the
+ * largest chunk end of the bins that overlap the region, and no later than the first chunk of a bin that starts at or
+ * past `end`.  The later entry points are, for a BAI, the linear-index entries of the windows the region covers and,
+ * for a CSI, the loffsets of the bins of any level that start inside it.  Without an index: one entry point at the
+ * first record and the range runs to the end of the file.  An empty contig gives n_entry = 0.  The arrays (and the
  * compressed range, when the file is not mapped) belong to the handle until its next plan. */
 int hm_bam_region_plan(hm_bam* b, int rid, int32_t start, int32_t end, hm_bgzf_plan* out);
 /* the ids of `n` NUL-terminated names (name i at blob + off[i]) in the handle's query-name table: the ids

@@ -12,7 +12,7 @@ gcc $SAN -Iinclude -o oracle/libhimut_oracle.so oracle/himut_oracle.c -lm
 LD_PRELOAD="$(gcc -print-file-name=libasan.so):$(gcc -print-file-name=libubsan.so)" ASAN_OPTIONS=detect_leaks=0 UBSAN_OPTIONS=print_stacktrace=1 \
   python -m pytest tests/test_bamdec.py tests/test_inflate.py tests/test_thresholds.py tests/test_host.py tests/test_worker_host.py \
   tests/test_oracle_golden.py tests/test_oracle_random.py tests/test_kat.py tests/test_edges.py tests/test_reflib.py \
-  tests/test_deflate_conformance.py tests/test_bam_writers.py tests/test_ref_ops.py -q -s -m "not gpu" > /tmp/sanitize_host.log 2>&1 || true
+  tests/test_deflate_conformance.py tests/test_bam_writers.py tests/test_ref_ops.py tests/test_csi.py -q -s -m "not gpu" > /tmp/sanitize_host.log 2>&1 || true
 tail -2 /tmp/sanitize_host.log
 echo "sanitizer reports: $(grep -c 'runtime error\|AddressSanitizer' /tmp/sanitize_host.log || true)"
 grep -A6 'runtime error\|AddressSanitizer' /tmp/sanitize_host.log || true
