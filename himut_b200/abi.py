@@ -115,6 +115,15 @@ SITE_DTYPE = np.dtype([
 ])
 assert SITE_DTYPE.itemsize == C.sizeof(hm_site_record)
 
+class hm_callable_run(C.Structure):
+    _fields_ = [("chunk", C.c_uint32), ("start", C.c_int32), ("end", C.c_int32), ("value", C.c_uint32)]
+
+
+# runs of the callable-base track (hm_last_callable_runs): positions [start, end) of chunk `chunk`, each counted with
+# `value` callable read bases
+RUN_DTYPE = np.dtype([("chunk", "<u4"), ("start", "<i4"), ("end", "<i4"), ("value", "<u4")])
+assert RUN_DTYPE.itemsize == C.sizeof(hm_callable_run)
+
 CHUNK_DTYPE = np.dtype([("start", "<i4"), ("end", "<i4"), ("read_lo", "<u4"), ("read_hi", "<u4"),
                         ("phase_set", "<i4"), ("reserved", "<i4")])
 assert CHUNK_DTYPE.itemsize == C.sizeof(hm_chunk)

@@ -27,6 +27,7 @@
 #include "normfast.cuh"
 #include "callfused.cuh"
 #include "normbits.cuh"
+#include "normtrack.cuh"
 #include "bamgpu.cuh"
 
 #define HM_BOUNDARY_CAP_DEFAULT 65536   // boundary records the device list holds (HIMUT_B200_BOUNDARY_CAP overrides: tests)
@@ -177,6 +178,11 @@ struct hm_ctx {
   uint64_t packed_pos = 0;                  // positions b_ref2 / b_tri8 cover for the reference now in b_ref (0: not packed)
   DevBuf b_cw_off, b_calw, b_impure, b_ref2, b_tri8, b_thr, b_span_off, b_exc_minmax, b_sdiff, b_cal_ok;
   bool compact_resident = false;            // the resident batch came as bitmap + exceptions: both are still on the device
+  // callable-base track of normcounts (HM_OPT_CALLABLE_TRACK, normtrack.cuh)
+  bool callable_track = false;
+  DevBuf b_track, b_track_off, b_track_cnt, b_track_runs;
+  uint64_t track_runs = 0;                  // runs of the last normcounts call (in b_track_runs)
+  unsigned long long* h_track_pin = nullptr; // mapped: the run count
   uint32_t modal = 0;
   // device BAM decoder (hm_decode_bam_*, bamgpu.cuh)
   DevBuf b_comp, b_pcoff, b_pcsize, b_pisize, b_puoff, b_pcrc, b_pentry, b_inflated, b_blk_code, b_derr, b_seg_cnt,
@@ -383,6 +389,7 @@ size_t hm_abi_sizeof(int which) {
     case 3: return sizeof(hm_site_record);
     case 4: return sizeof(hm_bq_compact);
     case 5: return sizeof(hm_bgzf_plan);
+    case 6: return sizeof(hm_callable_run);
     default: return 0;
   }
 }
@@ -431,6 +438,7 @@ void hm_destroy(hm_ctx* ctx) {
                     &ctx->b_records, &ctx->b_counters, &ctx->b_ref, &ctx->b_norm_out, &ctx->b_lut, &ctx->b_tile_off, &ctx->b_agg, &ctx->b_geom, &ctx->b_bidx, &ctx->b_brecs, &ctx->b_sites, &ctx->b_push, &ctx->b_span_cnt, &ctx->b_koff, &ctx->b_tile_info, &ctx->b_edge_counts, &ctx->b_edge_hpos, &ctx->b_edge_href, &ctx->b_bqmask, &ctx->b_bqexc, &ctx->b_bqexc_off,
                     &ctx->b_cgeom, &ctx->b_seg_keys, &ctx->b_seg_read, &ctx->b_keys_tmp, &ctx->b_gscratch, &ctx->b_czero, &ctx->b_tiles, &ctx->b_pair_c,
                     &ctx->b_cw_off, &ctx->b_calw, &ctx->b_impure, &ctx->b_ref2, &ctx->b_tri8, &ctx->b_thr, &ctx->b_span_off, &ctx->b_exc_minmax, &ctx->b_sdiff, &ctx->b_cal_ok,
+                    &ctx->b_track, &ctx->b_track_off, &ctx->b_track_cnt, &ctx->b_track_runs,
                     &ctx->b_comp, &ctx->b_pcoff, &ctx->b_pcsize, &ctx->b_pisize, &ctx->b_puoff, &ctx->b_pcrc, &ctx->b_pentry, &ctx->b_inflated,
                     &ctx->b_blk_code, &ctx->b_derr, &ctx->b_seg_cnt, &ctx->b_seg_off, &ctx->b_recoff, &ctx->b_recinfo, &ctx->b_cnt,
                     &ctx->b_scan, &ctx->b_ecode, &ctx->b_earg, &ctx->b_names, &ctx->b_name_off, &ctx->b_reflist};
@@ -438,6 +446,7 @@ void hm_destroy(hm_ctx* ctx) {
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_cnt_pin) cudaFreeHost(ctx->h_cnt_pin);
   if (ctx->h_geom_pin) cudaFreeHost(ctx->h_geom_pin);
+  if (ctx->h_track_pin) cudaFreeHost(ctx->h_track_pin);
   ctx->h_pmax.release(); ctx->h_cw_off.release();
   ctx->hd_tstart.release(); ctx->hd_tend.release(); ctx->hd_qstart.release(); ctx->hd_qlen.release(); ctx->hd_n_ops.release();
   ctx->hd_bq_off.release(); ctx->hd_op_off.release(); ctx->hd_name_off.release(); ctx->hd_seq_off.release(); ctx->hd_scal.release(); ctx->hd_names.release();
@@ -928,6 +937,7 @@ int hm_set_option(hm_ctx* ctx, int option, int value) {
   if (!ctx) return HM_ERR_ARG;
   if (option == HM_OPT_OMIT_RESTATEMENTS) { ctx->omit_restatements = value != 0; return HM_OK; }
   if (option == HM_OPT_KERNEL_TIMING) { ctx->ktiming = value != 0; return HM_OK; }
+  if (option == HM_OPT_CALLABLE_TRACK) { ctx->callable_track = value != 0; return HM_OK; }
   return fail(ctx, HM_ERR_ARG, "unknown option %d", option);
 }
 
@@ -1571,6 +1581,19 @@ int hm_normcounts_chunks(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len, con
   return hm_normcounts_impl(ctx, refseq, ref_len, chunks, n_chunks, ccs_tri, ref_tri, log, n_alt_tie);
 }
 
+/* runs of the callable-base track of the last hm_normcounts_chunks (HM_OPT_CALLABLE_TRACK), without recomputing */
+int hm_last_callable_runs(hm_ctx* ctx, hm_callable_run* out, size_t cap, size_t* n) {
+  if (!ctx || !n) return HM_ERR_ARG;
+  *n = (size_t)ctx->track_runs;
+  if (cap < *n || (!out && *n)) return fail(ctx, HM_ERR_CAPACITY, "output holds %zu runs, %zu needed", cap, *n);
+  if (*n) {
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaMemcpyAsync(out, ctx->b_track_runs.p, *n * sizeof(hm_callable_run), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+  }
+  return HM_OK;
+}
+
 /* per-qname_id flags of the last call: 1 where some record with that id passed the read gates in
  * a chunk that fetched it (the reads m.num_ccs counts, caller.py:318-320) */
 int hm_qname_seen(hm_ctx* ctx, uint8_t* out, size_t cap, size_t* n) {
@@ -1856,6 +1879,7 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
   memset(log, 0, sizeof(int64_t) * HM_NORM_LOG_LEN);
   if (n_alt_tie) *n_alt_tie = 0;
   ctx->last_norm_sites = 0;
+  ctx->track_runs = 0;
   t_reset(ctx);
   std::vector<uint64_t> pair_off;
   int rc = upload_chunks(ctx, chunks, n_chunks, pair_off);
@@ -1888,6 +1912,31 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     max_end = std::max<int64_t>(max_end, chunks[i].end);
   }
   const uint64_t n_spans = span_off[n_chunks];
+  // callable track (normtrack.cuh): chunk c owns slots [track_off[c], track_off[c + 1]) — its positions from its start,
+  // padded to a multiple of 32 — read back in pieces of 1024 slots (piece_off, uploaded behind track_off)
+  const bool track = ctx->callable_track;
+  std::vector<uint64_t> track_off;
+  uint64_t n_pieces = 0;
+  uint32_t* track_buf = nullptr;
+  const uint64_t* track_off_d = nullptr;
+  if (track) {
+    track_off.assign(2 * (n_chunks + 1), 0);
+    uint64_t* piece_off = track_off.data() + n_chunks + 1;
+    for (size_t i = 0; i < n_chunks; i++) {
+      const int64_t len = (int64_t)chunks[i].end - (int64_t)chunks[i].start;
+      const uint64_t slots = len > 0 ? (uint64_t)((len + 31) & ~31ll) : 0;
+      track_off[i + 1] = track_off[i] + slots;
+      piece_off[i + 1] = piece_off[i] + (slots + NB_SPAN - 1) / NB_SPAN;
+    }
+    const uint64_t n_slots = track_off[n_chunks];
+    n_pieces = piece_off[n_chunks];
+    if (n_slots >= (1ull << 32)) return fail(ctx, HM_ERR_ARG, "callable track: %llu positions in one call, at most 2^32 - 1", (unsigned long long)n_slots);
+    if ((rc = upload(ctx, ctx->b_track_off, track_off.data(), track_off.size()))) return rc;
+    CU(ctx->b_track.ensure(n_slots * 4 + 16));
+    CU(cudaMemsetAsync(ctx->b_track.p, 0, n_slots * 4, ctx->stream));
+    track_buf = ctx->b_track.as<uint32_t>();
+    track_off_d = ctx->b_track_off.as<uint64_t>();
+  }
   uint64_t imp_words = 0;
   if (use_bits) {
     const uint64_t need_pos = std::max<uint64_t>(std::max<uint64_t>((uint64_t)ref_len, (uint64_t)std::max(ctx->h_pmax.back(), 0) + 2), (uint64_t)max_end);
@@ -1941,18 +1990,19 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, ctx->device);
     if (!use_bits) {
       const size_t smem = sizeof(TileStage) * HM_NSTAGE;
-      static bool attr_set = false;
-      if (!attr_set) {
-        CU(cudaFuncSetAttribute(k_norm_tiles_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
+      static bool attr_set[2] = {false, false};
+      const auto k_tiles = track ? k_norm_tiles_tma<true> : k_norm_tiles_tma<false>;
+      if (!attr_set[track]) {
+        CU(cudaFuncSetAttribute(k_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_set[track] = true;
       }
       const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles, (uint64_t)n_sm);
       t_begin(ctx, "k_norm_tiles_tma");
-      k_norm_tiles_tma<<<grid, HM_TW + 32 * HM_NPROD, smem, ctx->stream>>>(ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(),
+      k_tiles<<<grid, HM_TW + 32 * HM_NPROD, smem, ctx->stream>>>(ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(),
                                                                 (uint32_t)n_chunks, ctx->b_pair_off.as<uint64_t>(),
                                                                 ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_off.as<uint64_t>(),
                                                                 (uint32_t)n_tiles, ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len,
-                                                                ctx->b_norm_out.as<NormOut>());
+                                                                ctx->b_norm_out.as<NormOut>(), track_buf, track_off_d);
       t_end(ctx);
     } else {
       // bit-vector pass over every position, then the exact pass over the listed sites
@@ -1975,11 +2025,13 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
         uint32_t* span_cnt = ctx->b_span_cnt.as<uint32_t>();
         uint32_t* span_dst = span_cnt + n_spans;
         t_begin(ctx, "k_norm_bits");
-        (ctx->params.phase ? k_norm_bits<true> : k_norm_bits<false>)<<<bgrid, 32 * NB_BITS_WARPS, 0, ctx->stream>>>(
+        const auto k_bits = ctx->params.phase ? (track ? k_norm_bits<true, true> : k_norm_bits<true, false>)
+                                              : (track ? k_norm_bits<false, true> : k_norm_bits<false, false>);
+        k_bits<<<bgrid, 32 * NB_BITS_WARPS, 0, ctx->stream>>>(
             ctx->db, ctx->dp, ctx->b_thr.as<uint16_t>(), (int)ctx->cert.n_min, md_k, ctx->b_chunks.as<hm_chunk>(), (uint32_t)n_chunks,
             ctx->b_pair_off.as<uint64_t>(), ctx->b_pair_hap.as<uint8_t>(), ctx->b_tile_info.as<uint4>(), n_spans, ctx->b_cw_off.as<uint32_t>(),
             ctx->b_calw.as<uint32_t>(), ctx->b_impure.as<uint32_t>(), ctx->b_tri8.as<uint8_t>(), ctx->b_norm_out.as<NormOut>(),
-            ctx->b_push.as<uint32_t>(), span_cnt);
+            ctx->b_push.as<uint32_t>(), span_cnt, track_buf, track_off_d);
         t_end(ctx);
         CU(cudaGetLastError());
         t_begin(ctx, "k_emit_sites");
@@ -2022,10 +2074,10 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
             ctx->b_ref2.as<uint32_t>(), ctx->compact_resident ? ctx->b_bqmask.as<uint16_t>() : nullptr, ctx->modal, n_slots);
         t_end(ctx);
         t_begin(ctx, "k_norm_reduce");
-        k_norm_reduce<<<(unsigned)((nb + 127) / 128), 128, 0, ctx->stream>>>(
+        (track ? k_norm_reduce<true> : k_norm_reduce<false>)<<<(unsigned)((nb + 127) / 128), 128, 0, ctx->stream>>>(
             ctx->db, ctx->dp, ctx->dsets, ctx->dlut, ctx->b_chunks.as<hm_chunk>(), ctx->b_pair_off.as<uint64_t>(),
             ctx->b_pair_hap.as<uint8_t>(), keys, nb, site_lo, site_n, entries, stride, ctx->b_ref.as<uint8_t>(), (uint64_t)ref_len,
-            ctx->b_norm_out.as<NormOut>(), n_slots);
+            ctx->b_norm_out.as<NormOut>(), n_slots, track_buf, track_off_d);
         t_end(ctx);
         CU(cudaGetLastError());
       }
@@ -2036,12 +2088,47 @@ static int hm_normcounts_impl(hm_ctx* ctx, const uint8_t* refseq, size_t ref_len
                                                 ctx->b_counters.as<unsigned long long>() + 2);
     t_end(ctx);
     CU(cudaGetLastError());
+    if (track && n_pieces) {
+      // the track as runs: begin / end counts per piece, their scans (the run total lands in mapped memory), records
+      const uint64_t* piece_off_d = track_off_d + n_chunks + 1;
+      CU(ctx->b_track_cnt.ensure((4 * n_pieces + 2) * 4 + 16));
+      uint32_t* bcnt = ctx->b_track_cnt.as<uint32_t>();
+      uint32_t* ecnt = bcnt + n_pieces;
+      uint32_t* bdst = ecnt + n_pieces;
+      uint32_t* edst = bdst + n_pieces + 1;
+      if (!ctx->h_track_pin) CU(cudaHostAlloc((void**)&ctx->h_track_pin, 16, cudaHostAllocMapped));
+      unsigned long long* d_pin = nullptr;
+      CU(cudaHostGetDevicePointer((void**)&d_pin, ctx->h_track_pin, 0));
+      const unsigned tgrid = (unsigned)((n_pieces * 32 + 255) / 256);
+      t_begin(ctx, "k_track_count");
+      k_track_count<<<tgrid, 256, 0, ctx->stream>>>(track_buf, track_off_d, piece_off_d, (uint32_t)n_chunks, ctx->b_chunks.as<hm_chunk>(),
+                                                    n_pieces, bcnt, ecnt);
+      k_span_scan<<<1, 1024, 0, ctx->stream>>>(bcnt, n_pieces, bdst, d_pin);
+      k_span_scan<<<1, 1024, 0, ctx->stream>>>(ecnt, n_pieces, edst, d_pin + 1);
+      t_end(ctx);
+      CU(cudaGetLastError());
+      CU(cudaStreamSynchronize(ctx->stream));
+      const uint64_t n_runs = ctx->h_track_pin[0];
+      if (ctx->h_track_pin[1] != n_runs) return fail(ctx, HM_ERR_CUDA, "callable track: %llu runs begin, %llu end", ctx->h_track_pin[0], ctx->h_track_pin[1]);
+      if (n_runs) {
+        CU(ctx->b_track_runs.ensure(n_runs * sizeof(hm_callable_run)));
+        t_begin(ctx, "k_track_emit");
+        k_track_emit<<<tgrid, 256, 0, ctx->stream>>>(track_buf, track_off_d, piece_off_d, (uint32_t)n_chunks, ctx->b_chunks.as<hm_chunk>(),
+                                                     n_pieces, bdst, edst, ctx->b_track_runs.as<uint32_t>());
+        t_end(ctx);
+        CU(cudaGetLastError());
+      }
+      ctx->track_runs = n_runs;
+    }
     CU(cudaMemcpyAsync(&h, ctx->b_norm_out.p, sizeof(NormOut), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaMemcpyAsync(h_cnt, ctx->b_counters.p, 32, cudaMemcpyDeviceToHost, ctx->stream));
   }
   CU(cudaStreamSynchronize(ctx->stream));
   t_collect(ctx);
-  if (h.err == HM_ERR_BQ_ZERO) return fail(ctx, HM_ERR_BQ_ZERO, "a base quality of 0 reached the genotype model (the reference raises ValueError: math.log10(0))");
+  if (h.err == HM_ERR_BQ_ZERO) {
+    ctx->track_runs = 0;
+    return fail(ctx, HM_ERR_BQ_ZERO, "a base quality of 0 reached the genotype model (the reference raises ValueError: math.log10(0))");
+  }
   for (int i = 0; i < HM_TRI_BINS; i++) { ccs_tri[i] = (int64_t)h.ccs_tri[i]; ref_tri[i] = (int64_t)h.ref_tri[i]; }
   for (int i = 1; i < HM_NORM_LOG_LEN; i++) log[i] = (int64_t)h.log[i];
   log[0] = (int64_t)h_cnt[2];

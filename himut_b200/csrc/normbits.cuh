@@ -614,12 +614,14 @@ __global__ void __launch_bounds__(256) k_span_ranges(DevBatch b, const hm_chunk*
 
 // thr[n]: the smallest callable count that certifies a pure position of depth n (host, make_norm_cert), 0xffff: none.
 // md_k: depth >= md_k is "read_depth > md_threshold" (256: never).
-template <bool kPhase>
+// kTrack: the callable count of every counted position also goes to the track (track_at, normcounts.cuh)
+template <bool kPhase, bool kTrack>
 __global__ void __launch_bounds__(32 * NB_BITS_WARPS, kPhase ? 4 : 6) k_norm_bits(DevBatch b, DevParams p, const uint16_t* thr, int n_min, int md_k, const hm_chunk* chunks,
                                                                    uint32_t n_chunks, const uint64_t* pair_off, const uint8_t* pair_flag,
                                                                    const uint4* span_info, uint64_t n_spans, const uint32_t* cw_off,
                                                                    const uint32_t* calw, const uint32_t* impure, const uint8_t* tri8,
-                                                                   NormOut* out, uint32_t* push_words, uint32_t* span_cnt) {
+                                                                   NormOut* out, uint32_t* push_words, uint32_t* span_cnt,
+                                                                   uint32_t* track, const uint64_t* track_off) {
   __shared__ unsigned long long s_ccs[HM_TRI_BINS], s_ref[HM_TRI_BINS], s_log[HM_NORM_LOG_LEN];
   __shared__ unsigned int s_wccs[NB_BITS_WARPS][HM_TRI_BINS + 1], s_wref[NB_BITS_WARPS][HM_TRI_BINS + 1];
   __shared__ uint16_t s_thr[256];
@@ -735,6 +737,7 @@ __global__ void __launch_bounds__(32 * NB_BITS_WARPS, kPhase ? 4 : 6) k_norm_bit
           const uint32_t tri = (tw[g] >> (8 * k)) & 255u;
           atomicAdd(&s_wref[wid][tri], 1u);
           atomicAdd(&s_wccs[wid][tri], (cw >> (8 * k)) & 255u);
+          if constexpr (kTrack) track[track_at(track_off, c, ch.start, P0 + 4 * g + k)] = (cw >> (8 * k)) & 255u;
         }
       }
     }

@@ -24,6 +24,14 @@ struct NormOut { // device tallies
   int err;
 };
 
+// Callable-base track (HM_OPT_CALLABLE_TRACK): one uint32 per position of every chunk, chunk-major — chunk c owns
+// [track_off[c], track_off[c + 1]), its positions from ch.start on, padded to a multiple of 32.  A counted position
+// holds the callable count update_tri2count gave it (>= 1), everything else stays 0.  Overlapping chunks do not share
+// a slot.  normtrack.cuh turns the buffer into runs.
+__device__ __forceinline__ uint64_t track_at(const uint64_t* track_off, uint32_t c, int32_t start, int32_t pos) {
+  return __ldg(track_off + c) + (uint64_t)((int64_t)pos - start);
+}
+
 // pair_flag bits
 #define HM_PF_FETCHED 1u
 #define HM_PF_PASS 2u
@@ -290,10 +298,16 @@ __device__ __forceinline__ int tri_bin3(uint8_t l, uint8_t m, uint8_t r, int64_t
   return t0 * 8 + (t1 == 3 ? 4 : 0) + t2;
 }
 
+// The dynamic shared memory every kernel of the library declares as smem_raw: its first declaration sets the alignment
+// for all of them, and a template's body is only seen when it is instantiated, so it is made here, at 128 bytes.
+extern __shared__ __align__(128) uint8_t smem_raw[];
+
+// kTrack: every counted position also stores its callable count into the track (track_at); nothing else changes
+template <bool kTrack>
 __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(DevBatch b, DevParams p, DevSets sets, DevLut lut, const hm_chunk* chunks,
                                                                    uint32_t n_chunks, const uint64_t* pair_off, const uint8_t* pair_flag,
                                                                    const uint64_t* tile_off, uint32_t n_tiles, const uint8_t* refseq,
-                                                                   uint64_t ref_len, NormOut* out) {
+                                                                   uint64_t ref_len, NormOut* out, uint32_t* track, const uint64_t* track_off) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   TileStage* stages = reinterpret_cast<TileStage*>(smem_raw);
   __shared__ double s_lut[3][256];
@@ -602,6 +616,7 @@ __global__ void __launch_bounds__(HM_TW + 32 * HM_NPROD, 1) k_norm_tiles_tma(Dev
       }
     }
     if (tri >= 0) { atomicAdd(&s_wref[tid >> 5][tri], 1u); atomicAdd(&s_wccs[tid >> 5][tri], (unsigned)callable); }
+    if constexpr (kTrack) { if (tri >= 0) track[track_at(track_off, c, ch.start, pos)] = (uint32_t)callable; }
     if (tie_alt) atomicAdd(&s_tie, 1ull);
     // move the warp's 32-bit bins into the CTA's 64-bit ones before they can overflow
     __syncwarp();

@@ -68,11 +68,14 @@ __device__ __forceinline__ uint32_t norm_entry(const DevBatch& b, const DevParam
   return a | (bq << 3) | ((uint32_t)min(ins, 255) << 11) | (((pf >> HM_PF_HAP_SHIFT) & 3u) << 19) | (cnt << 21);
 }
 
+// kTrack: a counted site also stores its callable count into the track (track_at, normcounts.cuh)
+template <bool kTrack>
 __global__ void __launch_bounds__(128) k_norm_reduce(DevBatch b, DevParams p, DevSets sets, DevLut lut, const hm_chunk* chunks,
                                                      const uint64_t* pair_off, const uint8_t* pair_flag,
                                                      const unsigned long long* keys, uint64_t n_keys, const uint32_t* site_lo,
                                                      const uint32_t* site_n, const uint32_t* entries, uint64_t stride,
-                                                     const uint8_t* refseq, uint64_t ref_len, NormOut* out, uint32_t n_slots) {
+                                                     const uint8_t* refseq, uint64_t ref_len, NormOut* out, uint32_t n_slots,
+                                                     uint32_t* track, const uint64_t* track_off) {
   __shared__ double s_lut[3][256];
   __shared__ unsigned long long s_ccs[HM_TRI_BINS], s_ref[HM_TRI_BINS], s_log[HM_NORM_LOG_LEN], s_tie;
   __shared__ int s_err;
@@ -171,6 +174,7 @@ __global__ void __launch_bounds__(128) k_norm_reduce(DevBatch b, DevParams p, De
         }
       }
     }
+    if constexpr (kTrack) { if (tri >= 0) track[track_at(track_off, c, ch.start, pos)] = (uint32_t)callable; }
   }
   {
     const unsigned cv = counted ? (unsigned)callable : 0u;

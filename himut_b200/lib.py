@@ -22,7 +22,7 @@ EXPORTS = [
     "hm_host_unregister", "hm_abi_sizeof", "hm_last_records", "hm_qname_seen", "hm_set_reference", "hm_ref_tricounts", "hm_last_norm_exact_sites",
     "hm_phase_edges_begin", "hm_phase_edges_add", "hm_phase_edges_end", "hm_upload_batch_compact", "hm_call_batch_compact", "hm_call_chunks_async", "hm_records_wait", "hm_set_option", "hm_last_call_path", "hm_call_chunks_submit", "hm_call_chunks_collect", "hm_device_count", "hm_upload_batch_compact_begin", "hm_upload_wait",
     "hm_decode_bam_begin", "hm_decode_bam_names", "hm_decode_bam_end", "hm_batch_read_back", "hm_inflate_device_test",
-    "hm_decode_bam_begin_opts", "hm_batch_read_back_seq",
+    "hm_decode_bam_begin_opts", "hm_batch_read_back_seq", "hm_last_callable_runs",
 ]
 
 
@@ -74,6 +74,7 @@ def load():
         lib.hm_set_reference.argtypes = [vp, vp, sz]
         lib.hm_ref_tricounts.argtypes = [vp, vp, sz, vp]
         lib.hm_last_norm_exact_sites.argtypes = [vp, C.POINTER(C.c_uint64)]
+        lib.hm_last_callable_runs.argtypes = [vp, vp, sz, C.POINTER(sz)]
         lib.hm_phase_edges_begin.argtypes = [vp, vp, vp, sz, C.c_uint32]
         lib.hm_phase_edges_add.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32)]
         lib.hm_phase_edges_end.argtypes = [vp, vp, sz]
@@ -361,6 +362,21 @@ class Context:
     def kernel_timing(self, on=True):
         """CUDA events around the kernels of a call (last_kernel_times); off saves a dozen driver calls per call"""
         self._chk(self.lib.hm_set_option(self.h, 2, 1 if on else 0))
+
+    def callable_track(self, on=True):
+        """normcounts_chunks also keeps the callable-base track (last_callable_runs); the tallies are the same"""
+        self._chk(self.lib.hm_set_option(self.h, 3, 1 if on else 0))
+
+    def last_callable_runs(self):
+        """runs of the callable-base track of the last normcounts_chunks (callable_track on; else none) -> abi.RUN_DTYPE
+        array: positions [start, end) of chunk `chunk` of that call's table, each counted with `value` callable bases"""
+        n = C.c_size_t(0)
+        rc = self.lib.hm_last_callable_runs(self.h, None, 0, C.byref(n))
+        if rc != abi.HM_ERR_CAPACITY:
+            self._chk(rc)
+        out = np.zeros(n.value, abi.RUN_DTYPE)
+        self._chk(self.lib.hm_last_callable_runs(self.h, _p(out), out.size, C.byref(n)))
+        return out
 
     def records_wait(self):
         self._chk(self.lib.hm_records_wait(self.h))

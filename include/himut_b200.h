@@ -226,6 +226,19 @@ typedef struct hm_site_record {
   int32_t phase_set;   /* --phase: chunk_start of the phase set for PASS rows, else -1       */
 } hm_site_record;
 
+/* One run of the callable-base track of hm_normcounts_chunks (HM_OPT_CALLABLE_TRACK): positions [start, end) (0-based)
+ * of chunk `chunk` (index into that call's chunk list) are all counted into the trinucleotide tallies, each with
+ * `value` callable read bases — the number ccs_callable_tri2count receives there (>= 1).  Runs are maximal, never
+ * cross a chunk, and come in chunk order, then position order; a position of two overlapping chunks appears in both,
+ * as the tallies count it.  So per trinucleotide bin, sum(end - start) = ref_tri and sum(value * (end - start)) =
+ * ccs_tri, and sum(value * (end - start)) over all runs = log[13].                                               */
+typedef struct hm_callable_run {
+  uint32_t chunk;
+  int32_t start;
+  int32_t end;
+  uint32_t value;
+} hm_callable_run;
+
 /* chrom2tsbs_log[chrom] (caller.py:625-641), same order */
 #define HM_CALL_LOG_LEN 15
 /* chrom2norm_log[chrom] (normcounts.py:404-419), same order */
@@ -241,7 +254,8 @@ int hm_abi_version(void);
 /* visible CUDA devices (cudaGetDeviceCount; 0 without a driver or a device): pool workers place themselves with it */
 int hm_device_count(void);
 /* sizeof of the ABI structs as the library was compiled: 0 hm_read_batch, 1 hm_chunk,
- * 2 hm_params, 3 hm_site_record (bindings check their own layout against it) */
+ * 2 hm_params, 3 hm_site_record, 4 hm_bq_compact, 5 hm_bgzf_plan, 6 hm_callable_run (bindings check their own
+ * layout against it) */
 size_t hm_abi_sizeof(int which);
 
 /* create / destroy a context bound to one CUDA device */
@@ -314,6 +328,10 @@ int hm_call_chunks_collect(hm_ctx* ctx, hm_site_record* out, size_t cap, size_t*
 /* HM_OPT_KERNEL_TIMING (default 1): CUDA events around the kernels of a call, read back by hm_last_timing /
  * hm_last_kernel_times.  0 saves the event records (a dozen driver calls per call); the figures are then not updated. */
 #define HM_OPT_KERNEL_TIMING 2
+/* HM_OPT_CALLABLE_TRACK (default 0): hm_normcounts_chunks also keeps where the callable territory is, as runs read back
+ * by hm_last_callable_runs.  Costs a store per counted position, two short passes and a device buffer of 4 bytes per
+ * chunk position; the tallies are the same either way. */
+#define HM_OPT_CALLABLE_TRACK 3
 int hm_set_option(hm_ctx* ctx, int option, int value);
 
 /* after hm_call_chunks / hm_call_batch returned HM_ERR_CAPACITY: copy the records of that call
@@ -366,6 +384,10 @@ int hm_qname_seen(hm_ctx* ctx, uint8_t* out, size_t cap, size_t* n);
  * fp64 genotype arithmetic; all the others were pure-reference positions whose verdict the integer
  * pass certified (DESIGN.md §4).  0 when the single-pass kernel ran.                            */
 int hm_last_norm_exact_sites(hm_ctx* ctx, uint64_t* n);
+
+/* after hm_normcounts_chunks with HM_OPT_CALLABLE_TRACK on: the runs of the callable-base track (hm_callable_run) of
+ * that call, *n of them (0 with the option off).  A buffer smaller than *n (or NULL): HM_ERR_CAPACITY, *n = the count. */
+int hm_last_callable_runs(hm_ctx* ctx, hm_callable_run* out, size_t cap, size_t* n);
 
 /* ---- `himut phase`: hetSNP pair tables (replaces phaselib.get_edges, src/himut/phaselib.py:16-67) -------
  * hpos: ascending 1-based hetSNP positions of the contig (vcflib.load_hetsnps), href: their reference base codes
